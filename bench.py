@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- headline benchmark of the receive path (contract in the task statement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one synthetic capture per GPU.  Default workload is
 BASELINE.json configs[3], the configuration the metric is quoted on: a 96 Msps wideband capture
@@ -12,6 +12,10 @@ one B200.  Rank 0 prints ONE JSON line.
   e2e        same metric through RxEngine.run() on a pinned HOST buffer (H2D + frame D2H inside)
   roofline   channelizer kernel: algorithmic 8 B/sample / its measured launch time vs MEASURED_PEAKS
   cpu_baseline  the CPU statement of the same path (oracle) timed on this box's host cores
+
+--dump-outputs DIR writes the frame records of the last timed step (see dump_frames) so that two builds can be compared
+output for output: the inputs are seeded and the same from run to run.  The benchmark writes nothing into the tree it
+runs from (no bytecode caches; the CPU arm's host-tuned oracle is compiled in a temporary directory).
 """
 import argparse
 import json
@@ -25,6 +29,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True
 
 WORKLOADS = {
     # name: (engine mode, BASELINE config, description)
@@ -178,6 +183,26 @@ def cpu_path(workload, sample, min_seconds=0.0):
     return time.perf_counter() - t0, done, frames, cores, kind
 
 
+def dump_frames(out_dir, frames, budget=64_000_000):
+    """Write the frame records a caller of the timed path receives (poll(): reference order, so the same computation gives
+    the same files): every field as out_dir/frames_<field>.npy, float64 (integers up to 2^53 are exact), the payload bytes
+    float32 [n, 132]; frames_count.npy holds the number of records.  A list larger than `budget` bytes is cut to a fixed,
+    seeded sample of its records, kept in order; frames_row.npy names the records kept."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(frames)
+    names = frames.dtype.names
+    row_bytes = 8 + sum(4 * frames.dtype[k].itemsize if k == "bytes" else 8 for k in names)
+    keep = np.arange(n)
+    cap = (budget - (1 << 16)) // row_bytes                       # room for the .npy headers
+    if n > cap:
+        keep = np.sort(np.random.default_rng(0).choice(n, cap, replace=False))
+    sub = frames[keep]
+    np.save(os.path.join(out_dir, "frames_count.npy"), np.array([n], np.float64))
+    np.save(os.path.join(out_dir, "frames_row.npy"), keep.astype(np.float64))
+    for k in names:
+        np.save(os.path.join(out_dir, f"frames_{k}.npy"), sub[k].astype(np.float32 if k == "bytes" else np.float64))
+
+
 def ncu_traffic(n_samples, kernel="k_pfb_ble", stem="pfb_ncu"):
     """dram__bytes_read.sum + dram__bytes_write.sum of one launch of the workload's dominant kernel from the committed
     ncu --set full summary (profiles/rNN_<stem>[_vM].json), valid when it was captured on this same workload size; else None."""
@@ -218,7 +243,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="CPU work timed for cpu_baseline (bounded sample)")
     ap.add_argument("--ref-step-seconds", type=float, default=1.5, help="--impl reference: CPU work per step")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the frame records of the last timed step to DIR/*.npy "
+                    "(rank 0; --workload c5: those of the last capture's shards, copied as they are polled)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -317,6 +346,8 @@ def main():
             d.barrier()
         torch.cuda.synchronize()
 
+    last_polled = [None]                 # the frame list of the step run_resident collected last (a view, see poll())
+
     def run_resident(k, min_seconds=0.0):
         """k steps, software pipelined two deep: batch i+1 is queued before batch i is collected, so
         the GPU never waits for the host.  Returns (frames of last step, front-end ms list, launches)."""
@@ -329,6 +360,7 @@ def main():
             queued += 1
         while queued:
             fr = eng.poll(copy=False)
+            last_polled[0] = fr
             queued -= 1
             done += 1
             nfr = len(fr)
@@ -380,6 +412,8 @@ def main():
     ev1.record()
     barrier()
     assert done == args.steps
+    if args.dump_outputs and rank == 0 and not c5_only:
+        dump_frames(args.dump_outputs, last_polled[0])   # nothing is queued after the last step: the view is still valid
     ms = ev0.elapsed_time(ev1)
     # keep the load on for the clock sampler a little longer, then stop it
     if world == 1:
@@ -474,13 +508,20 @@ def main():
         units = sdist.plan_job(1, len(xc), ceng, units_per_shard=body_units)
         halo = sum(u["hi"] - u["lo"] for u in units) / len(xc) - 1.0
 
+        def poll(stats):
+            fr = ceng.poll(copy=False)
+            if args.dump_outputs and c5_only and stats["polled"] >= stats["keep_from"]:
+                stats["kept"].append(fr.copy())         # a shard of the last capture (the view is reused two batches later)
+            stats["polled"] += 1
+            stats["queued"] -= 1
+            stats["frames"] += len(fr)
+            stats["launches"] += ceng.stats()["kernel_launches"]
+            return fr
+
         def one_capture(cid, pend, stats):
             for u in units:
                 if stats["queued"] == args.c5_depth:
-                    fr = ceng.poll(copy=False)
-                    stats["queued"] -= 1
-                    stats["frames"] += len(fr)
-                    stats["launches"] += ceng.stats()["kernel_launches"]
+                    fr = poll(stats)
                     if world > 1:
                         pend.append(cgather.start(fr, *ceng.polled_frames_device()[:2]))
                         if len(pend) >= gather_depth:
@@ -491,17 +532,14 @@ def main():
 
         def drain(pend, stats):
             while stats["queued"]:
-                fr = ceng.poll(copy=False)
-                stats["queued"] -= 1
-                stats["frames"] += len(fr)
-                stats["launches"] += ceng.stats()["kernel_launches"]
+                fr = poll(stats)
                 if world > 1:
                     pend.append(cgather.start(fr, *ceng.polled_frames_device()[:2]))
             while pend:
                 stats["gathered"] += sum(pend.pop(0).counts())
 
         def run(k):
-            pend, stats = [], dict(queued=0, frames=0, gathered=0, launches=0)
+            pend, stats = [], dict(queued=0, frames=0, gathered=0, launches=0, polled=0, keep_from=(k - 1) * len(units), kept=[])
             for cid in range(k):
                 one_capture(cid, pend, stats)
             drain(pend, stats)
@@ -514,6 +552,8 @@ def main():
         st = run(args.steps)
         e1.record()
         barrier()
+        if args.dump_outputs and rank == 0 and c5_only:
+            dump_frames(args.dump_outputs, np.concatenate(st["kept"]))
         cms = e0.elapsed_time(e1)
         if world > 1:
             import torch.distributed as d

@@ -13,9 +13,12 @@ Two kinds of oracle live here:
 """
 from __future__ import annotations
 
+import atexit
 import ctypes
 import os
+import shutil
 import subprocess
+import tempfile
 from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_uint8, c_uint32, c_void_p
 
 import numpy as np
@@ -37,15 +40,23 @@ def reference_available() -> bool:
     return os.path.isdir(os.path.join(REFERENCE_ROOT, "vendor", "BTLE"))
 
 
+_native_dir: str | None = None
+
+
 def build(ref: bool | None = None, native: bool = False, quiet: bool = True) -> None:
     """Compile the port oracle, and the reference oracle when /root/reference is present.  native=True also builds
-    _build/liboracle_native.so (-O3 -march=native on THIS host): the library the CPU baseline legs of bench.py time."""
+    liboracle_native.so (-O3 -march=native on THIS host): the library the CPU baseline legs of bench.py time.  It goes
+    to a temporary directory, removed at exit, so that the benchmark can run from a read-only tree."""
+    global _native_dir
     args = ["make", "-C", HERE]
     out = subprocess.run(args + ["all"], capture_output=True, text=True)
     if out.returncode != 0:
         raise RuntimeError("oracle build failed:\n" + out.stdout + out.stderr)
     if native:
-        out = subprocess.run(args + ["native"], capture_output=True, text=True)
+        if _native_dir is None:
+            _native_dir = tempfile.mkdtemp(prefix="snrx_oracle_native_")
+            atexit.register(shutil.rmtree, _native_dir, True)
+        out = subprocess.run(args + ["native", f"BUILD={_native_dir}"], capture_output=True, text=True)
         if out.returncode != 0:
             raise RuntimeError("native oracle build failed:\n" + out.stdout + out.stderr)
     if ref is None:
@@ -63,15 +74,15 @@ _libs: dict[str, ctypes.CDLL] = {}
 def _lib(name: str) -> ctypes.CDLL:
     if name in _libs:
         return _libs[name]
+    if name == "native" and _native_dir is None:
+        build(ref=False, native=True)
     path = {"port": os.path.join(HERE, "_build", "liboracle.so"),
-            "native": os.path.join(HERE, "_build", "liboracle_native.so"),
+            "native": os.path.join(_native_dir or "", "liboracle_native.so"),
             "btle_ref": os.path.join(HERE, "_ref", "libbtle_ref.so"),
             "zb_ref": os.path.join(HERE, "_ref", "libzbsink_ref.so")}[name]
     if not os.path.exists(path):
         if name == "port":
             build(ref=False)
-        elif name == "native":
-            build(ref=False, native=True)
         else:
             raise FileNotFoundError(f"{path} missing: run `make -C oracle ref` where /root/reference exists")
     lib = ctypes.CDLL(path)

@@ -108,7 +108,6 @@ def test_port_equals_reference_live(oracle_mod):
         assert_frames_equal(oracle_mod.ble_decode(q, ch), oracle_mod.ble_decode(q, ch, impl="reference"), what=f"seed {seed}")
 
 
-@ref
 def test_restated_loop_equals_real_receiver_stdout(oracle_mod, golden):
     """The harness obtains records by walking receiver()'s steps with the reference's functions;
     the text the real receiver() prints must describe the same frames."""
