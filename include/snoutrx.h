@@ -143,6 +143,7 @@ typedef struct snrx_config {
 } snrx_config_t;
 
 #define SNRX_F_KEEP_STREAMS 1u  /* also store channel streams so snrx_debug_stage can return them */
+#define SNRX_F_RF_METRICS   2u  /* compute per-frame radio metrics in every batch (snrx_frame_rf) */
 
 typedef struct snrx_stats {
     uint64_t samples_in;      /* input-rate samples consumed by the last snrx_process */
@@ -182,6 +183,9 @@ void snrx_destroy(snrx_t* h);
  * the result of one call on the whole capture, bit for bit.  Requirements (channel rate):
  *   BLE    pre halo multiple of 128 (>= 128 unless the shard starts the capture), post halo
  *          >= 2048, body on the 8192-sample window grid;
+ *          With SNRX_F_RF_METRICS and pfb_taps = 768 a wideband BLE shard that does not start the
+ *          capture needs a pre halo >= 256: the noise window of a frame at the start of the body
+ *          reaches 104 samples back and the channelizer needs 32 samples of history before it;
  *   Zigbee pre halo multiple of 2048 and >= 100352 + zb_prehalo unless the shard starts the
  *          capture (the DC tracker remembers 48 blocks of 2048 and the first block of a buffer
  *          starts without discriminator / channelizer history), post halo >= 16448, body on
@@ -379,6 +383,57 @@ typedef struct snrx_zbmac {         /* one per record of the batch, 40 bytes */
 /* Summaries of the batch most recently retired by snrx_poll / snrx_poll_view, computed on the GPU from the device frame
  * list (call before the second-next snrx_process).  *n_out = records of the batch (BLE records get SNRX_ZBMAC_NOT_ZIGBEE). */
 int  snrx_zb_mac_summary(snrx_t* h, snrx_zbmac_t* out, uint32_t cap, uint32_t* n_out);
+
+/* ---- Radio metrics of every decoded frame (engine created with SNRX_F_RF_METRICS): signal power, noise floor, SNR and
+ * carrier offset, what packet sniffers report beside each packet (the PHDR fields of LINKTYPE_BLUETOOTH_LE_LL_WITH_PHDR,
+ * the RFtap power / noise / snr / freqofs fields).  Computed inside the batch, from the input, by k_frame_rf.
+ *
+ * Definition.  s = the record's sample_index (channel rate, capture relative); y[m] = the frame's channel samples:
+ *   wideband modes    the channelizer's own definition (DESIGN.md "Channelizer") for the bin of the frame's channel
+ *                     (snrx_ble_channel_bin / snrx_zigbee_channel_bin) with the prototype of its protocol
+ *                     (snrx_pfb_prototype(mode, pfb_taps)); x = 0 outside the buffer;
+ *   narrow-band modes y = the input itself (sc8 input: q / 128, the value the engine expands it to).
+ * Windows, half-open [a, b) relative to s:
+ *   BLE       signal / CFO [s-24, s+120)   preamble bits 2..7 and access-address bits 0..29
+ *             noise        [s-104, s-40)   64 samples ending 8 before the preamble
+ *   802.15.4  signal / CFO [s-392, s-136)  4 whole preamble symbol periods ending 8 before the nominal SFD start s-128
+ *             noise        [s-720, s-656)  64 samples ending 16 before the nominal SHR start s-640
+ *   (Measured on synthetic bursts of known start, narrow band and through the synthesis filterbank at both prototype
+ *   lengths: the BLE sample_index lies 1 (narrow band) or 0.5 (wideband, after the filter delays) samples before the
+ *   nominal position of AA bit 0, the 802.15.4 one 3..5 samples before the nominal PHR start -- inside the guards, so the
+ *   windows stay where the nominal positions put them.)
+ *   power_dbfs = 10 log10(mean |y[m]|^2) over the signal window, noise_dbfs the same over the noise window (0 dBFS = |x| = 1
+ *   at the input; the prototypes have unity DC gain); a mean below 1e-20 reads -200.  snr_db = power_dbfs - noise_dbfs.
+ *   cfo_hz = fs / 2 pi * wrap(arg(sum_{m=a}^{b-1} y[m] conj(y[m-1])) - theta0), fs = 4e6, over the signal window (so it also
+ *   reads y[a-1]); theta0 = arg sum_m exp(j dtheta_ref[m]) over the same m, dtheta_ref = the per-sample phase increment of the
+ *   zero-offset reference waveform:
+ *     BLE       the GFSK waveform (h = 0.5, 4 samples per bit, the 16 Gaussian taps of BT 0.5 -- snrx_tx_burst_t, synth.py)
+ *               of the 40 known bits -- preamble (0xAA, or 0x55 when AA bit 0 is 1) then the record's access_addr, LSB first --
+ *               with the burst's first sample at s - 39 (the measured position above); computed per frame;
+ *     802.15.4  the preamble is periodic in 64 samples, so theta0 over whole periods is one constant: SNRX_RF_ZB_THETA0.
+ *   Positive cfo_hz = carrier above the channel centre (the sign of snrx_tx_burst_t.cfo_hz).
+ *   A window that reaches before channel sample 0 of the capture, or of the buffer, or past the buffer's end is not
+ *   evaluated: its values are NaN and its valid bits are clear (snr_db is NaN unless both windows are valid). */
+#define SNRX_RF_POWER 0x01     /* power_dbfs valid (the signal window lies inside the buffer)  */
+#define SNRX_RF_NOISE 0x02     /* noise_dbfs valid                                             */
+#define SNRX_RF_CFO   0x04     /* cfo_hz valid (same window as the power)                      */
+#define SNRX_RF_ZB_THETA0 0.12435499454676144   /* atan(1/8): 36 of every 64 preamble increments are +pi/4, 28 are -pi/4 */
+
+typedef struct snrx_frame_rf {      /* one per record of the batch, 40 bytes */
+    int64_t  sample_index;  /* key fields copied from the record, so that consumers can join after reordering / filtering */
+    uint32_t capture_id;
+    uint32_t frame;         /* index of the record in the batch                                                */
+    uint16_t channel;
+    uint8_t  proto;
+    uint8_t  valid;         /* SNRX_RF_*                                                                       */
+    float    power_dbfs, noise_dbfs, snr_db, cfo_hz;
+    uint32_t reserved;
+} snrx_frame_rf_t;
+
+/* Radio metrics of the records of the batch most recently retired by snrx_poll / snrx_poll_view, in record order
+ * (*n_out = records of the batch; out may be NULL; SNRX_ERANGE if cap is smaller than the batch).  Call before the
+ * second-next snrx_process.  SNRX_ESTATE if the engine was created without SNRX_F_RF_METRICS or nothing has been polled. */
+int  snrx_frame_rf(snrx_t* h, snrx_frame_rf_t* out, uint32_t cap, uint32_t* n_out);
 
 /* ---- SURVEY 8(e) / a19: the one exchange of the path -- every engine of a node gets every engine's frame records.
  * No reference counterpart (the reference runs on one host CPU); north_star: "NCCL over NVLink is used only to allgather

@@ -18,6 +18,7 @@ ABI_VERSION = 2
 
 MODE_BLE_NB, MODE_ZB_NB, MODE_ZB_WB16, MODE_BLE_WB40, MODE_MIXED_WB56 = 0, 1, 2, 3, 4
 F_KEEP_STREAMS = 1
+F_RF_METRICS = 2               # include/snoutrx.h SNRX_F_RF_METRICS
 ZB_SEGMENT_DEFAULT = 4096      # include/snoutrx.h SNRX_ZB_SEGMENT_DEFAULT / SNRX_ZB_PREHALO_DEFAULT
 ZB_PREHALO_DEFAULT = 2048
 ZB_IIR_BLOCK = 2048            # SNRX_ZB_IIR_BLOCK / SNRX_ZB_IIR_MEMORY_BLOCKS
@@ -45,6 +46,14 @@ ZBMAC_DTYPE = np.dtype([
     ("zll_command", "u1"), ("reserved", "u1"), ("cluster", "<u2"), ("profile", "<u2"), ("frame", "<u4"),
 ], align=True)
 assert ZBMAC_DTYPE.itemsize == 40
+
+# per-frame radio metrics (include/snoutrx.h snrx_frame_rf_t)
+RF_POWER, RF_NOISE, RF_CFO = 0x01, 0x02, 0x04
+RF_ZB_THETA0 = 0.12435499454676144
+RF_DTYPE = np.dtype([("sample_index", "<i8"), ("capture_id", "<u4"), ("frame", "<u4"), ("channel", "<u2"), ("proto", "u1"),
+                     ("valid", "u1"), ("power_dbfs", "<f4"), ("noise_dbfs", "<f4"), ("snr_db", "<f4"), ("cfo_hz", "<f4"),
+                     ("reserved", "<u4")], align=True)
+assert RF_DTYPE.itemsize == 40
 
 FRAME_DTYPE = np.dtype([
     ("sample_index", "<i8"), ("capture_id", "<u4"), ("window", "<u4"), ("channel", "<u2"),
@@ -120,6 +129,7 @@ SYMBOLS = [
     ("snrx_ble_connections", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_ble_follow", c_int, [c_void_p, c_uint32, c_uint32, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_zb_mac_summary", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
+    ("snrx_frame_rf", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_exchange_create", c_int, [c_void_p, c_uint32, c_uint32, c_uint32, c_void_p]),
     ("snrx_exchange_connect", c_int, [c_void_p, c_void_p]),
     ("snrx_allgather", c_int, [c_void_p, c_uint64, c_void_p, c_uint32, POINTER(c_uint32), POINTER(c_uint32), c_uint32]),

@@ -76,6 +76,9 @@ USAGE = """Usage:
       With --wideband: print frames of every channel, not just -c
     --device N
       CUDA device ordinal (default 0)
+    --rf
+      Measure signal power, noise floor and carrier offset of every frame; with -s the pcap's PHDR carries the
+      signal and noise power (dBFS, flags 0x0002 / 0x0004).  Stdout lines are unchanged
 
 See README for detailed information.
 """
@@ -99,6 +102,7 @@ class Options:
     all_channels = False
     device = 0
     shard_windows = 0
+    rf = False
 
 
 def _strtol(text: str, base: int) -> int:
@@ -130,7 +134,7 @@ def parse_commandline(argv: list[str], out=sys.stdout) -> Options | None:
         opts, rest = getopt.getopt(argv, "hc:g:a:k:vrf:m:os:",
                                    ["help", "chan=", "gain=", "access=", "crcinit=", "verbose", "raw", "freq_hz=",
                                     "access_mask=", "hop", "filename=", "iq=", "format=", "scale=", "wideband",
-                                    "all-channels", "device=", "shard-windows="])
+                                    "all-channels", "device=", "shard-windows=", "rf"])
     except getopt.GetoptError as e:
         out.write(f"btle_rx: {e}\n")
         out.write(USAGE)
@@ -173,6 +177,8 @@ def parse_commandline(argv: list[str], out=sys.stdout) -> Options | None:
             o.device = int(v)
         elif k == "--shard-windows":
             o.shard_windows = int(v)
+        elif k == "--rf":
+            o.rf = True
     if o.chan < 0 or o.chan > MAX_CHANNEL:
         out.write(f"channel number must be within 0~{MAX_CHANNEL}!\n")
         out.write(USAGE)
@@ -213,7 +219,7 @@ def run(o: Options, out=sys.stdout, engine_factory=None, blocks=None) -> int:
         fh_pcap.write(formats.PCAP_HDR_BLE)
     out.flush()
 
-    from .stream import ShardStreamer, iq_blocks
+    from .stream import ShardStreamer, iq_blocks, rf_of
     if engine_factory is None:
         from .engine import RxEngine
         engine_factory = RxEngine
@@ -228,7 +234,8 @@ def run(o: Options, out=sys.stdout, engine_factory=None, blocks=None) -> int:
         return 1
     try:
         eng = engine_factory(mode, channel=o.chan, device=o.device, max_samples=max_samples, access_addr=o.access_addr,
-                             crc_init=o.crc_init, quant_scale=o.scale, access_mask=o.access_mask)
+                             crc_init=o.crc_init, quant_scale=o.scale, access_mask=o.access_mask,
+                             **({"rf_metrics": True} if o.rf else {}))
     except Exception as e:                                             # no GPU / no library: there is no CPU path
         out.write(f"btle_rx (snout_b200): cannot start the GPU receive engine: {e}\n")
         return 1
@@ -236,9 +243,9 @@ def run(o: Options, out=sys.stdout, engine_factory=None, blocks=None) -> int:
     rc = 0
     track = {"conn": None, "first": False}                             # -o: the connection being followed
 
-    def lines(frames: np.ndarray, key=None):
+    def lines(frames: np.ndarray, key=None, rf=None):
         if fh_pcap:
-            fh_pcap.write(formats.ble_pcap_block(frames))              # the batch's records in one piece (same bytes)
+            fh_pcap.write(formats.ble_pcap_block(frames, rf=rf))       # the batch's records in one piece (same bytes)
         for f in frames:
             ch = int(f["channel"]) if key is None else key
             pkt_count[ch] = pkt_count.get(ch, 0) + 1                   # pkt_count++, btle_rx.c:2126
@@ -248,12 +255,14 @@ def run(o: Options, out=sys.stdout, engine_factory=None, blocks=None) -> int:
         st = ShardStreamer(eng, units_per_shard=windows)
 
         def emit(frames: np.ndarray):
+            rf = rf_of(frames, eng.frame_rf()) if o.rf else None
             if o.wideband and not o.all_channels:
-                frames = frames[frames["channel"] == o.chan]
+                sel = frames["channel"] == o.chan
+                frames, rf = frames[sel], (rf[sel] if rf is not None else None)
             if o.hop:
                 follow(frames)
             else:
-                lines(frames)
+                lines(frames, rf=rf)
             out.flush()                                                # fflush(stdout), btle_rx.c:2383
 
         def follow(frames: np.ndarray):

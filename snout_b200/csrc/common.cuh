@@ -126,6 +126,19 @@ SNRX_HD double d_add(double a, double b) {
 #endif
 }
 
+// ---- channel plan: centre frequencies (get_freq_by_channel_number, btle_rx.c:932-948; top_block.py:56) and the
+// channelizer bin of a centre frequency (bin k sits at 2440 + k MHz, modulo 96 MHz)
+SNRX_HD int ble_channel_mhz(int ch) {
+    if (ch == 37) return 2402;
+    if (ch == 38) return 2426;
+    if (ch == 39) return 2480;
+    if (ch >= 0 && ch <= 10) return 2404 + 2 * ch;
+    if (ch >= 11 && ch <= 36) return 2428 + 2 * (ch - 11);
+    return -1;
+}
+SNRX_HD int zb_channel_mhz(int ch) { return (ch >= 11 && ch <= 26) ? 2400 + 5 * (ch - 10) : -1; }
+SNRX_HD int pfb_bin_of_mhz(int mhz) { return mhz < 0 ? -1 : ((mhz - 2440) % 96 + 96) % 96; }
+
 // ---- BLE constants (vendor/BTLE/host/btle-tools/src/btle_rx.c) -------------------------------
 constexpr int kSps = 4;                    // SAMPLE_PER_SYMBOL, btle_rx.c:176
 constexpr int kWindow = SNRX_BLE_WINDOW;   // 8192 IQ per receiver() call, btle_rx.c:180-182, 2382

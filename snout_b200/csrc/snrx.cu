@@ -34,6 +34,7 @@
 #include "pfb_zb.cuh"
 #include "zb_mac.cuh"
 #include "synth.cuh"
+#include "frame_rf.cuh"
 
 using namespace snrx;
 
@@ -67,6 +68,8 @@ struct Lane {
     uint32_t* d_totals = nullptr;       // device: same layout; [5] CRC-ok frames, [6] arrival counter of k_export_frames' CTAs
     cudaEvent_t ev_start = nullptr, ev_front0 = nullptr, ev_front = nullptr, ev_done = nullptr, ev_in = nullptr;
     cudaEvent_t ev_handoff = nullptr;
+    snrx_frame_rf_t* d_rf = nullptr;     // radio metrics the current batch writes (SNRX_F_RF_METRICS): one of d_rf_buf, alternating
+    snrx_frame_rf_t* d_rf_buf[2] = {nullptr, nullptr};   // with d_frames_buf, so a polled batch's records outlive the next batch
     bool pending = false, done = false;
     uint32_t caps = 0, n_out = 0, n_frames = 0; uint64_t n_in = 0; int launches = 0;
     // BLE working set
@@ -132,12 +135,15 @@ struct snrx_handle {
     uint32_t *d_crc_tab = nullptr, *d_whiten = nullptr;
     int32_t* d_ble_channels = nullptr;
     float *d_taps_rho = nullptr, *d_taps_flat = nullptr, *d_taps_pass = nullptr;
+    float* d_rf_taps_zb = nullptr;       // 802.15.4 prototype in tap order (k_frame_rf, wideband modes with 802.15.4 channels)
+    double* d_rf_gauss = nullptr;        // Gaussian taps of the GFSK reference (k_frame_rf)
 
     // last batch
     bool batch_valid = false;
     int last_lane = 0;
     int polled_lane = -1;                // lane of the batch most recently retired by snrx_poll / snrx_poll_view
     const snrx_frame_t* polled_frames_dev = nullptr;   // its device frame list
+    const snrx_frame_rf_t* polled_rf_dev = nullptr;    // its radio metrics (SNRX_F_RF_METRICS)
     uint32_t b_caps = 0; uint64_t b_n_in = 0; uint32_t b_n_out = 0;
     snrx_stats_t stats{};
     int launches = 0;
@@ -203,16 +209,6 @@ uint32_t crc_init_internal(uint32_t k) {
     for (int i = 0; i < 24; i++) r |= ((sw >> i) & 1u) << (23 - i);
     return r;
 }
-
-int ble_mhz(int ch) {                           // get_freq_by_channel_number, btle_rx.c:932-948
-    if (ch == 37) return 2402;
-    if (ch == 38) return 2426;
-    if (ch == 39) return 2480;
-    if (ch >= 0 && ch <= 10) return 2404 + 2 * ch;
-    if (ch >= 11 && ch <= 36) return 2428 + 2 * (ch - 11);
-    return -1;
-}
-int zb_mhz(int ch) { return (ch >= 11 && ch <= 26) ? 2400 + 5 * (ch - 10) : -1; }   // top_block.py:56
 
 template <class T>
 int dev_alloc(snrx_handle* h, T** p, size_t count) {
@@ -408,10 +404,10 @@ int snrx_device_count(int* n) {
     return (e == cudaSuccess && c > 0) ? SNRX_OK : SNRX_ENODEV;
 }
 
-int snrx_ble_channel_mhz(int ch) { return ble_mhz(ch); }
-int snrx_zigbee_channel_mhz(int ch) { return zb_mhz(ch); }
-int snrx_ble_channel_bin(int ch) { int m = ble_mhz(ch); return m < 0 ? -1 : ((m - 2440) % 96 + 96) % 96; }
-int snrx_zigbee_channel_bin(int ch) { int m = zb_mhz(ch); return m < 0 ? -1 : ((m - 2440) % 96 + 96) % 96; }
+int snrx_ble_channel_mhz(int ch) { return ble_channel_mhz(ch); }
+int snrx_zigbee_channel_mhz(int ch) { return zb_channel_mhz(ch); }
+int snrx_ble_channel_bin(int ch) { return pfb_bin_of_mhz(ble_channel_mhz(ch)); }
+int snrx_zigbee_channel_bin(int ch) { return pfb_bin_of_mhz(zb_channel_mhz(ch)); }
 
 int snrx_pfb_prototype(int mode, uint32_t taps, double* out) {
     const bool zb = (mode == SNRX_MODE_ZB_WB16);
@@ -428,12 +424,14 @@ void snrx_destroy(snrx_t* h) {
     cudaSetDevice(h->device);
     for (auto& ln : h->lane) { if (ln.stream) cudaStreamSynchronize(ln.stream); if (ln.tail) cudaStreamSynchronize(ln.tail); }
     if (h->copy_stream) cudaStreamSynchronize(h->copy_stream);
-    void* bufs[] = {h->d_crc_tab, h->d_whiten, h->d_ble_channels, h->d_taps_rho, h->d_taps_flat, h->d_taps_pass};
+    void* bufs[] = {h->d_crc_tab, h->d_whiten, h->d_ble_channels, h->d_taps_rho, h->d_taps_flat, h->d_taps_pass, h->d_rf_taps_zb,
+                    h->d_rf_gauss};
     for (void* b : bufs) if (b) cudaFree(b);
     for (auto& ln : h->lane) {
         void* lb[] = {ln.d_x, ln.d_x8, ln.d_bits, ln.d_hits, ln.d_counts, ln.d_offsets, ln.d_scratch, ln.d_wcounts, ln.d_woffsets,
                       ln.d_cands, ln.d_decs, ln.d_totals, ln.d_q8, ln.d_cf,
-                      ln.d_frames_buf[0] ? ln.d_frames_buf[0] - 1 : nullptr, ln.d_frames_buf[1] ? ln.d_frames_buf[1] - 1 : nullptr};
+                      ln.d_frames_buf[0] ? ln.d_frames_buf[0] - 1 : nullptr, ln.d_frames_buf[1] ? ln.d_frames_buf[1] - 1 : nullptr,
+                      ln.d_rf_buf[0], ln.d_rf_buf[1]};
         for (void* b : lb) if (b) cudaFree(b);
         zb_free(ln.zb);
         if (ln.frames) cudaFreeHost(ln.frames);
@@ -542,6 +540,20 @@ int snrx_create(snrx_t** out, const snrx_config_t* cfg) {
                 if (r != SNRX_OK) return r;
             }
         }
+        if (c.flags & SNRX_F_RF_METRICS) {
+            double g[16];
+            rf_gauss_taps(g);
+            CKD(dev_alloc(h, &h->d_rf_gauss, 16));
+            CK(cudaMemcpy(h->d_rf_gauss, g, sizeof g, cudaMemcpyHostToDevice));
+            if (h->has_zb && h->wideband) {
+                const double* proto = (c.pfb_taps == 384) ? SNRX_PFB_ZB_384 : SNRX_PFB_ZB_768;
+                std::vector<float> flat(c.pfb_taps);
+                for (uint32_t n = 0; n < c.pfb_taps; n++) flat[n] = (float)proto[n];
+                CKD(dev_alloc(h, &h->d_rf_taps_zb, c.pfb_taps));
+                CK(cudaMemcpy(h->d_rf_taps_zb, flat.data(), sizeof(float) * c.pfb_taps, cudaMemcpyHostToDevice));
+            }
+            CK(cudaFuncSetAttribute(k_frame_rf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rf_smem_bytes(32)));
+        }
         for (auto& ln : h->lane) {
             int prio_lo = 0, prio_hi = 0;
             CK(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
@@ -559,6 +571,10 @@ int snrx_create(snrx_t** out, const snrx_config_t* cfg) {
             // so [header | records] can leave the GPU as one block (dist.PeerGather)
             for (auto& fb : ln.d_frames_buf) { CK(cudaMalloc((void**)&fb, sizeof(snrx_frame_t) * ((size_t)h->frame_cap + 1))); fb += 1; }
             ln.d_frames = ln.d_frames_buf[0];
+            if (c.flags & SNRX_F_RF_METRICS) {
+                for (auto& rb : ln.d_rf_buf) CKD(dev_alloc(h, &rb, h->frame_cap));
+                ln.d_rf = ln.d_rf_buf[0];
+            }
             CKD(dev_alloc(h, &ln.d_totals, 8));
             CK(cudaMemset(ln.d_totals, 0, 8 * sizeof(uint32_t)));
             if (h->has_ble) {
@@ -710,12 +726,17 @@ static int process_impl(snrx_t* h, const void* iq, int fmt, uint32_t n_captures,
         }
     }
 
+    if (shard && (h->cfg.flags & SNRX_F_RF_METRICS) && h->has_ble && h->wideband && h->pfb_nt == 32 && pre_out < 256 &&
+        (uint64_t)first_window * kWindow != pre_out)
+        return fail(h, SNRX_EINVAL, "radio metrics with 768 taps: a BLE shard that does not start the capture needs a pre halo of >= 256 channel samples");
+
     if (is_device_ptr && h->user_stream) {          // device input is produced on the caller's stream
         CK(cudaEventRecord(ln.ev_in, h->user_stream));
         CK(cudaStreamWaitEvent(st, ln.ev_in, 0));
     }
     CK(cudaEventRecord(ln.ev_start, st));
     CK(cudaMemsetAsync(ln.d_totals, 0, 8 * sizeof(uint32_t), st));
+    if (ln.d_rf_buf[0]) ln.d_rf = ln.d_rf_buf[ln.uses & 1];
     ln.d_frames = ln.d_frames_buf[ln.uses++ & 1];
 
     // ---- input: cf32 device pointer as is; host pointer staged in chunks overlapped with the front end;
@@ -861,6 +882,17 @@ static int process_impl(snrx_t* h, const void* iq, int fmt, uint32_t n_captures,
                            h->launches, h->err, h->has_ble ? nullptr : ln.ev_front);
         if (r != SNRX_OK) return r;
     }
+    if (h->cfg.flags & SNRX_F_RF_METRICS) {        // radio metrics of the final list, from the input the front end read
+        RfArgs ra{};
+        ra.x = x; ra.stride = x_stride; ra.n_in = (int64_t)n_samples; ra.n_out = (int32_t)n_out;
+        ra.nt = h->wideband ? h->pfb_nt : 0;
+        ra.origin = (int64_t)first_window * kWindow - (int64_t)pre_out; ra.first_capture = first_capture;
+        ra.taps_ble = h->d_taps_flat; ra.taps_zb = h->d_rf_taps_zb; ra.gauss = h->d_rf_gauss;
+        ra.frames = ln.d_frames; ra.totals = ln.d_totals; ra.frame_cap = h->frame_cap; ra.out = ln.d_rf;
+        k_frame_rf<<<h->sm_count * 2, 32 * kRfWarps, rf_smem_bytes(ra.nt), st>>>(ra);
+        h->launches++;
+        CK(cudaGetLastError());
+    }
     // export: device frame list -> pinned host memory; on this lane's stream, so it overlaps the other lane's front end
     ExportXchg xa{};
     if (h->xchg.connected) {
@@ -934,6 +966,7 @@ int snrx_poll(snrx_t* h, snrx_frame_t* out, uint32_t cap, uint32_t* n_out) {
         sl->pending = false;
         h->polled_lane = (int)(sl - h->lane);
         h->polled_frames_dev = sl->d_frames;
+        h->polled_rf_dev = sl->d_rf;
         h->seq_poll++;
     }
     return SNRX_OK;
@@ -949,6 +982,7 @@ int snrx_poll_view(snrx_t* h, const snrx_frame_t** frames, uint32_t* n_out) {
     sl->pending = false;
     h->polled_lane = (int)(sl - h->lane);
     h->polled_frames_dev = sl->d_frames;
+    h->polled_rf_dev = sl->d_rf;
     h->seq_poll++;
     return SNRX_OK;
 }
@@ -957,6 +991,19 @@ int snrx_polled_frames_device(snrx_t* h, const snrx_frame_t** frames_dev, uint32
     if (!h || h->polled_lane < 0) return SNRX_ESTATE;
     if (frames_dev) *frames_dev = h->polled_frames_dev;
     if (n_out) *n_out = h->lane[h->polled_lane].n_frames;
+    return SNRX_OK;
+}
+
+int snrx_frame_rf(snrx_t* h, snrx_frame_rf_t* out, uint32_t cap, uint32_t* n_out) {
+    if (!h) return SNRX_EINVAL;
+    if (!(h->cfg.flags & SNRX_F_RF_METRICS)) return fail(h, SNRX_ESTATE, "snrx_frame_rf: create the engine with SNRX_F_RF_METRICS");
+    if (h->polled_lane < 0) return fail(h, SNRX_ESTATE, "snrx_frame_rf needs a polled batch");
+    const uint32_t n = h->lane[h->polled_lane].n_frames;
+    if (n_out) *n_out = n;
+    if (!out || n == 0) return SNRX_OK;
+    if (cap < n) return fail(h, SNRX_ERANGE, "radio-metrics buffer smaller than the batch");
+    CK(cudaSetDevice(h->device));
+    CK(cudaMemcpy(out, h->polled_rf_dev, sizeof(snrx_frame_rf_t) * (size_t)n, cudaMemcpyDeviceToHost));
     return SNRX_OK;
 }
 

@@ -37,6 +37,20 @@ SNRX_HD uint32_t tx_zb_chips(int s) {
     return c;
 }
 
+// GFSK instantaneous frequency at sample i: freq[i] = sum_j gauss[i - 4 j] (2 bit_j - 1) over the bits whose impulse lies
+// under the 16 taps; the phase is (pi h / 4) sum_{m < i} freq[m], h = 0.5.  bit(j) returns bit j of the burst (0 / 1).
+constexpr double kGfskPhasePerFreq = 3.14159265358979323846 * 0.5 / 4.0;
+template <class Bit>
+SNRX_HD double gfsk_freq(const double* gauss, int64_t i, int64_t n_bits, Bit bit) {
+    double fr = 0.0;
+    for (int t = 0; t < 4; t++) {
+        const int64_t j = (i >> 2) - t;
+        const int tap = (int)(i - 4 * j);
+        if (j >= 0 && j < n_bits && tap < 16) fr += gauss[tap] * (bit(j) ? 1.0 : -1.0);
+    }
+    return fr;
+}
+
 #if defined(__CUDACC__)
 struct TxModArgs {
     const snrx_tx_burst_t* bursts; uint32_t n_bursts;
@@ -69,14 +83,7 @@ __global__ void __launch_bounds__(256) k_tx_modulate(TxModArgs a) {
         const int64_t i = base + threadIdx.x;
         double re = 0.0, im = 0.0, fr = 0.0;
         if (b.proto == SNRX_PROTO_BLE) {
-            // freq[i] = sum_j gauss[i - 4 j] (2 bit_j - 1) over the bits whose impulse lies under the 16 taps; phase[i] = (pi h / 4) sum_{m < i} freq[m]
-            if (i < n) {
-                for (int t = 0; t < 4; t++) {
-                    const int64_t j = (i >> 2) - t;
-                    const int tap = (int)(i - 4 * j);
-                    if (j >= 0 && j < (int64_t)b.n_units && tap < 16) fr += a.gauss[tap] * (((d[j >> 3] >> (j & 7)) & 1) ? 1.0 : -1.0);
-                }
-            }
+            if (i < n) fr = gfsk_freq(a.gauss, i, (int64_t)b.n_units, [&](int64_t j) { return (d[j >> 3] >> (j & 7)) & 1; });
             // exclusive prefix sum of fr over the burst (block scan, carry between rounds)
             scan[threadIdx.x] = fr;
             __syncthreads();
@@ -87,7 +94,7 @@ __global__ void __launch_bounds__(256) k_tx_modulate(TxModArgs a) {
                 __syncthreads();
             }
             const double incl = scan[threadIdx.x] + carry;
-            const double ph = (incl - fr) * (3.14159265358979323846 * 0.5 / 4.0);
+            const double ph = (incl - fr) * kGfskPhasePerFreq;
             __syncthreads();
             if (threadIdx.x == blockDim.x - 1) carry = incl;
             __syncthreads();

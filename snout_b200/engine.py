@@ -38,7 +38,7 @@ class RxEngine:
                  max_samples: int = 0, max_captures: int = 1, max_frames: int = 0,
                  access_addr: int = chanplan.BLE_ADV_AA, crc_init: int = chanplan.BLE_ADV_CRC_INIT,
                  zb_threshold: int = 10, quant_scale: float = 0.0, zb_segment: int = 0, zb_prehalo: int = 0,
-                 pfb_taps: int = 0, keep_streams: bool = False, access_mask: int = 0):
+                 pfb_taps: int = 0, keep_streams: bool = False, access_mask: int = 0, rf_metrics: bool = False):
         self.lib = _abi.load()
         self.mode = MODES[mode] if isinstance(mode, str) else int(mode)
         if channel is None:
@@ -58,7 +58,7 @@ class RxEngine:
         cfg.zb_segment = zb_segment
         cfg.zb_prehalo = zb_prehalo
         cfg.pfb_taps = pfb_taps
-        cfg.flags = _abi.F_KEEP_STREAMS if keep_streams else 0
+        cfg.flags = (_abi.F_KEEP_STREAMS if keep_streams else 0) | (_abi.F_RF_METRICS if rf_metrics else 0)
         cfg.access_mask = access_mask & 0xFFFFFFFF
         self.cfg = cfg
         self.handle = c_void_p()
@@ -298,6 +298,17 @@ class RxEngine:
         cap = int(self.cfg.max_frames) or (1 << 17)
         out = np.zeros(cap, dtype=_abi.ZBMAC_DTYPE)
         self._check(self.lib.snrx_zb_mac_summary(self.handle, out.ctypes.data_as(c_void_p), cap, byref(n)))
+        return out[: n.value].copy()
+
+    # ------------------------------------------------------------------ per-frame radio metrics
+    def frame_rf(self) -> np.ndarray:
+        """Signal power, noise floor, SNR (dBFS / dB) and carrier offset (Hz) of every record of the batch most recently
+        returned by poll(), aligned with it (_abi.RF_DTYPE; definition in include/snoutrx.h).  Needs rf_metrics=True;
+        call before the second-next process()."""
+        n = c_uint32(0)
+        cap = int(self.cfg.max_frames) or (1 << 17)
+        out = np.zeros(cap, dtype=_abi.RF_DTYPE)
+        self._check(self.lib.snrx_frame_rf(self.handle, out.ctypes.data_as(c_void_p), cap, byref(n)))
         return out[: n.value].copy()
 
     def frames_device(self) -> tuple[int, int]:

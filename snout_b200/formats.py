@@ -31,7 +31,7 @@ from typing import BinaryIO, Iterable
 
 import numpy as np
 
-from ._abi import PROTO_BLE, PROTO_ZIGBEE
+from ._abi import PROTO_BLE, PROTO_ZIGBEE, RF_CFO, RF_NOISE, RF_POWER
 
 # ---------------------------------------------------------------------------------- BLE text line
 ADV_PDU_TYPE_STR = (      # btle_rx.c:1081-1098
@@ -170,40 +170,65 @@ def strip_timestamp(line: str) -> str:
 PCAP_HDR_BLE = bytes.fromhex("a1b2c3d4" "0002" "0004" "00000000" "00000000" "000005dc" "00000100")   # btle_rx.c:129
 
 
-def ble_pcap_record(frame, ts: tuple[int, int] = (0, 0)) -> bytes:
+# LINKTYPE_BLUETOOTH_LE_LL_WITH_PHDR flags: de-whitened, signal power valid, noise power valid
+PHDR_DEWHITENED, PHDR_SIGNAL_VALID, PHDR_NOISE_VALID = 0x0001, 0x0002, 0x0004
+
+
+def _dbm_i8(db, offset: float) -> np.ndarray:
+    """int8(round(dB + offset)), clamped to the int8 range; NaN reads 0."""
+    v = np.nan_to_num(np.asarray(db, dtype=np.float64) + offset, nan=0.0)
+    return np.clip(np.rint(v), -128, 127).astype(np.int8).view(np.uint8)
+
+
+def ble_pcap_record(frame, ts: tuple[int, int] = (0, 0), rf=None, dbm_offset: float = 0.0) -> bytes:
     """One record of the file btle_rx -s writes (btle_rx.c:150-163): 16-byte record header whose
     lengths are big-endian (htonl) -- sec/usec are uninitialised stack in the reference, here the
     caller's `ts` in native order as fwrite() of the struct would store them -- then the 10-byte
     LINKTYPE_BLUETOOTH_LE_LL_WITH_PHDR header {channel,0,0,0,0,0,0,0,1,0}, the access address as
-    the host stores a uint32 (little endian), and header+payload (no CRC)."""
+    the host stores a uint32 (little endian), and header+payload (no CRC).
+    `rf`: the frame's radio metrics (_abi.RF_DTYPE record): signal / noise power go into PHDR bytes 1 / 2 as
+    int8(round(dBFS + dbm_offset)) and the flags gain 0x0002 / 0x0004 for the valid ones.  dBFS + an offset is not a
+    calibrated dBm: the offset is the caller's estimate of the front end's gain."""
     b = bytes(frame["bytes"][: int(frame["len"]) - 3])
     n = 10 + 4 + len(b)
     rec = struct.pack("<ii", ts[0], ts[1]) + struct.pack(">ii", n, n)
-    phdr = bytes([int(frame["channel"]) & 0xFF, 0, 0, 0, 0, 0, 0, 0, 1, 0])
-    return rec + phdr + struct.pack("<I", int(frame["access_addr"])) + b
+    phdr = bytearray([int(frame["channel"]) & 0xFF, 0, 0, 0, 0, 0, 0, 0, 1, 0])
+    if rf is not None:
+        valid = int(rf["valid"])
+        if valid & RF_POWER:
+            phdr[1] = int(_dbm_i8(rf["power_dbfs"], dbm_offset))
+            phdr[8] |= PHDR_SIGNAL_VALID
+        if valid & RF_NOISE:
+            phdr[2] = int(_dbm_i8(rf["noise_dbfs"], dbm_offset))
+            phdr[8] |= PHDR_NOISE_VALID
+    return rec + bytes(phdr) + struct.pack("<I", int(frame["access_addr"])) + b
 
 
-def _pack_records(prefix: np.ndarray, payload: np.ndarray, lens: np.ndarray) -> bytes:
-    """Concatenation of [prefix[i] | payload[i, :lens[i]]] over all i, built with numpy only (no per-record Python
-    objects): the batch form of the record writers below (SURVEY 8f N2: at 10^5..10^7 frames per second a Python object
-    per packet is the bottleneck of the pcap / RFtap consumers)."""
+def _pack_records(prefix: np.ndarray, payload: np.ndarray, lens: np.ndarray, plens: np.ndarray | None = None) -> bytes:
+    """Concatenation of [prefix[i, :plens[i]] | payload[i, :lens[i]]] over all i (plens None: whole prefix rows), built
+    with numpy only (no per-record Python objects): the batch form of the record writers below (SURVEY 8f N2: at
+    10^5..10^7 frames per second a Python object per packet is the bottleneck of the pcap / RFtap consumers)."""
     n, P = prefix.shape
     if n == 0:
         return b""
     lens = lens.astype(np.int64)
-    rec = P + lens
+    pl = np.full(n, P, dtype=np.int64) if plens is None else plens.astype(np.int64)
+    rec = pl + lens
     start = np.concatenate(([0], np.cumsum(rec)[:-1]))
     out = np.empty(int(rec.sum()), dtype=np.uint8)
-    out[(start[:, None] + np.arange(P)[None, :]).reshape(-1)] = prefix.reshape(-1)
+    keep = np.arange(P)[None, :] < pl[:, None]
+    out[(start[:, None] + np.arange(P)[None, :])[keep]] = prefix[keep]
     rows = np.repeat(np.arange(n), lens)
     cols = np.arange(int(lens.sum())) - np.repeat(np.cumsum(lens) - lens, lens)
-    out[np.repeat(start + P, lens) + cols] = payload[rows, cols]
+    out[np.repeat(start + pl, lens) + cols] = payload[rows, cols]
     return out.tobytes()
 
 
-def ble_pcap_block(frames: np.ndarray, ts: tuple[int, int] = (0, 0)) -> bytes:
-    """All BLE records of `frames` as btle_rx -s writes them: byte-identical to b"".join(ble_pcap_record(f, ts))."""
-    f = frames[frames["proto"] == PROTO_BLE]
+def ble_pcap_block(frames: np.ndarray, ts: tuple[int, int] = (0, 0), rf=None, dbm_offset: float = 0.0) -> bytes:
+    """All BLE records of `frames` as btle_rx -s writes them: byte-identical to b"".join(ble_pcap_record(f, ts, r)).
+    `rf`: radio metrics aligned with `frames` (RxEngine.frame_rf())."""
+    sel = frames["proto"] == PROTO_BLE
+    f = frames[sel]
     n = len(f)
     lens = f["len"].astype(np.int64) - 3
     prefix = np.zeros((n, 16 + 10 + 4), dtype=np.uint8)
@@ -211,31 +236,62 @@ def ble_pcap_block(frames: np.ndarray, ts: tuple[int, int] = (0, 0)) -> bytes:
     be = (10 + 4 + lens).astype(">i4").view(np.uint8).reshape(n, 4)
     prefix[:, 8:12], prefix[:, 12:16] = be, be
     prefix[:, 16] = f["channel"].astype(np.uint8)
-    prefix[:, 24] = 1
+    prefix[:, 24] = PHDR_DEWHITENED
+    if rf is not None:
+        r = np.asarray(rf)[sel]
+        p_ok, n_ok = (r["valid"] & RF_POWER) != 0, (r["valid"] & RF_NOISE) != 0
+        prefix[:, 17] = np.where(p_ok, _dbm_i8(r["power_dbfs"], dbm_offset), 0)
+        prefix[:, 18] = np.where(n_ok, _dbm_i8(r["noise_dbfs"], dbm_offset), 0)
+        prefix[:, 24] |= np.where(p_ok, PHDR_SIGNAL_VALID, 0).astype(np.uint8) | np.where(n_ok, PHDR_NOISE_VALID, 0).astype(np.uint8)
     prefix[:, 26:30] = f["access_addr"].astype("<u4").view(np.uint8).reshape(n, 4)
     return _pack_records(prefix, f["bytes"], lens)
 
 
-def write_ble_pcap(fh: BinaryIO, frames: Iterable, header: bool = True) -> int:
+def write_ble_pcap(fh: BinaryIO, frames: Iterable, header: bool = True, rf=None, dbm_offset: float = 0.0) -> int:
     if header:
         fh.write(PCAP_HDR_BLE)
     frames = np.asarray(frames)
-    fh.write(ble_pcap_block(frames))
+    fh.write(ble_pcap_block(frames, rf=rf, dbm_offset=dbm_offset))
     return int((frames["proto"] == PROTO_BLE).sum())
 
 
 # ---------------------------------------------------------------------------------- Zigbee datagrams
 RFTAP_MAGIC = b"RFta"
 DLT_IEEE802_15_4_WITHFCS = 195
+DLT_RFTAP = 215
 
 
-def rftap_datagram(frame) -> bytes:
+# RFtap flag bits of the fields written here (layers/rftap.py)
+RFTAP_DLT, RFTAP_FREQOFS, RFTAP_POWER, RFTAP_NOISE, RFTAP_SNR, RFTAP_QUAL = 0x0100, 0x0800, 0x2000, 0x4000, 0x8000, 0x0001
+
+
+def rftap_datagram(frame, rf=None, dbm_offset: float = 0.0) -> bytes:
     """RFtap header + PSDU: what rftap_encap(2, 195, '') emits for a PDU whose meta carries
     qual = lqi / 255.0 (epy_block_0.py:21).  16-byte header: magic, length32 = 4, flags = dlt | qual
-    (0x0101), dlt = 195, qual as float32 -- equal to the records of scapy's test/rftap.pcap."""
-    qual = np.float32(int(frame["lqi"]) / 255.0)
-    hdr = RFTAP_MAGIC + struct.pack("<HHI", 4, 0x0101, DLT_IEEE802_15_4_WITHFCS) + struct.pack("<f", qual)
-    return hdr + bytes(frame["bytes"][: int(frame["len"])])
+    (0x0101), dlt = 195, qual as float32 -- equal to the records of scapy's test/rftap.pcap.
+    `rf`: the frame's radio metrics (_abi.RF_DTYPE record): the valid ones are added as freqofs (float64, Hz), power and
+    noise (float32, dBFS + dbm_offset) and snr (float32, dB), in RFtap field order, and length32 grows to match."""
+    return _rftap_header(int(frame["lqi"]), rf, dbm_offset) + bytes(frame["bytes"][: int(frame["len"])])
+
+
+def _rftap_header(lqi: int, rf, dbm_offset: float) -> bytes:
+    flags, body = RFTAP_DLT | RFTAP_QUAL, struct.pack("<I", DLT_IEEE802_15_4_WITHFCS)
+    if rf is not None:
+        valid = int(rf["valid"])
+        if valid & RF_CFO:
+            flags |= RFTAP_FREQOFS
+            body += struct.pack("<d", float(rf["cfo_hz"]))
+        if valid & RF_POWER:
+            flags |= RFTAP_POWER
+            body += struct.pack("<f", float(rf["power_dbfs"]) + dbm_offset)
+        if valid & RF_NOISE:
+            flags |= RFTAP_NOISE
+            body += struct.pack("<f", float(rf["noise_dbfs"]) + dbm_offset)
+        if valid & RF_POWER and valid & RF_NOISE:
+            flags |= RFTAP_SNR
+            body += struct.pack("<f", float(rf["snr_db"]))
+    body += struct.pack("<f", np.float32(lqi / 255.0))
+    return RFTAP_MAGIC + struct.pack("<HH", 2 + len(body) // 4, flags) + body
 
 
 def gnuradio_packet(frame) -> bytes:
@@ -296,16 +352,49 @@ def zigbee_pcap_block(frames: np.ndarray, ts=None, sample_rate: float = 4e6) -> 
     return _pack_records(prefix, f["bytes"], lens)
 
 
-def rftap_block(frames: np.ndarray) -> tuple[bytes, np.ndarray]:
+def rftap_block(frames: np.ndarray, rf=None, dbm_offset: float = 0.0) -> tuple[bytes, np.ndarray]:
     """The RFtap datagrams (rftap_datagram) of all 802.15.4 records back to back + the offsets where each starts
-    (n + 1 entries), for senders that batch their socket writes."""
-    f = frames[frames["proto"] == PROTO_ZIGBEE]
+    (n + 1 entries), for senders that batch their socket writes.  `rf`: radio metrics aligned with `frames`."""
+    sel = frames["proto"] == PROTO_ZIGBEE
+    f = frames[sel]
     n = len(f)
     lens = f["len"].astype(np.int64)
+    if rf is not None:
+        return _rftap_block_rf(f, np.asarray(rf)[sel], lens, dbm_offset)
     prefix = np.zeros((n, 16), dtype=np.uint8)
     prefix[:, 0:12] = np.frombuffer(RFTAP_MAGIC + struct.pack("<HHI", 4, 0x0101, DLT_IEEE802_15_4_WITHFCS), dtype=np.uint8)
     prefix[:, 12:16] = (f["lqi"].astype(np.int64) / 255.0).astype("<f4").view(np.uint8).reshape(n, 4)
     return _pack_records(prefix, f["bytes"], lens), np.concatenate(([0], np.cumsum(16 + lens)))
+
+
+def _rftap_block_rf(f: np.ndarray, r: np.ndarray, lens: np.ndarray, dbm_offset: float) -> tuple[bytes, np.ndarray]:
+    """rftap_block with radio metrics: the header of every record holds the fields its valid bits allow."""
+    n = len(f)
+    v = r["valid"].astype(np.int64)
+    has_cfo, has_p, has_n = (v & RF_CFO) != 0, (v & RF_POWER) != 0, (v & RF_NOISE) != 0
+    has_snr = has_p & has_n
+    prefix = np.zeros((n, 40), dtype=np.uint8)
+    col = np.full(n, 12, dtype=np.int64)                       # magic, length32, flags, dlt written below
+    rows = np.arange(n)
+
+    def put(mask, values: np.ndarray):
+        b = values.view(np.uint8).reshape(n, -1)
+        w = b.shape[1]
+        idx = col[mask][:, None] + np.arange(w)[None, :]
+        prefix[rows[mask][:, None], idx] = b[mask]
+        col[mask] += w
+
+    put(has_cfo, r["cfo_hz"].astype("<f8"))
+    put(has_p, (r["power_dbfs"].astype(np.float64) + dbm_offset).astype("<f4"))
+    put(has_n, (r["noise_dbfs"].astype(np.float64) + dbm_offset).astype("<f4"))
+    put(has_snr, r["snr_db"].astype("<f4"))
+    put(np.ones(n, dtype=bool), (f["lqi"].astype(np.int64) / 255.0).astype("<f4"))
+    flags = (RFTAP_DLT | RFTAP_QUAL) + has_cfo * RFTAP_FREQOFS + has_p * RFTAP_POWER + has_n * RFTAP_NOISE + has_snr * RFTAP_SNR
+    prefix[:, 0:4] = np.frombuffer(RFTAP_MAGIC, dtype=np.uint8)
+    prefix[:, 4:6] = (col // 4).astype("<u2").view(np.uint8).reshape(n, 2)
+    prefix[:, 6:8] = flags.astype("<u2").view(np.uint8).reshape(n, 2)
+    prefix[:, 8:12] = np.frombuffer(struct.pack("<I", DLT_IEEE802_15_4_WITHFCS), dtype=np.uint8)
+    return _pack_records(prefix, f["bytes"], lens, col), np.concatenate(([0], np.cumsum(col + lens)))
 
 
 def write_zigbee_pcap(fh: BinaryIO, frames: Iterable, ts=None, sample_rate: float = 4e6, header: bool = True) -> int:

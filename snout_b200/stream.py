@@ -91,6 +91,21 @@ def zb_span_filter(frames: np.ndarray, state: dict | None = None) -> np.ndarray:
     return frames if keep.all() else frames[keep]
 
 
+def rf_of(frames: np.ndarray, rf: np.ndarray) -> np.ndarray:
+    """The radio-metrics records (RxEngine.frame_rf()) of `frames`, matched on their key fields (capture, sample index,
+    channel, protocol): the streamer filters and a caller may reorder the records of a batch.  A frame without a match gets
+    a record whose valid bits are clear."""
+    from ._abi import RF_DTYPE
+    out = np.zeros(len(frames), dtype=RF_DTYPE)
+    out[["power_dbfs", "noise_dbfs", "snr_db", "cfo_hz"]] = (np.nan, np.nan, np.nan, np.nan)
+    index = {(int(r["capture_id"]), int(r["sample_index"]), int(r["channel"]), int(r["proto"])): i for i, r in enumerate(rf)}
+    for i, f in enumerate(frames):
+        j = index.get((int(f["capture_id"]), int(f["sample_index"]), int(f["channel"]), int(f["proto"])))
+        if j is not None:
+            out[i] = rf[j]
+    return out
+
+
 class ShardStreamer:
     """Push IQ blocks in, get frame arrays out, in stream order.
 

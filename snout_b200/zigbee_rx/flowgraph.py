@@ -46,7 +46,8 @@ class top_block:
     def __init__(self, channel: int = 26, iq: str | None = None, fmt: str = "cf32", wideband: bool = False,
                  encap: str = "rftap", device: int = 0, xmlrpc_addr=XMLRPC_ADDR, udp_dest=UDP_DEST,
                  realtime: bool = False, all_channels: bool = False, engine_factory=None, blocks=None,
-                 segments_per_shard: int = 0, zb_segment: int = 0, serve_xmlrpc: bool = True, pcap: str | None = None):
+                 segments_per_shard: int = 0, zb_segment: int = 0, serve_xmlrpc: bool = True, pcap: str | None = None,
+                 rf: bool = False):
         self.channel = channel
         self.samp_rate = 4000000                                       # top_block.py:42
         self._iq, self._fmt, self._wideband, self._encap = iq, fmt, wideband, encap
@@ -54,12 +55,13 @@ class top_block:
         self._realtime, self._all = realtime, all_channels
         self._engine_factory, self._blocks = engine_factory, blocks
         self._segments, self._zb_segment = segments_per_shard, zb_segment
+        self._rf = rf                   # radio metrics: RFtap freqofs / power / noise / snr, and the pcap holds RFtap records
         self._stop = threading.Event()
         self._thread = None
         self._sock = socket.socket(socket.AF_INET, socket.SOCK_DGRAM)
         self._pcap = open(pcap, "wb") if pcap else None
         if self._pcap:
-            self._pcap.write(formats.pcap_global_header(formats.DLT_IEEE802_15_4_WITHFCS))
+            self._pcap.write(formats.pcap_global_header(formats.DLT_RFTAP if rf else formats.DLT_IEEE802_15_4_WITHFCS))
         self.frames_sent = 0
         self.error = None
         self.xmlrpc_server_0 = None
@@ -109,21 +111,23 @@ class top_block:
             self._pcap = None
 
     # ---- data path ----------------------------------------------------------------------------
-    def _emit(self, frames: np.ndarray):
-        for f in frames:
+    def _emit(self, frames: np.ndarray, rf=None):
+        for i, f in enumerate(frames):
             if self._wideband and not self._all and int(f["channel"]) != self.channel:
                 continue
             if not self._wideband:
                 f = f.copy()
                 f["channel"] = self.channel
-            data = formats.rftap_datagram(f) if self._encap == "rftap" else formats.gnuradio_packet(f)
+            r = rf[i] if rf is not None else None
+            data = formats.rftap_datagram(f, r) if self._encap == "rftap" else formats.gnuradio_packet(f)
             self._sock.sendto(data, self._udp_dest)
             if self._pcap:
-                self._pcap.write(formats.pcap_record(bytes(f["bytes"][: int(f["len"])]), time.time()))
+                rec = formats.rftap_datagram(f, r) if r is not None else bytes(f["bytes"][: int(f["len"])])
+                self._pcap.write(formats.pcap_record(rec, time.time()))
             self.frames_sent += 1
 
     def _run(self):
-        from ..stream import ShardStreamer, iq_blocks, shard_geometry
+        from ..stream import ShardStreamer, iq_blocks, rf_of, shard_geometry
         factory = self._engine_factory
         if factory is None:
             from ..engine import RxEngine
@@ -135,7 +139,7 @@ class top_block:
         nseg = self._segments or (262144 if self._wideband else 1048576) // unit
         try:
             eng = factory(mode, channel=self.channel, device=self._device, zb_segment=seg,
-                          max_samples=(nseg * unit + pre + post) * decim)
+                          max_samples=(nseg * unit + pre + post) * decim, **({"rf_metrics": True} if self._rf else {}))
         except Exception as e:                                         # no GPU / no library: there is no CPU path
             self.error = e
             sys.stderr.write(f"Zigbee_rx (snout_b200): cannot start the GPU receive engine: {e}\n")
@@ -149,14 +153,14 @@ class top_block:
                 if self._stop.is_set():
                     break
                 for frames in st.feed(block):
-                    self._emit(frames)
+                    self._emit(frames, rf_of(frames, eng.frame_rf()) if self._rf else None)
                 done += len(block)
                 if self._realtime:
                     lag = done / rate - (time.time() - t0)
                     if lag > 0:
                         time.sleep(lag)
             for frames in st.flush():
-                self._emit(frames)
+                self._emit(frames, rf_of(frames, eng.frame_rf()) if self._rf else None)
             st.close()
         except Exception as e:
             self.error = e
@@ -178,6 +182,8 @@ def argument_parser():
     p.add_argument("--device", type=int, default=0)
     p.add_argument("--pcap", default=None, help="also write the PSDUs to this DLT 195 pcap")
     p.add_argument("--no-stdin", action="store_true", help="do not wait for a newline on stdin; exit at end of the source")
+    p.add_argument("--rf", action="store_true", help="measure signal power, noise floor and carrier offset of every frame: the "
+                   "RFtap datagrams carry freqofs / power / noise / snr, and --pcap then holds RFtap records (LINKTYPE_RFTAP)")
     return p
 
 
@@ -188,7 +194,7 @@ def main(top_block_cls=top_block, argv=None):
         return 1
     stdin_is_source = (o.iq == "-")
     tb = top_block_cls(channel=o.channel, iq=o.iq, fmt=o.format, wideband=o.wideband, encap=o.encap, device=o.device,
-                       realtime=o.realtime, all_channels=o.all_channels, pcap=o.pcap)
+                       realtime=o.realtime, all_channels=o.all_channels, pcap=o.pcap, rf=o.rf)
     tb.start()
     if o.no_stdin or stdin_is_source:
         tb._thread.join()
