@@ -11,6 +11,7 @@ import numpy as np
 import pytest
 
 from conftest import assert_frames_equal
+from quant_rule import check_q8
 from snout_b200 import chanplan, synth
 
 P = lambda a: a.ctypes.data_as(ctypes.c_void_p)
@@ -142,8 +143,7 @@ def test_pfb_tile_kernel(emu, oracle_mod, nt, name):
     yd = oracle_mod.pfb(x, h, [chanplan.ble_channel_bin(c) for c in range(40)])
     rms = np.sqrt(np.mean(np.abs(yd) ** 2))
     assert np.abs(raw - yd).max() / rms < 1e-4                       # stated channelizer tolerance
-    qo = np.clip(np.rint(np.stack([yd.real, yd.imag], -1) * 100.0), -128, 127)
-    assert np.abs(q8.astype(int) - qo).max() <= 1
+    check_q8(q8, raw, yd, 100.0, what=f"{name} tile harness")
     n_frames = 0
     for c in range(40):
         b2, _, _ = _slice_nb(emu, q8[c].astype(np.float32) / 128.0, 128.0)

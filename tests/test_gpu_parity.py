@@ -9,6 +9,7 @@ import numpy as np
 import pytest
 
 from conftest import assert_frames_equal, ble_expected
+from quant_rule import check_q8
 from snout_b200 import _abi, chanplan, synth
 
 pytestmark = pytest.mark.gpu
@@ -194,8 +195,7 @@ def test_ble_wb40_stagewise_parity(Engine, oracle_mod, taps):
     yd = oracle_mod.pfb(x, h, [chanplan.ble_channel_bin(c) for c in range(40)])
     rms = np.sqrt(np.mean(np.abs(yd) ** 2))
     assert np.abs(y - yd).max() / rms < CHAN_TOL
-    qo = np.clip(np.rint(np.stack([yd.real, yd.imag], -1) * 100.0), -128, 127)
-    assert np.abs(q8.astype(int) - qo).max() <= 1
+    check_q8(q8, y, yd, 100.0, what=f"wideband {taps} taps")
     # S2: frames vs the oracle run on the engine's own quantised streams -- bit exact
     want = _wb_oracle_frames(oracle_mod, q8)
     assert len(want) > 300
