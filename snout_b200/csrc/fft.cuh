@@ -1,5 +1,6 @@
 // fft.cuh -- fully unrolled in-register inverse DFTs (kernel exp(+j 2 pi k r / N)) for the
-// channelizer: N = 3 * 2^p (48 for the even-bin BLE bank, 96 for the full bank).
+// channelizer: N = 3 * 2^p (48 for the even-bin BLE bank, 96 for the full bank).  Pfa48 is the twiddle-free
+// prime-factor form of the 48-point transform that the BLE channelizer runs.
 //
 // Everything is resolved at compile time: the recursion is template recursion, all array
 // indices are constants after unrolling (so the arrays live in registers) and the twiddles are
@@ -138,5 +139,42 @@ struct Idft3xQ {
         combine<0>(f0, f1, f2, out);
     }
 };
+
+// 48-point inverse DFT by the Good-Thomas prime-factor map, 48 = 3 * 16 with gcd(3, 16) = 1: no twiddles at all.
+//   r = (16 n1 + 3 n2) mod 48,   k = (33 k16 + 16 k3) mod 48        (33 = 1 mod 16 = 0 mod 3;  16 = 0 mod 16 = 1 mod 3)
+//   Y[k] = sum_{n1} W3^{k3 n1} F_{n1}[k16],   F_{n1}[k16] = sum_{n2} W16^{k16 n2} in[(16 n1 + 3 n2) mod 48]
+// Pass n1 reads the same inputs as pass r1 = n1 of Idft3xQ<48> (r = 3 r2 + n1), in the order r2 = (5 n1 + n2) mod 16.
+struct Pfa48 {
+    SNRX_HD static constexpr int rot(int n1) { return 5 * n1 % 16; }                 // r2 of input n2 = 0 of pass n1
+    SNRX_HD static constexpr int bin(int k16, int k3) { return (33 * k16 + 16 * k3) % 48; }
+    template <int K16>
+    SNRX_HD static void combine(const cf* f0, const cf* f1, const cf* f2, cf* out) {
+        constexpr float h = 0.86602540378443864676f;   // sqrt(3)/2
+        const float2 a = P(f0[K16]);
+        const float2 s = f2_add(P(f1[K16]), P(f2[K16]));
+        const float2 d = f2_fma(P(f2[K16]), make_float2(-1.0f, -1.0f), P(f1[K16]));
+        out[bin(K16, 0)] = C(f2_add(a, s));
+        const float2 m = f2_fma(make_float2(-0.5f, -0.5f), s, a);
+        // k3 = 1: a + w b + w^2 c, w = exp(+j 2pi/3) = -1/2 + j h  ->  m + j h d ;  k3 = 2: m - j h d
+        const float2 dsw = make_float2(d.y, d.x);
+        out[bin(K16, 1)] = C(f2_fma(make_float2(-h, h), dsw, m));
+        out[bin(K16, 2)] = C(f2_fma(make_float2(h, -h), dsw, m));
+        if constexpr (K16 + 1 < 16) combine<K16 + 1>(f0, f1, f2, out);
+    }
+    SNRX_HD static void run(const cf* in, cf* out) {
+        cf v[3][16], f[3][16];
+        for (int n1 = 0; n1 < 3; n1++)
+            for (int n2 = 0; n2 < 16; n2++) v[n1][n2] = in[(16 * n1 + 3 * n2) % 48];
+        for (int n1 = 0; n1 < 3; n1++) IdftPow2<16, 1>::run(v[n1], f[n1]);
+        combine<0>(f[0], f[1], f[2], out);
+    }
+};
+constexpr bool pfa48_passes_agree() {
+    for (int n1 = 0; n1 < 3; n1++)
+        for (int n2 = 0; n2 < 16; n2++)
+            if (3 * ((Pfa48::rot(n1) + n2) % 16) + n1 != (16 * n1 + 3 * n2) % 48) return false;
+    return true;
+}
+static_assert(pfa48_passes_agree(), "pass n1 of the prime-factor map = the branches r = n1 (mod 3), rotated");
 
 }  // namespace snrx

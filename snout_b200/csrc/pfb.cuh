@@ -23,10 +23,12 @@
 //            window) -- then a 4 KB transpose through shared memory (16-byte stores/loads, XOR swizzle) and,
 //            one lane per output time, the 16-point inverse DFT over the branches r = gi (mod 3), in
 //            registers.  Keeping only one third of the branch outputs in shared memory at a time is what
-//            lets 16 warps share an SM;
-//   phase 2  radix-3 combination of the three 16-point transforms (fft.cuh), bin rotation, quantisation of
-//            the 40 bins that carry a channel;
-//   phase 3  successor samples by warp shuffle, cross product, sign bit shifted into a per-lane word
+//            lets 16 warps share an SM.  Pass gi reads its branches in the rotated order of the prime-factor
+//            map (fft.cuh Pfa48), so that the 48-point transform needs no twiddles;
+//   phase 2  twiddle-free radix-3 combination of the three 16-point transforms (fft.cuh Pfa48), bin rotation,
+//            quantisation of the 40 bins that carry a channel, packing of each quantised (I, Q) into the two
+//            byte words of the integer slicer;
+//   phase 3  successor words by warp shuffle, cross product by one dp4a, sign bit shifted into a per-lane word
 //            (bit = channel); two 32x32 bit-matrix transposes by shuffle turn them into per-channel
 //            words (bit = time), which lanes OR into the global bit streams (natural sample order).
 // ncu: profiles/.
@@ -113,14 +115,49 @@ SNRX_HD int fir_base(int rho, int q) {
 
 // Quantiser of the wideband path: q = clamp(rint(y * scale), -128, 127) evaluated as
 //   u = sat(y * (scale/255) + 128/255)          one FFMA.SAT per component: the clamp is free
-//   q = rint(255 u) - 128                        (255 u + (1.5 * 2^23 - 128)) - 1.5 * 2^23, packed
+//   t = 1.5 * 2^23 + rint(255 u) - 128           255 u + (1.5 * 2^23 - 128), packed: t = 1.5 * 2^23 + q
 // u carries one extra rounding (<= 2^-25, i.e. 8e-6 of a quantiser step): part of this engine's definition of
 // its quantised channel streams (SNRX_STAGE_BLE_Q8), on which frame parity is stated (DESIGN.md 4).
-SNRX_HD float2 quant_pair(float2 y, float s255 /* +-scale/255, 0 beyond the capture end */) {
+// The kernel keeps the result biased: the slicer reads q from the bits of t (q8_of_biased, slicer_w / slicer_a).
+SNRX_HD float2 quant_pair_biased(float2 y, float s255 /* +-scale/255, 0 beyond the capture end */) {
     const float ux = f_sat(f_fma(y.x, s255, 128.0f / 255.0f));
     const float uy = f_sat(f_fma(y.y, s255, 128.0f / 255.0f));
-    const float2 t = f2_fma(make_float2(ux, uy), make_float2(255.0f, 255.0f), make_float2(kMagic - 128.0f, kMagic - 128.0f));
-    return f2_add(t, make_float2(-kMagic, -kMagic));
+    return f2_fma(make_float2(ux, uy), make_float2(255.0f, 255.0f), make_float2(kMagic - 128.0f, kMagic - 128.0f));
+}
+// q itself as an integer-valued float (the Cooley-Tukey statement below)
+SNRX_HD float2 quant_pair(float2 y, float s255) { return f2_add(quant_pair_biased(y, s255), make_float2(-kMagic, -kMagic)); }
+
+SNRX_HD uint32_t f_bits(float x) {
+#ifdef __CUDA_ARCH__
+    return __float_as_uint(x);
+#else
+    uint32_t u; memcpy(&u, &x, 4); return u;
+#endif
+}
+// t = 1.5 * 2^23 + q, q in [-128, 127], lies in [2^23, 2^24) with unit spacing: its bits are 0x4B400000 + q, so byte 3 is
+// always 0x4B and byte 0 is q as int8
+SNRX_HD int8_t q8_of_biased(uint32_t t_bits) { return (int8_t)(t_bits & 0xFFu); }
+
+// Bytes of the 64-bit value y:x picked by the selector nibbles of s (selector values 0..7 only)
+SNRX_HD uint32_t byte_perm(uint32_t x, uint32_t y, uint32_t s) {
+#ifdef __CUDA_ARCH__
+    return __byte_perm(x, y, s);
+#else
+    const uint64_t v = ((uint64_t)y << 32) | x;
+    uint32_t r = 0;
+    for (int i = 0; i < 4; i++) r |= (uint32_t)((v >> (8 * ((s >> (4 * i)) & 7u))) & 0xFFu) << (8 * i);
+    return r;
+#endif
+}
+// Sum of the four products of the signed bytes of a and b
+SNRX_HD int dp4a(uint32_t a, uint32_t b) {
+#ifdef __CUDA_ARCH__
+    return __dp4a((int)a, (int)b, 0);
+#else
+    int s = 0;
+    for (int i = 0; i < 4; i++) s += (int)(int8_t)(a >> (8 * i)) * (int)(int8_t)(b >> (8 * i));
+    return s;
+#endif
 }
 
 // V tile of one FIR pass: row rl (0..7), column = output time, float4 = (branch r2 = rl, branch r2 = rl + 8)
@@ -128,19 +165,61 @@ SNRX_HD float2 quant_pair(float2 y, float s255 /* +-scale/255, 0 beyond the capt
 // stores (8 rows at one column) and the DFT lanes' loads (one row, 32 columns) are bank-conflict free.
 SNRX_HD constexpr int v_pos(int row, int col) { return row * 32 + (col ^ row); }
 
-// One lane's column of the pass -> the 16 inputs of IdftPow2<16, 1>
-SNRX_HD void pfb_load_col16(const float4* V, int lane, cf (&v)[16]) {
+// One lane's column of pass gi -> the 16 inputs of IdftPow2<16, 1>, in the prime-factor order of fft.cuh Pfa48: branch r2
+// feeds input (r2 - Pfa48::rot(gi)) mod 16.  gi is a constant after unrolling, so the rotation is register naming only (as a
+// template parameter ptxas allocated the phase worse: one 8-byte spill in k_pfb_ble<16, false>).
+SNRX_HD void pfb_load_col16_pfa(const float4* V, int lane, int gi, cf (&v)[16]) {
+    const int rot = Pfa48::rot(gi);
+#pragma unroll
+    for (int r = 0; r < 8; r++) {
+        const float4 t = V[v_pos(r, lane)];
+        v[(r + 16 - rot) % 16].r = t.x; v[(r + 16 - rot) % 16].i = t.y;
+        v[(r + 24 - rot) % 16].r = t.z; v[(r + 24 - rot) % 16].i = t.w;
+    }
+}
+
+// Integer slicer on the quantiser's bits.  From t_i, t_q (bits of the biased I and Q of one sample), bytes low to high:
+//   slicer_w = [I, ~Q, 0, 1]     (0x4B ^ 0x4B, 0x4B ^ 0x4A)    the word the PREDECESSOR sample reads
+//   slicer_a = [Q, I, I, I]
+// dp4a(slicer_a of sample m, slicer_w of sample m+1) = Q0 I1 + I0 (-Q1 - 1) + I0 * 0 + I0 = -(I0 Q1 - I1 Q0), exact: its sign
+// bit is the decision b[m] = I0 Q1 - I1 Q0 > 0 (btle_rx.c:1357-1361).
+SNRX_HD uint32_t slicer_w(uint32_t t_i, uint32_t t_q) { return byte_perm(t_i, t_q, 0x3340u) ^ 0x4A4BFF00u; }
+SNRX_HD uint32_t slicer_a(uint32_t t_i, uint32_t t_q) { return byte_perm(t_i, t_q, 0x0004u); }
+SNRX_HD uint32_t slicer_sign_dp4a(uint32_t a0, uint32_t w1) { return (uint32_t)dp4a(a0, w1); }
+// the quantised (I, Q) back from slicer_a
+SNRX_HD int8_t slicer_a_i(uint32_t a) { return (int8_t)(a >> 8); }
+SNRX_HD int8_t slicer_a_q(uint32_t a) { return (int8_t)a; }
+
+// Twiddle-free radix-3 combination of the three 16-point transforms (fft.cuh Pfa48) + rotation + quantisation:
+// on return sw[q] / sa[q] hold slicer_w / slicer_a of the quantised (I, Q) of even bin 2q for the 40 bins that carry a BLE
+// channel (the other 8 are never computed: dead code for the compiler).
+// s_even / s_odd: quantiser scale with the sign of (-1)^(q m) folded in (0 beyond the capture end).
+SNRX_HD void pfb_combine_quant_pfa(const cf (&f0)[16], const cf (&f1)[16], const cf (&f2)[16], uint32_t (&sw)[48],
+                                   uint32_t (&sa)[48], float s_even, float s_odd, cf (&raw)[48], bool keep_raw) {
+    cf y[48];
+    Pfa48::template combine<0>(f0, f1, f2, y);
+    const float se = f_mul(s_even, 1.0f / 255.0f), so = f_mul(s_odd, 1.0f / 255.0f);
+#pragma unroll
+    for (int q = 0; q < 48; q++) {
+        if (ble_channel_of_q(q) < 0) { sw[q] = sa[q] = 0u; if (keep_raw) raw[q] = cf{0.f, 0.f}; continue; }
+        if (keep_raw) raw[q] = y[q];
+        const float2 t = quant_pair_biased(P(y[q]), (q & 1) ? so : se);
+        sw[q] = slicer_w(f_bits(t.x), f_bits(t.y));
+        sa[q] = slicer_a(f_bits(t.x), f_bits(t.y));
+    }
+}
+
+// ---- The same phases 1-3 in their Cooley-Tukey form (twiddled radix-3 combination, float slicer): the statement the kernel
+// ran before the prime-factor map.  The kernel no longer calls these; the CPU tile harness tests/emu/emu.cu steps them against
+// the oracle, and tests/test_pfb_factored.py checks the kernel's path above against them tile by tile.
+SNRX_HD void pfb_load_col16(const float4* V, int lane, cf (&v)[16]) {          // natural order r2 = n2
 #pragma unroll
     for (int r = 0; r < 8; r++) {
         const float4 t = V[v_pos(r, lane)];
         v[r].r = t.x; v[r].i = t.y; v[r + 8].r = t.z; v[r + 8].i = t.w;
     }
 }
-
-// Radix-3 combination of the three 16-point transforms + rotation + quantisation:
-// on return y[q] holds the quantised (I, Q) of even bin 2q as integer-valued floats for the 40 bins that
-// carry a BLE channel (the other 8 are never computed: dead code for the compiler).
-// s_even / s_odd: quantiser scale with the sign of (-1)^(q m) folded in (0 beyond the capture end).
+// on return y[q] holds the quantised (I, Q) of even bin 2q as integer-valued floats for the 40 bins that carry a BLE channel
 SNRX_HD void pfb_combine_quant(const cf (&f0)[16], const cf (&f1)[16], const cf (&f2)[16], cf (&y)[48], float s_even,
                                float s_odd, cf (&raw)[48], bool keep_raw) {
     Idft3xQ<48>::template combine<0>(f0, f1, f2, y);
@@ -152,6 +231,9 @@ SNRX_HD void pfb_combine_quant(const cf (&f0)[16], const cf (&f1)[16], const cf 
         y[q] = C(quant_pair(P(y[q]), (q & 1) ? so : se));
     }
 }
+// decision b[m] = I[m] Q[m+1] - I[m+1] Q[m] > 0 as the sign bit of 0.5 - cross: the operands are integers of magnitude <= 128,
+// so 0.5 - cross is exact and never zero
+SNRX_HD uint32_t slicer_sign(float i0, float q0, float i1, float q1) { return f_bits(f_fma(i1, q0, f_fma(-i0, q1, 0.5f))); }
 
 // The 40 used bins in the order the slicer packs them: slot L of word A (L = 0..23) and of word B (L = 0..15)
 SNRX_HD constexpr int ble_q_of_slot_a(int L) { return L < 21 ? L : L + 8; }     // q = 0..20, 29..31
@@ -167,16 +249,6 @@ constexpr bool ble_slot_channels_agree() {
 }
 static_assert(ble_slot_channels_agree(), "slot -> BLE channel shortcut");
 
-// Slicer decision b[m] = I[m] Q[m+1] - I[m+1] Q[m] > 0 (btle_rx.c:1357-1361) as the sign bit of
-// 0.5 - cross: the operands are integers of magnitude <= 128, so 0.5 - cross is exact and never zero.
-SNRX_HD uint32_t slicer_sign(float i0, float q0, float i1, float q1) {
-    const float t = f_fma(i1, q0, f_fma(-i0, q1, 0.5f));
-#ifdef __CUDA_ARCH__
-    return (uint32_t)__float_as_int(t);
-#else
-    uint32_t u; memcpy(&u, &t, 4); return u;
-#endif
-}
 SNRX_HD uint32_t shift_in_sign(uint32_t acc, uint32_t sign_word) {   // (acc << 1) | (sign_word >> 31): one SHF
 #ifdef __CUDA_ARCH__
     return __funnelshift_l(sign_word, acc, 1);
@@ -396,26 +468,26 @@ __device__ __forceinline__ void pfb_ble_tile(const PfbBleArgs& a, const float2* 
             __syncwarp();
             if (gi == 2) after_fir();
             cf v16[16];
-            pfb_load_col16(V, lane, v16);
+            pfb_load_col16_pfa(V, lane, gi, v16);
             __syncwarp();                                                  // V is rewritten by the next pass
             IdftPow2<16, 1>::run(v16, f[gi]);
         }
     }
 
-    // ---- phase 2: radix-3 combination + rotation + quantiser, one lane per output time
-    cf y[48];
+    // ---- phase 2: radix-3 combination + rotation + quantiser + slicer words, one lane per output time
+    uint32_t sw[48], sa[48];
     const int mg = g_first + lane;                           // channel-rate sample index in the capture
     {
         const float s = (mg < a.n_out) ? a.scale : 0.0f;
         cf raw[48];
-        pfb_combine_quant(f[0], f[1], f[2], y, s, (mg & 1) ? -s : s, raw, DEBUG);
+        pfb_combine_quant_pfa(f[0], f[1], f[2], sw, sa, s, (mg & 1) ? -s : s, raw, DEBUG);
         if (DEBUG && lane < B::kStride && mg < a.n_out) {
 #pragma unroll
             for (int qq = 0; qq < 48; qq++) {
                 const int ch = ble_channel_of_q(qq);
                 if (ch >= 0) {
                     const size_t o = ((size_t)cap * 40 + ch) * (size_t)a.n_out + mg;
-                    if (a.dbg_q8) { a.dbg_q8[2 * o] = (int8_t)y[qq].r; a.dbg_q8[2 * o + 1] = (int8_t)y[qq].i; }
+                    if (a.dbg_q8) { a.dbg_q8[2 * o] = slicer_a_i(sa[qq]); a.dbg_q8[2 * o + 1] = slicer_a_q(sa[qq]); }
                     if (a.dbg_cf) {
                         const float sg = ((qq & 1) && (mg & 1)) ? -1.0f : 1.0f;
                         a.dbg_cf[o] = make_float2(raw[qq].r * sg, raw[qq].i * sg);
@@ -427,10 +499,10 @@ __device__ __forceinline__ void pfb_ble_tile(const PfbBleArgs& a, const float2* 
 
 #ifdef SNRX_PROBE_NO_TAIL                                    // measurement builds only (tools/ab_probe.sh): what the tail costs
     {
-        float sacc = 0.f;
+        uint32_t sacc = 0u;
 #pragma unroll
-        for (int q = 0; q < 48; q++) if (ble_channel_of_q(q) >= 0) sacc += y[q].r + y[q].i;
-        if (sacc == 12345.678f) a.bits[0] = 1u;
+        for (int q = 0; q < 48; q++) if (ble_channel_of_q(q) >= 0) sacc += sw[q] ^ sa[q];
+        if (sacc == 0x12345678u) a.bits[0] = 1u;
         return;
     }
 #endif
@@ -440,14 +512,12 @@ __device__ __forceinline__ void pfb_ble_tile(const PfbBleArgs& a, const float2* 
 #pragma unroll
         for (int L = 23; L >= 0; L--) {
             const int qq = ble_q_of_slot_a(L);
-            const float i1 = __shfl_down_sync(0xffffffffu, y[qq].r, 1), q1 = __shfl_down_sync(0xffffffffu, y[qq].i, 1);
-            wa = shift_in_sign(wa, slicer_sign(y[qq].r, y[qq].i, i1, q1));
+            wa = shift_in_sign(wa, slicer_sign_dp4a(sa[qq], __shfl_down_sync(0xffffffffu, sw[qq], 1)));
         }
 #pragma unroll
         for (int L = 15; L >= 0; L--) {
             const int qq = ble_q_of_slot_b(L);
-            const float i1 = __shfl_down_sync(0xffffffffu, y[qq].r, 1), q1 = __shfl_down_sync(0xffffffffu, y[qq].i, 1);
-            wb = shift_in_sign(wb, slicer_sign(y[qq].r, y[qq].i, i1, q1));
+            wb = shift_in_sign(wb, slicer_sign_dp4a(sa[qq], __shfl_down_sync(0xffffffffu, sw[qq], 1)));
         }
         // rows = times (lanes), columns = slots  ->  rows = slots, columns = times
         {
