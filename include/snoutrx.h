@@ -138,7 +138,9 @@ typedef struct snrx_config {
     uint32_t pfb_taps;       /* WB: prototype length, 384 or 768 (0 = default 384)         */
     uint32_t flags;          /* SNRX_F_*                                                   */
     uint32_t access_mask;    /* BLE `-m`: access-address bits that take part in the match
-                                (0 = default 0xFFFFFFFF, btle_rx.c:1203,2301)                */
+                                (0 = default 0xFFFFFFFF, btle_rx.c:1203,2301).  access_addr & mask must not be 0
+                                (SNRX_EINVAL): such an address matches every run of zero decisions, so the
+                                reference would decode a frame at every search origin, past the capture too */
     uint32_t reserved;       /* must be 0                                                  */
 } snrx_config_t;
 
@@ -342,7 +344,8 @@ typedef struct snrx_conn {          /* one per CRC-ok CONNECT_REQ (ADV PDU type 
 int  snrx_ble_connections(snrx_t* h, snrx_conn_t* out, uint32_t cap, uint32_t* n_out);
 /* Searches and decodes the BLE channels of that same batch again with another access address / CRC init (`-a` / `-k` of a
  * connection learned from snrx_ble_connections): *n_out frames in reference order, copied to out (up to cap).  The batch's
- * slicer bit streams are reused: nothing is channelized twice.  Call before the second-next snrx_process. */
+ * slicer bit streams are reused: nothing is channelized twice.  Call before the second-next snrx_process.  access_addr 0 is
+ * refused (SNRX_EINVAL), like an all-zero compared address at snrx_create. */
 int  snrx_ble_follow(snrx_t* h, uint32_t access_addr, uint32_t crc_init, snrx_frame_t* out, uint32_t cap, uint32_t* n_out);
 
 /* ---- SURVEY 8(f) N2: the Zigbee consumer path on the decoded 802.15.4 records (what Snout does per datagram:

@@ -498,6 +498,10 @@ int snrx_create(snrx_t** out, const snrx_config_t* cfg) {
         h->pfb_nt = (int)c.pfb_taps / 24;
         if (h->has_ble && !h->wideband && (c.channel < 0 || c.channel > 39)) return fail(h, SNRX_EINVAL, "BLE channel 0..39");
         if (h->has_zb && !h->wideband && (c.channel < 11 || c.channel > 26)) return fail(h, SNRX_EINVAL, "802.15.4 channel 11..26");
+        // With no compared 1 bit, runs of zero decisions match the address: btle_rx.c then "finds" a frame at every search origin,
+        // in the zero samples past the end of a capture too, where the sliding correlation (k_aa_search) has no start positions.
+        if (h->has_ble && (c.access_addr & (c.access_mask ? c.access_mask : 0xFFFFFFFFu)) == 0u)
+            return fail(h, SNRX_EINVAL, "BLE access_addr & access_mask must have a bit set");
         if (h->wideband && (c.max_samples % (uint64_t)(kPfbD * 2)) != 0) c.max_samples += (kPfbD * 2) - c.max_samples % (kPfbD * 2);
         h->max_in = c.max_samples;
         h->max_caps = c.max_captures;
@@ -1091,6 +1095,7 @@ int snrx_ble_follow(snrx_t* h, uint32_t access_addr, uint32_t crc_init, snrx_fra
     Lane& ln = h->lane[h->polled_lane];
     if (!h->has_ble || !ln.last_ble) return fail(h, SNRX_ESTATE, "snrx_ble_follow: the polled batch has no BLE bit streams");
     if (ln.pending) return fail(h, SNRX_ESTATE, "snrx_ble_follow: the batch's bit streams have been overwritten (call before the second-next snrx_process)");
+    if (access_addr == 0u) return fail(h, SNRX_EINVAL, "snrx_ble_follow: access_addr must have a bit set (see snrx_create)");
     CK(cudaSetDevice(h->device));
     if (!h->d_follow) CK(cudaMalloc((void**)&h->d_follow, sizeof(snrx_frame_t) * (size_t)h->frame_cap));
     cudaStream_t st = ln.tail;                                   // the lane is idle: its working set and streams are free
