@@ -348,6 +348,81 @@ int  snrx_ble_connections(snrx_t* h, snrx_conn_t* out, uint32_t cap, uint32_t* n
  * refused (SNRX_EINVAL), like an all-zero compared address at snrx_create. */
 int  snrx_ble_follow(snrx_t* h, uint32_t access_addr, uint32_t crc_init, snrx_frame_t* out, uint32_t cap, uint32_t* n_out);
 
+/* ---- BLE 5 extended advertising: the auxiliary packets (AUX_ADV_IND, AUX_CHAIN_IND) that the ADV_EXT_INDs of a batch point
+ * at, on the 1M and 2M PHYs, found and decoded from the batch's slicer bit streams (wideband BLE modes; nothing is
+ * channelized twice).  No reference receiver exists for this: the definition below is the contract, and the GPU equals it
+ * bit for bit on the engine's own bit streams (oracle/aux_oracle.py restates it).
+ *
+ * Pointer sources.  Depth 0: the records of the batch most recently retired by snrx_poll / snrx_poll_view with proto BLE,
+ *   channel 37..39, crc_ok, access_addr 0x8E89BED6, PDU type 7 (header byte 0 & 0x0F), whose payload byte 0 gives an extended
+ *   header length L >= 1 (bits 0..5) with 1 + L <= payload length, whose extended header flags (payload byte 1) have the AuxPtr
+ *   bit (0x10) set, and whose extended header holds the fields in front of the AuxPtr (AdvA 6, TargetA 6, CTEInfo 1, ADI 2
+ *   bytes, each if its flag bit 0..3 is set) and the AuxPtr itself: 2 + those fields + 3 <= 1 + L.
+ *   Depth d > 0: the entries of depth d - 1 of this list with status OK, crc_ok, first == their own index, and the same
+ *   AuxPtr conditions on their PDU (type 7 with an AuxPtr; the length is the full header byte 1).
+ * AuxPtr (3 bytes a0 a1 a2): channel index a0 & 0x3F; CA (a0 >> 6) & 1; Offset Units (a0 >> 7): U = 30 or 300 us;
+ *   Aux Offset A = a1 | (a2 & 0x1F) << 8; Aux PHY a2 >> 5 (SNRX_AUX_PHY_*).
+ * Window.  s = the source's sample_index (AA bit 0, channel rate; for both PHYs AA bit 0 lies 32 samples after the first
+ *   preamble sample).  O = A * U, ppm = 50 if CA else 500; the candidate positions n of the auxiliary packet's AA bit 0 are
+ *     win_lo = s + floor(4 * O * (10^6 - ppm) / 10^6) - 8,   win_hi = s + ceil(4 * (O + U) * (10^6 + ppm) / 10^6) + 8
+ *   (integer arithmetic, inclusive).
+ * Search.  b[n] = the slicer decision of channel sample n of the aux channel (SNRX_STAGE_BLE_BITS); sps = 4 (1M) or 2 (2M).
+ *   Decision n is usable when n + 1 < the buffer's channel samples (it pairs sample n with n + 1).  The earliest n in the
+ *   window whose 32 decisions b[n + k sps] (k = 0..31) equal 0x8E89BED6 LSB first, all 32 bits compared.
+ * Decode.  Byte j bit i = b[n + (32 + 8 j + i) sps]; the 2-byte header, len = header byte 1 (all 8 bits), then len + 3 more
+ *   bytes; de-whitened with the x^7+x^4+1 LFSR seeded by the aux channel index (continued to 260 bytes); CRC-24 with
+ *   crc_init 0x555555 (as snrx_create maps it) over 2 + len bytes, compared with the 3 bytes that follow.
+ * Status (one per pointer, in this order of precedence):
+ *   SNRX_AUX_DEPTH_LIMIT     depth > 15: not searched (chains are followed to depth 15)
+ *   SNRX_AUX_BAD_CHANNEL     channel index > 36
+ *   SNRX_AUX_UNSUPPORTED_PHY Coded or reserved PHY: not searched
+ *   SNRX_AUX_OUTSIDE         win_lo or win_hi + 31 sps is not a usable decision of the buffer (the capture, or a shard's
+ *                            pre-halo to post-halo span): not searched
+ *   SNRX_AUX_NOT_FOUND       no match in the window
+ *   SNRX_AUX_TRUNCATED       found, but the header's or the packet's last decision is not usable
+ *   SNRX_AUX_OK              decoded; crc_ok says whether the CRC matches
+ * Order and duplicates.  The list is ordered by depth, then by parent.  first = the list index of the earliest entry with
+ *   status OK or TRUNCATED of the same (capture_id, channel, sample_index, phy), its own index if there is none; only
+ *   entries with first == their own index start chains (the three ADV_EXT_INDs of an event normally point at one packet,
+ *   and a chain that points back at itself ends there).
+ * Shards.  Indices are whole-capture indices, as in the records.  A pointer whose window and packet lie inside both buffers
+ *   gives the same entry in a time shard as in the whole capture; one that reaches past a shard's buffer is OUTSIDE there
+ *   (pointers are not carried across shard boundaries). */
+#define SNRX_AUX_OK              0
+#define SNRX_AUX_NOT_FOUND       1
+#define SNRX_AUX_OUTSIDE         2
+#define SNRX_AUX_TRUNCATED       3
+#define SNRX_AUX_UNSUPPORTED_PHY 4
+#define SNRX_AUX_BAD_CHANNEL     5
+#define SNRX_AUX_DEPTH_LIMIT     6
+#define SNRX_AUX_PHY_1M    0
+#define SNRX_AUX_PHY_2M    1
+#define SNRX_AUX_PHY_CODED 2
+#define SNRX_AUX_MAX_DEPTH 15
+#define SNRX_AUX_MAX_BYTES 260    /* 2 header + 255 payload + 3 CRC */
+
+typedef struct snrx_ble_aux {       /* one per pointer, 304 bytes */
+    int64_t  sample_index;  /* AA bit 0 of the auxiliary packet (channel rate, capture relative); -1 unless OK / TRUNCATED */
+    int64_t  win_lo, win_hi;/* the searched window of AA bit 0 positions, inclusive, capture relative                     */
+    uint32_t capture_id;
+    uint32_t parent;        /* depth 0: index of the ADV_EXT_IND record in the batch; deeper: index of the parent entry   */
+    uint32_t first;         /* list index of the earliest entry that found the same packet (own index if none)           */
+    uint8_t  depth;         /* 0 = pointed at by an ADV_EXT_IND, d = d links down a chain                                */
+    uint8_t  channel;       /* AuxPtr channel index                                                                      */
+    uint8_t  phy;           /* SNRX_AUX_PHY_*                                                                            */
+    uint8_t  phase;         /* sample_index mod sps (0 unless OK / TRUNCATED)                                            */
+    uint8_t  status;        /* SNRX_AUX_*                                                                                */
+    uint8_t  crc_ok;        /* status OK and the CRC matches                                                             */
+    uint16_t len;           /* valid bytes in bytes[]: 2 + header length + 3 (0 unless OK)                               */
+    uint8_t  bytes[SNRX_AUX_MAX_BYTES];   /* de-whitened header | payload | CRC, zero past len                           */
+} snrx_ble_aux_t;
+
+/* The auxiliary packets of the batch most recently retired by snrx_poll / snrx_poll_view (definition above): *n_out entries,
+ * copied to out (up to cap; out may be NULL to count).  Call before the second-next snrx_process.  SNRX_ESTATE without a
+ * polled wideband BLE batch (SNRX_MODE_BLE_WB40 / SNRX_MODE_MIXED_WB56) or once its bit streams have been overwritten;
+ * SNRX_ERANGE if cap is smaller than the list; SNRX_EOVERFLOW if the list would hold more than max_frames entries. */
+int  snrx_ble_aux(snrx_t* h, snrx_ble_aux_t* out, uint32_t cap, uint32_t* n_out);
+
 /* ---- SURVEY 8(f) N2: the Zigbee consumer path on the decoded 802.15.4 records (what Snout does per datagram:
  * RFtap(pkt) -> Dot15d4FCS dissection, snout/util/zigbee.py:194-202; ZigbeeMessage.fromraw, snout/core/message.py:258-304;
  * the touchlink scan's haslayer(ZLLScanResponse), zigbee.py:176-192) ---- */

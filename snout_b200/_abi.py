@@ -55,6 +55,15 @@ RF_DTYPE = np.dtype([("sample_index", "<i8"), ("capture_id", "<u4"), ("frame", "
                      ("reserved", "<u4")], align=True)
 assert RF_DTYPE.itemsize == 40
 
+# BLE 5 extended advertising: one entry per AuxPtr (include/snoutrx.h snrx_ble_aux_t)
+AUX_OK, AUX_NOT_FOUND, AUX_OUTSIDE, AUX_TRUNCATED, AUX_UNSUPPORTED_PHY, AUX_BAD_CHANNEL, AUX_DEPTH_LIMIT = range(7)
+AUX_PHY_1M, AUX_PHY_2M, AUX_PHY_CODED = 0, 1, 2
+AUX_MAX_DEPTH, AUX_MAX_BYTES = 15, 260
+AUX_DTYPE = np.dtype([("sample_index", "<i8"), ("win_lo", "<i8"), ("win_hi", "<i8"), ("capture_id", "<u4"), ("parent", "<u4"),
+                      ("first", "<u4"), ("depth", "u1"), ("channel", "u1"), ("phy", "u1"), ("phase", "u1"), ("status", "u1"),
+                      ("crc_ok", "u1"), ("len", "<u2"), ("bytes", "u1", (AUX_MAX_BYTES,))], align=True)
+assert AUX_DTYPE.itemsize == 304
+
 FRAME_DTYPE = np.dtype([
     ("sample_index", "<i8"), ("capture_id", "<u4"), ("window", "<u4"), ("channel", "<u2"),
     ("proto", "u1"), ("crc_ok", "u1"), ("lqi", "u1"), ("phase", "u1"), ("len", "<u2"),
@@ -128,6 +137,7 @@ SYMBOLS = [
     ("snrx_ble_devices", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32), c_int]),
     ("snrx_ble_connections", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_ble_follow", c_int, [c_void_p, c_uint32, c_uint32, c_void_p, c_uint32, POINTER(c_uint32)]),
+    ("snrx_ble_aux", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_zb_mac_summary", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_frame_rf", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_exchange_create", c_int, [c_void_p, c_uint32, c_uint32, c_uint32, c_void_p]),

@@ -27,6 +27,15 @@ and every LL PDU of the connection is printed with the channel it was heard on -
 missed events.  The `Hop:` status lines of the reference are printed where it prints them.  With
 one 4 Msps channel there is nothing to hop to and `-o` is refused.
 
+`--aux` (with `--wideband`) also receives BLE 5 extended advertising: every ADV_EXT_IND's AuxPtr is followed to its
+AUX_ADV_IND and down its AUX_CHAIN_INDs on the 1M and 2M PHYs (RxEngine.ble_aux), and every auxiliary packet found is
+printed, whatever `-c` selects, as one line of 8 tokens (formats.aux_line):
+
+    AUX Ch<ch> PHY<1M|2M> AdvA:<address or -> ADI:<DID hex>/<SID hex or -> Depth<d> PloadL<len> CRC<0|1>
+
+It starts with AUX instead of a timestamp and a Pkt token, so a parser of the reference's lines does not take it for one.
+With `-s` the packets also go to the pcap (formats.ble_pcap_aux_block).
+
 There is no CPU path: without a usable GPU / libsnoutrx.so the program exits with an error.
 """
 from __future__ import annotations
@@ -37,7 +46,7 @@ import sys
 
 import numpy as np
 
-from . import chanplan, formats
+from . import chanplan, formats, messages
 
 DEFAULT_CHANNEL, DEFAULT_GAIN, MAX_GAIN, MAX_CHANNEL = 37, 6, 62, 39        # btle_rx.c:187,486,485,190
 USAGE = """Usage:
@@ -76,6 +85,8 @@ USAGE = """Usage:
       With --wideband: print frames of every channel, not just -c
     --device N
       CUDA device ordinal (default 0)
+    --aux
+      With --wideband: also follow BLE 5 extended advertising to its auxiliary packets (1M and 2M PHYs) and print them
     --rf
       Measure signal power, noise floor and carrier offset of every frame; with -s the pcap's PHDR carries the
       signal and noise power (dBFS, flags 0x0002 / 0x0004).  Stdout lines are unchanged
@@ -103,6 +114,7 @@ class Options:
     device = 0
     shard_windows = 0
     rf = False
+    aux = False
 
 
 def _strtol(text: str, base: int) -> int:
@@ -134,7 +146,7 @@ def parse_commandline(argv: list[str], out=sys.stdout) -> Options | None:
         opts, rest = getopt.getopt(argv, "hc:g:a:k:vrf:m:os:",
                                    ["help", "chan=", "gain=", "access=", "crcinit=", "verbose", "raw", "freq_hz=",
                                     "access_mask=", "hop", "filename=", "iq=", "format=", "scale=", "wideband",
-                                    "all-channels", "device=", "shard-windows=", "rf"])
+                                    "all-channels", "device=", "shard-windows=", "rf", "aux"])
     except getopt.GetoptError as e:
         out.write(f"btle_rx: {e}\n")
         out.write(USAGE)
@@ -179,6 +191,8 @@ def parse_commandline(argv: list[str], out=sys.stdout) -> Options | None:
             o.shard_windows = int(v)
         elif k == "--rf":
             o.rf = True
+        elif k == "--aux":
+            o.aux = True
     if o.chan < 0 or o.chan > MAX_CHANNEL:
         out.write(f"channel number must be within 0~{MAX_CHANNEL}!\n")
         out.write(USAGE)
@@ -208,6 +222,9 @@ def run(o: Options, out=sys.stdout, engine_factory=None, blocks=None) -> int:
         return 1
     if o.hop and not o.wideband:
         out.write("btle_rx (snout_b200): -o/--hop needs --wideband (a 4 Msps single-channel capture holds no data channel to hop to)\n")
+        return 1
+    if o.aux and not o.wideband:
+        out.write("btle_rx (snout_b200): --aux needs --wideband (auxiliary packets are sent on the data channels)\n")
         return 1
     if o.iq is None and blocks is None:
         out.write("btle_rx (snout_b200): no IQ source; pass --iq FILE (or - for stdin)\n")
@@ -263,6 +280,12 @@ def run(o: Options, out=sys.stdout, engine_factory=None, blocks=None) -> int:
                 follow(frames)
             else:
                 lines(frames, rf=rf)
+            if o.aux:
+                aux = eng.ble_aux()
+                if fh_pcap:
+                    fh_pcap.write(formats.ble_pcap_aux_block(aux))
+                for d in messages.ble_ext_adv(aux):
+                    out.write(formats.aux_line(d))
             out.flush()                                                # fflush(stdout), btle_rx.c:2383
 
         def follow(frames: np.ndarray):

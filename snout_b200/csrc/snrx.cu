@@ -23,6 +23,7 @@
 #define SNRX_PFB_TILES_DEFAULT 0
 #endif
 #include "ble_adv.cuh"
+#include "ble_aux.cuh"
 #include "ble_back.cuh"
 #include "ble_conn.cuh"
 #include "ble_front.cuh"
@@ -100,6 +101,10 @@ struct snrx_handle {
     snrx_zbmac_t* d_zbmac = nullptr;
     snrx_conn_t* d_conn = nullptr; uint32_t *d_conn_flags = nullptr, *d_conn_offsets = nullptr, *d_conn_scratch = nullptr;
     snrx_frame_t* d_follow = nullptr;    // frames of snrx_ble_follow
+    // snrx_ble_aux, allocated by its first call: the list (max_frames entries), flags / offsets / scan scratch of a round, and
+    // the whitening sequences continued to 260 bytes
+    snrx_ble_aux_t* d_aux = nullptr; uint32_t *d_aux_flags = nullptr, *d_aux_offsets = nullptr, *d_aux_scratch = nullptr;
+    uint8_t* d_aux_whiten = nullptr;
     snrx::DevSlot* d_devtab = nullptr;
     snrx_device_t* d_devout = nullptr;
     uint32_t* d_adv_counters = nullptr;   // [0] records summarised (BLE), [1] new devices, [2] dropped (table full), [3] export count
@@ -179,24 +184,28 @@ void make_crc_table(uint32_t* t) {
         t[i] = r;
     }
 }
-// Whitening LFSR x^7+x^4+1, register = 1 | channel MSB first (Core spec Vol 6 Part B 3.2);
+// Whitening LFSR x^7+x^4+1, register = 1 | channel MSB first (Core spec Vol 6 Part B 3.2): the first n bytes of a channel's
+// sequence, LSB first.
+void make_whiten_bytes(int ch, uint8_t* bytes, int n) {
+    unsigned reg = 0;                           // bit p = register position p
+    reg |= 1u;
+    for (int k = 0; k < 6; k++) reg |= ((unsigned)(ch >> (5 - k)) & 1u) << (1 + k);
+    for (int i = 0; i < n; i++) {
+        uint8_t v = 0;
+        for (int b = 0; b < 8; b++) {
+            unsigned out = (reg >> 6) & 1u;
+            v |= (uint8_t)(out << b);
+            reg = ((reg << 1) & 0x7Fu) | out;
+            reg ^= out << 4;
+        }
+        bytes[i] = v;
+    }
+}
 // 42 bytes per channel packed little-endian into 11 words.  Equals scramble_table.h.
 void make_whiten_table(uint32_t* w /*[40][11]*/) {
     for (int ch = 0; ch < 40; ch++) {
         uint8_t bytes[44] = {0};
-        unsigned reg = 0;                       // bit p = register position p
-        reg |= 1u;
-        for (int k = 0; k < 6; k++) reg |= ((unsigned)(ch >> (5 - k)) & 1u) << (1 + k);
-        for (int i = 0; i < 42; i++) {
-            uint8_t v = 0;
-            for (int b = 0; b < 8; b++) {
-                unsigned out = (reg >> 6) & 1u;
-                v |= (uint8_t)(out << b);
-                reg = ((reg << 1) & 0x7Fu) | out;
-                reg ^= out << 4;
-            }
-            bytes[i] = v;
-        }
+        make_whiten_bytes(ch, bytes, 42);
         for (int c = 0; c < 11; c++)
             w[ch * 11 + c] = (uint32_t)bytes[4 * c] | ((uint32_t)bytes[4 * c + 1] << 8) |
                              ((uint32_t)bytes[4 * c + 2] << 16) | ((uint32_t)bytes[4 * c + 3] << 24);
@@ -448,7 +457,8 @@ void snrx_destroy(snrx_t* h) {
     if (h->xchg.d_recv) cudaFree(h->xchg.d_recv);
     if (h->xchg.h_hdr) cudaFreeHost(h->xchg.h_hdr);
     if (h->adv_stream) { cudaStreamSynchronize(h->adv_stream); cudaStreamDestroy(h->adv_stream); }
-    { void* ab[] = {h->d_adv, h->d_zbmac, h->d_conn, h->d_conn_flags, h->d_conn_offsets, h->d_conn_scratch, h->d_follow, h->d_devtab, h->d_devout, h->d_adv_counters}; for (void* b : ab) if (b) cudaFree(b); }
+    { void* ab[] = {h->d_adv, h->d_zbmac, h->d_conn, h->d_conn_flags, h->d_conn_offsets, h->d_conn_scratch, h->d_follow, h->d_devtab, h->d_devout, h->d_adv_counters,
+                    h->d_aux, h->d_aux_flags, h->d_aux_offsets, h->d_aux_scratch, h->d_aux_whiten}; for (void* b : ab) if (b) cudaFree(b); }
     delete h;
 }
 
@@ -1130,6 +1140,61 @@ int snrx_ble_follow(snrx_t* h, uint32_t access_addr, uint32_t crc_init, snrx_fra
     if (out && tot[0]) {
         if (cap < tot[0]) return fail(h, SNRX_ERANGE, "frame buffer smaller than the number of frames");
         CK(cudaMemcpy(out, h->d_follow, sizeof(snrx_frame_t) * (size_t)tot[0], cudaMemcpyDeviceToHost));
+    }
+    return SNRX_OK;
+}
+
+int snrx_ble_aux(snrx_t* h, snrx_ble_aux_t* out, uint32_t cap, uint32_t* n_out) {
+    if (!h) return SNRX_EINVAL;
+    if (n_out) *n_out = 0;
+    if (h->polled_lane < 0) return fail(h, SNRX_ESTATE, "snrx_ble_aux needs a polled batch");
+    Lane& ln = h->lane[h->polled_lane];
+    if (!h->has_ble || !h->wideband || !ln.last_ble) return fail(h, SNRX_ESTATE, "snrx_ble_aux: the polled batch has no wideband BLE bit streams");
+    if (ln.pending) return fail(h, SNRX_ESTATE, "snrx_ble_aux: the batch's bit streams have been overwritten (call before the second-next snrx_process)");
+    CK(cudaSetDevice(h->device));
+    if (!h->d_aux) {
+        CK(cudaMalloc((void**)&h->d_aux, sizeof(snrx_ble_aux_t) * (size_t)h->frame_cap));
+        CK(cudaMalloc((void**)&h->d_aux_flags, sizeof(uint32_t) * ((size_t)h->frame_cap + 1)));
+        CK(cudaMalloc((void**)&h->d_aux_offsets, sizeof(uint32_t) * ((size_t)h->frame_cap + 1)));
+        CK(cudaMalloc((void**)&h->d_aux_scratch, sizeof(uint32_t) * scan_scratch_items(h->frame_cap)));
+        std::vector<uint8_t> wh(40 * SNRX_AUX_MAX_BYTES);
+        for (int ch = 0; ch < 40; ch++) make_whiten_bytes(ch, wh.data() + ch * SNRX_AUX_MAX_BYTES, SNRX_AUX_MAX_BYTES);
+        CK(cudaMalloc((void**)&h->d_aux_whiten, wh.size()));
+        CK(cudaMemcpy(h->d_aux_whiten, wh.data(), wh.size(), cudaMemcpyHostToDevice));
+    }
+    cudaStream_t st = ln.tail;                                   // the lane is idle: its bit streams stay as the batch left them
+    const BleParams& p = ln.last_p;
+    AuxGeom g{};
+    g.bits = ln.d_bits; g.lay = ln.last_lay; g.n_out = p.n_out;
+    g.base = (int64_t)kWindow * p.first_window - p.m_origin;
+    g.first_capture = p.first_capture; g.n_captures = p.n_captures;
+    const AaTables tabs = make_aa_tables(kAuxAdvAa, 0xFFFFFFFFu);
+    const uint32_t crc_init = crc_init_internal(0x555555u);
+    AuxSrc src{};
+    src.frames = h->polled_frames_dev; src.list = h->d_aux; src.first = 0; src.n = ln.n_frames; src.depth = 0;
+    uint32_t total = 0;
+    // one round per depth: the pointers of depth d come from the entries of depth d - 1 (the records at d = 0)
+    while (src.n > 0 && src.depth <= SNRX_AUX_MAX_DEPTH + 1) {
+        k_ble_aux_flag<<<div_up(src.n, 256), 256, 0, st>>>(src, h->d_aux_flags);
+        exclusive_scan(h->d_aux_flags, src.n, h->d_aux_offsets, h->d_aux_scratch, st);
+        uint32_t m = 0;
+        CK(cudaMemcpyAsync(&m, h->d_aux_offsets + src.n, sizeof m, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        if (m == 0) break;
+        if ((uint64_t)total + m > h->frame_cap) return fail(h, SNRX_EOVERFLOW, "snrx_ble_aux: more auxiliary pointers than max_frames");
+        k_ble_aux_fill<<<div_up(src.n, 256), 256, 0, st>>>(src, h->d_aux_flags, h->d_aux_offsets, h->d_aux, total, g);
+        const int gs = grid_for(h, m, 4, 8);
+        k_ble_aux_search<<<gs, 128, 0, st>>>(h->d_aux, total, total + m, g, h->d_crc_tab, h->d_aux_whiten, crc_init, tabs);
+        k_ble_aux_first<<<grid_for(h, m, 8, 8), 256, 0, st>>>(h->d_aux, total, total + m);
+        CK(cudaGetLastError());
+        src.frames = nullptr; src.first = total; src.n = m; src.depth++;
+        total += m;
+    }
+    if (n_out) *n_out = total;
+    if (out && total) {
+        if (cap < total) return fail(h, SNRX_ERANGE, "snrx_ble_aux: buffer smaller than the list");
+        CK(cudaMemcpyAsync(out, h->d_aux, sizeof(snrx_ble_aux_t) * (size_t)total, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
     }
     return SNRX_OK;
 }

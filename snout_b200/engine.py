@@ -289,6 +289,18 @@ class RxEngine:
         self._check(self.lib.snrx_ble_follow(self.handle, access_addr & 0xFFFFFFFF, crc_init & 0xFFFFFF, out.ctypes.data_as(c_void_p), cap, byref(n)))
         return out[: n.value].copy()
 
+    # ------------------------------------------------------------------ BLE 5 extended advertising
+    def ble_aux(self) -> np.ndarray:
+        """The auxiliary packets (AUX_ADV_IND, AUX_CHAIN_IND) that the ADV_EXT_INDs of the batch most recently returned by
+        poll() point at, followed down their chains, on the 1M and 2M PHYs: one _abi.AUX_DTYPE entry per AuxPtr, found and
+        decoded on the GPU from the batch's slicer bit streams (definition in include/snoutrx.h).  Wideband BLE modes; call
+        before the second-next process()."""
+        n = c_uint32(0)
+        cap = int(self.cfg.max_frames) or (1 << 17)
+        out = np.zeros(cap, dtype=_abi.AUX_DTYPE)
+        self._check(self.lib.snrx_ble_aux(self.handle, out.ctypes.data_as(c_void_p), cap, byref(n)))
+        return out[: n.value].copy()
+
     # ------------------------------------------------------------------ SURVEY 8(f) N2: Zigbee consumer path
     def zb_mac_summary(self) -> np.ndarray:
         """Per-record MAC summaries (_abi.ZBMAC_DTYPE: frame type, sequence number, PAN ids, addresses, inter-PAN / ZLL

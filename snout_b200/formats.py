@@ -31,7 +31,7 @@ from typing import BinaryIO, Iterable
 
 import numpy as np
 
-from ._abi import PROTO_BLE, PROTO_ZIGBEE, RF_CFO, RF_NOISE, RF_POWER
+from ._abi import AUX_OK, PROTO_BLE, PROTO_ZIGBEE, RF_CFO, RF_NOISE, RF_POWER
 
 # ---------------------------------------------------------------------------------- BLE text line
 ADV_PDU_TYPE_STR = (      # btle_rx.c:1081-1098
@@ -245,6 +245,39 @@ def ble_pcap_block(frames: np.ndarray, ts: tuple[int, int] = (0, 0), rf=None, db
         prefix[:, 24] |= np.where(p_ok, PHDR_SIGNAL_VALID, 0).astype(np.uint8) | np.where(n_ok, PHDR_NOISE_VALID, 0).astype(np.uint8)
     prefix[:, 26:30] = f["access_addr"].astype("<u4").view(np.uint8).reshape(n, 4)
     return _pack_records(prefix, f["bytes"], lens)
+
+
+# LINKTYPE_BLUETOOTH_LE_LL_WITH_PHDR flags bits 7..9: PDU type (1 = auxiliary advertising); bits 14..15: PHY (0 = LE 1M,
+# 1 = LE 2M, 2 = LE Coded) -- the link-type definition published by tcpdump.org
+PHDR_PDU_TYPE_SHIFT, PHDR_PDU_AUX_ADV, PHDR_PHY_SHIFT = 7, 1, 14
+
+
+def ble_pcap_aux_block(aux: np.ndarray, ts: tuple[int, int] = (0, 0)) -> bytes:
+    """The auxiliary packets of RxEngine.ble_aux() that were decoded (status OK) by the first entry to find them, as records
+    of the file btle_rx -s writes (see ble_pcap_record): PHDR {channel, 0, 0, 0, 0, 0, 0, 0, flags}, flags = de-whitened |
+    PDU type 1 (auxiliary advertising) << 7 | PHY << 14, then the advertising access address and header | payload (no
+    CRC).  CRC-failed packets are written too, as btle_rx writes its CRC-failed frames."""
+    sel = (aux["status"] == AUX_OK) & (aux["first"] == np.arange(len(aux)))
+    a = aux[sel]
+    n = len(a)
+    lens = a["len"].astype(np.int64) - 3
+    prefix = np.zeros((n, 16 + 10 + 4), dtype=np.uint8)
+    prefix[:, 0:8] = np.frombuffer(struct.pack("<ii", ts[0], ts[1]), dtype=np.uint8)
+    be = (10 + 4 + lens).astype(">i4").view(np.uint8).reshape(n, 4)
+    prefix[:, 8:12], prefix[:, 12:16] = be, be
+    prefix[:, 16] = a["channel"]
+    flags = PHDR_DEWHITENED | (PHDR_PDU_AUX_ADV << PHDR_PDU_TYPE_SHIFT) | (a["phy"].astype(np.int64) << PHDR_PHY_SHIFT)
+    prefix[:, 24:26] = flags.astype("<u2").view(np.uint8).reshape(n, 2)
+    prefix[:, 26:30] = np.frombuffer(struct.pack("<I", 0x8E89BED6), dtype=np.uint8)
+    return _pack_records(prefix, a["bytes"], lens)
+
+
+def aux_line(d: dict) -> str:
+    """btle_rx --aux line of one decoded auxiliary packet (a messages.ble_ext_adv dictionary), 8 tokens:
+    AUX Ch<ch> PHY<1M|2M> AdvA:<address or -> ADI:<DID>/<SID> (hex, - if absent) Depth<d> PloadL<len> CRC<0 ok|1 failed>."""
+    adi = f"{d['did']:03x}/{d['sid']:x}" if d["adi"] is not None else "-/-"
+    return (f"AUX Ch{d['channel']} PHY{d['phy']} AdvA:{d['adv_a'] or '-'} ADI:{adi} Depth{d['depth']} "
+            f"PloadL{d['pload_len']} CRC{0 if d['crc_ok'] else 1}\n")
 
 
 def write_ble_pcap(fh: BinaryIO, frames: Iterable, header: bool = True, rf=None, dbm_offset: float = 0.0) -> int:

@@ -72,3 +72,71 @@ def device_fingerprints(devices: np.ndarray, company_names: dict | None = None) 
         out.append(dict(address=bytes(d["adv_a"])[::-1].hex(), tx_add=int(d["tx_add"]), vendor=vendor, model=_MODEL_TEXT[int(d["model"])],
                         os=_OS_TEXT[int(d["os"])]))
     return out
+
+
+# ----------------------------------------------------------------------------------------- BLE 5 extended advertising
+def _ext_fields(pdu: bytes) -> dict:
+    """Common extended advertising payload of a PDU of type 7 (header | payload | CRC): AdvMode and the flagged fields of the
+    extended header in their order (Core Vol 6 Part B 2.3.4), then AdvData.  A field the header is too short for is None."""
+    n_payload = pdu[1]
+    p = pdu[2:2 + n_payload]
+    out = dict(adv_mode=None, adv_a=None, target_a=None, adi=None, did=None, sid=None, tx_power=None, aux_ptr=None, adv_data=b"")
+    if not p:
+        return out
+    hlen, out["adv_mode"] = p[0] & 0x3F, p[0] >> 6
+    hdr = p[1:1 + hlen]
+    out["adv_data"] = bytes(p[1 + hlen:])
+    if not hdr:
+        return out
+    flags, at = hdr[0], 1
+    for bit, name, size in ((0, "adv_a", 6), (1, "target_a", 6), (2, "cte_info", 1), (3, "adi", 2), (4, "aux_ptr", 3),
+                            (5, "sync_info", 18), (6, "tx_power", 1)):
+        if not flags & (1 << bit):
+            continue
+        v = bytes(hdr[at:at + size])
+        at += size
+        if len(v) < size:
+            break
+        if name in ("adv_a", "target_a"):
+            out[name] = v[::-1].hex()                         # printed most significant byte first, as btle_rx prints AdvA
+        elif name == "adi":
+            a = int.from_bytes(v, "little")
+            out["adi"], out["did"], out["sid"] = a, a & 0x0FFF, a >> 12
+        elif name == "tx_power":
+            out["tx_power"] = v[0] - 256 if v[0] > 127 else v[0]
+        elif name == "aux_ptr":
+            out["aux_ptr"] = v
+    return out
+
+
+def ble_ext_adv(aux: np.ndarray) -> list[dict]:
+    """One dictionary per auxiliary packet of RxEngine.ble_aux() that was decoded (status OK) and is the first entry to have
+    found it: index, channel, phy ('1M' / '2M'), depth, crc_ok, tx_add, pload_len (header length field), adv_mode, adv_a, target_a, adi / did / sid, tx_power,
+    adv_data.  The AUX_ADV_INDs (depth 0) also carry `chain` (the list indices of the chain from it) and `chain_data`: the
+    AdvData of the whole chain reassembled in order, and `complete`: every link was received with a good CRC and the last
+    one points nowhere."""
+    out, by_index = [], {}
+    children = {int(r["parent"]): k for k, r in enumerate(aux) if int(r["depth"]) > 0}
+    for k, r in enumerate(aux):
+        if int(r["status"]) != _abi.AUX_OK or int(r["first"]) != k:
+            continue
+        pdu = bytes(r["bytes"][: int(r["len"])])
+        d = dict(index=k, channel=int(r["channel"]), phy="2M" if int(r["phy"]) == _abi.AUX_PHY_2M else "1M", depth=int(r["depth"]),
+                 crc_ok=bool(r["crc_ok"]), tx_add=(pdu[0] >> 6) & 1, pload_len=pdu[1], sample_index=int(r["sample_index"]),
+                 capture_id=int(r["capture_id"]), **_ext_fields(pdu))
+        out.append(d)
+        by_index[k] = d
+    for d in out:
+        if d["depth"] != 0:
+            continue
+        chain, data, k, complete = [d["index"]], d["adv_data"], d["index"], d["crc_ok"]
+        while complete and by_index[k]["aux_ptr"] is not None:
+            c = children.get(k)
+            if c is None or c not in by_index or not by_index[c]["crc_ok"]:
+                complete = False
+                break
+            chain.append(c)
+            data += by_index[c]["adv_data"]
+            k = c
+        d["chain"], d["chain_data"], d["complete"] = chain, data, complete
+    return out

@@ -86,15 +86,17 @@ def gaussian_taps(sps: int = 4, bt: float = 0.5, span: int = 4) -> np.ndarray:
 
 
 _GAUSS4 = gaussian_taps()
+_GAUSS2 = gaussian_taps(sps=2)          # LE 2M at 4 Msps: 2 samples per symbol, same BT and span in symbols
 
 
 def gfsk_modulate(bits: np.ndarray, sps: int = 4, h: float = 0.5) -> np.ndarray:
-    """Unit-amplitude complex GFSK of a 0/1 bit array; returns len(bits)*sps + 16 samples."""
+    """Unit-amplitude complex GFSK of a 0/1 bit array; returns len(bits)*sps + 4*sps samples (sps = 4: LE 1M, 2: LE 2M)."""
+    g = _GAUSS4 if sps == 4 else gaussian_taps(sps=sps)
     nrz = np.zeros(len(bits) * sps)
     nrz[::sps] = 2.0 * bits - 1.0
-    freq = np.convolve(nrz, _GAUSS4)
+    freq = np.convolve(nrz, g)
     phase = np.concatenate(([0.0], np.cumsum(freq[:-1]))) * (math.pi * h / sps)
-    return np.exp(1j * phase)[: len(bits) * sps + len(_GAUSS4)]
+    return np.exp(1j * phase)[: len(bits) * sps + len(g)]
 
 
 def bytes_to_bits_lsb(data: bytes) -> np.ndarray:
@@ -109,6 +111,13 @@ def ble_phy_bits(pdu: bytes, channel: int, access_addr: int = chanplan.BLE_ADV_A
     body = bytes(np.frombuffer(body, dtype=np.uint8) ^ w)
     preamble = 0xAA if (access_addr & 1) == 0 else 0x55
     return bytes_to_bits_lsb(bytes([preamble]) + access_addr.to_bytes(4, "little") + body)
+
+
+def ble_phy_bits_2m(pdu: bytes, channel: int, access_addr: int = chanplan.BLE_ADV_AA,
+                    crc_init: int = chanplan.BLE_ADV_CRC_INIT) -> np.ndarray:
+    """LE 2M: a 2-byte preamble, then as ble_phy_bits (Core Vol 6 Part B 2.1.1)."""
+    bits = ble_phy_bits(pdu, channel, access_addr, crc_init)
+    return np.concatenate([bits[:8], bits])
 
 
 def ble_adv_pdu(rng: np.random.Generator, pdu_type: int = 0, data_len: int | None = None) -> bytes:
@@ -562,3 +571,150 @@ def wideband_capture_gpu(seconds: float = 0.02, kind: str = "ble", seed: int = 4
     _abi.check(lib.snrx_synth_wideband(device, P(bursts), len(bursts), P(data), len(blob), P(bins), len(bins), P(taps), P(gauss),
                                        n_ch, ctypes.c_float(sigma), seed & 0xFFFFFFFFFFFFFFFF, dst, on_dev))
     return ret, truth
+
+
+# ------------------------------------------------------------- BLE 5 extended advertising (test input)
+# ADV_EXT_IND on the primary channels, AUX_ADV_IND / AUX_CHAIN_IND on a data channel, on LE 1M or LE 2M (Core Vol 6 Part B
+# 2.3.1.4, 2.3.2.1, 2.3.4).  The extended header: byte 0 = length (bits 0..5) | AdvMode << 6, then the flags byte and the
+# flagged fields in the order AdvA, TargetA, CTEInfo, ADI, AuxPtr, SyncInfo, TxPower.
+
+def ext_header(adv_mode: int = 0, adv_a: bytes | None = None, tx_add: int = 0, adi: int | None = None, aux_ptr: bytes | None = None,
+               tx_power: int | None = None) -> bytes:
+    flags, body = 0, b""
+    if adv_a is not None:
+        flags |= 0x01
+        body += bytes(adv_a)
+    if adi is not None:
+        flags |= 0x08
+        body += (adi & 0xFFFF).to_bytes(2, "little")
+    if aux_ptr is not None:
+        flags |= 0x10
+        body += bytes(aux_ptr)
+    if tx_power is not None:
+        flags |= 0x40
+        body += bytes([tx_power & 0xFF])
+    hdr = bytes([flags]) + body
+    return bytes([len(hdr) | (adv_mode << 6)]) + hdr
+
+
+def aux_ptr_bytes(channel: int, ca: int, units_us: int, offset: int, phy: int) -> bytes:
+    """AuxPtr: channel | CA << 6 | OffsetUnits << 7, then Aux Offset (13 bits) | Aux PHY << 13, little endian."""
+    v = (offset & 0x1FFF) | ((phy & 7) << 13)
+    return bytes([(channel & 0x3F) | ((ca & 1) << 6) | ((1 if units_us == 300 else 0) << 7), v & 0xFF, v >> 8])
+
+
+def ext_pdu(ext_hdr: bytes, adv_data: bytes = b"", tx_add: int = 0) -> bytes:
+    """PDU of type 7 (ADV_EXT_IND, AUX_ADV_IND, AUX_CHAIN_IND): header with an 8-bit length, then payload."""
+    payload = bytes(ext_hdr) + bytes(adv_data)
+    assert len(payload) <= 255
+    return bytes([7 | (tx_add << 6), len(payload)]) + payload
+
+
+def aux_offset_for(gap_samples: float, ca: int, rng: np.random.Generator) -> tuple[int, int, float]:
+    """AuxPtr (units, offset) a transmitter whose clock runs fast by `drift` (within its CA accuracy) states for a true gap of
+    gap_samples (4 Msps) between the starts of two packets: (units_us, offset, drift)."""
+    ppm = 50 if ca else 500
+    drift = float(rng.uniform(-0.9, 0.9)) * ppm * 1e-6
+    t_us = gap_samples / 4.0 * (1.0 + drift)
+    units = 30 if t_us < 8191 * 30 else 300
+    off = int(t_us // units)
+    assert off <= 8191, "aux packet too far"
+    return units, off, drift
+
+
+@dataclass
+class AuxTruth:
+    """A BLE 5 auxiliary packet placed into a synthetic capture."""
+    channel: int
+    phy: int              # 0 = LE 1M, 1 = LE 2M
+    start: int            # channel-rate sample of the first preamble sample
+    anchor: int           # nominal sample of AA bit 0 (preamble + Gaussian filter delay)
+    data: bytes           # pdu | crc (un-whitened)
+    depth: int            # 0 = AUX_ADV_IND, d = d-th AUX_CHAIN_IND
+    parents: list = field(default_factory=list)   # [(parent channel, parent start, units_us, offset, ca, drift, gap in samples)]
+
+
+def _put(streams: dict, n_ch: int, channel: int, pos: int, wave: np.ndarray, rng: np.random.Generator, cfo_hz: float) -> None:
+    b = chanplan.ble_channel_bin(channel)
+    if b not in streams:
+        streams[b] = np.zeros(n_ch, dtype=np.complex128)
+    cfo, ph0 = float(rng.uniform(-cfo_hz, cfo_hz)), float(rng.uniform(0, 2 * math.pi))
+    k = np.arange(len(wave))
+    streams[b][pos:pos + len(wave)] += wave * np.exp(1j * (ph0 + 2 * math.pi * cfo * k / chanplan.NB_RATE))
+
+
+def ext_adv_schedule(n_ch: int, rng: np.random.Generator, n_events: int = 8, phys=(0, 1), max_chain: int = 3, cfo_hz: float = 50e3,
+                     data_len=(0, 240), event_gap: int = 30_000):
+    """Extended advertising events laid end to end on a 4 Msps time line: per event an ADV_EXT_IND on 37, 38 and 39, each
+    pointing at one AUX_ADV_IND on a random data channel and PHY, which points down a chain of 0..max_chain AUX_CHAIN_INDs.
+    Each AuxPtr states the gap to its packet as a transmitter with a clock error inside its CA accuracy would (aux_offset_for).
+    Returns ({bin: stream}, [Truth] of the primary packets, [AuxTruth])."""
+    streams: dict = {}
+    prim, aux = [], []
+    pos = 2000
+    for _ in range(n_events):
+        adv_a = bytes(rng.integers(0, 256, 6, dtype=np.uint8))
+        did, sid = int(rng.integers(0, 4096)), int(rng.integers(0, 16))
+        adi = did | (sid << 12)
+        n_links = 1 + int(rng.integers(0, max_chain + 1))
+        chans = [int(c) for c in rng.integers(0, 37, n_links)]
+        phys_l = [int(rng.choice(phys)) for _ in range(n_links)]
+        cas = [int(rng.integers(0, 2)) for _ in range(n_links + 1)]
+        datas = [bytes(rng.integers(0, 256, int(rng.integers(data_len[0], data_len[1] + 1)), dtype=np.uint8)) for _ in range(n_links)]
+        # primary ADV_EXT_INDs: 7 payload bytes each, 37 -> 38 -> 39 about 500 us apart
+        p_len = (1 + 4 + 2 + 9 + 3) * 8 * 4 + 16
+        p_starts = [pos, pos + p_len + 1400, pos + 2 * (p_len + 1400)]
+        a_start = p_starts[2] + p_len + int(rng.integers(1200, 6000))
+        # aux packets: each link starts T_MAFS (300 us) or more after the previous one ends
+        starts, pdus = [], []
+        t = a_start
+        for k in range(n_links):
+            payload_len = len(ext_header(0, adv_a if k == 0 else None, 0, adi, b"\0\0\0" if k + 1 < n_links else None,
+                                         0 if k == 0 else None)) + len(datas[k])
+            sps = 2 if phys_l[k] == 1 else 4
+            nbits = (16 if sps == 2 else 8) + 32 + 8 * (2 + payload_len + 3)
+            starts.append(t)
+            t += nbits * sps + 16 + 1200 + int(rng.integers(0, 4000))
+        for k in range(n_links):
+            ptr = None
+            info = None
+            if k + 1 < n_links:
+                units, off, drift = aux_offset_for(starts[k + 1] - starts[k], cas[k + 1], rng)
+                ptr = aux_ptr_bytes(chans[k + 1], cas[k + 1], units, off, phys_l[k + 1])
+                info = (units, off, cas[k + 1], drift)
+            hdr = ext_header(0, adv_a if k == 0 else None, 0, adi, ptr, 0 if k == 0 else None)
+            pdus.append((ext_pdu(hdr, datas[k]), info))
+        for k in range(n_links):
+            sps = 2 if phys_l[k] == 1 else 4
+            pdu = pdus[k][0]
+            bits = ble_phy_bits_2m(pdu, chans[k]) if sps == 2 else ble_phy_bits(pdu, chans[k])
+            _put(streams, n_ch, chans[k], starts[k], gfsk_modulate(bits, sps=sps), rng, cfo_hz)
+            par = []
+            if k == 0:
+                for j, ps in enumerate(p_starts):
+                    units, off, drift = aux_offset_for(starts[0] - ps, cas[0], rng)
+                    ptr = aux_ptr_bytes(chans[0], cas[0], units, off, phys_l[0])
+                    pp = ext_pdu(ext_header(0, None, 0, adi, ptr))
+                    _put(streams, n_ch, 37 + j, ps, gfsk_modulate(ble_phy_bits(pp, 37 + j)), rng, cfo_hz)
+                    prim.append(Truth(37 + j, ps, ps + 8 * 4 + 8, pp + ble_crc24(pp), 3))
+                    par.append((37 + j, ps, units, off, cas[0], drift, starts[0] - ps))
+            else:
+                units, off, ca, drift = pdus[k - 1][1]
+                par.append((chans[k - 1], starts[k - 1], units, off, ca, drift, starts[k] - starts[k - 1]))
+            aux.append(AuxTruth(chans[k], phys_l[k], starts[k], starts[k] + 32 + 2 * sps, pdu + ble_crc24(pdu), k, par))
+        pos = t + event_gap
+        assert pos < n_ch, "capture too short for the events"
+    return streams, prim, aux
+
+
+def ext_adv_capture(seconds: float = 0.05, seed: int = 9000, esn0_db: float | None = 25.0, **kw) -> Capture:
+    """96 Msps capture (centre 2440 MHz) carrying ext_adv_schedule(...) events and nothing else; meta["aux"] holds the
+    AuxTruth list.  esn0_db=None: no noise."""
+    rng = np.random.default_rng(seed)
+    n_ch = int(round(seconds * chanplan.NB_RATE))
+    n_ch -= n_ch % chanplan.BLE_WINDOW
+    streams, prim, aux = ext_adv_schedule(n_ch, rng, **kw)
+    x = wideband_mix(streams)
+    if esn0_db is not None:
+        x = x + _awgn(len(x), np.random.default_rng(seed + 999), 4.0 * chanplan.WB_DECIM / (10.0 ** (esn0_db / 10.0))).astype(np.complex64)
+    return Capture(x.astype(np.complex64), chanplan.WB_RATE, prim, dict(kind="wb_ble_ext", seed=seed, esn0_db=esn0_db, aux=aux))
