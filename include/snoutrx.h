@@ -423,6 +423,79 @@ typedef struct snrx_ble_aux {       /* one per pointer, 304 bytes */
  * SNRX_ERANGE if cap is smaller than the list; SNRX_EOVERFLOW if the list would hold more than max_frames entries. */
 int  snrx_ble_aux(snrx_t* h, snrx_ble_aux_t* out, uint32_t cap, uint32_t* n_out);
 
+/* ---- BLE Long Range: the ADV_EXT_INDs sent on the LE Coded PHY on channels 37..39, found and Viterbi-decoded from the
+ * batch's slicer bit streams, and the auxiliary packets they point at on every PHY (wideband BLE modes; nothing is
+ * channelized twice).  No reference receiver exists for this: the definition below is the contract, and the GPU equals it
+ * bit for bit on the engine's own bit streams (oracle/coded_oracle.py restates it).  Integer arithmetic only.
+ *
+ * Notation.  b[m] = the slicer decision of channel sample m (SNRX_STAGE_BLE_BITS); decision m is usable when m + 1 < the
+ *   buffer's channel samples.  One LE Coded symbol is 4 channel samples (1 Msym/s, as LE 1M).
+ * PHY (Core Vol 6 Part B 2.2, 3.3, as read here).  Encoder: rate 1/2, K = 4, state D1 | D2 << 1 | D3 << 2 with D1 the most
+ *   recent input bit; a0 = u ^ D1 ^ D2 ^ D3 and a1 = u ^ D2 ^ D3 (G0 = 1+x+x^2+x^3, G1 = 1+x^2+x^3), a0 sent first.  Pattern
+ *   mapper: S=8 maps 0 -> 0011 and 1 -> 1100, S=2 is the identity.  Packet: 80 preamble symbols (00111100 repeated); FEC
+ *   block 1, always S=8, encoder from state 0: AA (32 bits) | CI (2 bits, LSB first) | TERM1 (3 zero bits); FEC block 2,
+ *   encoder from state 0 again: whitened PDU | CRC-24 | TERM2 (3 zero bits), at S=8 if CI = 0 and at S=2 if CI = 1.
+ *   Whitening and CRC (the channel's LFSR, init 0x555555) are applied before FEC.
+ * Coded access address.  c[0..255] = 0x8E89BED6 encoded and mapped at S=8; P[j] = c[j >> 2], j = 0..1023.
+ *   d(n) = the number of j in 0..1023 with b[n + j] != P[j], defined when n + 1023 is usable (otherwise infinite).
+ * Primary packets.  On channels 37, 38 and 39 of every capture of the batch, n is a packet when d(n) <= T = 400 (noise: mean
+ *   512, deviation 16), d(n) < d(m) for every m in [n - 16, n) and d(n) <= d(m) for every m in (n, n + 16] (a strict local
+ *   minimum; the earliest wins ties).  sample_index = n (whole-capture index, as the records); a time shard reports the n
+ *   inside its body only.  win_lo = win_hi = sample_index, parent = 0xFFFFFFFF, depth 0, phy SNRX_AUX_PHY_CODED.
+ * Coding indicator.  Samples [n + 1024, n + 1184) carry CI and TERM1 (10 coded bits at 16 decisions).  ci = the v in 0..3
+ *   whose coded (from the encoder state after the AA), mapped, sample-level pattern differs from b in the fewest places,
+ *   the lower v on ties.  v = 2 or 3 is SNRX_AUX_RESERVED_CI: not decoded.
+ * Viterbi.  Block 2 starts at n + 1184; coded bit k occupies the L = 16 (S=8) or L = 4 (S=2) decisions from n + 1184 + k L,
+ *   and its branch metric is the number of them that differ from its sample-level pattern.  Add-compare-select keeps the
+ *   predecessor with the smaller path metric, the one with D3 = 0 on ties; the start state has metric 0, the others 2^20.
+ *   Header run: 40 info bits, traced back from the lowest-metric state at step 40 (lowest index on ties); its bits 0..15 are
+ *   the whitened header and give len.  Full run: N = 8 len + 43 info bits, traced back from state 0 after TERM2.  The entry
+ *   holds the full run's 2 + len + 3 de-whitened bytes, the CRC check, its final metric and d(n) (aa_errors).  If CI's, the
+ *   header run's or the full run's last decision is not usable, the status is TRUNCATED.  The longest packet reaches
+ *   n + 67 840.
+ * Pointers.  Sources are the primary entries with status OK, crc_ok, first == own index and a PDU of type 7 with an AuxPtr
+ *   (as for snrx_ble_aux), then, one depth down per round, the pointed entries meeting the same conditions.  The window is
+ *   snrx_ble_aux's window shifted by the preamble lengths: s - P(source PHY) + P(target PHY) + [lo, hi], P = 32 for 1M and
+ *   2M and 320 for Coded.  A 1M or 2M target is searched and decoded exactly as snrx_ble_aux does it.  A Coded target is
+ *   OUTSIDE when win_lo or win_hi + 1023 is not a usable decision; else it takes the n of the window with the smallest
+ *   d(n) <= T (earliest on ties; NOT_FOUND if none), decoded as above.  first, OUTSIDE, NOT_FOUND, BAD_CHANNEL and the
+ *   depth limit follow snrx_ble_aux, with UNSUPPORTED_PHY for the reserved PHYs only and DEPTH_LIMIT beyond depth 16 (the
+ *   same 15 chain links).
+ * Order.  Primaries in (capture, channel, sample_index) order, then the pointer rounds by depth, then by parent.
+ * Shards.  A packet whose decisions lie inside both buffers gives the same entry in a time shard as in the whole capture;
+ *   one that reaches past a shard's buffer is TRUNCATED or OUTSIDE there (the default 2048-sample post-halo is shorter than
+ *   most Coded packets: a shard needs a post-halo of 67 840 samples to decode every packet of its body). */
+#define SNRX_AUX_RESERVED_CI     7
+#define SNRX_CODED_T             400
+#define SNRX_CODED_MAX_DEPTH     16
+
+typedef struct snrx_ble_coded {     /* one per primary packet or pointer, 320 bytes */
+    int64_t  sample_index;  /* start of the coded AA (Coded) or AA bit 0 (1M / 2M); -1 unless found                      */
+    int64_t  win_lo, win_hi;/* the searched window, inclusive, capture relative (primaries: sample_index)                 */
+    uint32_t capture_id;
+    uint32_t parent;        /* list index of the pointing entry; 0xFFFFFFFF for primaries                                */
+    uint32_t first;         /* list index of the earliest entry that found the same packet (own index if none)           */
+    uint8_t  depth;         /* 0 = primary ADV_EXT_IND, d = d links from it                                              */
+    uint8_t  channel;
+    uint8_t  phy;           /* SNRX_AUX_PHY_*                                                                            */
+    uint8_t  phase;         /* sample_index mod sps (4 for Coded)                                                        */
+    uint8_t  status;        /* SNRX_AUX_*                                                                                */
+    uint8_t  crc_ok;
+    uint16_t len;           /* valid bytes in bytes[]: 2 + header length + 3 (0 unless OK)                               */
+    uint8_t  ci;            /* coding indicator 0..3 of a Coded packet; 0xFF when not Coded or not reached               */
+    uint8_t  reserved0;
+    uint16_t aa_errors;     /* d(n) of a Coded packet                                                                    */
+    uint32_t metric;        /* final path metric of the full Viterbi run (0 unless a Coded packet is OK)                 */
+    uint8_t  bytes[SNRX_AUX_MAX_BYTES];   /* de-whitened header | payload | CRC, zero past len                           */
+    uint8_t  reserved[8];
+} snrx_ble_coded_t;
+
+/* The Long Range packets of the batch most recently retired by snrx_poll / snrx_poll_view (definition above): *n_out
+ * entries, copied to out (up to cap; out may be NULL to count).  State and capacity rules as snrx_ble_aux: SNRX_ESTATE
+ * without a polled wideband BLE batch or once its bit streams have been overwritten; SNRX_ERANGE if cap is smaller than the
+ * list; SNRX_EOVERFLOW if the list would hold more than max_frames entries. */
+int  snrx_ble_coded(snrx_t* h, snrx_ble_coded_t* out, uint32_t cap, uint32_t* n_out);
+
 /* ---- SURVEY 8(f) N2: the Zigbee consumer path on the decoded 802.15.4 records (what Snout does per datagram:
  * RFtap(pkt) -> Dot15d4FCS dissection, snout/util/zigbee.py:194-202; ZigbeeMessage.fromraw, snout/core/message.py:258-304;
  * the touchlink scan's haslayer(ZLLScanResponse), zigbee.py:176-192) ---- */

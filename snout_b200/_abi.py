@@ -64,6 +64,15 @@ AUX_DTYPE = np.dtype([("sample_index", "<i8"), ("win_lo", "<i8"), ("win_hi", "<i
                       ("crc_ok", "u1"), ("len", "<u2"), ("bytes", "u1", (AUX_MAX_BYTES,))], align=True)
 assert AUX_DTYPE.itemsize == 304
 
+# BLE Long Range: one entry per primary LE Coded packet or pointer (include/snoutrx.h snrx_ble_coded_t)
+AUX_RESERVED_CI = 7
+CODED_T, CODED_MAX_DEPTH = 400, 16
+CODED_DTYPE = np.dtype([("sample_index", "<i8"), ("win_lo", "<i8"), ("win_hi", "<i8"), ("capture_id", "<u4"), ("parent", "<u4"),
+                        ("first", "<u4"), ("depth", "u1"), ("channel", "u1"), ("phy", "u1"), ("phase", "u1"), ("status", "u1"),
+                        ("crc_ok", "u1"), ("len", "<u2"), ("ci", "u1"), ("reserved0", "u1"), ("aa_errors", "<u2"),
+                        ("metric", "<u4"), ("bytes", "u1", (AUX_MAX_BYTES,)), ("reserved", "u1", (8,))], align=True)
+assert CODED_DTYPE.itemsize == 320
+
 FRAME_DTYPE = np.dtype([
     ("sample_index", "<i8"), ("capture_id", "<u4"), ("window", "<u4"), ("channel", "<u2"),
     ("proto", "u1"), ("crc_ok", "u1"), ("lqi", "u1"), ("phase", "u1"), ("len", "<u2"),
@@ -138,6 +147,7 @@ SYMBOLS = [
     ("snrx_ble_connections", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_ble_follow", c_int, [c_void_p, c_uint32, c_uint32, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_ble_aux", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
+    ("snrx_ble_coded", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_zb_mac_summary", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_frame_rf", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_exchange_create", c_int, [c_void_p, c_uint32, c_uint32, c_uint32, c_void_p]),

@@ -36,6 +36,17 @@ printed, whatever `-c` selects, as one line of 8 tokens (formats.aux_line):
 It starts with AUX instead of a timestamp and a Pkt token, so a parser of the reference's lines does not take it for one.
 With `-s` the packets also go to the pcap (formats.ble_pcap_aux_block).
 
+`--coded` (with `--wideband`) also receives BLE Long Range advertising: the ADV_EXT_INDs sent on the LE Coded PHY on
+channels 37..39 are found by their coded access address, Viterbi-decoded, and followed down their AuxPtrs on every PHY
+(RxEngine.ble_coded).  Each primary with a good CRC is printed as one line of 8 tokens (formats.coded_line), each packet of
+its chains as an AUX line (PHYCoded for LE Coded; its Depth counts from the primary, so the AUX_ADV_IND is Depth1).
+Primaries whose CRC fails are left out of the lines and the pcap: most are positions inside an S=8 packet's own coded body
+that come under the detection threshold (DESIGN.md 4).
+
+    CODED Ch<37..39> S<8|2> AdvA:<address or -> ADI:<DID hex>/<SID hex or -> PloadL<len> CRC<0|1> AAerr<d>
+
+With `-s` they also go to the pcap (formats.ble_pcap_coded_block).
+
 There is no CPU path: without a usable GPU / libsnoutrx.so the program exits with an error.
 """
 from __future__ import annotations
@@ -85,6 +96,8 @@ USAGE = """Usage:
       With --wideband: print frames of every channel, not just -c
     --device N
       CUDA device ordinal (default 0)
+    --coded
+      With --wideband: also receive BLE Long Range (LE Coded) ADV_EXT_INDs on 37..39 and their auxiliary packets
     --aux
       With --wideband: also follow BLE 5 extended advertising to its auxiliary packets (1M and 2M PHYs) and print them
     --rf
@@ -115,6 +128,7 @@ class Options:
     shard_windows = 0
     rf = False
     aux = False
+    coded = False
 
 
 def _strtol(text: str, base: int) -> int:
@@ -146,7 +160,7 @@ def parse_commandline(argv: list[str], out=sys.stdout) -> Options | None:
         opts, rest = getopt.getopt(argv, "hc:g:a:k:vrf:m:os:",
                                    ["help", "chan=", "gain=", "access=", "crcinit=", "verbose", "raw", "freq_hz=",
                                     "access_mask=", "hop", "filename=", "iq=", "format=", "scale=", "wideband",
-                                    "all-channels", "device=", "shard-windows=", "rf", "aux"])
+                                    "all-channels", "device=", "shard-windows=", "rf", "aux", "coded"])
     except getopt.GetoptError as e:
         out.write(f"btle_rx: {e}\n")
         out.write(USAGE)
@@ -193,6 +207,8 @@ def parse_commandline(argv: list[str], out=sys.stdout) -> Options | None:
             o.rf = True
         elif k == "--aux":
             o.aux = True
+        elif k == "--coded":
+            o.coded = True
     if o.chan < 0 or o.chan > MAX_CHANNEL:
         out.write(f"channel number must be within 0~{MAX_CHANNEL}!\n")
         out.write(USAGE)
@@ -222,6 +238,9 @@ def run(o: Options, out=sys.stdout, engine_factory=None, blocks=None) -> int:
         return 1
     if o.hop and not o.wideband:
         out.write("btle_rx (snout_b200): -o/--hop needs --wideband (a 4 Msps single-channel capture holds no data channel to hop to)\n")
+        return 1
+    if o.coded and not o.wideband:
+        out.write("btle_rx (snout_b200): --coded needs --wideband (the Coded packets are found in the wideband bit streams)\n")
         return 1
     if o.aux and not o.wideband:
         out.write("btle_rx (snout_b200): --aux needs --wideband (auxiliary packets are sent on the data channels)\n")
@@ -286,6 +305,14 @@ def run(o: Options, out=sys.stdout, engine_factory=None, blocks=None) -> int:
                     fh_pcap.write(formats.ble_pcap_aux_block(aux))
                 for d in messages.ble_ext_adv(aux):
                     out.write(formats.aux_line(d))
+            if o.coded:
+                lst = eng.ble_coded()
+                if fh_pcap:
+                    fh_pcap.write(formats.ble_pcap_coded_block(lst, crc_failed_primaries=False))
+                for d in messages.ble_coded_adv(lst):
+                    if d["depth"] == 0 and not d["crc_ok"]:
+                        continue                      # mostly positions inside an S=8 packet's own body (DESIGN 4)
+                    out.write(formats.coded_line(d) if d["depth"] == 0 else formats.aux_line(d))
             out.flush()                                                # fflush(stdout), btle_rx.c:2383
 
         def follow(frames: np.ndarray):

@@ -3,7 +3,7 @@
 // batch left in HBM.  The contract (pointer sources, window, search, decode, statuses, order) is stated in include/snoutrx.h
 // above snrx_ble_aux_t; oracle/aux_oracle.py restates it.
 //
-// One round per chain depth, launched by snrx_ble_aux:
+// One round per chain depth, launched by snrx_ble_aux (and, templated on the entry type, by snrx_ble_coded: ble_coded.cuh):
 //   k_ble_aux_flag / exclusive_scan / k_ble_aux_fill   the pointers of the round, in source order, with their windows and the
 //                                                       statuses that need no search
 //   k_ble_aux_search                                    one warp per pointer: windowed access-address search, then the decode
@@ -90,15 +90,41 @@ struct AuxGeom {                  // the polled batch
     uint32_t first_capture, n_captures;
 };
 
-struct AuxSrc {                   // where the pointers of one round come from
-    const snrx_frame_t* frames;   // depth 0: the polled records [0, n)
-    const snrx_ble_aux_t* list;   // deeper: the entries [first, first + n) of the previous round
+// What the two lists that share the pointer rounds differ in.  snrx_ble_aux: AUX_ADV_IND = depth 0, 1M / 2M only, AA bit 0
+// 32 samples after the preamble on both PHYs.  snrx_ble_coded: primaries = depth 0, Coded targets too, preamble 320 samples
+// on Coded (the window is shifted by P(target) - P(source)).
+constexpr int kAuxList = 0, kCodedList = 1;
+template <int L> struct AuxKind;
+template <> struct AuxKind<kAuxList> {
+    using Entry = snrx_ble_aux_t;
+    static constexpr bool kCoded = false;
+    static constexpr uint32_t kMaxDepth = SNRX_AUX_MAX_DEPTH;
+    static constexpr int kMaxPhy = SNRX_AUX_PHY_2M;
+};
+template <> struct AuxKind<kCodedList> {
+    using Entry = snrx_ble_coded_t;
+    static constexpr bool kCoded = true;
+    static constexpr uint32_t kMaxDepth = SNRX_CODED_MAX_DEPTH;
+    static constexpr int kMaxPhy = SNRX_AUX_PHY_CODED;
+};
+template <int L> using AuxEntry = typename AuxKind<L>::Entry;
+template <int L>
+struct AuxSrcT {                  // where the pointers of one round come from
+    const snrx_frame_t* frames;   // snrx_ble_aux at depth 0: the polled records [0, n); else nullptr
+    const AuxEntry<L>* list;      // otherwise: the entries [first, first + n) of the previous round
     uint32_t first, n, depth;     // depth of the pointers the round creates
 };
+using AuxSrc = AuxSrcT<kAuxList>;
+
+SNRX_HD constexpr int aux_preamble(int phy) { return phy == SNRX_AUX_PHY_CODED ? 320 : 32; }
+constexpr uint8_t kCodedPending = 0xFE;        // internal: a Coded target, to be searched by k_ble_coded_window
+constexpr int kCodedAaSamples = 1024;          // the coded access address: 256 symbols of 4 samples
 
 #if defined(__CUDACC__)
-__device__ __forceinline__ bool aux_source(const AuxSrc& s, uint32_t i, AuxPtr& a, int64_t& at, uint32_t& cap_id) {
-    if (s.depth == 0) {
+template <int L>
+__device__ __forceinline__ bool aux_source(const AuxSrcT<L>& s, uint32_t i, AuxPtr& a, int64_t& at, uint32_t& cap_id, int& phy) {
+    phy = SNRX_AUX_PHY_1M;
+    if (s.frames) {
         const snrx_frame_t& f = s.frames[i];
         if (f.proto != SNRX_PROTO_BLE || !f.crc_ok || f.channel < 37 || f.channel > 39 || f.access_addr != kAuxAdvAa || f.len < 5)
             return false;
@@ -106,55 +132,66 @@ __device__ __forceinline__ bool aux_source(const AuxSrc& s, uint32_t i, AuxPtr& 
         return aux_ptr_parse(f.bytes, (int)f.len - 5, a);
     }
     const uint32_t k = s.first + i;
-    const snrx_ble_aux_t& r = s.list[k];
+    const AuxEntry<L>& r = s.list[k];
     if (r.status != SNRX_AUX_OK || !r.crc_ok || r.first != k || r.len < 5) return false;
-    at = r.sample_index; cap_id = r.capture_id;
+    at = r.sample_index; cap_id = r.capture_id; phy = r.phy;
     return aux_ptr_parse(r.bytes, (int)r.len - 5, a);
 }
 
-__global__ void __launch_bounds__(256) k_ble_aux_flag(AuxSrc s, uint32_t* __restrict__ flags) {
+template <int L>
+__global__ void __launch_bounds__(256) k_ble_aux_flag(AuxSrcT<L> s, uint32_t* __restrict__ flags) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= s.n) return;
-    AuxPtr a; int64_t at; uint32_t cap_id;
-    flags[i] = aux_source(s, i, a, at, cap_id) ? 1u : 0u;
+    AuxPtr a; int64_t at; uint32_t cap_id; int phy;
+    flags[i] = aux_source(s, i, a, at, cap_id, phy) ? 1u : 0u;
 }
 
 // the round's entries at list[k0 + offsets[i]]: windows, pre-search statuses, zero bytes
-__global__ void __launch_bounds__(256) k_ble_aux_fill(AuxSrc s, const uint32_t* __restrict__ flags, const uint32_t* __restrict__ offsets,
-                                                      snrx_ble_aux_t* __restrict__ list, uint32_t k0, AuxGeom g) {
+template <int L>
+__global__ void __launch_bounds__(256) k_ble_aux_fill(AuxSrcT<L> s, const uint32_t* __restrict__ flags, const uint32_t* __restrict__ offsets,
+                                                      AuxEntry<L>* __restrict__ list, uint32_t k0, AuxGeom g) {
+    using K = AuxKind<L>;
+    using E = AuxEntry<L>;
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= s.n || !flags[i]) return;
-    AuxPtr a; int64_t at; uint32_t cap_id;
-    aux_source(s, i, a, at, cap_id);
+    AuxPtr a; int64_t at; uint32_t cap_id; int src_phy;
+    aux_source(s, i, a, at, cap_id, src_phy);
     const uint32_t k = k0 + offsets[i];
-    snrx_ble_aux_t& r = list[k];
+    E& r = list[k];
     uint4* d = reinterpret_cast<uint4*>(&r);
 #pragma unroll
-    for (int q = 0; q < (int)(sizeof(snrx_ble_aux_t) / 16); q++) d[q] = make_uint4(0u, 0u, 0u, 0u);
+    for (int q = 0; q < (int)(sizeof(E) / 16); q++) d[q] = make_uint4(0u, 0u, 0u, 0u);
     int64_t lo, hi;
     aux_window(a, lo, hi);
+    if constexpr (K::kCoded) {
+        at += aux_preamble(a.phy) - aux_preamble(src_phy);
+        r.ci = 0xFF;
+    }
     r.sample_index = -1;
     r.win_lo = at + lo; r.win_hi = at + hi;
     r.capture_id = cap_id;
-    r.parent = s.depth == 0 ? i : s.first + i;
+    r.parent = s.frames ? i : s.first + i;
     r.first = k;
     r.depth = (uint8_t)s.depth;
     r.channel = (uint8_t)a.channel;
     r.phy = (uint8_t)a.phy;
     uint8_t st = kAuxPending;
-    if (s.depth > SNRX_AUX_MAX_DEPTH) st = SNRX_AUX_DEPTH_LIMIT;
+    if (s.depth > K::kMaxDepth) st = SNRX_AUX_DEPTH_LIMIT;
     else if (a.channel > 36) st = SNRX_AUX_BAD_CHANNEL;
-    else if (a.phy > SNRX_AUX_PHY_2M) st = SNRX_AUX_UNSUPPORTED_PHY;
+    else if (a.phy > K::kMaxPhy) st = SNRX_AUX_UNSUPPORTED_PHY;
     else {
         const int sps = a.phy == SNRX_AUX_PHY_2M ? 2 : 4;
-        const int64_t l = r.win_lo - g.base, e = r.win_hi - g.base + 31 * sps;    // local first / last decision of the search
+        const int span = (K::kCoded && a.phy == SNRX_AUX_PHY_CODED) ? kCodedAaSamples - 1 : 31 * sps;
+        const int64_t l = r.win_lo - g.base, e = r.win_hi - g.base + span;        // local first / last decision of the search
         if (l < 0 || e + 1 >= g.n_out) st = SNRX_AUX_OUTSIDE;
+        else if (K::kCoded && a.phy == SNRX_AUX_PHY_CODED) st = kCodedPending;
     }
     r.status = st;
 }
 
 // One warp per entry of [i0, i1) still pending: the earliest full access-address match in the window, then the decode.
-__global__ void __launch_bounds__(128) k_ble_aux_search(snrx_ble_aux_t* __restrict__ list, uint32_t i0, uint32_t i1, AuxGeom g,
+template <int L>
+__global__ void __launch_bounds__(128) k_ble_aux_search(AuxEntry<L>* __restrict__ list, uint32_t i0, uint32_t i1, AuxGeom g,
                                                         const uint32_t* __restrict__ crc_tab, const uint8_t* __restrict__ whiten /*[40][260]*/,
                                                         uint32_t crc_init_internal, const __grid_constant__ AaTables tabs) {
     __shared__ uint32_t crc_s[256];
@@ -165,7 +202,7 @@ __global__ void __launch_bounds__(128) k_ble_aux_search(snrx_ble_aux_t* __restri
     uint8_t* buf = buf_s[wib];
     const uint32_t warps = gridDim.x * (blockDim.x >> 5);
     for (uint32_t k = i0 + blockIdx.x * (blockDim.x >> 5) + wib; k < i1; k += warps) {
-        snrx_ble_aux_t& r = list[k];
+        AuxEntry<L>& r = list[k];
         if (r.status != kAuxPending) continue;                    // warp-uniform
         const int sps = r.phy == SNRX_AUX_PHY_2M ? 2 : 4;
         const int lo = (int)(r.win_lo - g.base), hi = (int)(r.win_hi - g.base);   // inside the buffer (k_ble_aux_fill)
@@ -231,21 +268,24 @@ __global__ void __launch_bounds__(128) k_ble_aux_search(snrx_ble_aux_t* __restri
     }
 }
 
-__device__ __forceinline__ bool aux_found(const snrx_ble_aux_t& r) { return r.status == SNRX_AUX_OK || r.status == SNRX_AUX_TRUNCATED; }
+template <class E>
+__device__ __forceinline__ bool aux_found(const E& r) { return r.status == SNRX_AUX_OK || r.status == SNRX_AUX_TRUNCATED; }
 
 // One warp per entry of [i0, i1): first = the smallest list index that found the same (capture, channel, AA bit 0, PHY).
-__global__ void __launch_bounds__(256) k_ble_aux_first(snrx_ble_aux_t* __restrict__ list, uint32_t i0, uint32_t i1) {
+template <int L>
+__global__ void __launch_bounds__(256) k_ble_aux_first(AuxEntry<L>* __restrict__ list, uint32_t i0, uint32_t i1) {
+    using E = AuxEntry<L>;
     const int lane = threadIdx.x & 31;
     const uint32_t warps = gridDim.x * (blockDim.x >> 5);
     for (uint32_t k = i0 + blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); k < i1; k += warps) {
-        const snrx_ble_aux_t& r = list[k];
+        const E& r = list[k];
         if (!aux_found(r)) continue;
         uint32_t first = k;
         for (uint32_t b = 0; b < k; b += 32) {
             const uint32_t j = b + lane;
             bool same = false;
             if (j < k) {
-                const snrx_ble_aux_t& o = list[j];
+                const E& o = list[j];
                 same = aux_found(o) && o.sample_index == r.sample_index && o.channel == r.channel && o.capture_id == r.capture_id && o.phy == r.phy;
             }
             const uint32_t m = __ballot_sync(0xffffffffu, same);

@@ -24,6 +24,7 @@
 #endif
 #include "ble_adv.cuh"
 #include "ble_aux.cuh"
+#include "ble_coded.cuh"
 #include "ble_back.cuh"
 #include "ble_conn.cuh"
 #include "ble_front.cuh"
@@ -105,6 +106,11 @@ struct snrx_handle {
     // the whitening sequences continued to 260 bytes
     snrx_ble_aux_t* d_aux = nullptr; uint32_t *d_aux_flags = nullptr, *d_aux_offsets = nullptr, *d_aux_scratch = nullptr;
     uint8_t* d_aux_whiten = nullptr;
+    // snrx_ble_coded, allocated by its first call: the list (max_frames entries) with its round buffers, the scan's per-tile
+    // counts / offsets / scan scratch (grown to the batch's tile count), and its own whitening sequences
+    snrx_ble_coded_t* d_coded = nullptr; uint32_t *d_coded_flags = nullptr, *d_coded_offsets = nullptr, *d_coded_scratch = nullptr;
+    uint32_t *d_coded_tcounts = nullptr, *d_coded_toffsets = nullptr, *d_coded_tscratch = nullptr; uint32_t coded_tiles_cap = 0;
+    uint8_t* d_coded_whiten = nullptr;
     snrx::DevSlot* d_devtab = nullptr;
     snrx_device_t* d_devout = nullptr;
     uint32_t* d_adv_counters = nullptr;   // [0] records summarised (BLE), [1] new devices, [2] dropped (table full), [3] export count
@@ -458,7 +464,9 @@ void snrx_destroy(snrx_t* h) {
     if (h->xchg.h_hdr) cudaFreeHost(h->xchg.h_hdr);
     if (h->adv_stream) { cudaStreamSynchronize(h->adv_stream); cudaStreamDestroy(h->adv_stream); }
     { void* ab[] = {h->d_adv, h->d_zbmac, h->d_conn, h->d_conn_flags, h->d_conn_offsets, h->d_conn_scratch, h->d_follow, h->d_devtab, h->d_devout, h->d_adv_counters,
-                    h->d_aux, h->d_aux_flags, h->d_aux_offsets, h->d_aux_scratch, h->d_aux_whiten}; for (void* b : ab) if (b) cudaFree(b); }
+                    h->d_aux, h->d_aux_flags, h->d_aux_offsets, h->d_aux_scratch, h->d_aux_whiten,
+                    h->d_coded, h->d_coded_flags, h->d_coded_offsets, h->d_coded_scratch, h->d_coded_tcounts, h->d_coded_toffsets,
+                    h->d_coded_tscratch, h->d_coded_whiten}; for (void* b : ab) if (b) cudaFree(b); }
     delete h;
 }
 
@@ -1184,8 +1192,8 @@ int snrx_ble_aux(snrx_t* h, snrx_ble_aux_t* out, uint32_t cap, uint32_t* n_out) 
         if ((uint64_t)total + m > h->frame_cap) return fail(h, SNRX_EOVERFLOW, "snrx_ble_aux: more auxiliary pointers than max_frames");
         k_ble_aux_fill<<<div_up(src.n, 256), 256, 0, st>>>(src, h->d_aux_flags, h->d_aux_offsets, h->d_aux, total, g);
         const int gs = grid_for(h, m, 4, 8);
-        k_ble_aux_search<<<gs, 128, 0, st>>>(h->d_aux, total, total + m, g, h->d_crc_tab, h->d_aux_whiten, crc_init, tabs);
-        k_ble_aux_first<<<grid_for(h, m, 8, 8), 256, 0, st>>>(h->d_aux, total, total + m);
+        k_ble_aux_search<kAuxList><<<gs, 128, 0, st>>>(h->d_aux, total, total + m, g, h->d_crc_tab, h->d_aux_whiten, crc_init, tabs);
+        k_ble_aux_first<kAuxList><<<grid_for(h, m, 8, 8), 256, 0, st>>>(h->d_aux, total, total + m);
         CK(cudaGetLastError());
         src.frames = nullptr; src.first = total; src.n = m; src.depth++;
         total += m;
@@ -1194,6 +1202,90 @@ int snrx_ble_aux(snrx_t* h, snrx_ble_aux_t* out, uint32_t cap, uint32_t* n_out) 
     if (out && total) {
         if (cap < total) return fail(h, SNRX_ERANGE, "snrx_ble_aux: buffer smaller than the list");
         CK(cudaMemcpyAsync(out, h->d_aux, sizeof(snrx_ble_aux_t) * (size_t)total, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+    }
+    return SNRX_OK;
+}
+
+int snrx_ble_coded(snrx_t* h, snrx_ble_coded_t* out, uint32_t cap, uint32_t* n_out) {
+    if (!h) return SNRX_EINVAL;
+    if (n_out) *n_out = 0;
+    if (h->polled_lane < 0) return fail(h, SNRX_ESTATE, "snrx_ble_coded needs a polled batch");
+    Lane& ln = h->lane[h->polled_lane];
+    if (!h->has_ble || !h->wideband || !ln.last_ble) return fail(h, SNRX_ESTATE, "snrx_ble_coded: the polled batch has no wideband BLE bit streams");
+    if (ln.pending) return fail(h, SNRX_ESTATE, "snrx_ble_coded: the batch's bit streams have been overwritten (call before the second-next snrx_process)");
+    CK(cudaSetDevice(h->device));
+    if (!h->d_coded) {
+        CK(cudaMalloc((void**)&h->d_coded, sizeof(snrx_ble_coded_t) * (size_t)h->frame_cap));
+        CK(cudaMalloc((void**)&h->d_coded_flags, sizeof(uint32_t) * ((size_t)h->frame_cap + 1)));
+        CK(cudaMalloc((void**)&h->d_coded_offsets, sizeof(uint32_t) * ((size_t)h->frame_cap + 1)));
+        CK(cudaMalloc((void**)&h->d_coded_scratch, sizeof(uint32_t) * scan_scratch_items(h->frame_cap)));
+        std::vector<uint8_t> wh(40 * SNRX_AUX_MAX_BYTES);
+        for (int ch = 0; ch < 40; ch++) make_whiten_bytes(ch, wh.data() + ch * SNRX_AUX_MAX_BYTES, SNRX_AUX_MAX_BYTES);
+        CK(cudaMalloc((void**)&h->d_coded_whiten, wh.size()));
+        CK(cudaMemcpy(h->d_coded_whiten, wh.data(), wh.size(), cudaMemcpyHostToDevice));
+    }
+    const BleParams& p = ln.last_p;
+    CodedGeom cg{};
+    AuxGeom& g = cg.g;
+    g.bits = ln.d_bits; g.lay = ln.last_lay; g.n_out = p.n_out;
+    g.base = (int64_t)kWindow * p.first_window - p.m_origin;
+    g.first_capture = p.first_capture; g.n_captures = p.n_captures;
+    cg.body_lo = p.m_origin; cg.body_hi = p.m_origin + p.n_windows * kWindow;
+    cg.tiles_per_stream = (uint32_t)div_up(p.n_out, kCodedTile);
+    const uint32_t n_tiles = cg.tiles_per_stream * 3u * p.n_captures;
+    if (n_tiles + 1 > h->coded_tiles_cap) {
+        for (void* b : {(void*)h->d_coded_tcounts, (void*)h->d_coded_toffsets, (void*)h->d_coded_tscratch}) if (b) cudaFree(b);
+        h->coded_tiles_cap = n_tiles + 1;
+        CK(cudaMalloc((void**)&h->d_coded_tcounts, sizeof(uint32_t) * (size_t)h->coded_tiles_cap));
+        CK(cudaMalloc((void**)&h->d_coded_toffsets, sizeof(uint32_t) * (size_t)h->coded_tiles_cap));
+        CK(cudaMalloc((void**)&h->d_coded_tscratch, sizeof(uint32_t) * scan_scratch_items(h->coded_tiles_cap)));
+    }
+    cudaStream_t st = ln.tail;                                   // the lane is idle: its bit streams stay as the batch left them
+    const CodedTables ct = make_coded_tables();
+    const AaTables tabs = make_aa_tables(kAuxAdvAa, 0xFFFFFFFFu);
+    const uint32_t crc_init = crc_init_internal(0x555555u);
+    // the primaries: count per tile, offsets, then the entries in (capture, channel, sample) order, decoded
+    uint32_t total = 0;
+    if (n_tiles) {
+        k_ble_coded_scan<false><<<n_tiles, kCodedScanThreads, 0, st>>>(cg, ct, h->d_coded_tcounts, nullptr, nullptr);
+        exclusive_scan(h->d_coded_tcounts, n_tiles, h->d_coded_toffsets, h->d_coded_tscratch, st);
+        CK(cudaMemcpyAsync(&total, h->d_coded_toffsets + n_tiles, sizeof total, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        if (total > h->frame_cap) return fail(h, SNRX_EOVERFLOW, "snrx_ble_coded: more entries than max_frames");
+        if (total) {
+            k_ble_coded_scan<true><<<n_tiles, kCodedScanThreads, 0, st>>>(cg, ct, h->d_coded_tcounts, h->d_coded_toffsets, h->d_coded);
+            k_ble_coded_decode<<<grid_for(h, total, kCodedGroups, 8), 8 * kCodedGroups, 0, st>>>(h->d_coded, 0, total, g, ct, h->d_crc_tab,
+                                                                                                h->d_coded_whiten, crc_init);
+            CK(cudaGetLastError());
+        }
+    }
+    AuxSrcT<kCodedList> src{};
+    src.frames = nullptr; src.list = h->d_coded; src.first = 0; src.n = total; src.depth = 1;
+    // one round per depth: the pointers of depth d come from the entries of depth d - 1 (the primaries at d = 1)
+    while (src.n > 0 && src.depth <= SNRX_CODED_MAX_DEPTH + 1) {
+        k_ble_aux_flag<<<div_up(src.n, 256), 256, 0, st>>>(src, h->d_coded_flags);
+        exclusive_scan(h->d_coded_flags, src.n, h->d_coded_offsets, h->d_coded_scratch, st);
+        uint32_t m = 0;
+        CK(cudaMemcpyAsync(&m, h->d_coded_offsets + src.n, sizeof m, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        if (m == 0) break;
+        if ((uint64_t)total + m > h->frame_cap) return fail(h, SNRX_EOVERFLOW, "snrx_ble_coded: more entries than max_frames");
+        k_ble_aux_fill<<<div_up(src.n, 256), 256, 0, st>>>(src, h->d_coded_flags, h->d_coded_offsets, h->d_coded, total, g);
+        const int gs = grid_for(h, m, 4, 8);
+        k_ble_aux_search<kCodedList><<<gs, 128, 0, st>>>(h->d_coded, total, total + m, g, h->d_crc_tab, h->d_coded_whiten, crc_init, tabs);
+        k_ble_coded_window<<<gs, 128, 0, st>>>(h->d_coded, total, total + m, g, ct);
+        k_ble_coded_decode<<<grid_for(h, m, kCodedGroups, 8), 8 * kCodedGroups, 0, st>>>(h->d_coded, total, total + m, g, ct, h->d_crc_tab,
+                                                                                          h->d_coded_whiten, crc_init);
+        k_ble_aux_first<kCodedList><<<grid_for(h, m, 8, 8), 256, 0, st>>>(h->d_coded, total, total + m);
+        CK(cudaGetLastError());
+        src.first = total; src.n = m; src.depth++;
+        total += m;
+    }
+    if (n_out) *n_out = total;
+    if (out && total) {
+        if (cap < total) return fail(h, SNRX_ERANGE, "snrx_ble_coded: buffer smaller than the list");
+        CK(cudaMemcpyAsync(out, h->d_coded, sizeof(snrx_ble_coded_t) * (size_t)total, cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
     }
     return SNRX_OK;

@@ -301,6 +301,18 @@ class RxEngine:
         self._check(self.lib.snrx_ble_aux(self.handle, out.ctypes.data_as(c_void_p), cap, byref(n)))
         return out[: n.value].copy()
 
+    # ------------------------------------------------------------------ BLE Long Range (LE Coded)
+    def ble_coded(self) -> np.ndarray:
+        """The ADV_EXT_INDs sent on the LE Coded PHY on channels 37..39 of the batch most recently returned by poll(),
+        Viterbi-decoded, and the auxiliary packets they point at on every PHY, followed down their chains: one
+        _abi.CODED_DTYPE entry per primary packet or AuxPtr, found and decoded on the GPU from the batch's slicer bit streams
+        (definition in include/snoutrx.h).  Wideband BLE modes; call before the second-next process()."""
+        n = c_uint32(0)
+        cap = int(self.cfg.max_frames) or (1 << 17)
+        out = np.zeros(cap, dtype=_abi.CODED_DTYPE)
+        self._check(self.lib.snrx_ble_coded(self.handle, out.ctypes.data_as(c_void_p), cap, byref(n)))
+        return out[: n.value].copy()
+
     # ------------------------------------------------------------------ SURVEY 8(f) N2: Zigbee consumer path
     def zb_mac_summary(self) -> np.ndarray:
         """Per-record MAC summaries (_abi.ZBMAC_DTYPE: frame type, sequence number, PAN ids, addresses, inter-PAN / ZLL

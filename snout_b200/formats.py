@@ -31,7 +31,7 @@ from typing import BinaryIO, Iterable
 
 import numpy as np
 
-from ._abi import AUX_OK, PROTO_BLE, PROTO_ZIGBEE, RF_CFO, RF_NOISE, RF_POWER
+from ._abi import AUX_OK, AUX_PHY_CODED, PROTO_BLE, PROTO_ZIGBEE, RF_CFO, RF_NOISE, RF_POWER
 
 # ---------------------------------------------------------------------------------- BLE text line
 ADV_PDU_TYPE_STR = (      # btle_rx.c:1081-1098
@@ -270,6 +270,44 @@ def ble_pcap_aux_block(aux: np.ndarray, ts: tuple[int, int] = (0, 0)) -> bytes:
     prefix[:, 24:26] = flags.astype("<u2").view(np.uint8).reshape(n, 2)
     prefix[:, 26:30] = np.frombuffer(struct.pack("<I", 0x8E89BED6), dtype=np.uint8)
     return _pack_records(prefix, a["bytes"], lens)
+
+
+PHDR_PDU_PRIMARY_ADV = 0
+
+
+def ble_pcap_coded_block(lst: np.ndarray, ts: tuple[int, int] = (0, 0), crc_failed_primaries: bool = True) -> bytes:
+    """The packets of RxEngine.ble_coded() that were decoded (status OK) by the first entry to find them, as records of the
+    file btle_rx -s writes: PHDR {channel, 0 x 7, flags}, flags = de-whitened | PDU type << 7 (0 = primary advertising for
+    the ADV_EXT_INDs of depth 0, 1 = auxiliary advertising) | PHY << 14, then the advertising access address, for LE Coded
+    one Coding Indicator byte (0 = S=8, 1 = S=2), then header | payload (no CRC).  crc_failed_primaries=False leaves out the
+    primaries whose CRC failed (most are positions inside an S=8 packet's own body: DESIGN 4)."""
+    sel = (lst["status"] == AUX_OK) & (lst["first"] == np.arange(len(lst)))
+    if not crc_failed_primaries:
+        sel &= (lst["depth"] > 0) | (lst["crc_ok"] == 1)
+    a = lst[sel]
+    n = len(a)
+    coded = a["phy"] == AUX_PHY_CODED
+    lens = a["len"].astype(np.int64) - 3
+    plens = 16 + 10 + 4 + coded.astype(np.int64)
+    prefix = np.zeros((n, 16 + 10 + 4 + 1), dtype=np.uint8)
+    prefix[:, 0:8] = np.frombuffer(struct.pack("<ii", ts[0], ts[1]), dtype=np.uint8)
+    be = (plens - 16 + lens).astype(">i4").view(np.uint8).reshape(n, 4)
+    prefix[:, 8:12], prefix[:, 12:16] = be, be
+    prefix[:, 16] = a["channel"]
+    pdu_type = np.where(a["depth"] == 0, PHDR_PDU_PRIMARY_ADV, PHDR_PDU_AUX_ADV).astype(np.int64)
+    flags = PHDR_DEWHITENED | (pdu_type << PHDR_PDU_TYPE_SHIFT) | (a["phy"].astype(np.int64) << PHDR_PHY_SHIFT)
+    prefix[:, 24:26] = flags.astype("<u2").view(np.uint8).reshape(n, 2)
+    prefix[:, 26:30] = np.frombuffer(struct.pack("<I", 0x8E89BED6), dtype=np.uint8)
+    prefix[:, 30] = a["ci"]
+    return _pack_records(prefix, a["bytes"], lens, plens)
+
+
+def coded_line(d: dict) -> str:
+    """btle_rx --coded line of one primary LE Coded ADV_EXT_IND (a messages.ble_coded_adv dictionary of depth 0), 8 tokens:
+    CODED Ch<37..39> S<8|2> AdvA:<address or -> ADI:<DID>/<SID> (hex, - if absent) PloadL<len> CRC<0 ok|1 failed> AAerr<d>."""
+    adi = f"{d['did']:03x}/{d['sid']:x}" if d["adi"] is not None else "-/-"
+    return (f"CODED Ch{d['channel']} S{d['s']} AdvA:{d['adv_a'] or '-'} ADI:{adi} PloadL{d['pload_len']} "
+            f"CRC{0 if d['crc_ok'] else 1} AAerr{d['aa_errors']}\n")
 
 
 def aux_line(d: dict) -> str:

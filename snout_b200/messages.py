@@ -109,25 +109,29 @@ def _ext_fields(pdu: bytes) -> dict:
     return out
 
 
-def ble_ext_adv(aux: np.ndarray) -> list[dict]:
+_PHY_NAMES = {_abi.AUX_PHY_1M: "1M", _abi.AUX_PHY_2M: "2M", _abi.AUX_PHY_CODED: "Coded"}
+
+
+def ble_ext_adv(aux: np.ndarray, head_depth: int = 0) -> list[dict]:
     """One dictionary per auxiliary packet of RxEngine.ble_aux() that was decoded (status OK) and is the first entry to have
-    found it: index, channel, phy ('1M' / '2M'), depth, crc_ok, tx_add, pload_len (header length field), adv_mode, adv_a, target_a, adi / did / sid, tx_power,
+    found it: index, channel, phy ('1M' / '2M' / 'Coded'), depth, crc_ok, tx_add, pload_len (header length field), adv_mode, adv_a, target_a, adi / did / sid, tx_power,
     adv_data.  The AUX_ADV_INDs (depth 0) also carry `chain` (the list indices of the chain from it) and `chain_data`: the
     AdvData of the whole chain reassembled in order, and `complete`: every link was received with a good CRC and the last
-    one points nowhere."""
+    one points nowhere.  head_depth: the depth of the AUX_ADV_INDs in the list (0 for RxEngine.ble_aux, 1 for
+    RxEngine.ble_coded, whose primaries are depth 0)."""
     out, by_index = [], {}
-    children = {int(r["parent"]): k for k, r in enumerate(aux) if int(r["depth"]) > 0}
+    children = {int(r["parent"]): k for k, r in enumerate(aux) if int(r["depth"]) > head_depth}
     for k, r in enumerate(aux):
         if int(r["status"]) != _abi.AUX_OK or int(r["first"]) != k:
             continue
         pdu = bytes(r["bytes"][: int(r["len"])])
-        d = dict(index=k, channel=int(r["channel"]), phy="2M" if int(r["phy"]) == _abi.AUX_PHY_2M else "1M", depth=int(r["depth"]),
+        d = dict(index=k, channel=int(r["channel"]), phy=_PHY_NAMES.get(int(r["phy"]), "1M"), depth=int(r["depth"]),
                  crc_ok=bool(r["crc_ok"]), tx_add=(pdu[0] >> 6) & 1, pload_len=pdu[1], sample_index=int(r["sample_index"]),
                  capture_id=int(r["capture_id"]), **_ext_fields(pdu))
         out.append(d)
         by_index[k] = d
     for d in out:
-        if d["depth"] != 0:
+        if d["depth"] != head_depth:
             continue
         chain, data, k, complete = [d["index"]], d["adv_data"], d["index"], d["crc_ok"]
         while complete and by_index[k]["aux_ptr"] is not None:
@@ -139,4 +143,15 @@ def ble_ext_adv(aux: np.ndarray) -> list[dict]:
             data += by_index[c]["adv_data"]
             k = c
         d["chain"], d["chain_data"], d["complete"] = chain, data, complete
+    return out
+
+
+def ble_coded_adv(lst: np.ndarray) -> list[dict]:
+    """ble_ext_adv of RxEngine.ble_coded(): the primary ADV_EXT_INDs (depth 0) and the auxiliary packets (chains from the
+    AUX_ADV_INDs at depth 1).  Coded packets also carry `s` (8 or 2, from the coding indicator) and `aa_errors` (d(n))."""
+    out = ble_ext_adv(lst, head_depth=1)
+    for d in out:
+        r = lst[d["index"]]
+        if int(r["phy"]) == _abi.AUX_PHY_CODED:
+            d["s"], d["aa_errors"] = 8 if int(r["ci"]) == 0 else 2, int(r["aa_errors"])
     return out

@@ -718,3 +718,137 @@ def ext_adv_capture(seconds: float = 0.05, seed: int = 9000, esn0_db: float | No
     if esn0_db is not None:
         x = x + _awgn(len(x), np.random.default_rng(seed + 999), 4.0 * chanplan.WB_DECIM / (10.0 ** (esn0_db / 10.0))).astype(np.complex64)
     return Capture(x.astype(np.complex64), chanplan.WB_RATE, prim, dict(kind="wb_ble_ext", seed=seed, esn0_db=esn0_db, aux=aux))
+
+
+# ------------------------------------------------------------- BLE Long Range (LE Coded PHY, test input)
+# Core Vol 6 Part B 2.2 and 3.3 as read here: rate-1/2 convolutional code with K = 4, G0 = 1 + x + x^2 + x^3 and
+# G1 = 1 + x^2 + x^3 (a0 first), pattern mapper S=8: 0 -> 0011, 1 -> 1100 (S=2: identity).  The packet: 80 symbols of
+# 00111100, FEC block 1 (AA | CI | TERM1, always S=8), FEC block 2 (whitened PDU | CRC | TERM2, S=8 if CI = 0, S=2 if CI = 1);
+# each block's encoder starts with an all-zero register.
+_CODED_G = ((1, 1, 1, 1), (1, 0, 1, 1))        # coefficients of x^0..x^3: the input and the three delay cells
+
+
+def coded_fec(bits) -> list[int]:
+    reg = [0, 0, 0]                             # x^1, x^2, x^3: the last three inputs, most recent first
+    out = []
+    for u in bits:
+        taps = [int(u)] + reg
+        out += [sum(g * t for g, t in zip(G, taps)) & 1 for G in _CODED_G]
+        reg = [int(u)] + reg[:2]
+    return out
+
+
+def coded_map(coded, s: int) -> list[int]:
+    if s == 2:
+        return list(coded)
+    return [v for c in coded for v in ((0, 0, 1, 1) if c == 0 else (1, 1, 0, 0))]
+
+
+def ble_phy_bits_coded(pdu: bytes, channel: int, s: int = 8, access_addr: int = chanplan.BLE_ADV_AA,
+                       crc_init: int = chanplan.BLE_ADV_CRC_INIT, ci: int | None = None) -> np.ndarray:
+    """LE Coded symbols (1 Msym/s) of a PDU: preamble | FEC block 1 | FEC block 2.  ci overrides the coding indicator sent
+    (default: 0 for S=8, 1 for S=2)."""
+    assert s in (8, 2)
+    ci = (0 if s == 8 else 1) if ci is None else ci
+    body = bytes(pdu) + ble_crc24(pdu, crc_init)
+    body = bytes(np.frombuffer(body, dtype=np.uint8) ^ ble_whitening(channel, len(body)))
+    aa = [(access_addr >> i) & 1 for i in range(32)]
+    b1 = coded_map(coded_fec(aa + [ci & 1, ci >> 1, 0, 0, 0]), 8)
+    b2 = coded_map(coded_fec(list(bytes_to_bits_lsb(body)) + [0, 0, 0]), s)
+    return np.array([0, 0, 1, 1, 1, 1, 0, 0] * 10 + b1 + b2, dtype=np.uint8)
+
+
+CODED_PREAMBLE = {0: 32, 1: 32, 2: 320}          # channel samples from the first preamble sample to the AA (bit 0 / coded)
+
+
+def _phy_symbols(pdu: bytes, channel: int, phy: int, s: int) -> tuple[np.ndarray, int]:
+    if phy == 2:
+        return ble_phy_bits_coded(pdu, channel, s), 4
+    return (ble_phy_bits_2m(pdu, channel), 2) if phy == 1 else (ble_phy_bits(pdu, channel), 4)
+
+
+@dataclass
+class CodedTruth:
+    """A BLE Long Range packet placed into a synthetic capture (a primary ADV_EXT_IND or a packet of its chain)."""
+    channel: int
+    phy: int              # 0 = LE 1M, 1 = LE 2M, 2 = LE Coded
+    s: int                # Coded: 8 or 2 (0 otherwise)
+    start: int            # channel-rate sample of the first preamble sample
+    anchor: int           # nominal start of the coded AA (Coded) or AA bit 0 (preamble + Gaussian filter delay)
+    data: bytes           # pdu | crc (un-whitened)
+    depth: int            # 0 = primary ADV_EXT_IND, d = d links from it
+    parents: list = field(default_factory=list)
+
+
+def coded_adv_schedule(n_ch: int, rng: np.random.Generator, n_events: int = 4, phys=(2, 0, 1), s_values=(8, 2),
+                       max_chain: int = 2, cfo_hz: float = 50e3, data_len=(0, 60), event_gap: int = 20_000):
+    """Long Range extended advertising laid end to end on a 4 Msps time line: per event an ADV_EXT_IND on LE Coded on 37, 38
+    and 39 (one S per event), each pointing at one AUX_ADV_IND on a random data channel and PHY (phys), which points down a
+    chain of 0..max_chain AUX_CHAIN_INDs.  Returns ({bin: stream}, [CodedTruth])."""
+    streams: dict = {}
+    out = []
+    pos = 2000
+
+    def length(phy, s, n_bytes):
+        if phy == 2:
+            return 4 * (80 + 296 + 2 * (8 * n_bytes + 3) * (4 if s == 8 else 1)) + 16
+        return ((16 + 32 + 8 * n_bytes) * 2 if phy == 1 else (8 + 32 + 8 * n_bytes) * 4) + 16
+
+    for _ in range(n_events):
+        adv_a = bytes(rng.integers(0, 256, 6, dtype=np.uint8))
+        did, sid = int(rng.integers(0, 4096)), int(rng.integers(0, 16))
+        adi = did | (sid << 12)
+        s_prim = int(rng.choice(s_values))
+        n_links = 1 + int(rng.integers(0, max_chain + 1))
+        chans = [int(c) for c in rng.integers(0, 37, n_links)]
+        phys_l = [int(rng.choice(phys)) for _ in range(n_links)]
+        ss = [int(rng.choice(s_values)) if p == 2 else 0 for p in phys_l]
+        cas = [int(rng.integers(0, 2)) for _ in range(n_links + 1)]
+        datas = [bytes(rng.integers(0, 256, int(rng.integers(data_len[0], data_len[1] + 1)), dtype=np.uint8)) for _ in range(n_links)]
+        p_len = length(2, s_prim, 2 + 7 + 3)
+        p_starts = [pos, pos + p_len + 1400, pos + 2 * (p_len + 1400)]
+        t = p_starts[2] + p_len + int(rng.integers(1200, 6000))
+        starts = []
+        for k in range(n_links):
+            payload_len = len(ext_header(0, adv_a if k == 0 else None, 0, adi, b"\0\0\0" if k + 1 < n_links else None,
+                                         0 if k == 0 else None)) + len(datas[k])
+            starts.append(t)
+            t += length(phys_l[k], ss[k], 2 + payload_len + 3) + 1200 + int(rng.integers(0, 4000))
+        pdus = []
+        for k in range(n_links):
+            ptr, info = None, None
+            if k + 1 < n_links:
+                units, off, drift = aux_offset_for(starts[k + 1] - starts[k], cas[k + 1], rng)
+                ptr = aux_ptr_bytes(chans[k + 1], cas[k + 1], units, off, phys_l[k + 1])
+                info = (units, off, cas[k + 1], drift)
+            pdus.append((ext_pdu(ext_header(0, adv_a if k == 0 else None, 0, adi, ptr, 0 if k == 0 else None), datas[k]), info))
+        for j, ps in enumerate(p_starts):
+            units, off, drift = aux_offset_for(starts[0] - ps, cas[0], rng)
+            pp = ext_pdu(ext_header(0, None, 0, adi, aux_ptr_bytes(chans[0], cas[0], units, off, phys_l[0])))
+            sym, sps = _phy_symbols(pp, 37 + j, 2, s_prim)
+            _put(streams, n_ch, 37 + j, ps, gfsk_modulate(sym, sps=sps), rng, cfo_hz)
+            out.append(CodedTruth(37 + j, 2, s_prim, ps, ps + 320 + 8, pp + ble_crc24(pp), 0))
+        prim = out[-3:]
+        for k in range(n_links):
+            pdu = pdus[k][0]
+            sym, sps = _phy_symbols(pdu, chans[k], phys_l[k], ss[k])
+            _put(streams, n_ch, chans[k], starts[k], gfsk_modulate(sym, sps=sps), rng, cfo_hz)
+            par = [p.start for p in prim] if k == 0 else [starts[k - 1]]
+            anchor = starts[k] + CODED_PREAMBLE[phys_l[k]] + 2 * sps
+            out.append(CodedTruth(chans[k], phys_l[k], ss[k], starts[k], anchor, pdu + ble_crc24(pdu), k + 1, par))
+        pos = t + event_gap
+        assert pos < n_ch, "capture too short for the events"
+    return streams, out
+
+
+def coded_adv_capture(seconds: float = 0.05, seed: int = 9600, esn0_db: float | None = 25.0, **kw) -> Capture:
+    """96 Msps capture (centre 2440 MHz) carrying coded_adv_schedule(...) events and nothing else; meta["coded"] holds the
+    CodedTruth list.  esn0_db=None: no noise."""
+    rng = np.random.default_rng(seed)
+    n_ch = int(round(seconds * chanplan.NB_RATE))
+    n_ch -= n_ch % chanplan.BLE_WINDOW
+    streams, truth = coded_adv_schedule(n_ch, rng, **kw)
+    x = wideband_mix(streams)
+    if esn0_db is not None:
+        x = x + _awgn(len(x), np.random.default_rng(seed + 999), 4.0 * chanplan.WB_DECIM / (10.0 ** (esn0_db / 10.0))).astype(np.complex64)
+    return Capture(x.astype(np.complex64), chanplan.WB_RATE, [], dict(kind="wb_ble_coded", seed=seed, esn0_db=esn0_db, coded=truth))
