@@ -43,9 +43,10 @@
  *               (scapy-radio/scapy/scapy/modules/gnuradio.py:67-73).
  *   snrx_set_channel
  *       Zigbee: top_block.set_channel() via XMLRPC (top_block.py:94-96).
- *   snrx_debug_stage
- *       no reference counterpart: exposes intermediate streams (quantised
- *       channel streams, discriminator output, soft chips) for parity tests.
+ *   snrx_debug_stage / snrx_debug_process_bits
+ *       no reference counterpart: expose intermediate streams (quantised
+ *       channel streams, discriminator output, soft chips) for parity tests,
+ *       and run the BLE back end on given slicer bit streams.
  */
 #ifndef SNOUTRX_H
 #define SNOUTRX_H
@@ -644,6 +645,17 @@ int  snrx_set_stream(snrx_t* h, void* cuda_stream);       /* run on a caller str
 int  snrx_sync(snrx_t* h);
 int  snrx_stats(snrx_t* h, snrx_stats_t* s);
 int  snrx_debug_stage(snrx_t* h, int stage, void* out, uint64_t cap_bytes, uint64_t* n_bytes);
+/* Test hook: queue a batch as snrx_process does, but with the BLE slicer bit streams given instead of computed from a
+ * capture. words: host memory in the SNRX_STAGE_BLE_BITS layout [n_captures][BLE channels][bits_words_for(n_out)],
+ * n_out = n_samples / decimation. The back end, snrx_poll and every call on the polled batch (snrx_ble_aux, snrx_ble_coded,
+ * snrx_ble_follow, summaries) then behave as if the channelizer had produced these words.  bits_words_for(n) =
+ * 4 lead words + ceil(n / 32) + 64 tail words; bit (m & 31) of word 4 + (m >> 5) is the decision of channel sample m.
+ * shard: as in snrx_process (pre_samples and body_samples in input samples).  SNRX_EINVAL for a NULL words, a mode with
+ * an 802.15.4 receiver, an engine created with SNRX_F_RF_METRICS or SNRX_F_KEEP_STREAMS (there is no input or channel
+ * stream), a wideband n_samples that is not a multiple of 24, or a set bit in the lead words or at a sample >= n_out (the
+ * front end never writes one); SNRX_ERANGE and SNRX_ESTATE as snrx_process. */
+int snrx_debug_process_bits(snrx_t* h, const uint32_t* words, uint32_t n_captures, uint64_t n_samples,
+                            const snrx_shard_t* shard);
 
 /* prototype low-pass of the wideband channelizer (taps = 384 or 768 doubles) */
 int  snrx_pfb_prototype(int mode, uint32_t taps, double* out);

@@ -160,6 +160,7 @@ SYMBOLS = [
     ("snrx_sync", c_int, [c_void_p]),
     ("snrx_stats", c_int, [c_void_p, POINTER(Stats)]),
     ("snrx_debug_stage", c_int, [c_void_p, c_int, c_void_p, c_uint64, POINTER(c_uint64)]),
+    ("snrx_debug_process_bits", c_int, [c_void_p, c_void_p, c_uint32, c_uint64, POINTER(Shard)]),
     ("snrx_pfb_prototype", c_int, [c_int, c_uint32, POINTER(c_double)]),
     ("snrx_host_alloc", c_int, [POINTER(c_void_p), c_uint64]),
     ("snrx_host_free", c_int, [c_void_p]),

@@ -708,15 +708,34 @@ static int launch_ble_front(snrx_handle* h, Lane& ln, const float2* x, uint32_t 
 
 enum { kFmtCf32 = 0, kFmtSc8 = 1 };
 
+// true if no bit is set in the lead words or at a sample >= n_out of any stream ([streams][bits_words_for(n_out)])
+static bool bits_outside_clear(const uint32_t* words, uint64_t n_streams, uint32_t n_out) {
+    const uint64_t wpp = bits_words_for(n_out);
+    const uint32_t body = (n_out + 31) / 32, partial = n_out & 31;
+    for (uint64_t st = 0; st < n_streams; st++) {
+        const uint32_t* w = words + st * wpp;
+        for (uint64_t i = 0; i < wpp; i++) {
+            const uint64_t b = i - kBitsLeadWords;                 // body word (wraps for the lead words)
+            const uint32_t allowed = b >= body ? 0u : (b + 1 == body && partial ? (1u << partial) - 1u : 0xFFFFFFFFu);
+            if (w[i] & ~allowed) return false;
+        }
+    }
+    return true;
+}
+
+// bits != nullptr: snrx_debug_process_bits -- the BLE slicer words are given (host memory, SNRX_STAGE_BLE_BITS layout)
+// instead of computed from iq; no input is staged and no front end runs.  Everything from the back end on is shared.
 static int process_impl(snrx_t* h, const void* iq, int fmt, uint32_t n_captures, uint64_t n_samples, uint64_t stride_samples,
-                        const snrx_shard_t* shard, int is_device_ptr) {
-    if (!h || !iq) return SNRX_EINVAL;
+                        const snrx_shard_t* shard, int is_device_ptr, const uint32_t* bits = nullptr) {
+    if (!h || !(iq || bits)) return SNRX_EINVAL;
     if (n_captures == 0 || n_samples == 0) return fail(h, SNRX_EINVAL, "empty batch");
     if (n_captures > h->max_caps || n_samples > h->max_in) return fail(h, SNRX_ERANGE, "batch exceeds max_captures/max_samples");
     if (stride_samples == 0) stride_samples = n_samples;
     if (stride_samples < n_samples) return fail(h, SNRX_EINVAL, "stride smaller than the capture");
-    if ((((uintptr_t)iq) & 15) || (n_captures > 1 && (stride_samples & 1))) return fail(h, SNRX_EINVAL, "captures must be 16-byte aligned (even stride)");
+    if (!bits && ((((uintptr_t)iq) & 15) || (n_captures > 1 && (stride_samples & 1)))) return fail(h, SNRX_EINVAL, "captures must be 16-byte aligned (even stride)");
     if (h->wideband && (n_samples % kPfbD) != 0) return fail(h, SNRX_EINVAL, "wideband captures must hold a multiple of 24 samples");
+    if (bits && !bits_outside_clear(bits, (uint64_t)n_captures * h->n_ble_ch, (uint32_t)(n_samples / h->decim)))
+        return fail(h, SNRX_EINVAL, "snrx_debug_process_bits: a bit is set in the lead words or past the capture's last sample");
     CK(cudaSetDevice(h->device));
     const int li = (int)(h->seq_process % kLanes);
     Lane& ln = h->lane[li];
@@ -765,8 +784,8 @@ static int process_impl(snrx_t* h, const void* iq, int fmt, uint32_t n_captures,
     //      sc8 input (host or device) is expanded to cf32 in ln.d_x by k_sc8_to_cf32, chunk by chunk
     const float2* x = reinterpret_cast<const float2*>(iq);
     uint64_t x_stride = stride_samples;
-    const bool staged = !is_device_ptr;
-    const bool sc8 = (fmt == kFmtSc8);
+    const bool staged = !is_device_ptr && !bits;
+    const bool sc8 = (fmt == kFmtSc8) && !bits;
     const uint64_t chunk_samples = sc8 ? (8ull << 20) : (4ull << 20);   // 16 MiB (sc8) / 32 MiB (cf32) per copy
     const size_t in_elem = sc8 ? 2 : sizeof(float2);                // bytes per input sample
     if (staged || sc8) {
@@ -798,7 +817,9 @@ static int process_impl(snrx_t* h, const void* iq, int fmt, uint32_t n_captures,
     if (h->has_ble) {
         lay.words_per_stream = bits_words_for(n_out);
         lay.n_channels = h->n_ble_ch;
-        CK(cudaMemsetAsync(ln.d_bits, 0, (size_t)n_captures * h->n_ble_ch * lay.words_per_stream * sizeof(uint32_t), st));
+        const size_t bytes = (size_t)n_captures * h->n_ble_ch * lay.words_per_stream * sizeof(uint32_t);
+        if (bits) CK(cudaMemcpyAsync(ln.d_bits, bits, bytes, cudaMemcpyHostToDevice, st));
+        else CK(cudaMemsetAsync(ln.d_bits, 0, bytes, st));
     }
 
     if (staged) {
@@ -842,8 +863,10 @@ static int process_impl(snrx_t* h, const void* iq, int fmt, uint32_t n_captures,
         const bool pipelined = staged && h->wideband && !h->has_zb && n_captures == 1;
         if (!pipelined) {
             CK(cudaEventRecord(ln.ev_front0, st));
-            int r = launch_ble_front(h, ln, x, n_captures, n_samples, x_stride, n_out, 0, (int)div_up(n_out, ble_tile_stride(h)), lay);
-            if (r != SNRX_OK) return r;
+            if (!bits) {
+                int r = launch_ble_front(h, ln, x, n_captures, n_samples, x_stride, n_out, 0, (int)div_up(n_out, ble_tile_stride(h)), lay);
+                if (r != SNRX_OK) return r;
+            }
         }
         CK(cudaEventRecord(ln.ev_front, st));
         CK(cudaEventRecord(ln.ev_handoff, st));
@@ -975,6 +998,16 @@ int snrx_process(snrx_t* h, const float* iq, uint32_t n_captures, uint64_t n_sam
 int snrx_process_sc8(snrx_t* h, const int8_t* iq, uint32_t n_captures, uint64_t n_samples, uint64_t stride_samples,
                      const snrx_shard_t* shard, int is_device_ptr) {
     return process_impl(h, iq, kFmtSc8, n_captures, n_samples, stride_samples, shard, is_device_ptr);
+}
+
+int snrx_debug_process_bits(snrx_t* h, const uint32_t* words, uint32_t n_captures, uint64_t n_samples,
+                            const snrx_shard_t* shard) {
+    if (!h) return SNRX_EINVAL;
+    if (!words) return fail(h, SNRX_EINVAL, "snrx_debug_process_bits: words is NULL");
+    if (h->has_zb) return fail(h, SNRX_EINVAL, "snrx_debug_process_bits: BLE-only modes (an 802.15.4 receiver needs its input)");
+    if (h->cfg.flags & (SNRX_F_RF_METRICS | SNRX_F_KEEP_STREAMS))
+        return fail(h, SNRX_EINVAL, "snrx_debug_process_bits: no input or channel stream to measure or keep");
+    return process_impl(h, nullptr, kFmtCf32, n_captures, n_samples, 0, shard, 0, words);
 }
 
 int snrx_poll(snrx_t* h, snrx_frame_t* out, uint32_t cap, uint32_t* n_out) {

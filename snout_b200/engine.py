@@ -171,6 +171,26 @@ class RxEngine:
         self.batches_queued += 1
         return self
 
+    def process_bits(self, words, n_samples: int, shard: dict | None = None):
+        """Test hook (snrx_debug_process_bits): queue a batch whose BLE slicer bit streams are `words` -- uint32
+        [captures, BLE channels, words] in the SNRX_STAGE_BLE_BITS layout, for n_samples input samples per capture --
+        instead of channelizing a capture.  poll() and every call on the polled batch then see these streams."""
+        sh = None
+        if shard:
+            sh = Shard(int(shard.get("pre_samples", 0)), int(shard.get("body_samples", 0)),
+                       int(shard.get("first_window", 0)), int(shard.get("first_capture_id", 0)))
+        w = np.ascontiguousarray(words, dtype=np.uint32)
+        caps = 1 if w.ndim < 3 else w.shape[0]
+        self._check(self.lib.snrx_debug_process_bits(self.handle, w.ctypes.data_as(c_void_p), caps, int(n_samples),
+                                                     byref(sh) if sh else None))
+        self._keepalive.append(w)
+        self._last = (caps, int(n_samples))
+        self.batches_queued += 1
+        return self
+
+    def run_bits(self, words, n_samples: int, **kw) -> np.ndarray:
+        return self.process_bits(words, n_samples, **kw).poll()
+
     def poll(self, copy: bool = True) -> np.ndarray:
         """Wait for the oldest queued batch (up to two may be queued) and return its frames in
         reference order (capture, channel, window, index).  copy=False returns a view of the engine's
