@@ -30,8 +30,11 @@
 namespace snrx {
 
 constexpr int kZbPostHalo = 16448;          // PHR + 127 bytes = 256 symbols * 64 samples, + 64
-constexpr int kZbMinSyncSpacing = 448;      // the sink can complete a sync every 7 symbols of 64 samples: one '0' symbol + SFD (2),
-                                            // PHR (2), one byte (2) -- packet_sink_scapy_impl.cc:204-241, 247-359
+constexpr int kZbMinSyncChips = 193;        // chips between the SFD-completing chips of two records of one chain, at least: PHR (64),
+                                            // one byte (64; a PHR of 0 still waits for one), >= 1 chip to re-lock on the register that
+                                            // enter_search() cleared, 7 (32) and 10 (32) -- packet_sink_scapy_impl.cc:55-65, 190-359.
+                                            // Not 7 symbols: the cleared register lets the search lock after k < 32 fresh chips (k = 14
+                                            // at threshold 10), and every chip advances the clock recovery by 1..3 samples
 constexpr int kZbSinkLead = 1024;           // the sink starts this many samples before the body: SHR (640) + alignment
                                             // slack; the clock recovery starts `prehalo` samples early (warm-up only)
 constexpr float kZbClamp = 16.0f;           // |z| <= pi + |DC| for any finite input; anything else (Inf / NaN samples in the
@@ -507,7 +510,9 @@ SNRX_HD uint32_t zb_filter_chain(snrx_frame_t* slots, uint32_t n, int64_t good_e
     return w;
 }
 SNRX_HD int zb_filter_lookback(int segment) { return (16384 + segment - 1) / segment + 1; }
-SNRX_HD uint32_t zb_slots_per_chain(uint32_t segment) { return segment / kZbMinSyncSpacing + 2; }
+// a body of `segment` samples holds at most this many syncs kZbMinSyncChips samples apart (22 at 4096); k_zb_rx still flags a
+// chain that finds more (SNRX_EOVERFLOW)
+SNRX_HD uint32_t zb_slots_per_chain(uint32_t segment) { return (segment - 1) / kZbMinSyncChips + 1; }
 
 #if defined(__CUDACC__)
 // ------------------------------------------------------------------------------------ kernels
@@ -647,7 +652,13 @@ constexpr int kZbLead = 64;           // samples the tracker starts ahead of the
                                       // tracker's position stays a multiple of 64 at every window start and a block boundary
                                       // of the tracker (2048) can only fall on a window start
 constexpr int kZbLeadMin = 44;        // a window may start with this much lead: 32 steps of 3 samples eat at most 32 of it, 8 are read
-constexpr int kZbLeadMax = 84;        // beyond it the tracker pauses for a window (the ring holds 128 >= 84 + 32 + 8)
+constexpr int kZbLeadMax = 84;        // beyond it the tracker pauses for a window (the ring holds 128 >= 84 + 32 + 8).  A paused
+                                      // window converts nothing, so its reads must stay behind conv on their own: |mm| <=
+                                      // max|out| <= 1.60 * 2 pi (largest sum of |taps| of a row, |z| <= 2 pi), so 31 steps advance
+                                      // at most 1 + 31 * (2.0004 + 0.03 * 10.06) = 72.4 samples and the last read still has
+                                      // 85 - 72.4 = 12.6 samples of lead against the 8 it reads: 4.6 to spare.  This is a
+                                      // derived bound: no test input comes near it (windows under 3e-3 chip-rate drift pause
+                                      // with a lead of 22 or more at every read)
 constexpr int kZbTapsPlane = (SNRX_MMSE_NSTEPS + 1) * 16;   // bytes of one plane of the interpolator table in shared memory
 constexpr int kZbRxWarps = 4;         // warps per CTA (they only share the interpolator table)
 #ifndef SNRX_ZB_RX_MINCTAS

@@ -302,7 +302,14 @@ void emu_zb_dc(const float* f, int64_t n, float* z) {
         }
     }
 }
-// chains over a DC-removed stream: zb_run_chain (the per-thread code of k_zb_rx) with the samples read straight from z
+uint32_t emu_zb_slots_per_chain(uint32_t segment) { return zb_slots_per_chain(segment); }
+void emu_zb_mmse_taps(float* out /*[129][8]*/) { memcpy(out, SNRX_MMSE_TAPS, sizeof(SNRX_MMSE_TAPS)); }
+// k_zb_rx's tracker pacing: kZbLead, kZbLeadMin, kZbLeadMax
+void emu_zb_lead_params(int* out) { out[0] = kZbLead; out[1] = kZbLeadMin; out[2] = kZbLeadMax; }
+
+// chains over a DC-removed stream: zb_run_chain (the per-thread code of k_zb_rx) with the samples read straight from z.
+// Returns the number of records, or -(seg + 1) when chain seg found more records than its slots hold (k_zb_rx sets the
+// overflow flag there and the batch fails with SNRX_EOVERFLOW).
 int emu_zb_chains(const float* z, int n_out, int origin, int body, int segment, int prehalo, uint32_t first_segment,
                   int threshold, int channel, snrx_frame_t* out, int cap, int64_t* nchips_out /* [n_segments] or null */) {
     ZbChainParams p{};
@@ -321,7 +328,8 @@ int emu_zb_chains(const float* z, int n_out, int origin, int body, int segment, 
         uint32_t nf = zb_run_chain<false>(src, p, seg, map.w, channel, 0, slots.data() + (size_t)seg * p.slots_per_chain, nullptr, 0,
                                           &nchips, &good_end[seg]);
         if (nchips_out) nchips_out[seg] = nchips;
-        counts[seg] = nf < p.slots_per_chain ? nf : p.slots_per_chain;
+        if (nf > p.slots_per_chain) return -(seg + 1);
+        counts[seg] = nf;
     }
     // k_zb_span_filter (one thread per chain), then k_zb_gather
     const int lookback = zb_filter_lookback(segment);
