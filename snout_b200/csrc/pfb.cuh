@@ -330,7 +330,7 @@ template <class G, int TT, bool INIT = false>
 __device__ __forceinline__ void pfb_stage_tile_bulk(float2* xs, const float2* xtile /* sample i' = 0 */, uint64_t* bar, int lane) {
     constexpr int kPer = 24 * TT;
     static_assert(G::kPieces <= 32 && G::kTileIn % 2 == 0, "one lane per piece");
-    // the barrier was initialised once per warp (count 1); every tile is one phase of it.  ONE elected lane issues all the
+    // the barrier has count 1 and the tile is one phase of it.  ONE elected lane issues all the
     // copies (compile-time offsets and sizes, warp-uniform addresses): with one lane per piece the compiler serialises them
     // anyway -- a bulk copy takes its operands from uniform registers, so it elects a lane, broadcasts that lane's operands,
     // issues, and loops (ELECT / R2UR / UBLKCP / BRA.U.ANY six times in the sampled profile).
@@ -406,9 +406,6 @@ struct PfbBleArgs {
     int32_t n_tiles;          // tiles per capture in this launch
     int32_t tile0;            // first tile of this launch
     int32_t n_caps;           // captures in this launch
-    int32_t tiles_per_cta;    // k_pfb_ble_run only
-    int32_t stagger_ns;       // k_pfb_ble_run only: start delay per CTA slot of an SM (SNRX_PFB_STAGGER_NS; 0 = none)
-    int32_t sm_count;         // k_pfb_ble_run only
     const float4* taps_pass;  // [3][NT/4][8] float4: element (gi, d4, rl) = h[rho + 24 (4 d4 + 0..3)], rho = gi + 3 rl --
                               // the 8 FIR rows of a pass read 128 contiguous bytes per load
     float scale;              // quantiser scale
@@ -422,29 +419,9 @@ struct PfbBleArgs {
 template <class G>
 SNRX_HD bool pfb_tile_interior(int64_t x0, int64_t n_in) { return x0 >= 0 && x0 + G::kTileIn <= n_in; }
 
-// The same bulk staging with every instruction PREDICATED instead of branched around (`on` = stage / do nothing): the
-// persistent kernel issues the next tile's copies from inside its tile loop, and a branch there makes ptxas duplicate the
-// rest of the loop body (see k_pfb_ble_run).  No __syncwarp between the expect_tx and the copies: complete_tx may run
-// ahead of expect_tx (the phase cannot complete before lane 0's arrival).
-template <class G, int TT>
-__device__ __forceinline__ void pfb_stage_tile_bulk_pred(float2* xs, const float2* xtile, uint64_t* bar, int lane, bool on) {
-    constexpr int kPer = 24 * TT;
-    const uint32_t p0 = (on && lane == 0) ? 1u : 0u;
-    asm volatile("{\n.reg .pred p;\nsetp.ne.u32 p, %2, 0;\n@p mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n}\n" ::"r"(smem_u32(bar)),
-                 "r"((uint32_t)(G::kTileIn * sizeof(float2))), "r"(p0)
-                 : "memory");
-    const int lo = lane == 0 ? 0 : kPer * lane - 12;
-    const int hi = min(kPer * (lane + 1) - 12, G::kTileIn);
-    const uint32_t p1 = (on && lane < G::kPieces) ? 1u : 0u;
-    asm volatile("{\n.reg .pred p;\nsetp.ne.u32 p, %4, 0;\n@p cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];\n}\n" ::"r"(
-                     smem_u32(xs + lo + 8 * lane)),
-                 "l"(xtile + lo), "r"((uint32_t)((hi - lo) * sizeof(float2))), "r"(smem_u32(bar)), "r"(p1)
-                 : "memory");
-}
-
-// One tile, staged in xs, through phases 1-3.  after_fir() runs once every lane has read the tile for the last time.
-template <int NT, bool DEBUG, class AfterFir>
-__device__ __forceinline__ void pfb_ble_tile(const PfbBleArgs& a, const float2* xs, float4* V, int lane, int cap, int g_first, AfterFir after_fir) {
+// One tile, staged in xs, through phases 1-3.
+template <int NT, bool DEBUG>
+__device__ __forceinline__ void pfb_ble_tile(const PfbBleArgs& a, const float2* xs, float4* V, int lane, int cap, int g_first) {
     using B = PfbBleGeom<NT>;
     // ---- phase 1: three passes of FIR (branches r = gi mod 3) -> transpose -> 16-point inverse DFT
     cf f[3][16];
@@ -466,7 +443,6 @@ __device__ __forceinline__ void pfb_ble_tile(const PfbBleArgs& a, const float2* 
             for (int e = 0; e < kChunkT; e++)
                 V[v_pos(rl, 8 * c + e)] = make_float4(acc[0][e].x, acc[0][e].y, acc[1][e].x, acc[1][e].y);
             __syncwarp();
-            if (gi == 2) after_fir();
             cf v16[16];
             pfb_load_col16_pfa(V, lane, gi, v16);
             __syncwarp();                                                  // V is rewritten by the next pass
@@ -497,15 +473,6 @@ __device__ __forceinline__ void pfb_ble_tile(const PfbBleArgs& a, const float2* 
         }
     }
 
-#ifdef SNRX_PROBE_NO_TAIL                                    // measurement builds only (tools/ab_probe.sh): what the tail costs
-    {
-        uint32_t sacc = 0u;
-#pragma unroll
-        for (int q = 0; q < 48; q++) if (ble_channel_of_q(q) >= 0) sacc += sw[q] ^ sa[q];
-        if (sacc == 0x12345678u) a.bits[0] = 1u;
-        return;
-    }
-#endif
     // ---- phase 3: slicer bits (btle_rx.c:1357-1361), transposed to one word per channel, OR-ed into the streams
     {
         uint32_t wa = 0, wb = 0;                             // bit L = decision of slot L (ble_q_of_slot_a / _b) at time `lane`
@@ -577,10 +544,6 @@ __global__ void __launch_bounds__(32, PfbBleGeom<NT>::kCtasPerSm) k_pfb_ble(PfbB
     const int64_t x0 = (int64_t)kPfbD * g_first - G::kHist;
     // (an L2 prefetch of the input a CTA `n` launches behind this one will stage -- cp.async.bulk.prefetch.L2, 1184 ... 9472 tiles
     // ahead -- was measured: 0.333 / 0.334 / 0.336 / 0.336 / 0.338 ms, no gain: what a fresh CTA waits for is not HBM-vs-L2 latency)
-#ifdef SNRX_PROBE_NO_STAGE                                   // measurement builds only: the tile is whatever shared memory holds
-    if (pfb_tile_interior<G>(x0, a.n_in)) {
-    } else
-#endif
     if (pfb_tile_interior<G>(x0, a.n_in)) {
         pfb_stage_tile_bulk<G, kChunkT, true>(xs, xcap + x0, bar, lane);
         __syncwarp();
@@ -590,64 +553,7 @@ __global__ void __launch_bounds__(32, PfbBleGeom<NT>::kCtasPerSm) k_pfb_ble(PfbB
         cp_async_commit_wait_all();
         __syncwarp();
     }
-    pfb_ble_tile<NT, DEBUG>(a, xs, V, lane, cap, g_first, [] {});
-}
-
-// INTERIOR tiles only (a.tile0 .. a.tile0 + a.n_tiles - 1 of every capture lie entirely inside it), several consecutive tiles per
-// one-warp CTA: the bulk copy of the NEXT tile is issued as soon as the last FIR pass has read the current one (no second tile
-// buffer), so only a CTA's first tile waits for memory with nothing else to do, and there is no CTA start per tile.
-// MEASURED and REJECTED twice (round 2, B200, 94.4 M samples); it stays off (SNRX_PFB_TILES=0):
-//   first version (tile index split by divisions, one lane per bulk-copy piece, predicated staging; 108 B of spills):
-//     alone 0.388-0.390 ms against 0.328 for one tile per CTA; in the two-lane pipeline 0.452 / 0.495 / 0.555 ms for 2 / 4 / 8 tiles;
-//     ncu (profiles/r02_pfb_run_ncu.json): same DRAM traffic, L2 hit 47 % vs 33 %, long-scoreboard 0.93 vs 0.60 per issue;
-//   this version (no division, one elected lane issues the copies, 20 B of spills, parity suite green with SNRX_PFB_TILES=4):
-//     alone 0.333 / 0.333 / 0.337 / 0.349 ms for 2 / 4 / 8 / 16 tiles per CTA against 0.313; steps of 0.395 / 0.405 / 0.509 ms
-//     against 0.383.
-//     One wave (54 tiles per CTA): 0.360 ms; with the CTAs of an SM started 400 / 800 ns apart (SNRX_PFB_STAGGER_NS): 0.357 / 0.359.
-// The wait for the tile (10 % of a one-tile CTA's life) and the CTA start are gone, and it is still slower -- the more tiles per
-// CTA, the slower -- and staggering the warps' phases changes nothing, so phase lock-step is not it.  What grows with the tiles
-// per CTA is the number of separate input regions read at once (2368 CTAs each walking its own stretch of the capture, where
-// the one-tile kernel's resident CTAs form ONE compact window moving through it): the first version's ncu capture already
-// showed the long-scoreboard stall at 0.93 per issue against 0.60.  Not measured with this version: grid-strided tiles (CTA b
-// takes tiles b, b + grid, ...), which keep the window compact.  Until then a fresh 7-microsecond CTA per tile IS the cheapest
-// software pipeline here.
-template <int NT>
-__global__ void __launch_bounds__(32, PfbBleGeom<NT>::kCtasPerSm) k_pfb_ble_run(PfbBleArgs a) {
-    using B = PfbBleGeom<NT>;
-    using G = typename B::G;
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    float2* xs = reinterpret_cast<float2*>(smem_raw);
-    float4* V = reinterpret_cast<float4*>(smem_raw + B::kXsBytes);
-    uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + B::kXsBytes + B::kVBytes);
-
-    // grid = (CTAs per capture, captures); a CTA takes tiles_per_cta CONSECUTIVE tiles of its capture: no division anywhere,
-    // the source pointer advances by a constant
-    const int lane = threadIdx.x;
-    if (lane == 0) mbar_init(bar, 1);
-    __syncwarp();
-    const int cap = (int)blockIdx.y;
-    // measurement switch: the CTAs of one SM (block b lands on SM b % sm_count in the first wave) start a fraction of a tile
-    // apart, so that persistent warps do not run through their phases in step
-    if (a.stagger_ns > 0) __nanosleep((unsigned)(((blockIdx.x / (unsigned)a.sm_count) & 15u) * (unsigned)a.stagger_ns));
-    const int t0 = a.tile0 + (int)blockIdx.x * a.tiles_per_cta;
-    const int t1 = min(a.tile0 + a.n_tiles, t0 + a.tiles_per_cta);
-    const float2* src = a.x + (size_t)cap * a.stride + ((int64_t)kPfbD * B::kStride * t0 - G::kHist);
-    pfb_stage_tile_bulk<G, kChunkT>(xs, src, bar, lane);
-    uint32_t parity = 0;
-#pragma unroll 1
-    for (int tile = t0; tile < t1; tile++) {
-        mbar_wait(bar, parity);
-        parity ^= 1u;
-        src += kPfbD * B::kStride;
-        const bool more = tile + 1 < t1;
-        pfb_ble_tile<NT, false>(a, xs, V, lane, cap, B::kStride * tile, [&] {
-            if (more) {
-                asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");  // generic reads before the async-proxy writes
-                pfb_stage_tile_bulk<G, kChunkT>(xs, src, bar, lane);
-            }
-        });
-        __syncwarp();                                            // V and the quantised values of this tile are done with
-    }
+    pfb_ble_tile<NT, DEBUG>(a, xs, V, lane, cap, g_first);
 }
 
 #endif  // __CUDACC__

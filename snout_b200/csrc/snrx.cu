@@ -16,12 +16,6 @@
 #ifndef SNRX_LANES
 #define SNRX_LANES 2
 #endif
-#ifndef SNRX_BACK_BPS_DEFAULT
-#define SNRX_BACK_BPS_DEFAULT 8
-#endif
-#ifndef SNRX_PFB_TILES_DEFAULT
-#define SNRX_PFB_TILES_DEFAULT 0
-#endif
 #include "ble_adv.cuh"
 #include "ble_aux.cuh"
 #include "ble_coded.cuh"
@@ -88,7 +82,7 @@ struct Lane {
     ZbState zb;
     std::vector<cudaEvent_t> ev_chunks;
     // the BLE back-end parameters of the lane's last batch (snrx_ble_follow searches its bit streams again)
-    BleParams last_p{}; BitsLayout last_lay{}; uint32_t last_chunks = 0; bool last_ble = false;
+    BleParams last_p{}; BitsLayout last_lay{}; bool last_ble = false;
 };
 
 struct snrx_handle {
@@ -102,15 +96,13 @@ struct snrx_handle {
     snrx_zbmac_t* d_zbmac = nullptr;
     snrx_conn_t* d_conn = nullptr; uint32_t *d_conn_flags = nullptr, *d_conn_offsets = nullptr, *d_conn_scratch = nullptr;
     snrx_frame_t* d_follow = nullptr;    // frames of snrx_ble_follow
-    // snrx_ble_aux, allocated by its first call: the list (max_frames entries), flags / offsets / scan scratch of a round, and
-    // the whitening sequences continued to 260 bytes
-    snrx_ble_aux_t* d_aux = nullptr; uint32_t *d_aux_flags = nullptr, *d_aux_offsets = nullptr, *d_aux_scratch = nullptr;
+    // the lists of snrx_ble_aux and snrx_ble_coded (max_frames entries each), allocated by their first call; and what the
+    // pointer rounds of both share, allocated by the first of either: flags / offsets / scan scratch of a round and the
+    // whitening sequences continued to 260 bytes.  Neither list outlives its call (each is copied out before it returns).
+    snrx_ble_aux_t* d_aux = nullptr;
+    snrx_ble_coded_t* d_coded = nullptr;
+    uint32_t *d_round_flags = nullptr, *d_round_offsets = nullptr, *d_round_scratch = nullptr;
     uint8_t* d_aux_whiten = nullptr;
-    // snrx_ble_coded, allocated by its first call: the list (max_frames entries) with its round buffers, the scan's per-tile
-    // counts / offsets / scan scratch (grown to the batch's tile count), and its own whitening sequences
-    snrx_ble_coded_t* d_coded = nullptr; uint32_t *d_coded_flags = nullptr, *d_coded_offsets = nullptr, *d_coded_scratch = nullptr;
-    uint32_t *d_coded_tcounts = nullptr, *d_coded_toffsets = nullptr, *d_coded_tscratch = nullptr; uint32_t coded_tiles_cap = 0;
-    uint8_t* d_coded_whiten = nullptr;
     snrx::DevSlot* d_devtab = nullptr;
     snrx_device_t* d_devout = nullptr;
     uint32_t* d_adv_counters = nullptr;   // [0] records summarised (BLE), [1] new devices, [2] dropped (table full), [3] export count
@@ -246,62 +238,22 @@ static AaTables aa_tables_of(const BleParams& p) {
     return make_aa_tables(p.aa, p.aa_mask & ~((1u << z) - 1u));
 }
 
-// blocks per SM of the BLE back-end kernels (see process_impl)
-static int back_bps() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("SNRX_BACK_BPS"); v = e ? atoi(e) : SNRX_BACK_BPS_DEFAULT; if (v < 1) v = 1; if (v > 8) v = 8; }
-    return v;
-}
-
-// tiles per CTA of the persistent interior-tile kernel; 0 = every tile through the one-tile kernel (SNRX_PFB_TILES overrides, A/B runs)
-static int pfb_tiles_per_cta() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("SNRX_PFB_TILES"); v = e ? atoi(e) : SNRX_PFB_TILES_DEFAULT; if (v < 0) v = 0; }
-    return v;
-}
-
 template <int NT>
 static int pfb_ble_go(snrx_handle* h, const PfbBleArgs* a, cudaStream_t st, uint32_t caps) {
     using B = PfbBleGeom<NT>;
-    using G = typename B::G;
     if (!a) {
         CK(cudaFuncSetAttribute(k_pfb_ble<NT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, B::kSmemBytes));
         CK(cudaFuncSetAttribute(k_pfb_ble<NT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, B::kSmemBytes));
-        CK(cudaFuncSetAttribute(k_pfb_ble_run<NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, B::kSmemBytes));
         CK(cudaFuncSetAttribute(k_pfb_ble<NT, false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        CK(cudaFuncSetAttribute(k_pfb_ble_run<NT>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         return SNRX_OK;
     }
-    PfbBleArgs args = *a;
-    args.n_caps = (int32_t)caps;
-    args.tiles_per_cta = 1; args.stagger_ns = 0; args.sm_count = h->sm_count;
-    const bool dbg = (h->cfg.flags & SNRX_F_KEEP_STREAMS) != 0;
-    auto one_tile = [&](int t0, int t1) {                       // tiles [t0, t1) of every capture, one per CTA, any position
-        if (t1 <= t0) return;
-        PfbBleArgs b = args;
-        b.tile0 = t0; b.n_tiles = t1 - t0;
-        const dim3 grid((unsigned)(t1 - t0), caps);             // x: tiles, y: captures (snrx_create bounds max_captures by 65535)
-        if (dbg) k_pfb_ble<NT, true><<<grid, B::kThreads, B::kSmemBytes, st>>>(b);
-        else k_pfb_ble<NT, false><<<grid, B::kThreads, B::kSmemBytes, st>>>(b);
-        h->launches++;
-    };
-    const int t0 = a->tile0, t1 = a->tile0 + a->n_tiles, per = pfb_tiles_per_cta();
-    // interior tiles: 24 * 31 * tile - kHist >= 0 and ... + kTileIn <= n_in
-    const int64_t step = (int64_t)kPfbD * B::kStride;
-    int lo = (int)((G::kHist + step - 1) / step);
-    int hi = a->n_in >= G::kTileIn ? (int)((a->n_in - G::kTileIn + G::kHist) / step) + 1 : 0;          // first tile past the interior
-    lo = std::max(lo, t0); hi = std::min(hi, t1);
-    if (dbg || per == 0 || hi - lo < 4 * per) { one_tile(t0, t1); return SNRX_OK; }
-    one_tile(t0, lo);
-    {
-        PfbBleArgs b = args;
-        b.tile0 = lo; b.n_tiles = hi - lo; b.tiles_per_cta = per;
-        { static const int ns = getenv("SNRX_PFB_STAGGER_NS") ? atoi(getenv("SNRX_PFB_STAGGER_NS")) : 0; b.stagger_ns = ns; b.sm_count = h->sm_count; }
-        const dim3 grid((unsigned)((hi - lo + per - 1) / per), caps);
-        k_pfb_ble_run<NT><<<grid, B::kThreads, B::kSmemBytes, st>>>(b);
-        h->launches++;
-    }
-    one_tile(hi, t1);
+    if (a->n_tiles <= 0) return SNRX_OK;
+    PfbBleArgs b = *a;
+    b.n_caps = (int32_t)caps;
+    const dim3 grid((unsigned)b.n_tiles, caps);                 // x: tiles, y: captures (snrx_create bounds max_captures by 65535)
+    if (h->cfg.flags & SNRX_F_KEEP_STREAMS) k_pfb_ble<NT, true><<<grid, B::kThreads, B::kSmemBytes, st>>>(b);
+    else k_pfb_ble<NT, false><<<grid, B::kThreads, B::kSmemBytes, st>>>(b);
+    h->launches++;
     return SNRX_OK;
 }
 static int pfb_ble_dispatch(snrx_handle* h, const PfbBleArgs* a, cudaStream_t st, uint32_t caps) {
@@ -464,9 +416,7 @@ void snrx_destroy(snrx_t* h) {
     if (h->xchg.h_hdr) cudaFreeHost(h->xchg.h_hdr);
     if (h->adv_stream) { cudaStreamSynchronize(h->adv_stream); cudaStreamDestroy(h->adv_stream); }
     { void* ab[] = {h->d_adv, h->d_zbmac, h->d_conn, h->d_conn_flags, h->d_conn_offsets, h->d_conn_scratch, h->d_follow, h->d_devtab, h->d_devout, h->d_adv_counters,
-                    h->d_aux, h->d_aux_flags, h->d_aux_offsets, h->d_aux_scratch, h->d_aux_whiten,
-                    h->d_coded, h->d_coded_flags, h->d_coded_offsets, h->d_coded_scratch, h->d_coded_tcounts, h->d_coded_toffsets,
-                    h->d_coded_tscratch, h->d_coded_whiten}; for (void* b : ab) if (b) cudaFree(b); }
+                    h->d_aux, h->d_coded, h->d_round_flags, h->d_round_offsets, h->d_round_scratch, h->d_aux_whiten}; for (void* b : ab) if (b) cudaFree(b); }
     delete h;
 }
 
@@ -723,6 +673,40 @@ static bool bits_outside_clear(const uint32_t* words, uint64_t n_streams, uint32
     return true;
 }
 
+// The BLE back end over a lane's bit streams, on stream st: access-address search -> scan -> candidate fill -> decode ->
+// resolve (count per window) -> scan -> resolve (write) into `frames` (frame_cap records).  snrx_process runs it on the
+// batch's streams, snrx_ble_follow again on the polled batch's streams with another address.  The kernels use grid-stride
+// loops, so the grids set the speed, not the result: 8 blocks per SM of the grid-limited kernels.  MEASURED
+// (tools/ab_serial.py, ms per step with two batches queued): 8 blocks 0.404 | 4 blocks 0.402 | 2 blocks 0.422 | 1 block
+// 0.471 -- smaller grids do not give the next batch's channelizer more of the machine, they only stretch the latency-bound
+// chain search -> scan -> fill -> decode -> resolve -> export until it no longer fits beside one channelizer launch.
+struct BackTotals {
+    const uint32_t* frames;       // device: frames the chain found (may exceed frame_cap: the list then holds frame_cap)
+    const uint32_t* cands;        // device: access-address candidates (may exceed cand_cap)
+};
+static int launch_ble_back(snrx_handle* h, Lane& ln, const BleParams& p, const BitsLayout& lay, snrx_frame_t* frames,
+                           cudaStream_t st, BackTotals* tot) {
+    const uint32_t n_chunks = div_up(lay.words_per_stream, 32);
+    const uint32_t aa_items = p.n_captures * h->n_ble_ch * n_chunks;
+    const uint32_t w_items = p.n_captures * h->n_ble_ch * (uint32_t)p.n_windows;
+    k_aa_search<<<grid_for(h, aa_items, 8, 8), 256, 0, st>>>(ln.d_bits, lay, p, n_chunks, ln.d_counts, ln.d_hits, aa_tables_of(p));
+    h->launches += 1 + exclusive_scan(ln.d_counts, aa_items, ln.d_offsets, ln.d_scratch, st);
+    k_aa_fill<<<grid_for(h, aa_items, 256, 8), 256, 0, st>>>(ln.d_bits, ln.d_hits, lay, p, n_chunks, ln.d_counts, ln.d_offsets, ln.d_cands, h->cand_cap);
+    k_ble_decode<<<h->sm_count * 16, 128, 0, st>>>(ln.d_bits, lay, p, ln.d_offsets + aa_items, h->cand_cap, ln.d_cands,
+                                               ln.d_decs, h->d_crc_tab, h->d_whiten, h->d_ble_channels);
+    const int g_w = grid_for(h, w_items, 256, 8);
+    k_ble_resolve<false><<<g_w, 256, 0, st>>>(ln.d_cands, ln.d_decs, ln.d_offsets, n_chunks, p, ln.d_wcounts, nullptr,
+                                             nullptr, 0, h->d_ble_channels, h->cand_cap);
+    h->launches += 3 + exclusive_scan(ln.d_wcounts, w_items, ln.d_woffsets, ln.d_scratch, st);
+    k_ble_resolve<true><<<g_w, 256, 0, st>>>(ln.d_cands, ln.d_decs, ln.d_offsets, n_chunks, p, ln.d_wcounts, ln.d_woffsets,
+                                            frames, h->frame_cap, h->d_ble_channels, h->cand_cap);
+    h->launches += 1;
+    CK(cudaGetLastError());
+    tot->frames = ln.d_woffsets + w_items;
+    tot->cands = ln.d_offsets + aa_items;
+    return SNRX_OK;
+}
+
 // bits != nullptr: snrx_debug_process_bits -- the BLE slicer words are given (host memory, SNRX_STAGE_BLE_BITS layout)
 // instead of computed from iq; no input is staged and no front end runs.  Everything from the back end on is shared.
 static int process_impl(snrx_t* h, const void* iq, int fmt, uint32_t n_captures, uint64_t n_samples, uint64_t stride_samples,
@@ -884,35 +868,12 @@ static int process_impl(snrx_t* h, const void* iq, int fmt, uint32_t n_captures,
         p.first_capture = first_capture;
         p.n_captures = n_captures;
         p.n_channels = h->n_ble_ch;
-        const uint32_t n_chunks = div_up(lay.words_per_stream, 32);
-        ln.last_p = p; ln.last_lay = lay; ln.last_chunks = n_chunks; ln.last_ble = true;
-        const uint32_t aa_items = n_captures * h->n_ble_ch * n_chunks;
-        const uint32_t w_items = n_captures * h->n_ble_ch * (uint32_t)p.n_windows;
-
-        // Blocks per SM of the back-end kernels: SNRX_BACK_BPS.  MEASURED (tools/ab_serial.py, ms per step with two batches
-        // queued): 8 blocks 0.404 | 4 blocks 0.402 | 2 blocks 0.422 | 1 block 0.471 -- smaller grids do not give the next
-        // batch's channelizer more of the machine, they only stretch the latency-bound chain search -> scan -> fill ->
-        // decode -> resolve -> export until it no longer fits beside one channelizer launch.
-        const int g_aa = grid_for(h, aa_items, 8, back_bps());
-#ifdef SNRX_PROBE_SKIP_BACK                                  // measurement builds only: no candidates, hence no back-end work (a step then
-        CK(cudaMemsetAsync(ln.d_counts, 0, sizeof(uint32_t) * aa_items, st));     // takes 0.345 ms instead of 0.397: DESIGN.md 6)
-#else
-        k_aa_search<<<g_aa, 256, 0, st>>>(ln.d_bits, lay, p, n_chunks, ln.d_counts, ln.d_hits, aa_tables_of(p));
-#endif
-        h->launches += 1 + exclusive_scan(ln.d_counts, aa_items, ln.d_offsets, ln.d_scratch, st);
-        k_aa_fill<<<grid_for(h, aa_items, 256, back_bps()), 256, 0, st>>>(ln.d_bits, ln.d_hits, lay, p, n_chunks, ln.d_counts, ln.d_offsets, ln.d_cands, h->cand_cap);
-        k_ble_decode<<<h->sm_count * 16, 128, 0, st>>>(ln.d_bits, lay, p, ln.d_offsets + aa_items, h->cand_cap, ln.d_cands,
-                                                   ln.d_decs, h->d_crc_tab, h->d_whiten, h->d_ble_channels);
-        const int g_w = grid_for(h, w_items, 256, back_bps());
-        k_ble_resolve<false><<<g_w, 256, 0, st>>>(ln.d_cands, ln.d_decs, ln.d_offsets, n_chunks, p, ln.d_wcounts, nullptr,
-                                                 nullptr, 0, h->d_ble_channels, h->cand_cap);
-        h->launches += 3 + exclusive_scan(ln.d_wcounts, w_items, ln.d_woffsets, ln.d_scratch, st);
-        k_ble_resolve<true><<<g_w, 256, 0, st>>>(ln.d_cands, ln.d_decs, ln.d_offsets, n_chunks, p, ln.d_wcounts, ln.d_woffsets,
-                                                ln.d_frames, h->frame_cap, h->d_ble_channels, h->cand_cap);
-        h->launches += 1;
-        CK(cudaGetLastError());
-        CK(cudaMemcpyAsync(ln.d_totals + 0, ln.d_woffsets + w_items, sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
-        CK(cudaMemcpyAsync(ln.d_totals + 1, ln.d_offsets + aa_items, sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
+        ln.last_p = p; ln.last_lay = lay; ln.last_ble = true;
+        BackTotals tot{};
+        int r = launch_ble_back(h, ln, p, lay, ln.d_frames, st, &tot);
+        if (r != SNRX_OK) return r;
+        CK(cudaMemcpyAsync(ln.d_totals + 0, tot.frames, sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
+        CK(cudaMemcpyAsync(ln.d_totals + 1, tot.cands, sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
     }
     if (h->has_zb && !h->has_ble) {
         CK(cudaEventRecord(ln.ev_handoff, st));        // Zigbee only: front end and chains all on the tail stream
@@ -1140,40 +1101,113 @@ int snrx_ble_connections(snrx_t* h, snrx_conn_t* out, uint32_t cap, uint32_t* n_
     return SNRX_OK;
 }
 
+}  // extern "C"
+
+// The lane of the polled batch, for the calls that search its BLE bit streams again (snrx_ble_follow, snrx_ble_aux,
+// snrx_ble_coded): it must hold BLE streams -- of a wideband mode if `wideband` -- that no later batch has overwritten.
+static int polled_bits_lane(snrx_handle* h, const char* name, bool wideband, Lane** out) {
+    const std::string n = name;
+    if (h->polled_lane < 0) return fail(h, SNRX_ESTATE, (n + " needs a polled batch").c_str());
+    Lane& ln = h->lane[h->polled_lane];
+    if (!h->has_ble || (wideband && !h->wideband) || !ln.last_ble)
+        return fail(h, SNRX_ESTATE, (n + (wideband ? ": the polled batch has no wideband BLE bit streams" : ": the polled batch has no BLE bit streams")).c_str());
+    if (ln.pending) return fail(h, SNRX_ESTATE, (n + ": the batch's bit streams have been overwritten (call before the second-next snrx_process)").c_str());
+    *out = &ln;
+    return SNRX_OK;
+}
+
+// the polled lane's bit streams as the pointer rounds read them
+static AuxGeom aux_geom_of(const Lane& ln) {
+    const BleParams& p = ln.last_p;
+    AuxGeom g{};
+    g.bits = ln.d_bits; g.lay = ln.last_lay; g.n_out = p.n_out;
+    g.base = (int64_t)kWindow * p.first_window - p.m_origin;
+    g.first_capture = p.first_capture; g.n_captures = p.n_captures;
+    return g;
+}
+
+// what the pointer rounds of snrx_ble_aux and snrx_ble_coded share, allocated by the first call of either
+static int round_buffers_init(snrx_handle* h) {
+    if (h->d_aux_whiten) return SNRX_OK;
+    CK(cudaMalloc((void**)&h->d_round_flags, sizeof(uint32_t) * ((size_t)h->frame_cap + 1)));
+    CK(cudaMalloc((void**)&h->d_round_offsets, sizeof(uint32_t) * ((size_t)h->frame_cap + 1)));
+    CK(cudaMalloc((void**)&h->d_round_scratch, sizeof(uint32_t) * scan_scratch_items(h->frame_cap)));
+    std::vector<uint8_t> wh(40 * SNRX_AUX_MAX_BYTES);
+    for (int ch = 0; ch < 40; ch++) make_whiten_bytes(ch, wh.data() + ch * SNRX_AUX_MAX_BYTES, SNRX_AUX_MAX_BYTES);
+    CK(cudaMalloc((void**)&h->d_aux_whiten, wh.size()));
+    CK(cudaMemcpy(h->d_aux_whiten, wh.data(), wh.size(), cudaMemcpyHostToDevice));
+    return SNRX_OK;
+}
+
+// The pointer rounds of snrx_ble_aux and snrx_ble_coded, one per depth: the pointers of depth d come from the entries of
+// depth d - 1, src are those of the first round.  Appends to `list` from *total on, up to the list kind's maximum depth, and
+// leaves the list's length in *total; SNRX_EOVERFLOW with `overflow` if it would pass max_frames.
+template <int L>
+static int run_pointer_rounds(snrx_handle* h, AuxSrcT<L> src, AuxEntry<L>* list, const AuxGeom& g, cudaStream_t st,
+                              uint32_t* total, const char* overflow) {
+    const AaTables tabs = make_aa_tables(kAuxAdvAa, 0xFFFFFFFFu);
+    const uint32_t crc_init = crc_init_internal(0x555555u);
+    uint32_t t = *total;
+    while (src.n > 0 && src.depth <= AuxKind<L>::kMaxDepth + 1) {
+        k_ble_aux_flag<<<div_up(src.n, 256), 256, 0, st>>>(src, h->d_round_flags);
+        exclusive_scan(h->d_round_flags, src.n, h->d_round_offsets, h->d_round_scratch, st);
+        uint32_t m = 0;
+        CK(cudaMemcpyAsync(&m, h->d_round_offsets + src.n, sizeof m, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        if (m == 0) break;
+        if ((uint64_t)t + m > h->frame_cap) return fail(h, SNRX_EOVERFLOW, overflow);
+        k_ble_aux_fill<<<div_up(src.n, 256), 256, 0, st>>>(src, h->d_round_flags, h->d_round_offsets, list, t, g);
+        const int gs = grid_for(h, m, 4, 8);
+        k_ble_aux_search<L><<<gs, 128, 0, st>>>(list, t, t + m, g, h->d_crc_tab, h->d_aux_whiten, crc_init, tabs);
+        if constexpr (AuxKind<L>::kCoded) {
+            const CodedTables ct = make_coded_tables();
+            k_ble_coded_window<<<gs, 128, 0, st>>>(list, t, t + m, g, ct);
+            k_ble_coded_decode<<<grid_for(h, m, kCodedGroups, 8), 8 * kCodedGroups, 0, st>>>(list, t, t + m, g, ct, h->d_crc_tab,
+                                                                                              h->d_aux_whiten, crc_init);
+        }
+        k_ble_aux_first<L><<<grid_for(h, m, 8, 8), 256, 0, st>>>(list, t, t + m);
+        CK(cudaGetLastError());
+        src.frames = nullptr; src.first = t; src.n = m; src.depth++;
+        t += m;
+    }
+    *total = t;
+    return SNRX_OK;
+}
+
+// *n_out = total; the list's entries into out (cap entries) if asked for
+template <class E>
+static int copy_list_out(snrx_handle* h, const char* name, const E* list, uint32_t total, E* out, uint32_t cap, uint32_t* n_out,
+                         cudaStream_t st) {
+    if (n_out) *n_out = total;
+    if (out && total) {
+        if (cap < total) return fail(h, SNRX_ERANGE, (std::string(name) + ": buffer smaller than the list").c_str());
+        CK(cudaMemcpyAsync(out, list, sizeof(E) * (size_t)total, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+    }
+    return SNRX_OK;
+}
+
+extern "C" {
+
 int snrx_ble_follow(snrx_t* h, uint32_t access_addr, uint32_t crc_init, snrx_frame_t* out, uint32_t cap, uint32_t* n_out) {
     if (!h) return SNRX_EINVAL;
-    if (h->polled_lane < 0) return fail(h, SNRX_ESTATE, "snrx_ble_follow needs a polled batch");
-    Lane& ln = h->lane[h->polled_lane];
-    if (!h->has_ble || !ln.last_ble) return fail(h, SNRX_ESTATE, "snrx_ble_follow: the polled batch has no BLE bit streams");
-    if (ln.pending) return fail(h, SNRX_ESTATE, "snrx_ble_follow: the batch's bit streams have been overwritten (call before the second-next snrx_process)");
+    Lane* ln = nullptr;
+    int r = polled_bits_lane(h, "snrx_ble_follow", false, &ln);
+    if (r != SNRX_OK) return r;
     if (access_addr == 0u) return fail(h, SNRX_EINVAL, "snrx_ble_follow: access_addr must have a bit set (see snrx_create)");
     CK(cudaSetDevice(h->device));
     if (!h->d_follow) CK(cudaMalloc((void**)&h->d_follow, sizeof(snrx_frame_t) * (size_t)h->frame_cap));
-    cudaStream_t st = ln.tail;                                   // the lane is idle: its working set and streams are free
-    BleParams p = ln.last_p;
+    cudaStream_t st = ln->tail;                                  // the lane is idle: its working set and streams are free
+    BleParams p = ln->last_p;
     p.aa = access_addr;
     p.aa_mask = 0xFFFFFFFFu;
     p.crc_init_internal = crc_init_internal(crc_init);
-    const BitsLayout lay = ln.last_lay;
-    const uint32_t n_chunks = ln.last_chunks;
-    const uint32_t aa_items = p.n_captures * h->n_ble_ch * n_chunks;
-    const uint32_t w_items = p.n_captures * h->n_ble_ch * (uint32_t)p.n_windows;
-    const int g_aa = grid_for(h, aa_items, 8, 8);
-    k_aa_search<<<g_aa, 256, 0, st>>>(ln.d_bits, lay, p, n_chunks, ln.d_counts, ln.d_hits, aa_tables_of(p));
-    exclusive_scan(ln.d_counts, aa_items, ln.d_offsets, ln.d_scratch, st);
-    k_aa_fill<<<grid_for(h, aa_items, 256, 8), 256, 0, st>>>(ln.d_bits, ln.d_hits, lay, p, n_chunks, ln.d_counts, ln.d_offsets, ln.d_cands, h->cand_cap);
-    k_ble_decode<<<h->sm_count * 2, 128, 0, st>>>(ln.d_bits, lay, p, ln.d_offsets + aa_items, h->cand_cap, ln.d_cands,
-                                               ln.d_decs, h->d_crc_tab, h->d_whiten, h->d_ble_channels);
-    const int g_w = grid_for(h, w_items, 256, 8);
-    k_ble_resolve<false><<<g_w, 256, 0, st>>>(ln.d_cands, ln.d_decs, ln.d_offsets, n_chunks, p, ln.d_wcounts, nullptr,
-                                             nullptr, 0, h->d_ble_channels, h->cand_cap);
-    exclusive_scan(ln.d_wcounts, w_items, ln.d_woffsets, ln.d_scratch, st);
-    k_ble_resolve<true><<<g_w, 256, 0, st>>>(ln.d_cands, ln.d_decs, ln.d_offsets, n_chunks, p, ln.d_wcounts, ln.d_woffsets,
-                                            h->d_follow, h->frame_cap, h->d_ble_channels, h->cand_cap);
-    CK(cudaGetLastError());
+    BackTotals dev{};
+    r = launch_ble_back(h, *ln, p, ln->last_lay, h->d_follow, st, &dev);
+    if (r != SNRX_OK) return r;
     uint32_t tot[2] = {0, 0};
-    CK(cudaMemcpyAsync(&tot[0], ln.d_woffsets + w_items, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(&tot[1], ln.d_offsets + aa_items, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&tot[0], dev.frames, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&tot[1], dev.cands, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     if (tot[1] > h->cand_cap) return fail(h, SNRX_EOVERFLOW, "access-address candidates exceed capacity (raise max_frames)");
     if (tot[0] > h->frame_cap) return fail(h, SNRX_EOVERFLOW, "frames exceed max_frames");
@@ -1188,140 +1222,62 @@ int snrx_ble_follow(snrx_t* h, uint32_t access_addr, uint32_t crc_init, snrx_fra
 int snrx_ble_aux(snrx_t* h, snrx_ble_aux_t* out, uint32_t cap, uint32_t* n_out) {
     if (!h) return SNRX_EINVAL;
     if (n_out) *n_out = 0;
-    if (h->polled_lane < 0) return fail(h, SNRX_ESTATE, "snrx_ble_aux needs a polled batch");
-    Lane& ln = h->lane[h->polled_lane];
-    if (!h->has_ble || !h->wideband || !ln.last_ble) return fail(h, SNRX_ESTATE, "snrx_ble_aux: the polled batch has no wideband BLE bit streams");
-    if (ln.pending) return fail(h, SNRX_ESTATE, "snrx_ble_aux: the batch's bit streams have been overwritten (call before the second-next snrx_process)");
+    Lane* ln = nullptr;
+    int r = polled_bits_lane(h, "snrx_ble_aux", true, &ln);
+    if (r != SNRX_OK) return r;
     CK(cudaSetDevice(h->device));
-    if (!h->d_aux) {
-        CK(cudaMalloc((void**)&h->d_aux, sizeof(snrx_ble_aux_t) * (size_t)h->frame_cap));
-        CK(cudaMalloc((void**)&h->d_aux_flags, sizeof(uint32_t) * ((size_t)h->frame_cap + 1)));
-        CK(cudaMalloc((void**)&h->d_aux_offsets, sizeof(uint32_t) * ((size_t)h->frame_cap + 1)));
-        CK(cudaMalloc((void**)&h->d_aux_scratch, sizeof(uint32_t) * scan_scratch_items(h->frame_cap)));
-        std::vector<uint8_t> wh(40 * SNRX_AUX_MAX_BYTES);
-        for (int ch = 0; ch < 40; ch++) make_whiten_bytes(ch, wh.data() + ch * SNRX_AUX_MAX_BYTES, SNRX_AUX_MAX_BYTES);
-        CK(cudaMalloc((void**)&h->d_aux_whiten, wh.size()));
-        CK(cudaMemcpy(h->d_aux_whiten, wh.data(), wh.size(), cudaMemcpyHostToDevice));
-    }
-    cudaStream_t st = ln.tail;                                   // the lane is idle: its bit streams stay as the batch left them
-    const BleParams& p = ln.last_p;
-    AuxGeom g{};
-    g.bits = ln.d_bits; g.lay = ln.last_lay; g.n_out = p.n_out;
-    g.base = (int64_t)kWindow * p.first_window - p.m_origin;
-    g.first_capture = p.first_capture; g.n_captures = p.n_captures;
-    const AaTables tabs = make_aa_tables(kAuxAdvAa, 0xFFFFFFFFu);
-    const uint32_t crc_init = crc_init_internal(0x555555u);
-    AuxSrc src{};
-    src.frames = h->polled_frames_dev; src.list = h->d_aux; src.first = 0; src.n = ln.n_frames; src.depth = 0;
+    if ((r = round_buffers_init(h)) != SNRX_OK) return r;
+    if (!h->d_aux) CK(cudaMalloc((void**)&h->d_aux, sizeof(snrx_ble_aux_t) * (size_t)h->frame_cap));
+    cudaStream_t st = ln->tail;                                  // the lane is idle: its bit streams stay as the batch left them
+    AuxSrc src{};                                                // depth 0: the pointers of the polled records
+    src.frames = h->polled_frames_dev; src.list = h->d_aux; src.first = 0; src.n = ln->n_frames; src.depth = 0;
     uint32_t total = 0;
-    // one round per depth: the pointers of depth d come from the entries of depth d - 1 (the records at d = 0)
-    while (src.n > 0 && src.depth <= SNRX_AUX_MAX_DEPTH + 1) {
-        k_ble_aux_flag<<<div_up(src.n, 256), 256, 0, st>>>(src, h->d_aux_flags);
-        exclusive_scan(h->d_aux_flags, src.n, h->d_aux_offsets, h->d_aux_scratch, st);
-        uint32_t m = 0;
-        CK(cudaMemcpyAsync(&m, h->d_aux_offsets + src.n, sizeof m, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        if (m == 0) break;
-        if ((uint64_t)total + m > h->frame_cap) return fail(h, SNRX_EOVERFLOW, "snrx_ble_aux: more auxiliary pointers than max_frames");
-        k_ble_aux_fill<<<div_up(src.n, 256), 256, 0, st>>>(src, h->d_aux_flags, h->d_aux_offsets, h->d_aux, total, g);
-        const int gs = grid_for(h, m, 4, 8);
-        k_ble_aux_search<kAuxList><<<gs, 128, 0, st>>>(h->d_aux, total, total + m, g, h->d_crc_tab, h->d_aux_whiten, crc_init, tabs);
-        k_ble_aux_first<kAuxList><<<grid_for(h, m, 8, 8), 256, 0, st>>>(h->d_aux, total, total + m);
-        CK(cudaGetLastError());
-        src.frames = nullptr; src.first = total; src.n = m; src.depth++;
-        total += m;
-    }
-    if (n_out) *n_out = total;
-    if (out && total) {
-        if (cap < total) return fail(h, SNRX_ERANGE, "snrx_ble_aux: buffer smaller than the list");
-        CK(cudaMemcpyAsync(out, h->d_aux, sizeof(snrx_ble_aux_t) * (size_t)total, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-    }
-    return SNRX_OK;
+    r = run_pointer_rounds(h, src, h->d_aux, aux_geom_of(*ln), st, &total, "snrx_ble_aux: more auxiliary pointers than max_frames");
+    if (r != SNRX_OK) return r;
+    return copy_list_out(h, "snrx_ble_aux", h->d_aux, total, out, cap, n_out, st);
 }
 
 int snrx_ble_coded(snrx_t* h, snrx_ble_coded_t* out, uint32_t cap, uint32_t* n_out) {
     if (!h) return SNRX_EINVAL;
     if (n_out) *n_out = 0;
-    if (h->polled_lane < 0) return fail(h, SNRX_ESTATE, "snrx_ble_coded needs a polled batch");
-    Lane& ln = h->lane[h->polled_lane];
-    if (!h->has_ble || !h->wideband || !ln.last_ble) return fail(h, SNRX_ESTATE, "snrx_ble_coded: the polled batch has no wideband BLE bit streams");
-    if (ln.pending) return fail(h, SNRX_ESTATE, "snrx_ble_coded: the batch's bit streams have been overwritten (call before the second-next snrx_process)");
+    Lane* ln = nullptr;
+    int r = polled_bits_lane(h, "snrx_ble_coded", true, &ln);
+    if (r != SNRX_OK) return r;
     CK(cudaSetDevice(h->device));
-    if (!h->d_coded) {
-        CK(cudaMalloc((void**)&h->d_coded, sizeof(snrx_ble_coded_t) * (size_t)h->frame_cap));
-        CK(cudaMalloc((void**)&h->d_coded_flags, sizeof(uint32_t) * ((size_t)h->frame_cap + 1)));
-        CK(cudaMalloc((void**)&h->d_coded_offsets, sizeof(uint32_t) * ((size_t)h->frame_cap + 1)));
-        CK(cudaMalloc((void**)&h->d_coded_scratch, sizeof(uint32_t) * scan_scratch_items(h->frame_cap)));
-        std::vector<uint8_t> wh(40 * SNRX_AUX_MAX_BYTES);
-        for (int ch = 0; ch < 40; ch++) make_whiten_bytes(ch, wh.data() + ch * SNRX_AUX_MAX_BYTES, SNRX_AUX_MAX_BYTES);
-        CK(cudaMalloc((void**)&h->d_coded_whiten, wh.size()));
-        CK(cudaMemcpy(h->d_coded_whiten, wh.data(), wh.size(), cudaMemcpyHostToDevice));
-    }
-    const BleParams& p = ln.last_p;
+    if ((r = round_buffers_init(h)) != SNRX_OK) return r;
+    if (!h->d_coded) CK(cudaMalloc((void**)&h->d_coded, sizeof(snrx_ble_coded_t) * (size_t)h->frame_cap));
+    const BleParams& p = ln->last_p;
     CodedGeom cg{};
-    AuxGeom& g = cg.g;
-    g.bits = ln.d_bits; g.lay = ln.last_lay; g.n_out = p.n_out;
-    g.base = (int64_t)kWindow * p.first_window - p.m_origin;
-    g.first_capture = p.first_capture; g.n_captures = p.n_captures;
+    cg.g = aux_geom_of(*ln);
     cg.body_lo = p.m_origin; cg.body_hi = p.m_origin + p.n_windows * kWindow;
     cg.tiles_per_stream = (uint32_t)div_up(p.n_out, kCodedTile);
     const uint32_t n_tiles = cg.tiles_per_stream * 3u * p.n_captures;
-    if (n_tiles + 1 > h->coded_tiles_cap) {
-        for (void* b : {(void*)h->d_coded_tcounts, (void*)h->d_coded_toffsets, (void*)h->d_coded_tscratch}) if (b) cudaFree(b);
-        h->coded_tiles_cap = n_tiles + 1;
-        CK(cudaMalloc((void**)&h->d_coded_tcounts, sizeof(uint32_t) * (size_t)h->coded_tiles_cap));
-        CK(cudaMalloc((void**)&h->d_coded_toffsets, sizeof(uint32_t) * (size_t)h->coded_tiles_cap));
-        CK(cudaMalloc((void**)&h->d_coded_tscratch, sizeof(uint32_t) * scan_scratch_items(h->coded_tiles_cap)));
-    }
-    cudaStream_t st = ln.tail;                                   // the lane is idle: its bit streams stay as the batch left them
+    cudaStream_t st = ln->tail;                                  // the lane is idle: its bit streams stay as the batch left them
     const CodedTables ct = make_coded_tables();
-    const AaTables tabs = make_aa_tables(kAuxAdvAa, 0xFFFFFFFFu);
     const uint32_t crc_init = crc_init_internal(0x555555u);
-    // the primaries: count per tile, offsets, then the entries in (capture, channel, sample) order, decoded
+    // the primaries: count per tile, offsets, then the entries in (capture, channel, sample) order, decoded.  The tile scan
+    // runs in the lane's access-address scan buffers, which sit idle once the batch is polled: n_tiles + 1 =
+    // 3 caps ceil(n_out / 2048) + 1 <= caps 40 ceil(bits_words_for(max_out) / 32) + 1 items of d_counts / d_offsets, and
+    // scan_scratch_items is monotonic, so d_scratch is large enough too.
     uint32_t total = 0;
     if (n_tiles) {
-        k_ble_coded_scan<false><<<n_tiles, kCodedScanThreads, 0, st>>>(cg, ct, h->d_coded_tcounts, nullptr, nullptr);
-        exclusive_scan(h->d_coded_tcounts, n_tiles, h->d_coded_toffsets, h->d_coded_tscratch, st);
-        CK(cudaMemcpyAsync(&total, h->d_coded_toffsets + n_tiles, sizeof total, cudaMemcpyDeviceToHost, st));
+        k_ble_coded_scan<false><<<n_tiles, kCodedScanThreads, 0, st>>>(cg, ct, ln->d_counts, nullptr, nullptr);
+        exclusive_scan(ln->d_counts, n_tiles, ln->d_offsets, ln->d_scratch, st);
+        CK(cudaMemcpyAsync(&total, ln->d_offsets + n_tiles, sizeof total, cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
         if (total > h->frame_cap) return fail(h, SNRX_EOVERFLOW, "snrx_ble_coded: more entries than max_frames");
         if (total) {
-            k_ble_coded_scan<true><<<n_tiles, kCodedScanThreads, 0, st>>>(cg, ct, h->d_coded_tcounts, h->d_coded_toffsets, h->d_coded);
-            k_ble_coded_decode<<<grid_for(h, total, kCodedGroups, 8), 8 * kCodedGroups, 0, st>>>(h->d_coded, 0, total, g, ct, h->d_crc_tab,
-                                                                                                h->d_coded_whiten, crc_init);
+            k_ble_coded_scan<true><<<n_tiles, kCodedScanThreads, 0, st>>>(cg, ct, ln->d_counts, ln->d_offsets, h->d_coded);
+            k_ble_coded_decode<<<grid_for(h, total, kCodedGroups, 8), 8 * kCodedGroups, 0, st>>>(h->d_coded, 0, total, cg.g, ct, h->d_crc_tab,
+                                                                                                h->d_aux_whiten, crc_init);
             CK(cudaGetLastError());
         }
     }
-    AuxSrcT<kCodedList> src{};
+    AuxSrcT<kCodedList> src{};                                   // depth 1: the pointers of the primaries
     src.frames = nullptr; src.list = h->d_coded; src.first = 0; src.n = total; src.depth = 1;
-    // one round per depth: the pointers of depth d come from the entries of depth d - 1 (the primaries at d = 1)
-    while (src.n > 0 && src.depth <= SNRX_CODED_MAX_DEPTH + 1) {
-        k_ble_aux_flag<<<div_up(src.n, 256), 256, 0, st>>>(src, h->d_coded_flags);
-        exclusive_scan(h->d_coded_flags, src.n, h->d_coded_offsets, h->d_coded_scratch, st);
-        uint32_t m = 0;
-        CK(cudaMemcpyAsync(&m, h->d_coded_offsets + src.n, sizeof m, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        if (m == 0) break;
-        if ((uint64_t)total + m > h->frame_cap) return fail(h, SNRX_EOVERFLOW, "snrx_ble_coded: more entries than max_frames");
-        k_ble_aux_fill<<<div_up(src.n, 256), 256, 0, st>>>(src, h->d_coded_flags, h->d_coded_offsets, h->d_coded, total, g);
-        const int gs = grid_for(h, m, 4, 8);
-        k_ble_aux_search<kCodedList><<<gs, 128, 0, st>>>(h->d_coded, total, total + m, g, h->d_crc_tab, h->d_coded_whiten, crc_init, tabs);
-        k_ble_coded_window<<<gs, 128, 0, st>>>(h->d_coded, total, total + m, g, ct);
-        k_ble_coded_decode<<<grid_for(h, m, kCodedGroups, 8), 8 * kCodedGroups, 0, st>>>(h->d_coded, total, total + m, g, ct, h->d_crc_tab,
-                                                                                          h->d_coded_whiten, crc_init);
-        k_ble_aux_first<kCodedList><<<grid_for(h, m, 8, 8), 256, 0, st>>>(h->d_coded, total, total + m);
-        CK(cudaGetLastError());
-        src.first = total; src.n = m; src.depth++;
-        total += m;
-    }
-    if (n_out) *n_out = total;
-    if (out && total) {
-        if (cap < total) return fail(h, SNRX_ERANGE, "snrx_ble_coded: buffer smaller than the list");
-        CK(cudaMemcpyAsync(out, h->d_coded, sizeof(snrx_ble_coded_t) * (size_t)total, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-    }
-    return SNRX_OK;
+    r = run_pointer_rounds(h, src, h->d_coded, cg.g, st, &total, "snrx_ble_coded: more entries than max_frames");
+    if (r != SNRX_OK) return r;
+    return copy_list_out(h, "snrx_ble_coded", h->d_coded, total, out, cap, n_out, st);
 }
 
 int snrx_zb_mac_summary(snrx_t* h, snrx_zbmac_t* out, uint32_t cap, uint32_t* n_out) {

@@ -61,6 +61,7 @@ class RxEngine:
         cfg.flags = (_abi.F_KEEP_STREAMS if keep_streams else 0) | (_abi.F_RF_METRICS if rf_metrics else 0)
         cfg.access_mask = access_mask & 0xFFFFFFFF
         self.cfg = cfg
+        self.max_frames = int(cfg.max_frames) or (1 << 17)     # records per batch; 1 << 17: the library default
         self.handle = c_void_p()
         rc = self.lib.snrx_create(byref(self.handle), byref(cfg))
         if rc != 0:
@@ -98,6 +99,14 @@ class RxEngine:
     def _check(self, rc: int):
         if rc != 0:
             raise SnrxError(rc, self.lib.snrx_strerror(rc).decode(), self.lib.snrx_last_error(self.handle).decode())
+
+    def _polled_list(self, fn, dtype, *args) -> np.ndarray:
+        """A list about the batch most recently returned by poll(): fn(handle, *args, out, cap, &n) of the C ABI, with
+        room for max_frames entries."""
+        n = c_uint32(0)
+        out = np.zeros(self.max_frames, dtype=dtype)
+        self._check(fn(self.handle, *args, out.ctypes.data_as(c_void_p), self.max_frames, byref(n)))
+        return out[: n.value].copy()
 
     # ------------------------------------------------------------------ control
     def set_channel(self, channel: int):
@@ -230,7 +239,7 @@ class RxEngine:
         sends over NVLink."""
         f, n = c_void_p(), c_uint32(0)
         self._check(self.lib.snrx_polled_frames_device(self.handle, byref(f), byref(n)))
-        return int(f.value or 0), int(self.cfg.max_frames) or (1 << 17), int(n.value)   # 1 << 17: the library default
+        return int(f.value or 0), self.max_frames, int(n.value)
 
     # ------------------------------------------------------------------ SURVEY 8(e): frame exchange between engines
     def exchange_create(self, rank: int, world: int, cap_records: int = 1 << 15) -> bytes:
@@ -254,7 +263,7 @@ class RxEngine:
         n = c_uint32(0)
         out, ptr, cap = None, None, 0
         if want_frames:
-            cap = (int(self.cfg.max_frames) or (1 << 17)) * self._xchg_world
+            cap = self.max_frames * self._xchg_world
             out = np.zeros(cap, dtype=FRAME_DTYPE)
             ptr = out.ctypes.data_as(c_void_p)
         rc = self.lib.snrx_allgather(self.handle, batch_no, ptr, cap, counts, byref(n), timeout_ms)
@@ -269,14 +278,10 @@ class RxEngine:
         returned by poll(), computed on the GPU from the HBM frame list; also folds the batch into the sender table.
         This is what Snout builds per btle_rx line (BtleMessage.fromraw -> BtlePDUPayload, message.py:205-237,
         advertising.py:113-307).  Call before the second-next process().  want=False only updates the table."""
-        n = c_uint32(0)
         if not want:
-            self._check(self.lib.snrx_ble_adv_summary(self.handle, None, 0, byref(n)))
+            self._check(self.lib.snrx_ble_adv_summary(self.handle, None, 0, byref(c_uint32(0))))
             return np.zeros(0, dtype=_abi.ADV_DTYPE)
-        cap = int(self.cfg.max_frames) or (1 << 17)
-        out = np.zeros(cap, dtype=_abi.ADV_DTYPE)
-        self._check(self.lib.snrx_ble_adv_summary(self.handle, out.ctypes.data_as(c_void_p), cap, byref(n)))
-        return out[: n.value].copy()
+        return self._polled_list(self.lib.snrx_ble_adv_summary, _abi.ADV_DTYPE)
 
     def devices(self, reset: bool = False) -> np.ndarray:
         """The sender table (one _abi.DEVICE_DTYPE row per (AdvA, TxAdd), sorted by address) accumulated over every
@@ -294,20 +299,12 @@ class RxEngine:
     def connections(self) -> np.ndarray:
         """The CRC-ok CONNECT_REQs (_abi.CONN_DTYPE: AA, CRCInit, ChM, Hop, Interval, ...) among the records of the batch most
         recently returned by poll(): what btle_rx -o starts tracking (btle_rx.c:1476-1557, 2167-2282)."""
-        n = c_uint32(0)
-        cap = int(self.cfg.max_frames) or (1 << 17)
-        out = np.zeros(cap, dtype=_abi.CONN_DTYPE)
-        self._check(self.lib.snrx_ble_connections(self.handle, out.ctypes.data_as(c_void_p), cap, byref(n)))
-        return out[: n.value].copy()
+        return self._polled_list(self.lib.snrx_ble_connections, _abi.CONN_DTYPE)
 
     def follow(self, access_addr: int, crc_init: int) -> np.ndarray:
         """Search and decode the BLE channels of that batch again with a connection's access address and CRC init: the
         data-channel PDUs of the connection, from the slicer bit streams already in HBM (nothing is channelized twice)."""
-        n = c_uint32(0)
-        cap = int(self.cfg.max_frames) or (1 << 17)
-        out = np.zeros(cap, dtype=FRAME_DTYPE)
-        self._check(self.lib.snrx_ble_follow(self.handle, access_addr & 0xFFFFFFFF, crc_init & 0xFFFFFF, out.ctypes.data_as(c_void_p), cap, byref(n)))
-        return out[: n.value].copy()
+        return self._polled_list(self.lib.snrx_ble_follow, FRAME_DTYPE, access_addr & 0xFFFFFFFF, crc_init & 0xFFFFFF)
 
     # ------------------------------------------------------------------ BLE 5 extended advertising
     def ble_aux(self) -> np.ndarray:
@@ -315,11 +312,7 @@ class RxEngine:
         poll() point at, followed down their chains, on the 1M and 2M PHYs: one _abi.AUX_DTYPE entry per AuxPtr, found and
         decoded on the GPU from the batch's slicer bit streams (definition in include/snoutrx.h).  Wideband BLE modes; call
         before the second-next process()."""
-        n = c_uint32(0)
-        cap = int(self.cfg.max_frames) or (1 << 17)
-        out = np.zeros(cap, dtype=_abi.AUX_DTYPE)
-        self._check(self.lib.snrx_ble_aux(self.handle, out.ctypes.data_as(c_void_p), cap, byref(n)))
-        return out[: n.value].copy()
+        return self._polled_list(self.lib.snrx_ble_aux, _abi.AUX_DTYPE)
 
     # ------------------------------------------------------------------ BLE Long Range (LE Coded)
     def ble_coded(self) -> np.ndarray:
@@ -327,33 +320,21 @@ class RxEngine:
         Viterbi-decoded, and the auxiliary packets they point at on every PHY, followed down their chains: one
         _abi.CODED_DTYPE entry per primary packet or AuxPtr, found and decoded on the GPU from the batch's slicer bit streams
         (definition in include/snoutrx.h).  Wideband BLE modes; call before the second-next process()."""
-        n = c_uint32(0)
-        cap = int(self.cfg.max_frames) or (1 << 17)
-        out = np.zeros(cap, dtype=_abi.CODED_DTYPE)
-        self._check(self.lib.snrx_ble_coded(self.handle, out.ctypes.data_as(c_void_p), cap, byref(n)))
-        return out[: n.value].copy()
+        return self._polled_list(self.lib.snrx_ble_coded, _abi.CODED_DTYPE)
 
     # ------------------------------------------------------------------ SURVEY 8(f) N2: Zigbee consumer path
     def zb_mac_summary(self) -> np.ndarray:
         """Per-record MAC summaries (_abi.ZBMAC_DTYPE: frame type, sequence number, PAN ids, addresses, inter-PAN / ZLL
         scan-response flags) of the batch most recently returned by poll(), computed on the GPU from the HBM frame list:
         what Snout reads off a scapy Dot15d4FCS tree per packet (zigbee.py:194-202, message.py:258-304)."""
-        n = c_uint32(0)
-        cap = int(self.cfg.max_frames) or (1 << 17)
-        out = np.zeros(cap, dtype=_abi.ZBMAC_DTYPE)
-        self._check(self.lib.snrx_zb_mac_summary(self.handle, out.ctypes.data_as(c_void_p), cap, byref(n)))
-        return out[: n.value].copy()
+        return self._polled_list(self.lib.snrx_zb_mac_summary, _abi.ZBMAC_DTYPE)
 
     # ------------------------------------------------------------------ per-frame radio metrics
     def frame_rf(self) -> np.ndarray:
         """Signal power, noise floor, SNR (dBFS / dB) and carrier offset (Hz) of every record of the batch most recently
         returned by poll(), aligned with it (_abi.RF_DTYPE; definition in include/snoutrx.h).  Needs rf_metrics=True;
         call before the second-next process()."""
-        n = c_uint32(0)
-        cap = int(self.cfg.max_frames) or (1 << 17)
-        out = np.zeros(cap, dtype=_abi.RF_DTYPE)
-        self._check(self.lib.snrx_frame_rf(self.handle, out.ctypes.data_as(c_void_p), cap, byref(n)))
-        return out[: n.value].copy()
+        return self._polled_list(self.lib.snrx_frame_rf, _abi.RF_DTYPE)
 
     def frames_device(self) -> tuple[int, int]:
         f, c = c_void_p(), c_void_p()

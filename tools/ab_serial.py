@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
 """Front-end kernel time of one resident ble_wb40 capture-second, ONE batch at a time (no other lane on the GPU) and two in
-flight: separates the kernel itself from what it suffers next to the other lane's kernels.  Env: SNRX_PFB_TILES, SNRX_PFB_ORDER."""
+flight: separates the kernel itself from what it suffers next to the other lane's kernels."""
 import os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -27,4 +27,4 @@ def piped(n, depth=2):
     return np.median(fe[3:]), (time.perf_counter() - t0) / n * 1e3
 a = serial(25); b = piped(40)
 c = piped(60, 3) if os.environ.get('AB_DEPTH3') else (float('nan'), float('nan'))
-print(f"tiles={os.environ.get('SNRX_PFB_TILES','-')} order={os.environ.get('SNRX_PFB_ORDER','-')} serial: frontend {a[0]:.4f} ms, batch {a[1]:.4f} ms | two in flight: frontend {b[0]:.4f} ms, wall/step {b[1]:.4f} ms | three in flight: frontend {c[0]:.4f} ms, wall/step {c[1]:.4f} ms")
+print(f"serial: frontend {a[0]:.4f} ms, batch {a[1]:.4f} ms | two in flight: frontend {b[0]:.4f} ms, wall/step {b[1]:.4f} ms | three in flight: frontend {c[0]:.4f} ms, wall/step {c[1]:.4f} ms")
