@@ -497,6 +497,78 @@ typedef struct snrx_ble_coded {     /* one per primary packet or pointer, 320 by
  * list; SNRX_EOVERFLOW if the list would hold more than max_frames entries. */
 int  snrx_ble_coded(snrx_t* h, snrx_ble_coded_t* out, uint32_t cap, uint32_t* n_out);
 
+/* ---- BLE periodic advertising: the AUX_SYNC_IND trains that the SyncInfo fields of a batch's AUX_ADV_INDs describe, on the
+ * 1M and 2M PHYs, found and decoded from the batch's slicer bit streams (wideband BLE modes; nothing is channelized twice
+ * and nothing hops).  No reference receiver exists for this: the definition below is the contract, and the GPU equals it
+ * bit for bit on the engine's own bit streams (oracle/periodic_oracle.py restates it).  Integer arithmetic only.
+ *
+ * Train sources.  The entries of the list snrx_ble_aux returns for the same batch with status OK, crc_ok, first == their own
+ *   index and a PDU of type 7 whose extended header (length L >= 1, 1 + L <= payload length) has the SyncInfo flag (0x20)
+ *   set and holds the fields in front of it (AdvA 6, TargetA 6, CTEInfo 1, ADI 2, AuxPtr 3 bytes, each if flagged) and the
+ *   18-byte SyncInfo: 2 + those fields + 18 <= 1 + L.  A SyncInfo with Sync Packet Offset 0, Interval < 6 or fewer than 2
+ *   used channels is not a source.  One train per distinct (capture_id, access address): its source is the candidate with
+ *   the smallest sample_index, the lower list index on ties.  Trains are ordered by their source's list index.
+ * SyncInfo (18 bytes, little endian; Core Vol 6 Part B 2.3.4.6 as read here).  Bytes 0..1: Sync Packet Offset (13 bits) |
+ *   Offset Units << 13 (U = 30 or 300 us) | Offset Adjust << 14 (adds 2 457 600 us).  Bytes 2..3: Interval (x 1.25 ms).
+ *   Bytes 4..8: ChM (bits 0..36, bit c = data channel c used) | SCA << 37 (3 bits: ppm = 500, 250, 150, 100, 75, 50, 30,
+ *   20).  Bytes 9..12: AA.  Bytes 13..15: CRCInit, reported and used as crc_init = c0 << 16 | c1 << 8 | c2 (c0..c2 in
+ *   transmit order: snrx_conn_t.crc_init's and snrx_ble_follow's convention).  Bytes 16..17: paEventCounter.
+ * Events.  Event k (any integer) has event_counter = (paEventCounter + k) mod 2^16, the source's PHY, and the channel of
+ *   Channel Selection Algorithm #2 (Core Vol 6 Part B 4.5.8.3) for that counter: channelIdentifier = AA[31:16] ^ AA[15:0];
+ *   prn_e = three rounds of PERM (bit reversal within each byte) then MAM (17 a + b mod 2^16, b = channelIdentifier) on
+ *   counter ^ channelIdentifier, then ^ channelIdentifier; unmapped = prn_e mod 37; if unmapped is not used, the channel is
+ *   used channel number (N prn_e) >> 16 in ascending order, N = the number of used channels.
+ * Window.  s = the source's sample_index (AA bit 0 lies 32 samples after the first preamble sample on both PHYs), O = offset
+ *   * U (+ 2 457 600 if Offset Adjust), I' = 1250 Interval us, p = the SCA's ppm, D_lo = O + k I', D_hi = O + U + k I':
+ *     win_lo = s + early(D_lo) - 8,   win_hi = s + late(D_hi) + 8,
+ *     early(D) = floor(4 D (10^6 - p) / 10^6) for D >= 0 and floor(4 D (10^6 + p) / 10^6) for D < 0,
+ *     late(D)  = ceil(4 D (10^6 + p) / 10^6)  for D >= 0 and ceil(4 D (10^6 - p) / 10^6)  for D < 0
+ *   (mathematical floor and ceiling, inclusive).  For k = 0 this is snrx_ble_aux's window with p from the SCA.
+ * Listed events.  Every k with (a) win_hi - win_lo + 1 <= 2500 Interval (half the interval in samples) and (b)
+ *   [win_lo, win_hi + 31 sps] meeting the buffer's usable decisions, in ascending k.  The width grows with |D| on both sides
+ *   of D = 0 by 8 I' p / 10^6 >= 1.2 samples per event, more than the two roundings can take back, so both rules and the
+ *   list hold one contiguous range of k.  Rule (a) keeps a train's windows (with the 31 sps span) disjoint, and two trains
+ *   never share an AA, so no packet is listed twice.
+ * Search, decode and status.  As snrx_ble_aux, with the train's AA (all 32 bits compared) and crc_init, the earliest match in
+ *   the window, len = header byte 1 (all 8 bits), de-whitened by the event's channel:
+ *   SNRX_AUX_OUTSIDE (win_lo or win_hi + 31 sps is not a usable decision: not searched), SNRX_AUX_NOT_FOUND,
+ *   SNRX_AUX_TRUNCATED (the header's or the packet's last decision is not usable), SNRX_AUX_OK (crc_ok says whether the CRC
+ *   matches).
+ * Order.  Trains in source order, each train's events in ascending k.
+ * Shards.  Indices are whole-capture indices.  Each shard predicts from its own sources; trains are not carried across
+ *   shards, and an event whose window leaves a shard's buffer is OUTSIDE there or not listed.
+ * Not covered: AUX_CHAIN_INDs an AUX_SYNC_IND points at (its bytes are kept), trains on LE Coded, periodic advertising with
+ *   responses, BIG / BIS data, and re-anchoring on found events (windows are predicted from the source alone). */
+#define SNRX_SYNC_MIN_INTERVAL 6
+
+typedef struct snrx_ble_sync {      /* one per listed event of a train, 320 bytes */
+    int64_t  sample_index;  /* AA bit 0 of the AUX_SYNC_IND (channel rate, capture relative); -1 unless OK / TRUNCATED       */
+    int64_t  win_lo, win_hi;/* the searched window of AA bit 0 positions, inclusive, capture relative                     */
+    uint32_t capture_id;
+    uint32_t source;        /* index in the snrx_ble_aux list of the AUX_ADV_IND whose SyncInfo the train comes from      */
+    uint32_t access_addr;   /* the train's AA                                                                            */
+    uint32_t crc_init;      /* the train's CRCInit as c0 << 16 | c1 << 8 | c2 (the value snrx_ble_follow takes)            */
+    int32_t  event;         /* k: events after (negative: before) the one the SyncInfo points at                         */
+    uint16_t event_counter; /* (paEventCounter + k) mod 2^16                                                              */
+    uint16_t interval;      /* in 1.25 ms units                                                                          */
+    uint8_t  channel;       /* CSA#2 channel of the event                                                                */
+    uint8_t  phy;           /* SNRX_AUX_PHY_1M or SNRX_AUX_PHY_2M (the source's)                                        */
+    uint8_t  phase;         /* sample_index mod sps (0 unless OK / TRUNCATED)                                            */
+    uint8_t  status;        /* SNRX_AUX_OK, _NOT_FOUND, _OUTSIDE or _TRUNCATED                                           */
+    uint8_t  crc_ok;        /* status OK and the CRC matches                                                             */
+    uint8_t  sca;           /* SyncInfo SCA 0..7                                                                         */
+    uint16_t len;           /* valid bytes in bytes[]: 2 + header length + 3 (0 unless OK)                               */
+    uint8_t  bytes[SNRX_AUX_MAX_BYTES];   /* de-whitened header | payload | CRC, zero past len                           */
+    uint8_t  reserved[4];
+} snrx_ble_sync_t;
+
+/* The periodic-advertising events of the batch most recently retired by snrx_poll / snrx_poll_view (definition above):
+ * *n_out entries, copied to out (up to cap; out may be NULL to count).  Builds the snrx_ble_aux list itself first.  State
+ * and capacity rules as snrx_ble_aux: SNRX_ESTATE without a polled wideband BLE batch or once its bit streams have been
+ * overwritten; SNRX_ERANGE if cap is smaller than the list; SNRX_EOVERFLOW if the aux list or this list would hold more than
+ * max_frames entries. */
+int  snrx_ble_periodic(snrx_t* h, snrx_ble_sync_t* out, uint32_t cap, uint32_t* n_out);
+
 /* ---- SURVEY 8(f) N2: the Zigbee consumer path on the decoded 802.15.4 records (what Snout does per datagram:
  * RFtap(pkt) -> Dot15d4FCS dissection, snout/util/zigbee.py:194-202; ZigbeeMessage.fromraw, snout/core/message.py:258-304;
  * the touchlink scan's haslayer(ZLLScanResponse), zigbee.py:176-192) ---- */

@@ -73,6 +73,14 @@ CODED_DTYPE = np.dtype([("sample_index", "<i8"), ("win_lo", "<i8"), ("win_hi", "
                         ("metric", "<u4"), ("bytes", "u1", (AUX_MAX_BYTES,)), ("reserved", "u1", (8,))], align=True)
 assert CODED_DTYPE.itemsize == 320
 
+# BLE periodic advertising: one entry per listed event of an AUX_SYNC_IND train (include/snoutrx.h snrx_ble_sync_t)
+SYNC_MIN_INTERVAL = 6
+SYNC_DTYPE = np.dtype([("sample_index", "<i8"), ("win_lo", "<i8"), ("win_hi", "<i8"), ("capture_id", "<u4"), ("source", "<u4"),
+                       ("access_addr", "<u4"), ("crc_init", "<u4"), ("event", "<i4"), ("event_counter", "<u2"), ("interval", "<u2"),
+                       ("channel", "u1"), ("phy", "u1"), ("phase", "u1"), ("status", "u1"), ("crc_ok", "u1"), ("sca", "u1"),
+                       ("len", "<u2"), ("bytes", "u1", (AUX_MAX_BYTES,)), ("reserved", "u1", (4,))], align=True)
+assert SYNC_DTYPE.itemsize == 320
+
 FRAME_DTYPE = np.dtype([
     ("sample_index", "<i8"), ("capture_id", "<u4"), ("window", "<u4"), ("channel", "<u2"),
     ("proto", "u1"), ("crc_ok", "u1"), ("lqi", "u1"), ("phase", "u1"), ("len", "<u2"),
@@ -148,6 +156,7 @@ SYMBOLS = [
     ("snrx_ble_follow", c_int, [c_void_p, c_uint32, c_uint32, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_ble_aux", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_ble_coded", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
+    ("snrx_ble_periodic", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_zb_mac_summary", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_frame_rf", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_exchange_create", c_int, [c_void_p, c_uint32, c_uint32, c_uint32, c_void_p]),

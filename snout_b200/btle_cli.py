@@ -47,6 +47,15 @@ that come under the detection threshold (DESIGN.md 4).
 
 With `-s` they also go to the pcap (formats.ble_pcap_coded_block).
 
+`--periodic` (with `--wideband`) also receives BLE periodic advertising: the SyncInfo of every AUX_ADV_IND that ble_aux
+finds describes a train of AUX_SYNC_INDs (its own access address and CRC init, a fixed interval, a CSA#2 channel per
+event), and every event of the train inside the capture is searched for at its predicted place (RxEngine.ble_periodic).
+Each AUX_SYNC_IND found is printed as one line of 8 tokens (formats.sync_line):
+
+    SYNC Ch<ch> PHY<1M|2M> AA:<access address hex> Evt<paEventCounter> Int<interval, 1.25 ms units> PloadL<len> CRC<0|1>
+
+With `-s` they also go to the pcap, with the train's access address (formats.ble_pcap_sync_block).
+
 There is no CPU path: without a usable GPU / libsnoutrx.so the program exits with an error.
 """
 from __future__ import annotations
@@ -100,6 +109,8 @@ USAGE = """Usage:
       With --wideband: also receive BLE Long Range (LE Coded) ADV_EXT_INDs on 37..39 and their auxiliary packets
     --aux
       With --wideband: also follow BLE 5 extended advertising to its auxiliary packets (1M and 2M PHYs) and print them
+    --periodic
+      With --wideband: also follow the SyncInfo of every AUX_ADV_IND to its periodic advertising train (AUX_SYNC_IND)
     --rf
       Measure signal power, noise floor and carrier offset of every frame; with -s the pcap's PHDR carries the
       signal and noise power (dBFS, flags 0x0002 / 0x0004).  Stdout lines are unchanged
@@ -129,6 +140,7 @@ class Options:
     rf = False
     aux = False
     coded = False
+    periodic = False
 
 
 def _strtol(text: str, base: int) -> int:
@@ -160,7 +172,7 @@ def parse_commandline(argv: list[str], out=sys.stdout) -> Options | None:
         opts, rest = getopt.getopt(argv, "hc:g:a:k:vrf:m:os:",
                                    ["help", "chan=", "gain=", "access=", "crcinit=", "verbose", "raw", "freq_hz=",
                                     "access_mask=", "hop", "filename=", "iq=", "format=", "scale=", "wideband",
-                                    "all-channels", "device=", "shard-windows=", "rf", "aux", "coded"])
+                                    "all-channels", "device=", "shard-windows=", "rf", "aux", "coded", "periodic"])
     except getopt.GetoptError as e:
         out.write(f"btle_rx: {e}\n")
         out.write(USAGE)
@@ -209,6 +221,8 @@ def parse_commandline(argv: list[str], out=sys.stdout) -> Options | None:
             o.aux = True
         elif k == "--coded":
             o.coded = True
+        elif k == "--periodic":
+            o.periodic = True
     if o.chan < 0 or o.chan > MAX_CHANNEL:
         out.write(f"channel number must be within 0~{MAX_CHANNEL}!\n")
         out.write(USAGE)
@@ -244,6 +258,9 @@ def run(o: Options, out=sys.stdout, engine_factory=None, blocks=None) -> int:
         return 1
     if o.aux and not o.wideband:
         out.write("btle_rx (snout_b200): --aux needs --wideband (auxiliary packets are sent on the data channels)\n")
+        return 1
+    if o.periodic and not o.wideband:
+        out.write("btle_rx (snout_b200): --periodic needs --wideband (periodic advertising is sent on the data channels)\n")
         return 1
     if o.iq is None and blocks is None:
         out.write("btle_rx (snout_b200): no IQ source; pass --iq FILE (or - for stdin)\n")
@@ -313,6 +330,13 @@ def run(o: Options, out=sys.stdout, engine_factory=None, blocks=None) -> int:
                     if d["depth"] == 0 and not d["crc_ok"]:
                         continue                      # mostly positions inside an S=8 packet's own body (DESIGN 4)
                     out.write(formats.coded_line(d) if d["depth"] == 0 else formats.aux_line(d))
+            if o.periodic:
+                sync = eng.ble_periodic()
+                if fh_pcap:
+                    fh_pcap.write(formats.ble_pcap_sync_block(sync))
+                for t in messages.ble_periodic_adv(sync):
+                    for ev in t["events"]:
+                        out.write(formats.sync_line(t, ev))
             out.flush()                                                # fflush(stdout), btle_rx.c:2383
 
         def follow(frames: np.ndarray):

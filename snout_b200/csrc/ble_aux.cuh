@@ -189,6 +189,75 @@ __global__ void __launch_bounds__(256) k_ble_aux_fill(AuxSrcT<L> s, const uint32
     r.status = st;
 }
 
+// The earliest n in [lo, hi] (local samples, inside the buffer) whose 32 decisions at stride sps equal the address of
+// `tabs`, or -1: one warp, 32 words per pass.  Shared by snrx_ble_aux and snrx_ble_periodic.
+__device__ __forceinline__ int aux_find(const uint32_t* pw, uint32_t nw, int lo, int hi, int sps, const AaTables& tabs, int lane) {
+    for (int wb = kBitsLeadWords + (lo >> 5); wb <= kBitsLeadWords + (hi >> 5); wb += 32) {
+        const int w = wb + lane;
+        const int s0 = 32 * (w - kBitsLeadWords);                 // sample of bit 0 of word w
+        uint32_t h;
+        auto keep = [](uint32_t m) { return __any_sync(0xffffffffu, m != 0u) != 0; };
+        if (sps == 4) {
+            uint32_t ww[5];
+#pragma unroll
+            for (int d = 0; d < 5; d++) ww[d] = ((uint32_t)(w + d) < nw) ? __ldg(pw + w + d) : 0u;
+            h = aa_word_hits(ww, tabs, keep);
+        } else {
+            uint32_t ww[3];
+#pragma unroll
+            for (int d = 0; d < 3; d++) ww[d] = ((uint32_t)(w + d) < nw) ? __ldg(pw + w + d) : 0u;
+            h = aa_word_hits2(ww, tabs, keep);
+        }
+        // keep start positions lo..hi
+        if (s0 + 31 < lo || s0 > hi) h = 0u;
+        else {
+            if (s0 < lo) h &= 0xFFFFFFFFu << (lo - s0);
+            if (s0 + 31 > hi) h &= 0xFFFFFFFFu >> (s0 + 31 - hi);
+        }
+        const uint32_t any = __ballot_sync(0xffffffffu, h != 0u);
+        if (any) {
+            const int src = __ffs(any) - 1;
+            return __shfl_sync(0xffffffffu, s0 + __ffs(h) - 1, src);
+        }
+    }
+    return -1;
+}
+
+// One warp: the packet whose AA bit 0 is at local sample n (found by aux_find) read, de-whitened by `channel` and checked
+// with the CRC seeded by crc_init_internal, into the entry's sample_index / phase / len / crc_ok / status / bytes.  buf is
+// the warp's SNRX_AUX_MAX_BYTES of shared memory, crc_s the CRC table in shared memory.
+template <class E>
+__device__ __forceinline__ void aux_decode(E& r, const uint32_t* pw, int n, int sps, int channel, const AuxGeom& g,
+                                           const uint32_t* crc_s, const uint8_t* __restrict__ whiten, uint32_t crc_init_internal,
+                                           uint8_t* buf, int lane) {
+    const int last_usable = g.n_out - 2;
+    uint8_t status = SNRX_AUX_TRUNCATED;
+    int nb = 0;
+    if (n + 47 * sps <= last_usable) {                            // the header's last decision
+        const int len = (int)((aux_read_byte(pw, n, 1, sps) ^ whiten[channel * SNRX_AUX_MAX_BYTES + 1]) & 0xFFu);
+        if (n + (32 + 8 * (len + 5) - 1) * sps <= last_usable) { nb = len + 5; status = SNRX_AUX_OK; }
+    }
+    for (int j = lane; j < nb; j += 32) buf[j] = (uint8_t)(aux_read_byte(pw, n, j, sps) ^ whiten[channel * SNRX_AUX_MAX_BYTES + j]);
+    __syncwarp();
+    for (int j = lane; j < nb; j += 32) r.bytes[j] = buf[j];
+    if (lane == 0) {
+        uint32_t ok = 0;
+        if (nb) {
+            uint32_t crc = crc_init_internal;
+            for (int j = 0; j < nb - 3; j++) crc = (crc_s[(crc ^ buf[j]) & 0xFFu] ^ (crc >> 8)) & 0xFFFFFFu;
+            const uint32_t recv = (uint32_t)buf[nb - 3] | ((uint32_t)buf[nb - 2] << 8) | ((uint32_t)buf[nb - 1] << 16);
+            ok = crc == recv;
+        }
+        const int64_t si = g.base + n;
+        r.sample_index = si;
+        r.phase = (uint8_t)(si % sps);
+        r.len = (uint16_t)nb;
+        r.crc_ok = (uint8_t)ok;
+        r.status = status;
+    }
+    __syncwarp();                                                 // buf is reused by the warp's next entry
+}
+
 // One warp per entry of [i0, i1) still pending: the earliest full access-address match in the window, then the decode.
 template <int L>
 __global__ void __launch_bounds__(128) k_ble_aux_search(AuxEntry<L>* __restrict__ list, uint32_t i0, uint32_t i1, AuxGeom g,
@@ -199,7 +268,6 @@ __global__ void __launch_bounds__(128) k_ble_aux_search(AuxEntry<L>* __restrict_
     for (int i = threadIdx.x; i < 256; i += blockDim.x) crc_s[i] = crc_tab[i];
     __syncthreads();
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-    uint8_t* buf = buf_s[wib];
     const uint32_t warps = gridDim.x * (blockDim.x >> 5);
     for (uint32_t k = i0 + blockIdx.x * (blockDim.x >> 5) + wib; k < i1; k += warps) {
         AuxEntry<L>& r = list[k];
@@ -207,64 +275,9 @@ __global__ void __launch_bounds__(128) k_ble_aux_search(AuxEntry<L>* __restrict_
         const int sps = r.phy == SNRX_AUX_PHY_2M ? 2 : 4;
         const int lo = (int)(r.win_lo - g.base), hi = (int)(r.win_hi - g.base);   // inside the buffer (k_ble_aux_fill)
         const uint32_t* pw = g.bits + g.lay.index(r.capture_id - g.first_capture, r.channel, 0);
-        const uint32_t nw = g.lay.words_per_stream;
-        int n = -1;
-        for (int wb = kBitsLeadWords + (lo >> 5); wb <= kBitsLeadWords + (hi >> 5); wb += 32) {
-            const int w = wb + lane;
-            const int s0 = 32 * (w - kBitsLeadWords);             // sample of bit 0 of word w
-            uint32_t h;
-            auto keep = [](uint32_t m) { return __any_sync(0xffffffffu, m != 0u) != 0; };
-            if (sps == 4) {
-                uint32_t ww[5];
-#pragma unroll
-                for (int d = 0; d < 5; d++) ww[d] = ((uint32_t)(w + d) < nw) ? __ldg(pw + w + d) : 0u;
-                h = aa_word_hits(ww, tabs, keep);
-            } else {
-                uint32_t ww[3];
-#pragma unroll
-                for (int d = 0; d < 3; d++) ww[d] = ((uint32_t)(w + d) < nw) ? __ldg(pw + w + d) : 0u;
-                h = aa_word_hits2(ww, tabs, keep);
-            }
-            // keep start positions lo..hi
-            if (s0 + 31 < lo || s0 > hi) h = 0u;
-            else {
-                if (s0 < lo) h &= 0xFFFFFFFFu << (lo - s0);
-                if (s0 + 31 > hi) h &= 0xFFFFFFFFu >> (s0 + 31 - hi);
-            }
-            const uint32_t any = __ballot_sync(0xffffffffu, h != 0u);
-            if (any) {
-                const int src = __ffs(any) - 1;
-                n = __shfl_sync(0xffffffffu, s0 + __ffs(h) - 1, src);
-                break;
-            }
-        }
+        const int n = aux_find(pw, g.lay.words_per_stream, lo, hi, sps, tabs, lane);
         if (n < 0) { if (lane == 0) r.status = SNRX_AUX_NOT_FOUND; continue; }
-        const int last_usable = g.n_out - 2;
-        uint8_t status = SNRX_AUX_TRUNCATED;
-        int nb = 0;
-        if (n + 47 * sps <= last_usable) {                        // the header's last decision
-            const int len = (int)((aux_read_byte(pw, n, 1, sps) ^ whiten[r.channel * SNRX_AUX_MAX_BYTES + 1]) & 0xFFu);
-            if (n + (32 + 8 * (len + 5) - 1) * sps <= last_usable) { nb = len + 5; status = SNRX_AUX_OK; }
-        }
-        for (int j = lane; j < nb; j += 32) buf[j] = (uint8_t)(aux_read_byte(pw, n, j, sps) ^ whiten[r.channel * SNRX_AUX_MAX_BYTES + j]);
-        __syncwarp();
-        for (int j = lane; j < nb; j += 32) r.bytes[j] = buf[j];
-        if (lane == 0) {
-            uint32_t ok = 0;
-            if (nb) {
-                uint32_t crc = crc_init_internal;
-                for (int j = 0; j < nb - 3; j++) crc = (crc_s[(crc ^ buf[j]) & 0xFFu] ^ (crc >> 8)) & 0xFFFFFFu;
-                const uint32_t recv = (uint32_t)buf[nb - 3] | ((uint32_t)buf[nb - 2] << 8) | ((uint32_t)buf[nb - 1] << 16);
-                ok = crc == recv;
-            }
-            const int64_t si = g.base + n;
-            r.sample_index = si;
-            r.phase = (uint8_t)(si % sps);
-            r.len = (uint16_t)nb;
-            r.crc_ok = (uint8_t)ok;
-            r.status = status;
-        }
-        __syncwarp();                                             // buf is reused by the warp's next entry
+        aux_decode(r, pw, n, sps, r.channel, g, crc_s, whiten, crc_init_internal, buf_s[wib], lane);
     }
 }
 

@@ -19,6 +19,7 @@
 #include "ble_adv.cuh"
 #include "ble_aux.cuh"
 #include "ble_coded.cuh"
+#include "ble_sync.cuh"
 #include "ble_back.cuh"
 #include "ble_conn.cuh"
 #include "ble_front.cuh"
@@ -101,6 +102,10 @@ struct snrx_handle {
     // whitening sequences continued to 260 bytes.  Neither list outlives its call (each is copied out before it returns).
     snrx_ble_aux_t* d_aux = nullptr;
     snrx_ble_coded_t* d_coded = nullptr;
+    // snrx_ble_periodic: its trains and its list (max_frames entries each), allocated by its first call; it builds the aux
+    // list into d_aux first, and its scans reuse the round buffers once the rounds are done
+    snrx::SyncTrain* d_sync_trains = nullptr;
+    snrx_ble_sync_t* d_sync = nullptr;
     uint32_t *d_round_flags = nullptr, *d_round_offsets = nullptr, *d_round_scratch = nullptr;
     uint8_t* d_aux_whiten = nullptr;
     snrx::DevSlot* d_devtab = nullptr;
@@ -210,12 +215,7 @@ void make_whiten_table(uint32_t* w /*[40][11]*/) {
     }
 }
 // crc_init_reorder(), btle_rx.c:1801-1825: byte swap then 24-bit bit reversal
-uint32_t crc_init_internal(uint32_t k) {
-    uint32_t sw = ((k & 0xFFu) << 16) | (k & 0xFF00u) | ((k >> 16) & 0xFFu);
-    uint32_t r = 0;
-    for (int i = 0; i < 24; i++) r |= ((sw >> i) & 1u) << (23 - i);
-    return r;
-}
+uint32_t crc_init_internal(uint32_t k) { return crc_seed_of(k); }
 
 template <class T>
 int dev_alloc(snrx_handle* h, T** p, size_t count) {
@@ -416,7 +416,8 @@ void snrx_destroy(snrx_t* h) {
     if (h->xchg.h_hdr) cudaFreeHost(h->xchg.h_hdr);
     if (h->adv_stream) { cudaStreamSynchronize(h->adv_stream); cudaStreamDestroy(h->adv_stream); }
     { void* ab[] = {h->d_adv, h->d_zbmac, h->d_conn, h->d_conn_flags, h->d_conn_offsets, h->d_conn_scratch, h->d_follow, h->d_devtab, h->d_devout, h->d_adv_counters,
-                    h->d_aux, h->d_coded, h->d_round_flags, h->d_round_offsets, h->d_round_scratch, h->d_aux_whiten}; for (void* b : ab) if (b) cudaFree(b); }
+                    h->d_aux, h->d_coded, h->d_round_flags, h->d_round_offsets, h->d_round_scratch, h->d_aux_whiten,
+                    h->d_sync_trains, h->d_sync}; for (void* b : ab) if (b) cudaFree(b); }
     delete h;
 }
 
@@ -1104,7 +1105,7 @@ int snrx_ble_connections(snrx_t* h, snrx_conn_t* out, uint32_t cap, uint32_t* n_
 }  // extern "C"
 
 // The lane of the polled batch, for the calls that search its BLE bit streams again (snrx_ble_follow, snrx_ble_aux,
-// snrx_ble_coded): it must hold BLE streams -- of a wideband mode if `wideband` -- that no later batch has overwritten.
+// snrx_ble_coded, snrx_ble_periodic): it must hold BLE streams -- of a wideband mode if `wideband` -- that no later batch has overwritten.
 static int polled_bits_lane(snrx_handle* h, const char* name, bool wideband, Lane** out) {
     const std::string n = name;
     if (h->polled_lane < 0) return fail(h, SNRX_ESTATE, (n + " needs a polled batch").c_str());
@@ -1126,7 +1127,8 @@ static AuxGeom aux_geom_of(const Lane& ln) {
     return g;
 }
 
-// what the pointer rounds of snrx_ble_aux and snrx_ble_coded share, allocated by the first call of either
+// what the pointer rounds of snrx_ble_aux and snrx_ble_coded (and snrx_ble_periodic's scans) share, allocated by the first
+// call of any of them
 static int round_buffers_init(snrx_handle* h) {
     if (h->d_aux_whiten) return SNRX_OK;
     CK(cudaMalloc((void**)&h->d_round_flags, sizeof(uint32_t) * ((size_t)h->frame_cap + 1)));
@@ -1278,6 +1280,52 @@ int snrx_ble_coded(snrx_t* h, snrx_ble_coded_t* out, uint32_t cap, uint32_t* n_o
     r = run_pointer_rounds(h, src, h->d_coded, cg.g, st, &total, "snrx_ble_coded: more entries than max_frames");
     if (r != SNRX_OK) return r;
     return copy_list_out(h, "snrx_ble_coded", h->d_coded, total, out, cap, n_out, st);
+}
+
+int snrx_ble_periodic(snrx_t* h, snrx_ble_sync_t* out, uint32_t cap, uint32_t* n_out) {
+    if (!h) return SNRX_EINVAL;
+    if (n_out) *n_out = 0;
+    Lane* ln = nullptr;
+    int r = polled_bits_lane(h, "snrx_ble_periodic", true, &ln);
+    if (r != SNRX_OK) return r;
+    CK(cudaSetDevice(h->device));
+    if ((r = round_buffers_init(h)) != SNRX_OK) return r;
+    if (!h->d_aux) CK(cudaMalloc((void**)&h->d_aux, sizeof(snrx_ble_aux_t) * (size_t)h->frame_cap));
+    if (!h->d_sync) {
+        CK(cudaMalloc((void**)&h->d_sync_trains, sizeof(SyncTrain) * (size_t)h->frame_cap));
+        CK(cudaMalloc((void**)&h->d_sync, sizeof(snrx_ble_sync_t) * (size_t)h->frame_cap));
+    }
+    cudaStream_t st = ln->tail;                                  // the lane is idle: its bit streams stay as the batch left them
+    const AuxGeom g = aux_geom_of(*ln);
+    AuxSrc src{};                                                // the aux list, exactly as snrx_ble_aux builds it
+    src.frames = h->polled_frames_dev; src.list = h->d_aux; src.first = 0; src.n = ln->n_frames; src.depth = 0;
+    uint32_t n_aux = 0;
+    r = run_pointer_rounds(h, src, h->d_aux, g, st, &n_aux, "snrx_ble_periodic: more auxiliary pointers than max_frames");
+    if (r != SNRX_OK) return r;
+    uint32_t total = 0;
+    if (n_aux) {
+        // the trains: flags / offsets over the aux list (n_aux <= max_frames fits the round buffers)
+        k_ble_sync_flag<<<grid_for(h, n_aux, 8, 8), 256, 0, st>>>(h->d_aux, n_aux, h->d_round_flags);
+        exclusive_scan(h->d_round_flags, n_aux, h->d_round_offsets, h->d_round_scratch, st);
+        k_ble_sync_fill<<<div_up(n_aux, 256), 256, 0, st>>>(h->d_aux, n_aux, h->d_round_flags, h->d_round_offsets, h->d_sync_trains);
+        uint32_t n_trains = 0;
+        CK(cudaMemcpyAsync(&n_trains, h->d_round_offsets + n_aux, sizeof n_trains, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        if (n_trains) {
+            // the events: counts / offsets per train, then one entry per listed event, then the search
+            k_ble_sync_count<<<div_up(n_trains, 256), 256, 0, st>>>(h->d_sync_trains, n_trains, g, h->d_round_flags);
+            exclusive_scan(h->d_round_flags, n_trains, h->d_round_offsets, h->d_round_scratch, st);
+            CK(cudaMemcpyAsync(&total, h->d_round_offsets + n_trains, sizeof total, cudaMemcpyDeviceToHost, st));
+            CK(cudaStreamSynchronize(st));
+            if (total > h->frame_cap) return fail(h, SNRX_EOVERFLOW, "snrx_ble_periodic: more periodic events than max_frames");
+            if (total) {
+                k_ble_sync_events<<<div_up(total, 256), 256, 0, st>>>(h->d_sync_trains, n_trains, h->d_round_offsets, total, g, h->d_sync);
+                k_ble_sync_search<<<grid_for(h, total, 4, 8), 128, 0, st>>>(h->d_sync, total, g, h->d_crc_tab, h->d_aux_whiten);
+            }
+        }
+        CK(cudaGetLastError());
+    }
+    return copy_list_out(h, "snrx_ble_periodic", h->d_sync, total, out, cap, n_out, st);
 }
 
 int snrx_zb_mac_summary(snrx_t* h, snrx_zbmac_t* out, uint32_t cap, uint32_t* n_out) {

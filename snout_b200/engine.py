@@ -322,6 +322,14 @@ class RxEngine:
         (definition in include/snoutrx.h).  Wideband BLE modes; call before the second-next process()."""
         return self._polled_list(self.lib.snrx_ble_coded, _abi.CODED_DTYPE)
 
+    # ------------------------------------------------------------------ BLE periodic advertising
+    def ble_periodic(self) -> np.ndarray:
+        """The AUX_SYNC_IND trains that the SyncInfo fields of the batch's AUX_ADV_INDs (as ble_aux() finds them) describe, on
+        the 1M and 2M PHYs: one _abi.SYNC_DTYPE entry per predicted event of a train inside the batch, with its counter,
+        CSA#2 channel and window, found and decoded on the GPU from the batch's slicer bit streams (definition in
+        include/snoutrx.h).  Wideband BLE modes; call before the second-next process()."""
+        return self._polled_list(self.lib.snrx_ble_periodic, _abi.SYNC_DTYPE)
+
     # ------------------------------------------------------------------ SURVEY 8(f) N2: Zigbee consumer path
     def zb_mac_summary(self) -> np.ndarray:
         """Per-record MAC summaries (_abi.ZBMAC_DTYPE: frame type, sequence number, PAN ids, addresses, inter-PAN / ZLL

@@ -302,6 +302,31 @@ def ble_pcap_coded_block(lst: np.ndarray, ts: tuple[int, int] = (0, 0), crc_fail
     return _pack_records(prefix, a["bytes"], lens, plens)
 
 
+def ble_pcap_sync_block(sync: np.ndarray, ts: tuple[int, int] = (0, 0)) -> bytes:
+    """The AUX_SYNC_INDs of RxEngine.ble_periodic() that were decoded (status OK), as records of the file btle_rx -s writes:
+    PHDR {channel, 0 x 7, flags}, flags = de-whitened | PDU type 1 (auxiliary advertising) << 7 | PHY << 14, then the
+    train's access address and header | payload (no CRC).  CRC-failed packets are written too."""
+    a = sync[sync["status"] == AUX_OK]
+    n = len(a)
+    lens = a["len"].astype(np.int64) - 3
+    prefix = np.zeros((n, 16 + 10 + 4), dtype=np.uint8)
+    prefix[:, 0:8] = np.frombuffer(struct.pack("<ii", ts[0], ts[1]), dtype=np.uint8)
+    be = (10 + 4 + lens).astype(">i4").view(np.uint8).reshape(n, 4)
+    prefix[:, 8:12], prefix[:, 12:16] = be, be
+    prefix[:, 16] = a["channel"]
+    flags = PHDR_DEWHITENED | (PHDR_PDU_AUX_ADV << PHDR_PDU_TYPE_SHIFT) | (a["phy"].astype(np.int64) << PHDR_PHY_SHIFT)
+    prefix[:, 24:26] = flags.astype("<u2").view(np.uint8).reshape(n, 2)
+    prefix[:, 26:30] = a["access_addr"].astype("<u4").view(np.uint8).reshape(n, 4)
+    return _pack_records(prefix, a["bytes"], lens)
+
+
+def sync_line(train: dict, ev: dict) -> str:
+    """btle_rx --periodic line of one decoded AUX_SYNC_IND (a train of messages.ble_periodic_adv and one of its events),
+    8 tokens: SYNC Ch<ch> PHY<1M|2M> AA:<hex> Evt<counter> Int<interval> PloadL<len> CRC<0 ok|1 failed>."""
+    return (f"SYNC Ch{ev['channel']} PHY{train['phy']} AA:{train['access_addr']:08x} Evt{ev['event_counter']} Int{train['interval']} "
+            f"PloadL{ev['pload_len']} CRC{0 if ev['crc_ok'] else 1}\n")
+
+
 def coded_line(d: dict) -> str:
     """btle_rx --coded line of one primary LE Coded ADV_EXT_IND (a messages.ble_coded_adv dictionary of depth 0), 8 tokens:
     CODED Ch<37..39> S<8|2> AdvA:<address or -> ADI:<DID>/<SID> (hex, - if absent) PloadL<len> CRC<0 ok|1 failed> AAerr<d>."""

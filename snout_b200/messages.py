@@ -78,16 +78,22 @@ def device_fingerprints(devices: np.ndarray, company_names: dict | None = None) 
 def _ext_fields(pdu: bytes) -> dict:
     """Common extended advertising payload of a PDU of type 7 (header | payload | CRC): AdvMode and the flagged fields of the
     extended header in their order (Core Vol 6 Part B 2.3.4), then AdvData.  A field the header is too short for is None."""
+    return _ext_walk(pdu)[0]
+
+
+def _ext_walk(pdu: bytes) -> tuple[dict, bytes, bytes | None]:
+    """(_ext_fields, the extended header bytes past its flagged fields -- the ACAD --, the 18-byte SyncInfo or None)."""
     n_payload = pdu[1]
     p = pdu[2:2 + n_payload]
     out = dict(adv_mode=None, adv_a=None, target_a=None, adi=None, did=None, sid=None, tx_power=None, aux_ptr=None, adv_data=b"")
+    sync_info = None
     if not p:
-        return out
+        return out, b"", sync_info
     hlen, out["adv_mode"] = p[0] & 0x3F, p[0] >> 6
     hdr = p[1:1 + hlen]
     out["adv_data"] = bytes(p[1 + hlen:])
     if not hdr:
-        return out
+        return out, b"", sync_info
     flags, at = hdr[0], 1
     for bit, name, size in ((0, "adv_a", 6), (1, "target_a", 6), (2, "cte_info", 1), (3, "adi", 2), (4, "aux_ptr", 3),
                             (5, "sync_info", 18), (6, "tx_power", 1)):
@@ -106,7 +112,9 @@ def _ext_fields(pdu: bytes) -> dict:
             out["tx_power"] = v[0] - 256 if v[0] > 127 else v[0]
         elif name == "aux_ptr":
             out["aux_ptr"] = v
-    return out
+        elif name == "sync_info":
+            sync_info = v
+    return out, bytes(hdr[at:]), sync_info
 
 
 _PHY_NAMES = {_abi.AUX_PHY_1M: "1M", _abi.AUX_PHY_2M: "2M", _abi.AUX_PHY_CODED: "Coded"}
@@ -155,3 +163,63 @@ def ble_coded_adv(lst: np.ndarray) -> list[dict]:
         if int(r["phy"]) == _abi.AUX_PHY_CODED:
             d["s"], d["aa_errors"] = 8 if int(r["ci"]) == 0 else 2, int(r["aa_errors"])
     return out
+
+
+# ----------------------------------------------------------------------------------------- BLE periodic advertising
+SCA_PPM = (500, 250, 150, 100, 75, 50, 30, 20)
+AD_BIGINFO = 0x2C
+
+
+def sync_info_fields(b: bytes) -> dict:
+    """The fields of an 18-byte SyncInfo (Core Vol 6 Part B 2.3.4.6 as read in include/snoutrx.h): offset_us (Sync Packet
+    Offset x units, + 2 457 600 us with Offset Adjust), interval (1.25 ms units), used channels, sca / ppm, access_addr,
+    crc_init (c0 << 16 | c1 << 8 | c2, the value RxEngine.follow takes) and pa_event_counter."""
+    o = b[0] | (b[1] << 8)
+    units = 300 if o & 0x2000 else 30
+    v = int.from_bytes(bytes(b[4:9]), "little")
+    sca = (v >> 37) & 7
+    return dict(offset_us=(o & 0x1FFF) * units + (2_457_600 if o & 0x4000 else 0), offset_units_us=units,
+                interval=b[2] | (b[3] << 8), channels=[c for c in range(37) if v >> c & 1], sca=sca, ppm=SCA_PPM[sca],
+                access_addr=int.from_bytes(bytes(b[9:13]), "little"), crc_init=(b[13] << 16) | (b[14] << 8) | b[15],
+                pa_event_counter=b[16] | (b[17] << 8))
+
+
+def _ad_types(data: bytes) -> list[int]:
+    """AD types of the AD structures of `data` (length | type | value), up to the first malformed one."""
+    out, at = [], 0
+    while at < len(data) and data[at] != 0 and at + 1 + data[at] <= len(data):
+        out.append(data[at + 1])
+        at += 1 + data[at]
+    return out
+
+
+def ble_periodic_adv(sync: np.ndarray, aux: np.ndarray | None = None) -> list[dict]:
+    """One dictionary per train of RxEngine.ble_periodic() (in list order): source (aux list index), capture_id,
+    access_addr, crc_init, interval (1.25 ms units) and interval_ms, channels (used), sca, ppm, phy ('1M' / '2M') and, when
+    the aux list of the same batch is given, the source's adv_a / adi / did / sid.  `events` holds the train's decoded events
+    (status OK), each with event (k), event_counter, channel, sample_index, crc_ok, pload_len, the extended-header fields of
+    _ext_fields, adv_data, acad (the raw Additional Controller Advertising Data), big_info (an ACAD AD structure of type
+    0x2C) and chained (the packet carries an AuxPtr to an AUX_CHAIN_IND, which is not followed)."""
+    trains: dict = {}
+    for r in sync:
+        key = int(r["source"])
+        if key not in trains:
+            t = dict(source=key, capture_id=int(r["capture_id"]), access_addr=int(r["access_addr"]), crc_init=int(r["crc_init"]),
+                     interval=int(r["interval"]), interval_ms=1.25 * int(r["interval"]), sca=int(r["sca"]), ppm=SCA_PPM[int(r["sca"])],
+                     phy=_PHY_NAMES.get(int(r["phy"]), "1M"), channels=None, adv_a=None, adi=None, did=None, sid=None, events=[])
+            if aux is not None and key < len(aux):
+                a = aux[key]
+                fields, _, si = _ext_walk(bytes(a["bytes"][: int(a["len"])]))
+                t.update(adv_a=fields["adv_a"], adi=fields["adi"], did=fields["did"], sid=fields["sid"])
+                if si is not None:
+                    t["channels"] = sync_info_fields(si)["channels"]
+            trains[key] = t
+        if int(r["status"]) != _abi.AUX_OK:
+            continue
+        pdu = bytes(r["bytes"][: int(r["len"])])
+        fields, acad, _ = _ext_walk(pdu)
+        trains[key]["events"].append(dict(event=int(r["event"]), event_counter=int(r["event_counter"]), channel=int(r["channel"]),
+                                          sample_index=int(r["sample_index"]), crc_ok=bool(r["crc_ok"]), pload_len=pdu[1],
+                                          **fields, acad=acad, big_info=AD_BIGINFO in _ad_types(acad),
+                                          chained=fields["aux_ptr"] is not None))
+    return list(trains.values())

@@ -579,7 +579,7 @@ def wideband_capture_gpu(seconds: float = 0.02, kind: str = "ble", seed: int = 4
 # flagged fields in the order AdvA, TargetA, CTEInfo, ADI, AuxPtr, SyncInfo, TxPower.
 
 def ext_header(adv_mode: int = 0, adv_a: bytes | None = None, tx_add: int = 0, adi: int | None = None, aux_ptr: bytes | None = None,
-               tx_power: int | None = None) -> bytes:
+               tx_power: int | None = None, sync_info: bytes | None = None, acad: bytes = b"") -> bytes:
     flags, body = 0, b""
     if adv_a is not None:
         flags |= 0x01
@@ -590,10 +590,13 @@ def ext_header(adv_mode: int = 0, adv_a: bytes | None = None, tx_add: int = 0, a
     if aux_ptr is not None:
         flags |= 0x10
         body += bytes(aux_ptr)
+    if sync_info is not None:
+        flags |= 0x20
+        body += bytes(sync_info)
     if tx_power is not None:
         flags |= 0x40
         body += bytes([tx_power & 0xFF])
-    hdr = bytes([flags]) + body
+    hdr = bytes([flags]) + body + bytes(acad)
     return bytes([len(hdr) | (adv_mode << 6)]) + hdr
 
 
@@ -718,6 +721,176 @@ def ext_adv_capture(seconds: float = 0.05, seed: int = 9000, esn0_db: float | No
     if esn0_db is not None:
         x = x + _awgn(len(x), np.random.default_rng(seed + 999), 4.0 * chanplan.WB_DECIM / (10.0 ** (esn0_db / 10.0))).astype(np.complex64)
     return Capture(x.astype(np.complex64), chanplan.WB_RATE, prim, dict(kind="wb_ble_ext", seed=seed, esn0_db=esn0_db, aux=aux))
+
+
+# ------------------------------------------------------------- BLE periodic advertising (test input)
+# An AUX_ADV_IND whose extended header carries a SyncInfo (Core Vol 6 Part B 2.3.4.6 as read in include/snoutrx.h) describes
+# a train of AUX_SYNC_INDs with their own access address and CRC init, one per interval, on the channel Channel Selection
+# Algorithm #2 (Vol 6 Part B 4.5.8.3) gives the event counter.
+SCA_PPM = (500, 250, 150, 100, 75, 50, 30, 20)
+OFFSET_ADJUST_US = 2_457_600
+
+
+def sync_info_bytes(offset: int, units_us: int, interval: int, chm: int, sca: int, access_addr: int, crc_init: int,
+                    pa_counter: int, adjust: int = 0) -> bytes:
+    """SyncInfo: offset (13 bits) | units << 13 | adjust << 14, Interval, ChM (37 bits) | SCA << 37, AA, CRCInit, paEventCounter,
+    little endian.  crc_init = c0 << 16 | c1 << 8 | c2 with c0 sent first (the value btle_rx's -k and RxEngine.follow take)."""
+    o = (offset & 0x1FFF) | ((1 if units_us == 300 else 0) << 13) | ((adjust & 1) << 14)
+    return (o.to_bytes(2, "little") + (interval & 0xFFFF).to_bytes(2, "little") + ((chm & ((1 << 37) - 1)) | ((sca & 7) << 37)).to_bytes(5, "little")
+            + (access_addr & 0xFFFFFFFF).to_bytes(4, "little") + (crc_init & 0xFFFFFF).to_bytes(3, "big") + (pa_counter & 0xFFFF).to_bytes(2, "little"))
+
+
+def sync_crc_seed(crc_init: int) -> int:
+    """The ble_crc24 `init` (CRCInit least significant byte first) of a SyncInfo crc_init (first byte most significant)."""
+    return int.from_bytes((crc_init & 0xFFFFFF).to_bytes(3, "big"), "little")
+
+
+def csa2_channel(counter: int, access_addr: int, used: list[int]) -> int:
+    """Channel Selection Algorithm #2: channelIdentifier = AA[31:16] ^ AA[15:0]; three rounds of MAM(PERM(.)) on
+    counter ^ channelIdentifier; prn_e = that ^ channelIdentifier; channel prn_e mod 37, or used[(N prn_e) >> 16] when that
+    channel is not used."""
+    ci = (access_addr >> 16) ^ (access_addr & 0xFFFF)
+    x = counter ^ ci
+    for _ in range(3):
+        lo, hi = x & 0xFF, x >> 8
+        x = (int(bin(lo)[2:].zfill(8)[::-1], 2) | (int(bin(hi)[2:].zfill(8)[::-1], 2) << 8))
+        x = (17 * x + ci) % 65536
+    e = x ^ ci
+    return e % 37 if e % 37 in used else sorted(used)[(len(used) * e) // 65536]
+
+
+def sync_offset_for(gap_samples: float, drift: float) -> tuple[int, int, int]:
+    """SyncInfo (offset, units_us, adjust) an advertiser whose clock runs fast by `drift` states for a true gap of gap_samples
+    (4 Msps) between the AUX_ADV_IND and the AUX_SYNC_IND."""
+    t_us = gap_samples / 4.0 * (1.0 + drift)
+    adjust = 1 if t_us >= 8191 * 300 + 300 else 0
+    t_us -= adjust * OFFSET_ADJUST_US
+    units = 30 if t_us < 8191 * 30 else 300
+    off = int(t_us // units)
+    assert 1 <= off <= 8191, "sync packet too near or too far"
+    return off, units, adjust
+
+
+@dataclass
+class SyncTruth:
+    """An AUX_SYNC_IND placed into a synthetic capture."""
+    access_addr: int
+    crc_init: int
+    counter: int          # paEventCounter of the event
+    channel: int
+    phy: int              # 0 = LE 1M, 1 = LE 2M
+    start: int            # channel-rate sample of the first preamble sample
+    anchor: int           # nominal sample of AA bit 0
+    data: bytes           # pdu | crc (un-whitened)
+    clash: bool = False   # another packet overlaps it on its channel
+
+
+def periodic_adv_schedule(n_ch: int, rng: np.random.Generator, n_trains: int = 3, phys=(0, 1), intervals=(6, 80),
+                          adv_interval=(60_000, 120_000), data_len=(0, 120), big_info: bool = True, cfo_hz: float = 50e3):
+    """Periodic advertising trains on a 4 Msps time line.  Each train has a random AA and CRC init, an Interval in `intervals`,
+    a channel map of 2..37 used channels, an SCA and an advertiser clock error inside the SCA's bound, a PHY, and a first
+    paEventCounter that makes some trains wrap past 0xFFFF inside the capture; its AUX_SYNC_INDs run from before its first
+    advertising event to the end of the capture.  Every adv_interval samples (per train, interleaved) an ADV_EXT_IND on 37,
+    38 and 39 points at an AUX_ADV_IND on the train's PHY whose SyncInfo points at the next AUX_SYNC_IND.  Some trains carry
+    a BIGInfo in their ACAD.  Returns ({bin: stream}, [Truth] of the primaries, [SyncTruth], [AuxTruth] of the AUX_ADV_INDs);
+    a SyncTruth is marked `clash` when another packet overlaps it on its channel."""
+    streams: dict = {}
+    prim, syncs, auxs = [], [], []
+    busy: dict[int, list] = {}                       # channel -> [(start, end)] of every packet placed
+    trains = []
+    for t in range(n_trains):
+        phy = int(phys[t % len(phys)])
+        sps = 2 if phy == 1 else 4
+        aa = int(rng.integers(1, 1 << 32))
+        while aa == chanplan.BLE_ADV_AA:
+            aa = int(rng.integers(1, 1 << 32))
+        n_used = int(rng.integers(2, 38))
+        used = sorted(int(c) for c in rng.choice(37, n_used, replace=False))
+        chm = sum(1 << c for c in used)
+        sca = int(rng.integers(0, 8))
+        drift = float(rng.uniform(-0.9, 0.9)) * SCA_PPM[sca] * 1e-6
+        interval = int(rng.integers(intervals[0], intervals[1] + 1))
+        pa0 = int(rng.integers(65536 - 3, 65536)) if t % 2 == 0 else int(rng.integers(0, 65536))
+        step = 5000.0 * interval / (1.0 + drift)     # receiver samples per event
+        t0 = float(rng.uniform(500, 500 + step))
+        crc_init = int(rng.integers(0, 1 << 24))
+        acad = b""
+        if big_info and t % 3 == 1:
+            acad = bytes([34, 0x2C]) + bytes(rng.integers(0, 256, 33, dtype=np.uint8))
+        adv_a = bytes(rng.integers(0, 256, 6, dtype=np.uint8))
+        adi = int(rng.integers(0, 4096)) | (int(rng.integers(0, 16)) << 12)
+        events = []
+        j = 0
+        while True:
+            start = int(round(t0 + j * step))
+            data = bytes(rng.integers(0, 256, int(rng.integers(data_len[0], data_len[1] + 1)), dtype=np.uint8))
+            pdu = ext_pdu(ext_header(0, None, 0, None, None, None if j % 2 else -10, acad=acad), data)
+            nbits = (16 if sps == 2 else 8) + 32 + 8 * (len(pdu) + 3)
+            if start + nbits * sps + 64 >= n_ch:
+                break
+            counter = (pa0 + j) % 65536
+            ch = csa2_channel(counter, aa, used)
+            syncs.append(SyncTruth(aa, crc_init, counter, ch, phy, start, start + 32 + 2 * sps, pdu + ble_crc24(pdu, sync_crc_seed(crc_init))))
+            events.append((start, start + nbits * sps, len(syncs) - 1, pdu))
+            busy.setdefault(ch, []).append((start, start + nbits * sps, len(syncs) - 1))
+            j += 1
+        trains.append(dict(phy=phy, sps=sps, aa=aa, used=used, chm=chm, sca=sca, drift=drift, interval=interval, pa0=pa0,
+                           crc_init=crc_init, adv_a=adv_a, adi=adi, events=events))
+    # advertising events on a shared time line, the trains taking turns; each AUX_ADV_IND on a data channel that is free then
+    pos = 2000 + int(rng.integers(0, 4000))
+    p_len = (1 + 4 + 2 + 9 + 3) * 8 * 4 + 16
+    order = 0
+    while True:
+        tr = trains[order % n_trains]
+        order += 1
+        p_starts = [pos, pos + p_len + 1400, pos + 2 * (p_len + 1400)]
+        a_start = p_starts[2] + p_len + int(rng.integers(1200, 6000))
+        sps = tr["sps"]
+        nxt = [e for e in tr["events"] if e[0] >= a_start + 6000]
+        if not nxt or a_start + 6000 >= n_ch:
+            break
+        e_start, _, e_idx, _ = nxt[0]
+        off, units, adjust = sync_offset_for(e_start - a_start, tr["drift"])
+        si = sync_info_bytes(off, units, tr["interval"], tr["chm"], tr["sca"], tr["aa"], tr["crc_init"], syncs[e_idx].counter, adjust)
+        pdu = ext_pdu(ext_header(0, tr["adv_a"], 0, tr["adi"], None, 0, sync_info=si))
+        nbits = (16 if sps == 2 else 8) + 32 + 8 * (len(pdu) + 3)
+        a_end = a_start + nbits * sps
+        free = [c for c in range(37) if not any(s < a_end + 64 and a_start < e + 64 for s, e, *_ in busy.get(c, []))]
+        ch = int(rng.choice(free))
+        bits = ble_phy_bits_2m(pdu, ch) if sps == 2 else ble_phy_bits(pdu, ch)
+        _put(streams, n_ch, ch, a_start, gfsk_modulate(bits, sps=sps), rng, cfo_hz)
+        busy.setdefault(ch, []).append((a_start, a_end, -1))
+        par = []
+        ca = 1
+        for j, ps in enumerate(p_starts):
+            units_p, off_p, drift_p = aux_offset_for(a_start - ps, ca, rng)
+            pp = ext_pdu(ext_header(0, None, 0, tr["adi"], aux_ptr_bytes(ch, ca, units_p, off_p, tr["phy"])))
+            _put(streams, n_ch, 37 + j, ps, gfsk_modulate(ble_phy_bits(pp, 37 + j)), rng, cfo_hz)
+            prim.append(Truth(37 + j, ps, ps + 8 * 4 + 8, pp + ble_crc24(pp), 3))
+            par.append((37 + j, ps, units_p, off_p, ca, drift_p, a_start - ps))
+        auxs.append(AuxTruth(ch, tr["phy"], a_start, a_start + 32 + 2 * sps, pdu + ble_crc24(pdu), 0, par))
+        pos = max(a_end, p_starts[2] + p_len) + int(rng.integers(adv_interval[0], adv_interval[1] + 1)) // n_trains
+    for tr in trains:
+        for start, end, k, pdu in tr["events"]:
+            s = syncs[k]
+            bits = (ble_phy_bits_2m if s.phy == 1 else ble_phy_bits)(pdu, s.channel, access_addr=tr["aa"],
+                                                                     crc_init=sync_crc_seed(tr["crc_init"]))
+            _put(streams, n_ch, s.channel, start, gfsk_modulate(bits, sps=tr["sps"]), rng, cfo_hz)
+            s.clash = any(o != k and a < end + 64 and start < b + 64 for a, b, o in busy[s.channel])
+    return streams, prim, syncs, auxs
+
+
+def periodic_adv_capture(seconds: float = 0.1, seed: int = 9700, esn0_db: float | None = 25.0, **kw) -> Capture:
+    """96 Msps capture (centre 2440 MHz) carrying periodic_adv_schedule(...) and nothing else; meta["sync"] holds the
+    SyncTruth list, meta["aux"] the AUX_ADV_INDs.  esn0_db=None: no noise."""
+    rng = np.random.default_rng(seed)
+    n_ch = int(round(seconds * chanplan.NB_RATE))
+    n_ch -= n_ch % chanplan.BLE_WINDOW
+    streams, prim, syncs, auxs = periodic_adv_schedule(n_ch, rng, **kw)
+    x = wideband_mix(streams)
+    if esn0_db is not None:
+        x = x + _awgn(len(x), np.random.default_rng(seed + 999), 4.0 * chanplan.WB_DECIM / (10.0 ** (esn0_db / 10.0))).astype(np.complex64)
+    return Capture(x.astype(np.complex64), chanplan.WB_RATE, prim, dict(kind="wb_ble_periodic", seed=seed, esn0_db=esn0_db, sync=syncs, aux=auxs))
 
 
 # ------------------------------------------------------------- BLE Long Range (LE Coded PHY, test input)
