@@ -569,6 +569,97 @@ typedef struct snrx_ble_sync {      /* one per listed event of a train, 320 byte
  * max_frames entries. */
 int  snrx_ble_periodic(snrx_t* h, snrx_ble_sync_t* out, uint32_t cap, uint32_t* n_out);
 
+/* ---- BLE broadcast isochronous streams: the BIS subevents that the BIGInfo in a batch's AUX_SYNC_INDs describes, on the 1M
+ * and 2M PHYs, found and decoded from the batch's slicer bit streams (wideband BLE modes; nothing is channelized twice and
+ * nothing hops).  No reference receiver exists for this: the definition below is the contract, and the GPU equals it bit for
+ * bit on the engine's own bit streams (oracle/bis_oracle.py restates it).  Integer arithmetic only.
+ *
+ * Carriers.  The entries of the list snrx_ble_periodic returns for the same batch with status OK, crc_ok and a PDU of type 7
+ *   whose extended header has length L >= 1 with 1 + L <= payload length and holds its flagged fields (AdvA 6, TargetA 6,
+ *   CTEInfo 1, ADI 2, AuxPtr 3, SyncInfo 18, TxPower 1 bytes); the header bytes past them are the ACAD.  The ACAD is walked
+ *   as AD structures (length | type | value), stopping at a length-0 structure or one that overruns it; its first structure
+ *   of type 0x2C must have length byte 34 (an unencrypted BIGInfo, 33 bytes) or 58 (encrypted, 57 bytes), and that BIGInfo
+ *   must be valid (below).
+ * BIGInfo (little endian; Core Vol 6 Part B 2.3.4.8 as read here).  Bytes 0..3: BIG_Offset (14 bits) | BIG_Offset_Units << 14
+ *   (U = 30 or 300 us) | ISO_Interval << 15 (12 bits, x 1.25 ms) | Num_BIS << 27 (5).  Bytes 4..7: NSE (5) | BN << 5 (3) |
+ *   Sub_Interval << 8 (20, us) | PTO << 28 (4).  Bytes 8..11: BIS_Spacing (20, us) | IRC << 20 (4) | Max_PDU << 24 (8).
+ *   Byte 12: RFU.  Bytes 13..16: SeedAccessAddress (SAA).  Bytes 17..20: SDU_Interval (20) | Max_SDU << 20 (12).  Bytes
+ *   21..22: BaseCRCInit.  Bytes 23..27: ChM (bits 0..36) | PHY << 37 (3: 0 = 1M, 1 = 2M, 2 = Coded).  Bytes 28..32:
+ *   bisPayloadCount (39 bits) | Framing << 39.  Bytes 33..56 (encrypted only): GIV (8) and GSKD (16).
+ *   Valid: Num_BIS, BN, NSE >= 1, NSE mod BN = 0, 1 <= IRC <= NSE / BN; ISO_Interval >= 4; PHY 1M or 2M; at least 2 used
+ *   channels; (Num_BIS - 1) BIS_Spacing + (NSE - 1) Sub_Interval < 1250 ISO_Interval; S_min > 0, where S_min (the spacing of
+ *   two packets of one BIS, us) = min(Sub_Interval, 1250 ISO_Interval - (NSE - 1) Sub_Interval), or 1250 ISO_Interval when
+ *   NSE = 1.
+ * BIGs.  One per distinct (capture_id, SAA): its source is the carrier with the smallest sample_index, the lower list index
+ *   on ties; BIGs are ordered by their source's index in the periodic list.  Everything is predicted from the source alone.
+ * BIS n = 1..Num_BIS (Vol 6 Part B 2.1.2 as read here).  AA_n = SAA ^ DW_n with D = (35 n + 42) mod 128 (bits D6..D0) and
+ *   the diversifier word DW_n, from bit 31 down to bit 0: D0 D0 D0 D0 D0 D0 D1 D6 | D1 0 D5 D4 0 D3 D2 0 | 16 zero bits.
+ *   The 24-bit CRCInit is BaseCRCInit << 8 | n, sent least significant byte first, so crc_init (c0 << 16 | c1 << 8 | c2 in
+ *   transmit order: snrx_conn_t.crc_init's and snrx_ble_follow's convention) = n << 16 | (BaseCRCInit & 0xFF) << 8 |
+ *   BaseCRCInit >> 8.  A BIS whose AA_n is 0 is not searched (its entries are NOT_FOUND): an all-zero address would match
+ *   any run of 32 zero decisions.
+ * Events.  Event k (any integer) has event_counter E_k = (floor(bisPayloadCount / BN) + k) mod 2^16.  Its subevent (n, se),
+ *   se = 0..NSE-1, has D_lo = O + 1250 k ISO_Interval + (n - 1) BIS_Spacing + se Sub_Interval (us), O = BIG_Offset U,
+ *   D_hi = D_lo + U, measured from s = the source's sample_index (AA bit 0 lies 32 samples after the first preamble sample on
+ *   both PHYs), and p = the ppm of the source's train's SCA (the BIGInfo carries no SCA; this is the reading used here):
+ *     win_lo = s + early(D_lo) - 8,   win_hi = s + late(D_hi) + 8   (early / late as snrx_ble_sync_t's windows).
+ * Channel (Vol 6 Part B 4.5.8.3 as read here).  Subevent 0: CSA#2 of E_k with AA_n and ChM (as snrx_ble_sync_t's events).
+ *   Subevents se >= 1: prnSubEvent_lu starts at the event's prn_s (prn_e before its final ^ channelIdentifier); each
+ *   subevent sets prnSubEvent_lu = MAM(PERM(prnSubEvent_lu)), prnSubEvent_se = prnSubEvent_lu ^ channelIdentifier, and takes
+ *   used channel number index = (lastIndex + d + ((prnSubEvent_se (N - 2 d + 1)) >> 16)) mod N in ascending order, with
+ *   d = max(1, max(min(3, N - 5), min(11, (N - 10) / 2))), N = the number of used channels and lastIndex the used-channel
+ *   number of the previous subevent (of subevent 0 to start).
+ * Payload number (Vol 6 Part B 4.4.6.6 as read here).  g = se / BN, i = se mod BN:
+ *   payload_number = ((floor(bisPayloadCount / BN) + k + (g < IRC ? 0 : PTO (g - IRC + 1))) mod 2^39) BN + i.
+ * Listed events.  k_c = the first k with D_lo(1, 0) >= 0.  Event k is listed when (a) every subevent window of every event
+ *   from k to k_c (inclusive) is at most 2 S_min samples long, and (b) [win_lo(1, 0), win_hi(Num_BIS, NSE - 1) + 31 sps]
+ *   meets the buffer's usable decisions.  A listed event contributes all its Num_BIS x NSE entries; an entry whose own
+ *   [win_lo, win_hi + 31 sps] leaves the usable decisions is OUTSIDE.  Two packets of one BIS are at least S_min us =
+ *   4 S_min samples apart, so a window of at most 2 S_min samples (with the 31 sps address span) ends before the next one
+ *   of its BIS starts: no packet is listed twice.
+ * Search, decode and status.  As snrx_ble_sync_t's, with AA_n (all 32 bits), crc_init_n and the subevent's channel, at 4
+ *   samples per symbol on 1M and 2 on 2M (the BIGInfo's PHY): OUTSIDE, NOT_FOUND, TRUNCATED or OK with crc_ok.  The payload
+ *   of an encrypted BIS is reported as sent (its MIC is part of len).
+ * Order.  BIGs in source order; within a BIG ascending k, then BIS number, then subevent.
+ * Shards.  Indices are whole-capture indices.  Each shard predicts from its own carriers; BIGs are not carried across shards.
+ * Spec-dependent pieces, unverified here against the specification's sample data: the BIGInfo bit layout, the diversifier
+ *   word, the subevent channel mapping and the payload numbering (DESIGN.md section 4).
+ * Not covered: decrypting encrypted BISes (needs the Broadcast_Code), BIG Control subevents (after a channel map update the
+ *   entries are NOT_FOUND), BIGs on LE Coded, re-anchoring on found events, ISOAL SDU reassembly, connected isochronous
+ *   streams. */
+#define SNRX_BIS_ENCRYPTED 0x01     /* snrx_ble_bis_t.flags */
+#define SNRX_BIS_FRAMED    0x02
+
+typedef struct snrx_ble_bis_entry { /* one per subevent of a listed BIG event, 336 bytes */
+    int64_t  sample_index;  /* AA bit 0 of the BIS PDU (channel rate, capture relative); -1 unless OK / TRUNCATED            */
+    int64_t  win_lo, win_hi;/* the searched window of AA bit 0 positions, inclusive, capture relative                     */
+    uint64_t payload_number;/* the payload this subevent carries (definition above)                                      */
+    uint32_t capture_id;
+    uint32_t source;        /* index in the snrx_ble_periodic list of the AUX_SYNC_IND whose BIGInfo the BIG comes from   */
+    uint32_t access_addr;   /* AA_n                                                                                      */
+    uint32_t crc_init;      /* crc_init_n as c0 << 16 | c1 << 8 | c2 (the value snrx_ble_follow takes)                     */
+    int32_t  event;         /* k: BIG events after (negative: before) the one the BIGInfo points at                      */
+    uint16_t event_counter; /* E_k                                                                                         */
+    uint8_t  bis;           /* n, 1..Num_BIS                                                                              */
+    uint8_t  subevent;      /* se, 0..NSE-1                                                                               */
+    uint8_t  channel;       /* the subevent's data channel                                                               */
+    uint8_t  phy;           /* SNRX_AUX_PHY_1M or SNRX_AUX_PHY_2M (the BIGInfo's)                                       */
+    uint8_t  phase;         /* sample_index mod sps (0 unless OK / TRUNCATED)                                            */
+    uint8_t  status;        /* SNRX_AUX_OK, _NOT_FOUND, _OUTSIDE or _TRUNCATED                                           */
+    uint8_t  crc_ok;        /* status OK and the CRC matches                                                             */
+    uint8_t  flags;         /* SNRX_BIS_ENCRYPTED (a 57-byte BIGInfo) | SNRX_BIS_FRAMED                                   */
+    uint16_t len;           /* valid bytes in bytes[]: 2 + length byte + 3 (0 unless OK)                                 */
+    uint8_t  bytes[SNRX_AUX_MAX_BYTES];   /* de-whitened header | payload | CRC, zero past len                           */
+    uint8_t  reserved[12];
+} snrx_ble_bis_t;
+
+/* The BIS subevents of the batch most recently retired by snrx_poll / snrx_poll_view (definition above): *n_out entries,
+ * copied to out (up to cap; out may be NULL to count).  Builds the snrx_ble_aux and snrx_ble_periodic lists itself first.
+ * State and capacity rules as snrx_ble_periodic: SNRX_ESTATE without a polled wideband BLE batch or once its bit streams
+ * have been overwritten; SNRX_ERANGE if cap is smaller than the list; SNRX_EOVERFLOW if the aux list, the periodic list or
+ * this list would hold more than max_frames entries. */
+int  snrx_ble_bis(snrx_t* h, snrx_ble_bis_t* out, uint32_t cap, uint32_t* n_out);
+
 /* ---- SURVEY 8(f) N2: the Zigbee consumer path on the decoded 802.15.4 records (what Snout does per datagram:
  * RFtap(pkt) -> Dot15d4FCS dissection, snout/util/zigbee.py:194-202; ZigbeeMessage.fromraw, snout/core/message.py:258-304;
  * the touchlink scan's haslayer(ZLLScanResponse), zigbee.py:176-192) ---- */

@@ -81,6 +81,15 @@ SYNC_DTYPE = np.dtype([("sample_index", "<i8"), ("win_lo", "<i8"), ("win_hi", "<
                        ("len", "<u2"), ("bytes", "u1", (AUX_MAX_BYTES,)), ("reserved", "u1", (4,))], align=True)
 assert SYNC_DTYPE.itemsize == 320
 
+# BLE broadcast isochronous streams: one entry per subevent of a listed BIG event (include/snoutrx.h snrx_ble_bis_t)
+BIS_ENCRYPTED, BIS_FRAMED = 0x01, 0x02
+BIS_DTYPE = np.dtype([("sample_index", "<i8"), ("win_lo", "<i8"), ("win_hi", "<i8"), ("payload_number", "<u8"), ("capture_id", "<u4"),
+                      ("source", "<u4"), ("access_addr", "<u4"), ("crc_init", "<u4"), ("event", "<i4"), ("event_counter", "<u2"),
+                      ("bis", "u1"), ("subevent", "u1"), ("channel", "u1"), ("phy", "u1"), ("phase", "u1"), ("status", "u1"),
+                      ("crc_ok", "u1"), ("flags", "u1"), ("len", "<u2"), ("bytes", "u1", (AUX_MAX_BYTES,)), ("reserved", "u1", (12,))],
+                     align=True)
+assert BIS_DTYPE.itemsize == 336
+
 FRAME_DTYPE = np.dtype([
     ("sample_index", "<i8"), ("capture_id", "<u4"), ("window", "<u4"), ("channel", "<u2"),
     ("proto", "u1"), ("crc_ok", "u1"), ("lqi", "u1"), ("phase", "u1"), ("len", "<u2"),
@@ -157,6 +166,7 @@ SYMBOLS = [
     ("snrx_ble_aux", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_ble_coded", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_ble_periodic", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
+    ("snrx_ble_bis", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_zb_mac_summary", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_frame_rf", c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint32)]),
     ("snrx_exchange_create", c_int, [c_void_p, c_uint32, c_uint32, c_uint32, c_void_p]),

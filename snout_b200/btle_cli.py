@@ -56,6 +56,16 @@ Each AUX_SYNC_IND found is printed as one line of 8 tokens (formats.sync_line):
 
 With `-s` they also go to the pcap, with the train's access address (formats.ble_pcap_sync_block).
 
+`--bis` (with `--wideband`) also receives BLE broadcast isochronous streams (LE Audio broadcast): the BIGInfo in the ACAD
+of every AUX_SYNC_IND that ble_periodic finds describes a BIG (its BISes' access addresses and CRC inits, an ISO interval,
+NSE subevents per BIS on CSA#2 subevent channels), and every subevent of the BIG inside the capture is searched for at its
+predicted place (RxEngine.ble_bis).  Each BIS PDU found is printed as one line of 9 tokens (formats.bis_line):
+
+    BIS Ch<ch> PHY<1M|2M> AA:<access address hex> BIS<n> Evt<BIG event counter> Se<subevent> PloadL<len> CRC<0|1>
+
+Encrypted BISes are printed as sent (they are not decrypted).  With `-s` they also go to the pcap, with the BIS's access
+address (formats.ble_pcap_bis_block).
+
 There is no CPU path: without a usable GPU / libsnoutrx.so the program exits with an error.
 """
 from __future__ import annotations
@@ -111,6 +121,8 @@ USAGE = """Usage:
       With --wideband: also follow BLE 5 extended advertising to its auxiliary packets (1M and 2M PHYs) and print them
     --periodic
       With --wideband: also follow the SyncInfo of every AUX_ADV_IND to its periodic advertising train (AUX_SYNC_IND)
+    --bis
+      With --wideband: also follow the BIGInfo of every AUX_SYNC_IND to its broadcast isochronous streams (BIS PDUs)
     --rf
       Measure signal power, noise floor and carrier offset of every frame; with -s the pcap's PHDR carries the
       signal and noise power (dBFS, flags 0x0002 / 0x0004).  Stdout lines are unchanged
@@ -141,6 +153,7 @@ class Options:
     aux = False
     coded = False
     periodic = False
+    bis = False
 
 
 def _strtol(text: str, base: int) -> int:
@@ -172,7 +185,7 @@ def parse_commandline(argv: list[str], out=sys.stdout) -> Options | None:
         opts, rest = getopt.getopt(argv, "hc:g:a:k:vrf:m:os:",
                                    ["help", "chan=", "gain=", "access=", "crcinit=", "verbose", "raw", "freq_hz=",
                                     "access_mask=", "hop", "filename=", "iq=", "format=", "scale=", "wideband",
-                                    "all-channels", "device=", "shard-windows=", "rf", "aux", "coded", "periodic"])
+                                    "all-channels", "device=", "shard-windows=", "rf", "aux", "coded", "periodic", "bis"])
     except getopt.GetoptError as e:
         out.write(f"btle_rx: {e}\n")
         out.write(USAGE)
@@ -223,6 +236,8 @@ def parse_commandline(argv: list[str], out=sys.stdout) -> Options | None:
             o.coded = True
         elif k == "--periodic":
             o.periodic = True
+        elif k == "--bis":
+            o.bis = True
     if o.chan < 0 or o.chan > MAX_CHANNEL:
         out.write(f"channel number must be within 0~{MAX_CHANNEL}!\n")
         out.write(USAGE)
@@ -261,6 +276,9 @@ def run(o: Options, out=sys.stdout, engine_factory=None, blocks=None) -> int:
         return 1
     if o.periodic and not o.wideband:
         out.write("btle_rx (snout_b200): --periodic needs --wideband (periodic advertising is sent on the data channels)\n")
+        return 1
+    if o.bis and not o.wideband:
+        out.write("btle_rx (snout_b200): --bis needs --wideband (broadcast isochronous streams are sent on the data channels)\n")
         return 1
     if o.iq is None and blocks is None:
         out.write("btle_rx (snout_b200): no IQ source; pass --iq FILE (or - for stdin)\n")
@@ -337,6 +355,14 @@ def run(o: Options, out=sys.stdout, engine_factory=None, blocks=None) -> int:
                 for t in messages.ble_periodic_adv(sync):
                     for ev in t["events"]:
                         out.write(formats.sync_line(t, ev))
+            if o.bis:
+                bis = eng.ble_bis()
+                if fh_pcap:
+                    fh_pcap.write(formats.ble_pcap_bis_block(bis))
+                for g in messages.ble_broadcast_iso(bis):
+                    for st in g["streams"]:
+                        for p in st["pdus"]:
+                            out.write(formats.bis_line(g, st, p))
             out.flush()                                                # fflush(stdout), btle_rx.c:2383
 
         def follow(frames: np.ndarray):

@@ -94,13 +94,19 @@ SNRX_HD int64_t floor_div(int64_t a, int64_t b) {                 // b > 0
 }
 SNRX_HD int64_t ceil_div(int64_t a, int64_t b) { return -floor_div(-a, b); }
 
+// [early(d_lo) - 8, late(d_hi) + 8]: the AA bit 0 positions (4 Msps) of a packet due d_lo..d_hi us after a reference
+// packet, by a clock of p ppm either way (mathematical floor and ceiling; shared by the periodic and the BIS windows)
+SNRX_HD void drift_window(int64_t d_lo, int64_t d_hi, int64_t p, int64_t& lo, int64_t& hi) {
+    lo = (d_lo >= 0 ? floor_div(4 * d_lo * (1000000 - p), 1000000) : floor_div(4 * d_lo * (1000000 + p), 1000000)) - kAuxGuard;
+    hi = (d_hi >= 0 ? ceil_div(4 * d_hi * (1000000 + p), 1000000) : ceil_div(4 * d_hi * (1000000 - p), 1000000)) + kAuxGuard;
+}
+
 // [lo, hi] of AA bit 0 positions of event k, relative to the source's AA bit 0
 SNRX_HD void sync_window(const SyncInfo& si, int64_t k, int64_t& lo, int64_t& hi) {
     const int64_t U = si.units_us, p = sca_ppm(si.sca);
     const int64_t O = (int64_t)si.offset * U + (si.adjust ? kSyncOffsetAdjustUs : 0);
-    const int64_t d_lo = O + k * 1250 * (int64_t)si.interval, d_hi = d_lo + U;
-    lo = (d_lo >= 0 ? floor_div(4 * d_lo * (1000000 - p), 1000000) : floor_div(4 * d_lo * (1000000 + p), 1000000)) - kAuxGuard;
-    hi = (d_hi >= 0 ? ceil_div(4 * d_hi * (1000000 + p), 1000000) : ceil_div(4 * d_hi * (1000000 - p), 1000000)) + kAuxGuard;
+    const int64_t d_lo = O + k * 1250 * (int64_t)si.interval;
+    drift_window(d_lo, d_lo + U, p, lo, hi);
 }
 
 // rule (a): the window is at most half the interval long
@@ -247,9 +253,10 @@ __global__ void __launch_bounds__(256) k_ble_sync_events(const SyncTrain* __rest
     r.status = (l < 0 || x + 1 >= g.n_out) ? SNRX_AUX_OUTSIDE : kAuxPending;
 }
 
-// One warp per pending event of [0, n): the earliest full match of the train's access address in the window, then the
-// decode with the train's CRC init.
-__global__ void __launch_bounds__(128) k_ble_sync_search(snrx_ble_sync_t* __restrict__ list, uint32_t n, AuxGeom g,
+// One warp per pending entry of [0, n): the earliest full match of the entry's access address in its window, then the
+// decode with its CRC init.  E is snrx_ble_sync_t (a periodic event) or snrx_ble_bis_t (a BIS subevent, ble_bis.cuh).
+template <class E>
+__global__ void __launch_bounds__(128) k_ble_sync_search(E* __restrict__ list, uint32_t n, AuxGeom g,
                                                          const uint32_t* __restrict__ crc_tab, const uint8_t* __restrict__ whiten /*[40][260]*/) {
     __shared__ uint32_t crc_s[256];
     __shared__ uint8_t buf_s[4][SNRX_AUX_MAX_BYTES];
@@ -259,7 +266,7 @@ __global__ void __launch_bounds__(128) k_ble_sync_search(snrx_ble_sync_t* __rest
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const uint32_t warps = gridDim.x * (blockDim.x >> 5);
     for (uint32_t k = blockIdx.x * (blockDim.x >> 5) + wib; k < n; k += warps) {
-        snrx_ble_sync_t& r = list[k];
+        E& r = list[k];
         if (r.status != kAuxPending) continue;                    // warp-uniform
         const uint32_t aa = r.access_addr;
         tabs_s[wib].want0[lane] = ((aa >> lane) & 1u) - 1u;

@@ -20,6 +20,7 @@
 #include "ble_aux.cuh"
 #include "ble_coded.cuh"
 #include "ble_sync.cuh"
+#include "ble_bis.cuh"
 #include "ble_back.cuh"
 #include "ble_conn.cuh"
 #include "ble_front.cuh"
@@ -106,6 +107,10 @@ struct snrx_handle {
     // list into d_aux first, and its scans reuse the round buffers once the rounds are done
     snrx::SyncTrain* d_sync_trains = nullptr;
     snrx_ble_sync_t* d_sync = nullptr;
+    // snrx_ble_bis: its BIGs and its list (max_frames entries each), allocated by its first call; it builds the periodic list
+    // into d_sync first
+    snrx::BigGroup* d_bigs = nullptr;
+    snrx_ble_bis_t* d_bis = nullptr;
     uint32_t *d_round_flags = nullptr, *d_round_offsets = nullptr, *d_round_scratch = nullptr;
     uint8_t* d_aux_whiten = nullptr;
     snrx::DevSlot* d_devtab = nullptr;
@@ -417,7 +422,7 @@ void snrx_destroy(snrx_t* h) {
     if (h->adv_stream) { cudaStreamSynchronize(h->adv_stream); cudaStreamDestroy(h->adv_stream); }
     { void* ab[] = {h->d_adv, h->d_zbmac, h->d_conn, h->d_conn_flags, h->d_conn_offsets, h->d_conn_scratch, h->d_follow, h->d_devtab, h->d_devout, h->d_adv_counters,
                     h->d_aux, h->d_coded, h->d_round_flags, h->d_round_offsets, h->d_round_scratch, h->d_aux_whiten,
-                    h->d_sync_trains, h->d_sync}; for (void* b : ab) if (b) cudaFree(b); }
+                    h->d_sync_trains, h->d_sync, h->d_bigs, h->d_bis}; for (void* b : ab) if (b) cudaFree(b); }
     delete h;
 }
 
@@ -1105,7 +1110,7 @@ int snrx_ble_connections(snrx_t* h, snrx_conn_t* out, uint32_t cap, uint32_t* n_
 }  // extern "C"
 
 // The lane of the polled batch, for the calls that search its BLE bit streams again (snrx_ble_follow, snrx_ble_aux,
-// snrx_ble_coded, snrx_ble_periodic): it must hold BLE streams -- of a wideband mode if `wideband` -- that no later batch has overwritten.
+// snrx_ble_coded, snrx_ble_periodic, snrx_ble_bis): it must hold BLE streams -- of a wideband mode if `wideband` -- that no later batch has overwritten.
 static int polled_bits_lane(snrx_handle* h, const char* name, bool wideband, Lane** out) {
     const std::string n = name;
     if (h->polled_lane < 0) return fail(h, SNRX_ESTATE, (n + " needs a polled batch").c_str());
@@ -1186,6 +1191,56 @@ static int copy_list_out(snrx_handle* h, const char* name, const E* list, uint32
         CK(cudaMemcpyAsync(out, list, sizeof(E) * (size_t)total, cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
     }
+    return SNRX_OK;
+}
+
+// The snrx_ble_periodic list of the polled batch into h->d_sync (*total entries), the aux list it comes from built into
+// h->d_aux first with the pointer rounds of snrx_ble_aux; *ln is the polled lane.  Shared by snrx_ble_periodic and
+// snrx_ble_bis (`name` in their errors).
+static int periodic_list(snrx_handle* h, const char* name, Lane** ln_out, uint32_t* total_out) {
+    const std::string nm = name;
+    Lane* ln = nullptr;
+    int r = polled_bits_lane(h, name, true, &ln);
+    if (r != SNRX_OK) return r;
+    *ln_out = ln;
+    CK(cudaSetDevice(h->device));
+    if ((r = round_buffers_init(h)) != SNRX_OK) return r;
+    if (!h->d_aux) CK(cudaMalloc((void**)&h->d_aux, sizeof(snrx_ble_aux_t) * (size_t)h->frame_cap));
+    if (!h->d_sync) {
+        CK(cudaMalloc((void**)&h->d_sync_trains, sizeof(SyncTrain) * (size_t)h->frame_cap));
+        CK(cudaMalloc((void**)&h->d_sync, sizeof(snrx_ble_sync_t) * (size_t)h->frame_cap));
+    }
+    cudaStream_t st = ln->tail;                                  // the lane is idle: its bit streams stay as the batch left them
+    const AuxGeom g = aux_geom_of(*ln);
+    AuxSrc src{};                                                // the aux list, exactly as snrx_ble_aux builds it
+    src.frames = h->polled_frames_dev; src.list = h->d_aux; src.first = 0; src.n = ln->n_frames; src.depth = 0;
+    uint32_t n_aux = 0;
+    r = run_pointer_rounds(h, src, h->d_aux, g, st, &n_aux, (nm + ": more auxiliary pointers than max_frames").c_str());
+    if (r != SNRX_OK) return r;
+    uint32_t total = 0;
+    if (n_aux) {
+        // the trains: flags / offsets over the aux list (n_aux <= max_frames fits the round buffers)
+        k_ble_sync_flag<<<grid_for(h, n_aux, 8, 8), 256, 0, st>>>(h->d_aux, n_aux, h->d_round_flags);
+        exclusive_scan(h->d_round_flags, n_aux, h->d_round_offsets, h->d_round_scratch, st);
+        k_ble_sync_fill<<<div_up(n_aux, 256), 256, 0, st>>>(h->d_aux, n_aux, h->d_round_flags, h->d_round_offsets, h->d_sync_trains);
+        uint32_t n_trains = 0;
+        CK(cudaMemcpyAsync(&n_trains, h->d_round_offsets + n_aux, sizeof n_trains, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        if (n_trains) {
+            // the events: counts / offsets per train, then one entry per listed event, then the search
+            k_ble_sync_count<<<div_up(n_trains, 256), 256, 0, st>>>(h->d_sync_trains, n_trains, g, h->d_round_flags);
+            exclusive_scan(h->d_round_flags, n_trains, h->d_round_offsets, h->d_round_scratch, st);
+            CK(cudaMemcpyAsync(&total, h->d_round_offsets + n_trains, sizeof total, cudaMemcpyDeviceToHost, st));
+            CK(cudaStreamSynchronize(st));
+            if (total > h->frame_cap) return fail(h, SNRX_EOVERFLOW, (nm + ": more periodic events than max_frames").c_str());
+            if (total) {
+                k_ble_sync_events<<<div_up(total, 256), 256, 0, st>>>(h->d_sync_trains, n_trains, h->d_round_offsets, total, g, h->d_sync);
+                k_ble_sync_search<<<grid_for(h, total, 4, 8), 128, 0, st>>>(h->d_sync, total, g, h->d_crc_tab, h->d_aux_whiten);
+            }
+        }
+        CK(cudaGetLastError());
+    }
+    *total_out = total;
     return SNRX_OK;
 }
 
@@ -1286,46 +1341,56 @@ int snrx_ble_periodic(snrx_t* h, snrx_ble_sync_t* out, uint32_t cap, uint32_t* n
     if (!h) return SNRX_EINVAL;
     if (n_out) *n_out = 0;
     Lane* ln = nullptr;
-    int r = polled_bits_lane(h, "snrx_ble_periodic", true, &ln);
+    uint32_t total = 0;
+    const int r = periodic_list(h, "snrx_ble_periodic", &ln, &total);
     if (r != SNRX_OK) return r;
-    CK(cudaSetDevice(h->device));
-    if ((r = round_buffers_init(h)) != SNRX_OK) return r;
-    if (!h->d_aux) CK(cudaMalloc((void**)&h->d_aux, sizeof(snrx_ble_aux_t) * (size_t)h->frame_cap));
-    if (!h->d_sync) {
-        CK(cudaMalloc((void**)&h->d_sync_trains, sizeof(SyncTrain) * (size_t)h->frame_cap));
-        CK(cudaMalloc((void**)&h->d_sync, sizeof(snrx_ble_sync_t) * (size_t)h->frame_cap));
+    return copy_list_out(h, "snrx_ble_periodic", h->d_sync, total, out, cap, n_out, ln->tail);
+}
+
+int snrx_ble_bis(snrx_t* h, snrx_ble_bis_t* out, uint32_t cap, uint32_t* n_out) {
+    if (!h) return SNRX_EINVAL;
+    if (n_out) *n_out = 0;
+    Lane* ln = nullptr;
+    uint32_t n_sync = 0;
+    int r = periodic_list(h, "snrx_ble_bis", &ln, &n_sync);
+    if (r != SNRX_OK) return r;
+    if (!h->d_bis) {
+        CK(cudaMalloc((void**)&h->d_bigs, sizeof(BigGroup) * (size_t)h->frame_cap));
+        CK(cudaMalloc((void**)&h->d_bis, sizeof(snrx_ble_bis_t) * (size_t)h->frame_cap));
     }
     cudaStream_t st = ln->tail;                                  // the lane is idle: its bit streams stay as the batch left them
     const AuxGeom g = aux_geom_of(*ln);
-    AuxSrc src{};                                                // the aux list, exactly as snrx_ble_aux builds it
-    src.frames = h->polled_frames_dev; src.list = h->d_aux; src.first = 0; src.n = ln->n_frames; src.depth = 0;
-    uint32_t n_aux = 0;
-    r = run_pointer_rounds(h, src, h->d_aux, g, st, &n_aux, "snrx_ble_periodic: more auxiliary pointers than max_frames");
-    if (r != SNRX_OK) return r;
     uint32_t total = 0;
-    if (n_aux) {
-        // the trains: flags / offsets over the aux list (n_aux <= max_frames fits the round buffers)
-        k_ble_sync_flag<<<grid_for(h, n_aux, 8, 8), 256, 0, st>>>(h->d_aux, n_aux, h->d_round_flags);
-        exclusive_scan(h->d_round_flags, n_aux, h->d_round_offsets, h->d_round_scratch, st);
-        k_ble_sync_fill<<<div_up(n_aux, 256), 256, 0, st>>>(h->d_aux, n_aux, h->d_round_flags, h->d_round_offsets, h->d_sync_trains);
-        uint32_t n_trains = 0;
-        CK(cudaMemcpyAsync(&n_trains, h->d_round_offsets + n_aux, sizeof n_trains, cudaMemcpyDeviceToHost, st));
+    if (n_sync) {
+        // the BIGs: flags / offsets over the periodic list (n_sync <= max_frames fits the round buffers)
+        k_ble_big_flag<<<grid_for(h, n_sync, 8, 8), 256, 0, st>>>(h->d_sync, n_sync, h->d_round_flags);
+        exclusive_scan(h->d_round_flags, n_sync, h->d_round_offsets, h->d_round_scratch, st);
+        k_ble_big_fill<<<div_up(n_sync, 256), 256, 0, st>>>(h->d_sync, n_sync, h->d_round_flags, h->d_round_offsets, h->d_bigs);
+        uint32_t n_bigs = 0;
+        CK(cudaMemcpyAsync(&n_bigs, h->d_round_offsets + n_sync, sizeof n_bigs, cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
-        if (n_trains) {
-            // the events: counts / offsets per train, then one entry per listed event, then the search
-            k_ble_sync_count<<<div_up(n_trains, 256), 256, 0, st>>>(h->d_sync_trains, n_trains, g, h->d_round_flags);
-            exclusive_scan(h->d_round_flags, n_trains, h->d_round_offsets, h->d_round_scratch, st);
-            CK(cudaMemcpyAsync(&total, h->d_round_offsets + n_trains, sizeof total, cudaMemcpyDeviceToHost, st));
+        if (n_bigs) {
+            // the subevents: counts / offsets per BIG, then one entry per subevent of a listed event, then the search
+            // The counts are summed on the host in 64 bits before the (32-bit) scan: each is at most max_frames + 1, but
+            // n_bigs of them could wrap a 32-bit sum past the overflow test.  Once the sum is at most max_frames the scan
+            // cannot wrap.
+            k_ble_big_count<<<div_up(n_bigs, 256), 256, 0, st>>>(h->d_bigs, n_bigs, g, h->frame_cap, h->d_round_flags);
+            std::vector<uint32_t> counts(n_bigs);
+            CK(cudaMemcpyAsync(counts.data(), h->d_round_flags, sizeof(uint32_t) * (size_t)n_bigs, cudaMemcpyDeviceToHost, st));
             CK(cudaStreamSynchronize(st));
-            if (total > h->frame_cap) return fail(h, SNRX_EOVERFLOW, "snrx_ble_periodic: more periodic events than max_frames");
+            uint64_t sum = 0;
+            for (uint32_t c : counts) sum += c;
+            if (sum > h->frame_cap) return fail(h, SNRX_EOVERFLOW, "snrx_ble_bis: more BIS subevents than max_frames");
+            total = (uint32_t)sum;
+            exclusive_scan(h->d_round_flags, n_bigs, h->d_round_offsets, h->d_round_scratch, st);
             if (total) {
-                k_ble_sync_events<<<div_up(total, 256), 256, 0, st>>>(h->d_sync_trains, n_trains, h->d_round_offsets, total, g, h->d_sync);
-                k_ble_sync_search<<<grid_for(h, total, 4, 8), 128, 0, st>>>(h->d_sync, total, g, h->d_crc_tab, h->d_aux_whiten);
+                k_ble_bis_events<<<div_up(total, 256), 256, 0, st>>>(h->d_bigs, n_bigs, h->d_round_offsets, total, g, h->d_bis);
+                k_ble_sync_search<<<grid_for(h, total, 4, 8), 128, 0, st>>>(h->d_bis, total, g, h->d_crc_tab, h->d_aux_whiten);
             }
         }
         CK(cudaGetLastError());
     }
-    return copy_list_out(h, "snrx_ble_periodic", h->d_sync, total, out, cap, n_out, st);
+    return copy_list_out(h, "snrx_ble_bis", h->d_bis, total, out, cap, n_out, st);
 }
 
 int snrx_zb_mac_summary(snrx_t* h, snrx_zbmac_t* out, uint32_t cap, uint32_t* n_out) {

@@ -330,6 +330,14 @@ class RxEngine:
         include/snoutrx.h).  Wideband BLE modes; call before the second-next process()."""
         return self._polled_list(self.lib.snrx_ble_periodic, _abi.SYNC_DTYPE)
 
+    # ------------------------------------------------------------------ BLE broadcast isochronous streams
+    def ble_bis(self) -> np.ndarray:
+        """The BIS subevents that the BIGInfo of the batch's AUX_SYNC_INDs (as ble_periodic() finds them) describes, on the
+        1M and 2M PHYs: one _abi.BIS_DTYPE entry per subevent of a predicted BIG event inside the batch, with its BIS access
+        address, CRC init, counter, channel, payload number and window, found and decoded on the GPU from the batch's slicer
+        bit streams (definition in include/snoutrx.h).  Wideband BLE modes; call before the second-next process()."""
+        return self._polled_list(self.lib.snrx_ble_bis, _abi.BIS_DTYPE)
+
     # ------------------------------------------------------------------ SURVEY 8(f) N2: Zigbee consumer path
     def zb_mac_summary(self) -> np.ndarray:
         """Per-record MAC summaries (_abi.ZBMAC_DTYPE: frame type, sequence number, PAN ids, addresses, inter-PAN / ZLL

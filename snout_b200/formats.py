@@ -327,6 +327,36 @@ def sync_line(train: dict, ev: dict) -> str:
             f"PloadL{ev['pload_len']} CRC{0 if ev['crc_ok'] else 1}\n")
 
 
+# the LINKTYPE_BLUETOOTH_LE_LL_WITH_PHDR PDU type of broadcast isochronous PDUs, as read from the link-type page (not checked
+# against a dissector here)
+PHDR_PDU_BIS = 6
+
+
+def ble_pcap_bis_block(bis: np.ndarray, ts: tuple[int, int] = (0, 0)) -> bytes:
+    """The BIS PDUs of RxEngine.ble_bis() that were decoded (status OK), as records of the file btle_rx -s writes: PHDR
+    {channel, 0 x 7, flags}, flags = de-whitened | PDU type 6 (broadcast isochronous) << 7 | PHY << 14, then the BIS's access
+    address and header | payload (no CRC).  CRC-failed PDUs are written too; an encrypted payload is written as sent."""
+    a = bis[bis["status"] == AUX_OK]
+    n = len(a)
+    lens = a["len"].astype(np.int64) - 3
+    prefix = np.zeros((n, 16 + 10 + 4), dtype=np.uint8)
+    prefix[:, 0:8] = np.frombuffer(struct.pack("<ii", ts[0], ts[1]), dtype=np.uint8)
+    be = (10 + 4 + lens).astype(">i4").view(np.uint8).reshape(n, 4)
+    prefix[:, 8:12], prefix[:, 12:16] = be, be
+    prefix[:, 16] = a["channel"]
+    flags = PHDR_DEWHITENED | (PHDR_PDU_BIS << PHDR_PDU_TYPE_SHIFT) | (a["phy"].astype(np.int64) << PHDR_PHY_SHIFT)
+    prefix[:, 24:26] = flags.astype("<u2").view(np.uint8).reshape(n, 2)
+    prefix[:, 26:30] = a["access_addr"].astype("<u4").view(np.uint8).reshape(n, 4)
+    return _pack_records(prefix, a["bytes"], lens)
+
+
+def bis_line(big: dict, stream: dict, pdu: dict) -> str:
+    """btle_rx --bis line of one decoded BIS PDU (a BIG of messages.ble_broadcast_iso, one of its streams and one of its
+    PDUs), 9 tokens: BIS Ch<ch> PHY<1M|2M> AA:<hex> BIS<n> Evt<counter> Se<subevent> PloadL<len> CRC<0 ok|1 failed>."""
+    return (f"BIS Ch{pdu['channel']} PHY{big['phy']} AA:{stream['access_addr']:08x} BIS{stream['bis']} Evt{pdu['event_counter']} "
+            f"Se{pdu['subevent']} PloadL{pdu['pload_len']} CRC{0 if pdu['crc_ok'] else 1}\n")
+
+
 def coded_line(d: dict) -> str:
     """btle_rx --coded line of one primary LE Coded ADV_EXT_IND (a messages.ble_coded_adv dictionary of depth 0), 8 tokens:
     CODED Ch<37..39> S<8|2> AdvA:<address or -> ADI:<DID>/<SID> (hex, - if absent) PloadL<len> CRC<0 ok|1 failed> AAerr<d>."""

@@ -223,3 +223,75 @@ def ble_periodic_adv(sync: np.ndarray, aux: np.ndarray | None = None) -> list[di
                                           **fields, acad=acad, big_info=AD_BIGINFO in _ad_types(acad),
                                           chained=fields["aux_ptr"] is not None))
     return list(trains.values())
+
+
+# ----------------------------------------------------------------------------------------- BLE broadcast isochronous streams
+def big_info_fields(b: bytes) -> dict:
+    """The fields of a 33-byte (or, encrypted, 57-byte) BIGInfo (Core Vol 6 Part B 2.3.4.8 as read in include/snoutrx.h):
+    big_offset_us (BIG_Offset x units), iso_interval (1.25 ms units) and iso_interval_ms, num_bis, nse, bn, sub_interval_us,
+    pto, bis_spacing_us, irc, max_pdu, seed_access_addr, sdu_interval_us, max_sdu, base_crc_init, channels (used), phy
+    ('1M' / '2M' / 'Coded' / the raw value), payload_count, framed, encrypted and, when encrypted, giv and gskd."""
+    def le(a, n):
+        return int.from_bytes(bytes(b[a:a + n]), "little")
+    w0, w1, w2, w5, w7, w8 = le(0, 4), le(4, 4), le(8, 4), le(17, 4), le(23, 5), le(28, 5)
+    units = 300 if w0 >> 14 & 1 else 30
+    iso = w0 >> 15 & 0xFFF
+    phy = w7 >> 37 & 7
+    d = dict(big_offset_us=(w0 & 0x3FFF) * units, big_offset_units_us=units, iso_interval=iso, iso_interval_ms=1.25 * iso,
+             num_bis=w0 >> 27 & 0x1F, nse=w1 & 0x1F, bn=w1 >> 5 & 7, sub_interval_us=w1 >> 8 & 0xFFFFF, pto=w1 >> 28 & 0xF,
+             bis_spacing_us=w2 & 0xFFFFF, irc=w2 >> 20 & 0xF, max_pdu=w2 >> 24 & 0xFF, seed_access_addr=le(13, 4),
+             sdu_interval_us=w5 & 0xFFFFF, max_sdu=w5 >> 20 & 0xFFF, base_crc_init=le(21, 2),
+             channels=[c for c in range(37) if w7 >> c & 1], phy=_PHY_NAMES.get(phy, phy), payload_count=w8 & ((1 << 39) - 1),
+             framed=bool(w8 >> 39 & 1), encrypted=len(b) >= 57, giv=None, gskd=None)
+    if d["encrypted"]:
+        d["giv"], d["gskd"] = bytes(b[33:41]), bytes(b[41:57])
+    return d
+
+
+def _big_info_of(pdu: bytes) -> bytes | None:
+    """The BIGInfo bytes of the first AD structure of type 0x2C in a PDU's ACAD (33 or 57 bytes), or None."""
+    _, acad, _ = _ext_walk(pdu)
+    at = 0
+    while at < len(acad) and acad[at] != 0 and at + 1 + acad[at] <= len(acad):
+        if acad[at + 1] == AD_BIGINFO:
+            return bytes(acad[at + 2:at + 1 + acad[at]]) if acad[at] in (34, 58) else None
+        at += 1 + acad[at]
+    return None
+
+
+def ble_broadcast_iso(bis: np.ndarray, sync: np.ndarray | None = None) -> list[dict]:
+    """One dictionary per BIG of RxEngine.ble_bis() (in list order): source (periodic list index), capture_id, phy ('1M' /
+    '2M'), encrypted, framed and, when the periodic list of the same batch is given, big_info (big_info_fields of the source's
+    BIGInfo; None otherwise).  `streams` holds one dictionary per BIS (bis, access_addr, crc_init) with its decoded PDUs
+    (status OK) in list order, each with event (k), event_counter, subevent, channel, sample_index, payload_number, llid,
+    cssn, cstf, pload_len, payload (as sent: an encrypted payload keeps its MIC), crc_ok and encrypted."""
+    bigs: dict = {}
+    for r in bis:
+        key = int(r["source"])
+        if key not in bigs:
+            flags = int(r["flags"])
+            g = dict(source=key, capture_id=int(r["capture_id"]), phy=_PHY_NAMES.get(int(r["phy"]), "1M"),
+                     encrypted=bool(flags & _abi.BIS_ENCRYPTED), framed=bool(flags & _abi.BIS_FRAMED), big_info=None, streams={})
+            if sync is not None and key < len(sync):
+                s = sync[key]
+                b = _big_info_of(bytes(s["bytes"][: int(s["len"])]))
+                if b is not None:
+                    g["big_info"] = big_info_fields(b)
+            bigs[key] = g
+        g = bigs[key]
+        n = int(r["bis"])
+        if n not in g["streams"]:
+            g["streams"][n] = dict(bis=n, access_addr=int(r["access_addr"]), crc_init=int(r["crc_init"]), pdus=[])
+        if int(r["status"]) != _abi.AUX_OK:
+            continue
+        pdu = bytes(r["bytes"][: int(r["len"])])
+        g["streams"][n]["pdus"].append(dict(event=int(r["event"]), event_counter=int(r["event_counter"]), subevent=int(r["subevent"]),
+                                            channel=int(r["channel"]), sample_index=int(r["sample_index"]),
+                                            payload_number=int(r["payload_number"]), llid=pdu[0] & 3, cssn=pdu[0] >> 2 & 7,
+                                            cstf=pdu[0] >> 5 & 1, pload_len=pdu[1], payload=pdu[2:2 + pdu[1]],
+                                            crc_ok=bool(r["crc_ok"]), encrypted=g["encrypted"]))
+    out = []
+    for g in bigs.values():
+        g["streams"] = [g["streams"][n] for n in sorted(g["streams"])]
+        out.append(g)
+    return out

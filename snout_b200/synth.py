@@ -893,6 +893,255 @@ def periodic_adv_capture(seconds: float = 0.1, seed: int = 9700, esn0_db: float 
     return Capture(x.astype(np.complex64), chanplan.WB_RATE, prim, dict(kind="wb_ble_periodic", seed=seed, esn0_db=esn0_db, sync=syncs, aux=auxs))
 
 
+# ------------------------------------------------------------- BLE broadcast isochronous streams (test input)
+# An AUX_SYNC_IND whose ACAD carries a BIGInfo (Core Vol 6 Part B 2.3.4.8 as read in include/snoutrx.h) describes a BIG:
+# Num_BIS streams, each with its own access address (Vol 6 Part B 2.1.2) and CRC init, NSE subevents per ISO interval on the
+# channels of the CSA#2 subevent mapping (Vol 6 Part B 4.5.8.3).  Stated here separately from oracle/bis_oracle.py.
+
+def big_info_bytes(offset: int, units_us: int, iso_interval: int, num_bis: int, nse: int, bn: int, sub_interval: int, pto: int,
+                   bis_spacing: int, irc: int, max_pdu: int, saa: int, sdu_interval: int, max_sdu: int, base_crc: int, chm: int,
+                   phy: int, payload_count: int, framing: int = 0, giv: bytes | None = None, gskd: bytes | None = None) -> bytes:
+    """BIGInfo, little endian: BIG_Offset (14) | units << 14 | ISO_Interval << 15 (12) | Num_BIS << 27 (5); NSE (5) | BN << 5
+    (3) | Sub_Interval << 8 (20) | PTO << 28 (4); BIS_Spacing (20) | IRC << 20 (4) | Max_PDU << 24; RFU; SeedAccessAddress;
+    SDU_Interval (20) | Max_SDU << 20 (12); BaseCRCInit (16); ChM (37) | PHY << 37 (3); bisPayloadCount (39) | Framing << 39;
+    then GIV (8) and GSKD (16) when encrypted (33 or 57 bytes)."""
+    u = 1 if units_us == 300 else 0
+    w0 = (offset & 0x3FFF) | (u << 14) | ((iso_interval & 0xFFF) << 15) | ((num_bis & 0x1F) << 27)
+    w1 = (nse & 0x1F) | ((bn & 7) << 5) | ((sub_interval & 0xFFFFF) << 8) | ((pto & 0xF) << 28)
+    w2 = (bis_spacing & 0xFFFFF) | ((irc & 0xF) << 20) | ((max_pdu & 0xFF) << 24)
+    w5 = (sdu_interval & 0xFFFFF) | ((max_sdu & 0xFFF) << 20)
+    out = (w0.to_bytes(4, "little") + w1.to_bytes(4, "little") + w2.to_bytes(4, "little") + b"\0" + (saa & 0xFFFFFFFF).to_bytes(4, "little")
+           + w5.to_bytes(4, "little") + (base_crc & 0xFFFF).to_bytes(2, "little")
+           + ((chm & ((1 << 37) - 1)) | ((phy & 7) << 37)).to_bytes(5, "little")
+           + ((payload_count & ((1 << 39) - 1)) | ((framing & 1) << 39)).to_bytes(5, "little"))
+    if giv is not None:
+        out += bytes(giv) + bytes(gskd)
+    return out
+
+
+def bis_access_address(saa: int, n: int) -> int:
+    """SAA ^ the diversifier word of BIS n: D = (35 n + 42) mod 128; bits 31..26 = D0, 25 = D1, 24 = D6, 23 = D1, 21 = D5,
+    20 = D4, 18 = D3, 17 = D2, the rest 0."""
+    d = (35 * n + 42) % 128
+    dw = 0
+    for pos, bit in ((31, 0), (30, 0), (29, 0), (28, 0), (27, 0), (26, 0), (25, 1), (24, 6), (23, 1), (21, 5), (20, 4), (18, 3), (17, 2)):
+        dw |= ((d >> bit) & 1) << pos
+    return (saa ^ dw) & 0xFFFFFFFF
+
+
+def bis_crc_seed(base_crc: int, n: int) -> int:
+    """The ble_crc24 `init` of BIS n: the 24-bit CRCInit BaseCRCInit << 8 | n."""
+    return ((base_crc & 0xFFFF) << 8) | (n & 0xFF)
+
+
+def csa2_subevent_channels(counter: int, access_addr: int, used: list[int], nse: int) -> list[int]:
+    """Channels of subevents 0..nse-1: subevent 0 is csa2_channel; then prnSubEvent_lu = MAM(PERM(.)) from prn_s (the
+    three-round value before ^ channelIdentifier), prnSubEvent_se = that ^ channelIdentifier, and the used-channel index moves
+    to (last + d + ((prnSubEvent_se (N - 2d + 1)) >> 16)) mod N, d = max(1, max(min(3, N - 5), min(11, (N - 10) / 2)))."""
+    used = sorted(used)
+    ci = (access_addr >> 16) ^ (access_addr & 0xFFFF)
+
+    def perm_mam(x):
+        lo, hi = x & 0xFF, x >> 8
+        x = int(bin(lo)[2:].zfill(8)[::-1], 2) | (int(bin(hi)[2:].zfill(8)[::-1], 2) << 8)
+        return (17 * x + ci) % 65536
+    x = counter ^ ci
+    for _ in range(3):
+        x = perm_mam(x)
+    ch = csa2_channel(counter, access_addr, used)
+    out, idx, n = [ch], used.index(ch), len(used)
+    d = max(1, min(3, n - 5), min(11, (n - 10) // 2))
+    for _ in range(nse - 1):
+        x = perm_mam(x)
+        idx = (idx + d + (((x ^ ci) * (n - 2 * d + 1)) >> 16)) % n
+        out.append(used[idx])
+    return out
+
+
+def bis_payload_number(payload_count: int, bn: int, irc: int, pto: int, k: int, se: int) -> int:
+    """The payload subevent se of BIG event k (counted from the event bisPayloadCount belongs to) carries: groups of BN
+    subevents; groups below IRC carry the event's own payloads, group g >= IRC those PTO (g - IRC + 1) events ahead."""
+    g, i = se // bn, se % bn
+    ev = payload_count // bn + k + (pto * (g - irc + 1) if g >= irc else 0)
+    return (ev % (1 << 39)) * bn + i
+
+
+@dataclass
+class BisTruth:
+    """A BIS PDU placed into a synthetic capture."""
+    access_addr: int
+    bis: int
+    counter: int          # BIG event counter
+    subevent: int
+    payload_number: int
+    channel: int
+    phy: int              # 0 = LE 1M, 1 = LE 2M
+    start: int            # channel-rate sample of the first preamble sample
+    data: bytes           # pdu | crc (un-whitened)
+    clash: bool = False   # another packet overlaps it on its channel
+
+
+def broadcast_iso_schedule(n_ch: int, rng: np.random.Generator, n_bigs: int = 2, phys=(0, 1), iso_intervals=(6, 8),
+                           num_bis=(2, 4), nse=(2, 6), data_len=(0, 24), adv_interval=(60_000, 120_000), encrypted=(False, True),
+                           cfo_hz: float = 50e3):
+    """BIGs on a 4 Msps time line, each announced by its own periodic train.  BIG b has a random SAA, BaseCRCInit, channel
+    map (2..37 channels), ISO_Interval from `iso_intervals`, Num_BIS and NSE from their ranges (NSE a multiple of BN, with IRC
+    and PTO drawn so that some subevents carry pretransmissions), the sequential arrangement for even b and the interleaved
+    one for odd b, the PHY phys[b mod len], an SCA of 100 ppm or better and a clock error inside it, an encrypted BIGInfo for encrypted[b mod len],
+    and a first event counter that makes some BIGs wrap past 0xFFFF.  Its train (Interval = m ISO_Interval) sends an
+    AUX_SYNC_IND in the idle time of every m-th BIG event whose BIGInfo points at the next event; advertising events
+    (ADV_EXT_IND on 37..39 -> AUX_ADV_IND with the SyncInfo) announce the trains as periodic_adv_schedule's do.  A BIS PDU's
+    payload depends only on its BIS and payload number, so repeats carry the same bytes.  Returns ({bin: stream}, [Truth] of
+    the primaries, [BisTruth], [SyncTruth] of the AUX_SYNC_INDs, [AuxTruth] of the AUX_ADV_INDs, [dict] of the BIGs)."""
+    streams: dict = {}
+    prim, bises, syncs, auxs, bigs = [], [], [], [], []
+    busy: dict[int, list] = {}                       # channel -> [(start, end, ("bis" | "sync", index))]
+    waves = []                                       # (channel, start, bits, sps) placed after all clash marks are known
+    trains = []
+    for b in range(n_bigs):
+        phy = int(phys[b % len(phys)])
+        sps = 2 if phy == 1 else 4
+        tphy = int(phys[(b + 1) % len(phys)])
+        tsps = 2 if tphy == 1 else 4
+        iso = int(iso_intervals[b % len(iso_intervals)])
+        saa = int(rng.integers(1, 1 << 32))
+        aa_t = int(rng.integers(1, 1 << 32))
+        base_crc = int(rng.integers(0, 1 << 16))
+        n_used = int(rng.integers(2, 38))
+        used = sorted(int(c) for c in rng.choice(37, n_used, replace=False))
+        chm = sum(1 << c for c in used)
+        sca = int(rng.integers(3, 8))                                    # 100 ppm or better, as broadcast sources state
+        drift = float(rng.uniform(-0.9, 0.9)) * SCA_PPM[sca] * 1e-6
+        enc = bool(encrypted[b % len(encrypted)])
+        max_len = data_len[1] + (4 if enc else 0)
+        air_us = ((16 if sps == 2 else 8) + 32 + 8 * (2 + max_len + 3)) // (2 if sps == 2 else 1)
+        slot = air_us + 150 + 40
+        sync_us = 8 + 32 + 8 * (2 + 2 + 2 + 59 + 1 + 4 + 3)          # the AUX_SYNC_IND's air time on 1M, an upper bound
+        for _ in range(100):
+            nb = int(rng.integers(num_bis[0], num_bis[1] + 1))
+            bn = int(rng.integers(1, 3))
+            ns = bn * int(rng.integers(max(1, -(-nse[0] // bn)), nse[1] // bn + 1))
+            if nb * ns * slot + sync_us + 600 < 1250 * iso:
+                break
+        else:
+            raise AssertionError("no BIG fits the ISO interval")
+        irc = int(rng.integers(1, ns // bn + 1))
+        pto = int(rng.integers(1, 3)) if irc < ns // bn else 0
+        if b % 2 == 0:
+            sub, spacing = slot, ns * slot                               # sequential
+        else:
+            spacing, sub = slot, nb * slot                               # interleaved
+        span = (nb - 1) * spacing + (ns - 1) * sub + slot
+        m = int(rng.integers(2, 4))
+        e0 = int(rng.integers(65536 - 4, 65536)) + (int(rng.integers(0, 1 << 20)) << 16) if b % 2 == 0 else int(rng.integers(0, 1 << 30))
+        scale = 4.0 / (1.0 + drift)                                      # receiver samples per advertiser us
+        t0 = float(rng.uniform(500, 500 + 5000 * iso))
+        pa0 = int(rng.integers(0, 65536))
+        giv = bytes(rng.integers(0, 256, 8, dtype=np.uint8)) if enc else None
+        gskd = bytes(rng.integers(0, 256, 16, dtype=np.uint8)) if enc else None
+        payloads: dict = {}
+        big = dict(saa=saa, base_crc=base_crc, used=used, chm=chm, iso_interval=iso, num_bis=nb, nse=ns, bn=bn, irc=irc, pto=pto,
+                   sub_interval=sub, bis_spacing=spacing, phy=phy, encrypted=enc, sequential=b % 2 == 0, train_aa=aa_t, sca=sca)
+        bigs.append(big)
+        events = []
+        j = 0
+        while True:
+            a_us = 1250 * iso * j
+            if t0 + (a_us + span + sync_us + 400) * scale + 64 >= n_ch:
+                break
+            counter = (e0 + j) % 65536
+            for n in range(1, nb + 1):
+                aa = bis_access_address(saa, n)
+                chans = csa2_subevent_channels(counter, aa, used, ns)
+                for se in range(ns):
+                    pn = bis_payload_number(e0 * bn, bn, irc, pto, j, se)
+                    if (n, pn) not in payloads:
+                        ln = int(rng.integers(data_len[0], data_len[1] + 1)) + (4 if enc else 0)
+                        hdr0 = (2 if ln else 0) | (int(rng.integers(0, 8)) << 2)
+                        payloads[(n, pn)] = bytes([hdr0, ln]) + bytes(rng.integers(0, 256, ln, dtype=np.uint8))
+                    pdu = payloads[(n, pn)]
+                    start = int(round(t0 + (a_us + (n - 1) * spacing + se * sub) * scale))
+                    bits = (ble_phy_bits_2m if sps == 2 else ble_phy_bits)(pdu, chans[se], access_addr=aa, crc_init=bis_crc_seed(base_crc, n))
+                    bises.append(BisTruth(aa, n, counter, se, pn, chans[se], phy, start, pdu + ble_crc24(pdu, bis_crc_seed(base_crc, n))))
+                    busy.setdefault(chans[se], []).append((start, start + len(bits) * sps, ("bis", len(bises) - 1)))
+                    waves.append((chans[se], start, bits, sps, ("bis", len(bises) - 1)))
+            if j % m == 0:                                               # the train's AUX_SYNC_IND in this event's idle time
+                i = j // m
+                s_us = a_us + span + 300
+                gap_us = 1250 * iso * (j + 1) - s_us                      # to the next event's anchor
+                bi = big_info_bytes(gap_us // 30, 30, iso, nb, ns, bn, sub, pto, spacing, irc, max_len, saa, 1250 * iso, max_len,
+                                    base_crc, chm, phy, ((e0 + j + 1) * bn) % (1 << 39), 0, giv, gskd)
+                acad = bytes([len(bi) + 1, 0x2C]) + bi
+                pdu = ext_pdu(ext_header(0, None, 0, None, None, -5 if i % 2 else None, acad=acad), bytes(rng.integers(0, 256, 4, dtype=np.uint8)))
+                counter_t = (pa0 + i) % 65536
+                ch = csa2_channel(counter_t, aa_t, used)
+                start = int(round(t0 + s_us * scale))
+                bits = (ble_phy_bits_2m if tsps == 2 else ble_phy_bits)(pdu, ch, access_addr=aa_t, crc_init=sync_crc_seed(base_crc << 8 | 0x5A))
+                syncs.append(SyncTruth(aa_t, base_crc << 8 | 0x5A, counter_t, ch, tphy, start, start + 32 + 2 * tsps,
+                                       pdu + ble_crc24(pdu, sync_crc_seed(base_crc << 8 | 0x5A))))
+                busy.setdefault(ch, []).append((start, start + len(bits) * tsps, ("sync", len(syncs) - 1)))
+                waves.append((ch, start, bits, tsps, ("sync", len(syncs) - 1)))
+                events.append((start, len(syncs) - 1))
+            j += 1
+        trains.append(dict(phy=tphy, sps=tsps, aa=aa_t, chm=chm, sca=sca, drift=drift, interval=m * iso, adi=int(rng.integers(0, 1 << 16)),
+                           adv_a=bytes(rng.integers(0, 256, 6, dtype=np.uint8)), crc_init=base_crc << 8 | 0x5A, events=events))
+    # advertising events on a shared time line, the trains taking turns (as periodic_adv_schedule)
+    pos = 2000 + int(rng.integers(0, 4000))
+    p_len = (1 + 4 + 2 + 9 + 3) * 8 * 4 + 16
+    order = 0
+    while True:
+        tr = trains[order % n_bigs]
+        order += 1
+        p_starts = [pos, pos + p_len + 1400, pos + 2 * (p_len + 1400)]
+        a_start = p_starts[2] + p_len + int(rng.integers(1200, 6000))
+        sps = tr["sps"]
+        nxt = [e for e in tr["events"] if e[0] >= a_start + 6000]
+        if not nxt or a_start + 6000 >= n_ch:
+            break
+        e_start, e_idx = nxt[0]
+        off, units, adjust = sync_offset_for(e_start - a_start, tr["drift"])
+        si = sync_info_bytes(off, units, tr["interval"], tr["chm"], tr["sca"], tr["aa"], tr["crc_init"], syncs[e_idx].counter, adjust)
+        pdu = ext_pdu(ext_header(0, tr["adv_a"], 0, tr["adi"], None, 0, sync_info=si))
+        nbits = (16 if sps == 2 else 8) + 32 + 8 * (len(pdu) + 3)
+        a_end = a_start + nbits * sps
+        free = [c for c in range(37) if not any(s < a_end + 64 and a_start < e + 64 for s, e, _ in busy.get(c, []))]
+        ch = int(rng.choice(free))
+        bits = ble_phy_bits_2m(pdu, ch) if sps == 2 else ble_phy_bits(pdu, ch)
+        _put(streams, n_ch, ch, a_start, gfsk_modulate(bits, sps=sps), rng, cfo_hz)
+        busy.setdefault(ch, []).append((a_start, a_end, ("aux", -1)))
+        par = []
+        ca = 1
+        for j, ps in enumerate(p_starts):
+            units_p, off_p, drift_p = aux_offset_for(a_start - ps, ca, rng)
+            pp = ext_pdu(ext_header(0, None, 0, tr["adi"], aux_ptr_bytes(ch, ca, units_p, off_p, tr["phy"])))
+            _put(streams, n_ch, 37 + j, ps, gfsk_modulate(ble_phy_bits(pp, 37 + j)), rng, cfo_hz)
+            prim.append(Truth(37 + j, ps, ps + 8 * 4 + 8, pp + ble_crc24(pp), 3))
+            par.append((37 + j, ps, units_p, off_p, ca, drift_p, a_start - ps))
+        auxs.append(AuxTruth(ch, tr["phy"], a_start, a_start + 32 + 2 * sps, pdu + ble_crc24(pdu), 0, par))
+        pos = max(a_end, p_starts[2] + p_len) + int(rng.integers(adv_interval[0], adv_interval[1] + 1)) // n_bigs
+    for ch, start, bits, sps, who in waves:
+        _put(streams, n_ch, ch, start, gfsk_modulate(bits, sps=sps), rng, cfo_hz)
+        end = start + len(bits) * sps
+        clash = any(o != who and a < end + 64 and start < e + 64 for a, e, o in busy[ch])
+        (bises[who[1]] if who[0] == "bis" else syncs[who[1]]).clash = clash
+    return streams, prim, bises, syncs, auxs, bigs
+
+
+def broadcast_iso_capture(seconds: float = 0.1, seed: int = 9900, esn0_db: float | None = 25.0, **kw) -> Capture:
+    """96 Msps capture (centre 2440 MHz) carrying broadcast_iso_schedule(...) and nothing else; meta["bis"] holds the
+    BisTruth list, meta["sync"] the AUX_SYNC_INDs, meta["aux"] the AUX_ADV_INDs and meta["bigs"] the BIGs.  esn0_db=None: no
+    noise."""
+    rng = np.random.default_rng(seed)
+    n_ch = int(round(seconds * chanplan.NB_RATE))
+    n_ch -= n_ch % chanplan.BLE_WINDOW
+    streams, prim, bises, syncs, auxs, bigs = broadcast_iso_schedule(n_ch, rng, **kw)
+    x = wideband_mix(streams)
+    if esn0_db is not None:
+        x = x + _awgn(len(x), np.random.default_rng(seed + 999), 4.0 * chanplan.WB_DECIM / (10.0 ** (esn0_db / 10.0))).astype(np.complex64)
+    return Capture(x.astype(np.complex64), chanplan.WB_RATE, prim, dict(kind="wb_ble_bis", seed=seed, esn0_db=esn0_db, bis=bises, sync=syncs,
+                                                                       aux=auxs, bigs=bigs))
+
+
 # ------------------------------------------------------------- BLE Long Range (LE Coded PHY, test input)
 # Core Vol 6 Part B 2.2 and 3.3 as read here: rate-1/2 convolutional code with K = 4, G0 = 1 + x + x^2 + x^3 and
 # G1 = 1 + x^2 + x^3 (a0 first), pattern mapper S=8: 0 -> 0011, 1 -> 1100 (S=2: identity).  The packet: 80 symbols of
