@@ -24,17 +24,32 @@ struct AuxPtr {
     int channel, ca, units_us, offset, phy;
 };
 
+// The fields of the extended header by their flag bit (AdvA 6, TargetA 6, CTEInfo 1, ADI 2, AuxPtr 3, SyncInfo 18, TxPower
+// 1 bytes), and the ACAD behind them.
+constexpr int kExtAuxPtr = 4, kExtSyncInfo = 5, kExtAcad = 7;
+
 // pdu = header(2) | payload as stored in the records; n_payload = payload bytes.  True if this is a PDU of type 7 whose extended
-// header carries an AuxPtr (with every field in front of it inside the header).
-SNRX_HD bool aux_ptr_parse(const uint8_t* pdu, int n_payload, AuxPtr& a) {
+// header (length hlen >= 1, 1 + hlen <= n_payload) flags `field` (the ACAD is always there, maybe empty): off = where the
+// field starts and end = 1 + hlen, where the header ends, both counted from the payload's first byte.  Whether the field
+// fits inside the header is the caller's test.
+SNRX_HD bool ext_header_field(const uint8_t* pdu, int n_payload, int field, int& off, int& end) {
     if ((pdu[0] & 0x0F) != 7 || n_payload < 2) return false;
     const uint8_t* p = pdu + 2;
     const int hlen = p[0] & 0x3F;
     if (hlen < 1 || 1 + hlen > n_payload) return false;
-    const int flags = p[1];
-    if (!(flags & 0x10)) return false;
-    const int off = 2 + ((flags & 1) ? 6 : 0) + ((flags & 2) ? 6 : 0) + ((flags & 4) ? 1 : 0) + ((flags & 8) ? 2 : 0);
-    if (off + 3 > 1 + hlen) return false;
+    if (field < kExtAcad && !((p[1] >> field) & 1)) return false;
+    const int flags = p[1] & ((1 << field) - 1);                 // the fields in front
+    off = 2 + ((flags & 1) ? 6 : 0) + ((flags & 2) ? 6 : 0) + ((flags & 4) ? 1 : 0) + ((flags & 8) ? 2 : 0) +
+          ((flags & 0x10) ? 3 : 0) + ((flags & 0x20) ? 18 : 0) + ((flags & 0x40) ? 1 : 0);
+    end = 1 + hlen;
+    return true;
+}
+
+// True if pdu carries an AuxPtr inside its extended header (ext_header_field).
+SNRX_HD bool aux_ptr_parse(const uint8_t* pdu, int n_payload, AuxPtr& a) {
+    int off, end;
+    if (!ext_header_field(pdu, n_payload, kExtAuxPtr, off, end) || off + 3 > end) return false;
+    const uint8_t* p = pdu + 2;
     const int a0 = p[off], a1 = p[off + 1], a2 = p[off + 2];
     a.channel = a0 & 0x3F;
     a.ca = (a0 >> 6) & 1;

@@ -3,14 +3,15 @@
 // (carriers, BIGInfo fields, BIS access addresses and CRC inits, subevent channels, payload numbers, windows, listed events,
 // search, decode, statuses, order) is stated in include/snoutrx.h above snrx_ble_bis_t; oracle/bis_oracle.py restates it.
 //
-// Launched by snrx_ble_bis after the periodic list is built, no atomics and no sort:
-//   k_ble_big_flag / exclusive_scan / k_ble_big_fill     the BIGs, in source order (one warp per periodic entry: the earliest
-//                                                        carrier of its (capture, SAA) by a ballot over the other carriers)
-//   k_ble_big_count / exclusive_scan / k_ble_bis_events  the listed events of every BIG, Num_BIS x NSE entries each, with
-//                                                        their AAs, CRC inits, counters, channels, payload numbers, windows
-//                                                        and OUTSIDE
-//   k_ble_sync_search<snrx_ble_bis_t>                    one warp per entry: windowed search with AA_n, then the decode
-//                                                        with crc_init_n
+// Launched by snrx_ble_bis after the periodic list is built, no atomics and no sort: the schedule kernels of ble_sync.cuh
+// with BigSched,
+//   k_ble_sched_flag / exclusive_scan / k_ble_sched_fill   the BIGs, in source order (one warp per periodic entry: the
+//                                                          earliest carrier of its (capture, SAA) by a ballot over the others)
+//   k_ble_sched_count / exclusive_scan / k_ble_sched_entries  the listed events of every BIG, Num_BIS x NSE entries each,
+//                                                          with their AAs, CRC inits, counters, channels, payload numbers,
+//                                                          windows and OUTSIDE
+//   k_ble_sync_search<snrx_ble_bis_t>                      one warp per entry: windowed search with AA_n, then the decode
+//                                                          with crc_init_n
 #pragma once
 #include "ble_sync.cuh"
 
@@ -58,14 +59,9 @@ SNRX_HD void big_info_decode(const uint8_t* b, int n, BigInfo& bi) {
 // flagged fields and an ACAD whose first AD structure of type 0x2C is a BIGInfo of 33 or 57 bytes (the walk stops at a
 // length-0 structure or one that overruns the ACAD).
 SNRX_HD bool big_info_find(const uint8_t* pdu, int n_payload, BigInfo& bi) {
-    if ((pdu[0] & 0x0F) != 7 || n_payload < 2) return false;
+    int off, end;                                                 // the ACAD is p[off, end)
+    if (!ext_header_field(pdu, n_payload, kExtAcad, off, end)) return false;
     const uint8_t* p = pdu + 2;
-    const int hlen = p[0] & 0x3F;
-    if (hlen < 1 || 1 + hlen > n_payload) return false;
-    const int flags = p[1];
-    const int end = 1 + hlen;                                     // the ACAD is p[off, end)
-    const int off = 2 + ((flags & 1) ? 6 : 0) + ((flags & 2) ? 6 : 0) + ((flags & 4) ? 1 : 0) + ((flags & 8) ? 2 : 0) +
-                    ((flags & 0x10) ? 3 : 0) + ((flags & 0x20) ? 18 : 0) + ((flags & 0x40) ? 1 : 0);
     for (int at = off; at < end && p[at] != 0 && at + 1 + p[at] <= end; at += 1 + p[at]) {
         if (p[at + 1] != kAdBigInfo) continue;
         if (p[at] != 34 && p[at] != 58) return false;
@@ -105,12 +101,6 @@ SNRX_HD uint32_t bis_crc_init(uint32_t base_crc, int n) {
     return ((uint32_t)n << 16) | ((base_crc & 0xFFu) << 8) | ((base_crc >> 8) & 0xFFu);
 }
 
-SNRX_HD uint32_t csa2_perm_mam(uint32_t u, uint32_t cid) {
-    uint32_t v = 0;                                               // PERM: the bits of each byte reversed
-    for (int i = 0; i < 8; i++) v |= (((u >> i) & 0x0101u)) << (7 - i);
-    return (17u * v + cid) & 0xFFFFu;                             // MAM
-}
-
 // The channel of subevent se of the event with counter `counter`, for access address aa and the used channels chm (at least
 // 2): subevent 0 is csa2_channel, each later one steps prnSubEvent_lu from the event's prn_s and moves at least d used
 // channels on from the previous one (Core Vol 6 Part B 4.5.8.3 as read in include/snoutrx.h).
@@ -118,8 +108,7 @@ SNRX_HD int bis_channel(uint32_t counter, uint32_t aa, uint64_t chm, int se) {
     const int ch0 = csa2_channel(counter, aa, chm);
     if (se == 0) return ch0;
     const uint32_t cid = ((aa >> 16) ^ aa) & 0xFFFFu;
-    uint32_t u = (counter ^ cid) & 0xFFFFu;
-    for (int r = 0; r < 3; r++) u = csa2_perm_mam(u, cid);        // prn_s
+    uint32_t u = csa2_prn_s(counter, cid);
     const int n = popcount64(chm);
     const int d3 = n - 5 < 3 ? n - 5 : 3, d11 = (n - 10) / 2 < 11 ? (n - 10) / 2 : 11;
     const int d = d3 > d11 ? (d3 > 1 ? d3 : 1) : (d11 > 1 ? d11 : 1);
@@ -129,9 +118,7 @@ SNRX_HD int bis_channel(uint32_t counter, uint32_t aa, uint64_t chm, int se) {
         const uint32_t prn_se = u ^ cid;
         idx = (int)(((uint32_t)idx + (uint32_t)d + ((prn_se * (uint32_t)(n - 2 * d + 1)) >> 16)) % (uint32_t)n);
     }
-    for (int c = 0; c < 37; c++)
-        if ((chm >> c) & 1u) { if (idx == 0) return c; idx--; }
-    return -1;                                                    // not reached: idx < n
+    return csa2_used_channel(chm, idx);
 }
 
 // the payload number subevent se of event k carries: group g = se / BN (g >= IRC: pretransmissions PTO (g - IRC + 1) events
@@ -185,8 +172,7 @@ SNRX_HD bool big_event_ok(const BigInfo& bi, int p, int64_t k) {
 //   4 S (10^6 - p) / 10^6 - 1 samples past early() of the earlier one, whose window (at most 2 S_min samples, which rule (a)
 //   needs to be at least 4 U + 17 >= 137) then ends more than 2 S_min - 0.002 S_min - 1 > 31 * 4 samples before the later
 //   window starts.
-//   Rule (b).  win_hi(Num_BIS, NSE - 1) + 31 sps >= base (false, then true as k grows) and win_lo(1, 0) <= base + n_out - 2
-//   (true, then false): each bound is stepped from an estimate, as sync_k_range does.
+//   Rule (b).  rule_b_range with the first window's start, win_lo(1, 0), and the last window's end, win_hi(Num_BIS, NSE - 1).
 SNRX_HD void big_k_range(const BigInfo& bi, int p, int64_t s, int sps, int64_t base, int64_t n_out, int64_t& k_lo, int64_t& k_hi) {
     const int64_t I = 1250 * (int64_t)bi.iso_interval, O = (int64_t)bi.offset * bi.units_us, smin = big_s_min(bi);
     const int nb = bi.num_bis, se_last = bi.nse - 1;
@@ -205,124 +191,62 @@ SNRX_HD void big_k_range(const BigInfo& bi, int p, int64_t s, int sps, int64_t b
         if (bis_window_ok(bi, p, a_lo, 1, 0)) { while (bis_window_ok(bi, p, a_lo - 1, 1, 0)) a_lo--; }
         else { while (a_lo < kc - 2 && !bis_window_ok(bi, p, a_lo, 1, 0)) a_lo++; }
     }
-    const int64_t last = base + n_out - 2;
-    auto meets_lo = [&](int64_t k) { int64_t lo, hi; bis_window(bi, p, k, nb, se_last, lo, hi); return s + hi + 31 * sps >= base; };
-    auto meets_hi = [&](int64_t k) { int64_t lo, hi; bis_window(bi, p, k, 1, 0, lo, hi); return s + lo <= last; };
-    auto clamp = [](int64_t k, int64_t a, int64_t b) { return k < a ? a : (k > b ? b : k); };
-    int64_t k = clamp(floor_div(floor_div(base - s, 4) - O, I), a_lo, a_hi);
-    while (k > a_lo && meets_lo(k - 1)) k--;
-    while (k <= a_hi && !meets_lo(k)) k++;
-    k_lo = k;
-    if (k_lo > a_hi) { k_hi = k_lo - 1; return; }
-    k = clamp(floor_div(floor_div(last - s, 4) - O, I), k_lo, a_hi);
-    while (k < a_hi && meets_hi(k + 1)) k++;
-    while (k >= k_lo && !meets_hi(k)) k--;
-    k_hi = k;
+    rule_b_range(a_lo, a_hi, O, I, [&](int64_t k) { int64_t lo, hi; bis_window(bi, p, k, 1, 0, lo, hi); return lo; },
+                 [&](int64_t k) { int64_t lo, hi; bis_window(bi, p, k, nb, se_last, lo, hi); return hi; }, s, sps, base, n_out, k_lo, k_hi);
 }
 
 struct BigGroup {
     BigInfo bi;
     int64_t s;                    // the source's sample_index
-    int64_t k_lo;                 // first listed event (k_ble_big_count)
+    int64_t k_lo;                 // first listed event (k_ble_sched_count)
     uint32_t capture_id, source;
     int ppm;                      // of the source's train's SCA
 };
 
 #if defined(__CUDACC__)
-// periodic entry i is a carrier (status OK, crc_ok, a valid BIGInfo)
-__device__ __forceinline__ bool big_carrier(const snrx_ble_sync_t& r, BigInfo& bi) {
-    return r.status == SNRX_AUX_OK && r.crc_ok && r.len >= 5 && big_info_find(r.bytes, (int)r.len - 5, bi) && big_info_valid(bi);
-}
-
-// One warp per periodic entry of [0, n): flags[i] = 1 when entry i is the source of its (capture, SAA) BIG -- no other
-// carrier of the same (capture, SAA) has a smaller sample_index, or the same one and a lower index.
-__global__ void __launch_bounds__(256) k_ble_big_flag(const snrx_ble_sync_t* __restrict__ sync, uint32_t n, uint32_t* __restrict__ flags) {
-    const int lane = threadIdx.x & 31;
-    const uint32_t warps = gridDim.x * (blockDim.x >> 5);
-    for (uint32_t i = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); i < n; i += warps) {
-        const snrx_ble_sync_t& r = sync[i];
+// snrx_ble_bis: periodic entry -> BigGroup -> Num_BIS x NSE entries per listed event (the schedule kernels of ble_sync.cuh)
+struct BigSched {
+    using Src = snrx_ble_sync_t;
+    using Group = BigGroup;
+    using Entry = snrx_ble_bis_t;
+    // a carrier (status OK, crc_ok, a valid BIGInfo); grouped by its SAA
+    static __device__ __forceinline__ bool candidate(const Src& r, uint32_t, uint32_t& key) {
         BigInfo bi;
-        bool src = big_carrier(r, bi);                            // warp-uniform
-        for (uint32_t b = 0; src && b < n; b += 32) {
-            const uint32_t j = b + lane;
-            bool earlier = false;
-            if (j < n && j != i) {
-                const snrx_ble_sync_t& o = sync[j];
-                BigInfo bo;
-                earlier = o.capture_id == r.capture_id && (o.sample_index < r.sample_index || (o.sample_index == r.sample_index && j < i)) &&
-                          big_carrier(o, bo) && bo.saa == bi.saa;
-            }
-            if (__ballot_sync(0xffffffffu, earlier)) src = false;
-        }
-        if (lane == 0) flags[i] = src ? 1u : 0u;
+        if (!(r.status == SNRX_AUX_OK && r.crc_ok && r.len >= 5 && big_info_find(r.bytes, (int)r.len - 5, bi) && big_info_valid(bi))) return false;
+        key = bi.saa;
+        return true;
     }
-}
-
-__global__ void __launch_bounds__(256) k_ble_big_fill(const snrx_ble_sync_t* __restrict__ sync, uint32_t n, const uint32_t* __restrict__ flags,
-                                                      const uint32_t* __restrict__ offsets, BigGroup* __restrict__ bigs) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n || !flags[i]) return;
-    const snrx_ble_sync_t& r = sync[i];
-    BigGroup b{};
-    big_info_find(r.bytes, (int)r.len - 5, b.bi);
-    b.s = r.sample_index; b.capture_id = r.capture_id; b.source = i; b.ppm = sca_ppm(r.sca);
-    bigs[offsets[i]] = b;
-}
-
-// one thread per BIG: its listed k range, counts[t] = events x Num_BIS x NSE entries, capped at max_frames + 1 (the caller
-// sums the counts in 64 bits and refuses more than max_frames before it scans them)
-__global__ void __launch_bounds__(256) k_ble_big_count(BigGroup* __restrict__ bigs, uint32_t n_bigs, AuxGeom g, uint32_t cap,
-                                                       uint32_t* __restrict__ counts) {
-    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= n_bigs) return;
-    BigGroup& b = bigs[t];
-    int64_t k_lo, k_hi;
-    big_k_range(b.bi, b.ppm, b.s, b.bi.phy == SNRX_AUX_PHY_2M ? 2 : 4, g.base, g.n_out, k_lo, k_hi);
-    b.k_lo = k_lo;
-    const int64_t m = k_hi >= k_lo ? (k_hi - k_lo + 1) * b.bi.num_bis * b.bi.nse : 0;
-    counts[t] = (uint32_t)(m > (int64_t)cap ? (int64_t)cap + 1 : m);
-}
-
-// one thread per entry: its BIS, subevent, AA, CRC init, counter, channel, payload number, window and OUTSIDE (or pending);
-// offsets[0..n_bigs] are the BIGs' first entries
-__global__ void __launch_bounds__(256) k_ble_bis_events(const BigGroup* __restrict__ bigs, uint32_t n_bigs,
-                                                        const uint32_t* __restrict__ offsets, uint32_t total, AuxGeom g,
-                                                        snrx_ble_bis_t* __restrict__ list) {
-    const uint32_t e = blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= total) return;
-    uint32_t a = 0, b = n_bigs;                                   // the last t with offsets[t] <= e
-    while (b - a > 1) { const uint32_t m = (a + b) >> 1; if (offsets[m] <= e) a = m; else b = m; }
-    const BigGroup& big = bigs[a];
-    const BigInfo& bi = big.bi;
-    const uint32_t local = e - offsets[a], per_event = (uint32_t)(bi.num_bis * bi.nse);
-    const int64_t k = big.k_lo + (int64_t)(local / per_event);
-    const int n = (int)((local % per_event) / (uint32_t)bi.nse) + 1, se = (int)(local % (uint32_t)bi.nse);
-    snrx_ble_bis_t& r = list[e];
-    uint4* d = reinterpret_cast<uint4*>(&r);
-#pragma unroll
-    for (int q = 0; q < (int)(sizeof(snrx_ble_bis_t) / 16); q++) d[q] = make_uint4(0u, 0u, 0u, 0u);
-    int64_t lo, hi;
-    bis_window(bi, big.ppm, k, n, se, lo, hi);
-    const uint32_t counter = ((uint32_t)(bi.payload_count / (uint64_t)bi.bn) + (uint32_t)k) & 0xFFFFu;
-    const uint32_t aa = bis_access_address(bi.saa, n);
-    r.sample_index = -1;
-    r.win_lo = big.s + lo; r.win_hi = big.s + hi;
-    r.payload_number = bis_payload_number(bi, k, se);
-    r.capture_id = big.capture_id;
-    r.source = big.source;
-    r.access_addr = aa;
-    r.crc_init = bis_crc_init(bi.base_crc, n);
-    r.event = (int32_t)k;
-    r.event_counter = (uint16_t)counter;
-    r.bis = (uint8_t)n;
-    r.subevent = (uint8_t)se;
-    r.channel = (uint8_t)bis_channel(counter, aa, bi.chm, se);
-    r.phy = (uint8_t)bi.phy;
-    r.flags = (uint8_t)((bi.encrypted ? SNRX_BIS_ENCRYPTED : 0) | (bi.framing ? SNRX_BIS_FRAMED : 0));
-    const int sps = bi.phy == SNRX_AUX_PHY_2M ? 2 : 4;
-    const int64_t l = r.win_lo - g.base, x = r.win_hi - g.base + 31 * sps;      // local first / last decision of the search
-    r.status = (l < 0 || x + 1 >= g.n_out) ? SNRX_AUX_OUTSIDE : (aa == 0u ? SNRX_AUX_NOT_FOUND : kAuxPending);
-}
+    static __device__ __forceinline__ Group group(const Src& r, uint32_t i) {
+        BigGroup b{};
+        big_info_find(r.bytes, (int)r.len - 5, b.bi);
+        b.s = r.sample_index; b.capture_id = r.capture_id; b.source = i; b.ppm = sca_ppm(r.sca);
+        return b;
+    }
+    static __device__ __forceinline__ void k_range(const Group& b, const AuxGeom& g, int64_t& k_lo, int64_t& k_hi) {
+        big_k_range(b.bi, b.ppm, b.s, b.bi.phy == SNRX_AUX_PHY_2M ? 2 : 4, g.base, g.n_out, k_lo, k_hi);
+    }
+    static __device__ __forceinline__ uint32_t per_event(const Group& b) { return (uint32_t)(b.bi.num_bis * b.bi.nse); }
+    // entry j = (n - 1) NSE + se: BIS n, subevent se.  A BIS whose AA is 0 is not searched.
+    static __device__ __forceinline__ uint8_t entry(const Group& b, int64_t k, uint32_t j, Entry& r) {
+        const BigInfo& bi = b.bi;
+        const int n = (int)(j / (uint32_t)bi.nse) + 1, se = (int)(j % (uint32_t)bi.nse);
+        int64_t lo, hi;
+        bis_window(bi, b.ppm, k, n, se, lo, hi);
+        const uint32_t counter = ((uint32_t)(bi.payload_count / (uint64_t)bi.bn) + (uint32_t)k) & 0xFFFFu;
+        const uint32_t aa = bis_access_address(bi.saa, n);
+        r.win_lo = b.s + lo; r.win_hi = b.s + hi;
+        r.payload_number = bis_payload_number(bi, k, se);
+        r.access_addr = aa;
+        r.crc_init = bis_crc_init(bi.base_crc, n);
+        r.event_counter = (uint16_t)counter;
+        r.bis = (uint8_t)n;
+        r.subevent = (uint8_t)se;
+        r.channel = (uint8_t)bis_channel(counter, aa, bi.chm, se);
+        r.phy = (uint8_t)bi.phy;
+        r.flags = (uint8_t)((bi.encrypted ? SNRX_BIS_ENCRYPTED : 0) | (bi.framing ? SNRX_BIS_FRAMED : 0));
+        return aa == 0u ? SNRX_AUX_NOT_FOUND : kAuxPending;
+    }
+};
 #endif  // __CUDACC__
 
 }  // namespace snrx

@@ -3,10 +3,11 @@
 // (train sources, SyncInfo fields, CSA#2, windows, listed events, search, decode, statuses, order) is stated in
 // include/snoutrx.h above snrx_ble_sync_t; oracle/periodic_oracle.py restates it.
 //
-// Launched by snrx_ble_periodic after the pointer rounds of snrx_ble_aux, no atomics and no sort:
-//   k_ble_sync_flag / exclusive_scan / k_ble_sync_fill   the trains, in source order (one warp per aux entry: the earliest
+// Launched by snrx_ble_periodic after the pointer rounds of snrx_ble_aux, no atomics and no sort; the schedule kernels are
+// shared with snrx_ble_bis (ble_bis.cuh), SyncSched is this list's instance:
+//   k_ble_sched_flag / exclusive_scan / k_ble_sched_fill   the trains, in source order (one warp per aux entry: the earliest
 //                                                         source of its (capture, AA) by a ballot over the other candidates)
-//   k_ble_sync_count / exclusive_scan / k_ble_sync_events  the listed events of every train, in ascending k, with their
+//   k_ble_sched_count / exclusive_scan / k_ble_sched_entries  the listed events of every train, in ascending k, with their
 //                                                         counters, CSA#2 channels, windows and OUTSIDE
 //   k_ble_sync_search                                    one warp per event: windowed search with the train's AA, then the
 //                                                         decode that k_ble_aux_search uses, with the train's CRC init
@@ -26,18 +27,12 @@ struct SyncInfo {
     uint32_t pa_counter;
 };
 
-// pdu = header(2) | payload; n_payload = payload bytes.  True if this is a PDU of type 7 whose extended header carries a
-// SyncInfo (with every field in front of it inside the header).
+// pdu = header(2) | payload; n_payload = payload bytes.  True if pdu carries a SyncInfo inside its extended header
+// (ext_header_field).
 SNRX_HD bool sync_info_parse(const uint8_t* pdu, int n_payload, SyncInfo& si) {
-    if ((pdu[0] & 0x0F) != 7 || n_payload < 2) return false;
-    const uint8_t* p = pdu + 2;
-    const int hlen = p[0] & 0x3F;
-    if (hlen < 1 || 1 + hlen > n_payload) return false;
-    const int flags = p[1];
-    if (!(flags & 0x20)) return false;
-    const int off = 2 + ((flags & 1) ? 6 : 0) + ((flags & 2) ? 6 : 0) + ((flags & 4) ? 1 : 0) + ((flags & 8) ? 2 : 0) + ((flags & 0x10) ? 3 : 0);
-    if (off + 18 > 1 + hlen) return false;
-    const uint8_t* b = p + off;
+    int off, end;
+    if (!ext_header_field(pdu, n_payload, kExtSyncInfo, off, end) || off + 18 > end) return false;
+    const uint8_t* b = pdu + 2 + off;
     const int o = b[0] | (b[1] << 8);
     si.offset = o & 0x1FFF;
     si.units_us = (o & 0x2000) ? 300 : 30;
@@ -69,23 +64,34 @@ SNRX_HD int sca_ppm(int sca) {
     return ppm[sca & 7];
 }
 
-// Channel Selection Algorithm #2 (Core Vol 6 Part B 4.5.8.3): the channel of event counter `counter` for access address aa
-// and the used channels chm (at least one).
-SNRX_HD int csa2_channel(uint32_t counter, uint32_t aa, uint64_t chm) {
-    const uint32_t cid = ((aa >> 16) ^ aa) & 0xFFFFu;
+// Channel Selection Algorithm #2 (Core Vol 6 Part B 4.5.8.3), shared by the periodic events and the BIS subevents.
+SNRX_HD uint32_t csa2_perm_mam(uint32_t u, uint32_t cid) {
+    uint32_t v = 0;                                               // PERM: the bits of each byte reversed
+    for (int i = 0; i < 8; i++) v |= (((u >> i) & 0x0101u)) << (7 - i);
+    return (17u * v + cid) & 0xFFFFu;                             // MAM
+}
+
+// prn_s of event counter `counter` for channel identifier cid
+SNRX_HD uint32_t csa2_prn_s(uint32_t counter, uint32_t cid) {
     uint32_t u = (counter ^ cid) & 0xFFFFu;
-    for (int r = 0; r < 3; r++) {
-        uint32_t v = 0;                                           // PERM: the bits of each byte reversed
-        for (int i = 0; i < 8; i++) v |= (((u >> i) & 0x0101u)) << (7 - i);
-        u = (17u * v + cid) & 0xFFFFu;                            // MAM
-    }
-    const uint32_t prn_e = u ^ cid;
-    const int unmapped = (int)(prn_e % 37u);
-    if ((chm >> unmapped) & 1u) return unmapped;
-    int idx = (int)(((uint32_t)popcount64(chm) * prn_e) >> 16);
+    for (int r = 0; r < 3; r++) u = csa2_perm_mam(u, cid);
+    return u;
+}
+
+// the idx-th used channel of chm (idx below the number of used channels)
+SNRX_HD int csa2_used_channel(uint64_t chm, int idx) {
     for (int c = 0; c < 37; c++)
         if ((chm >> c) & 1u) { if (idx == 0) return c; idx--; }
-    return -1;                                                    // not reached: idx < the number of used channels
+    return -1;                                                    // not reached
+}
+
+// the channel of event counter `counter` for access address aa and the used channels chm (at least one)
+SNRX_HD int csa2_channel(uint32_t counter, uint32_t aa, uint64_t chm) {
+    const uint32_t cid = ((aa >> 16) ^ aa) & 0xFFFFu;
+    const uint32_t prn_e = csa2_prn_s(counter, cid) ^ cid;
+    const int unmapped = (int)(prn_e % 37u);
+    if ((chm >> unmapped) & 1u) return unmapped;
+    return csa2_used_channel(chm, (int)(((uint32_t)popcount64(chm) * prn_e) >> 16));
 }
 
 SNRX_HD int64_t floor_div(int64_t a, int64_t b) {                 // b > 0
@@ -116,25 +122,18 @@ SNRX_HD bool sync_rule_a(const SyncInfo& si, int64_t k) {
     return hi - lo + 1 <= 2500 * (int64_t)si.interval;
 }
 
-// The listed k of a train whose source's AA bit 0 is at capture index s, in a buffer of local decisions [0, n_out - 2] whose
-// sample 0 is capture index base: [k_lo, k_hi], empty when k_lo > k_hi.  Rule (a) holds on one contiguous range around the
-// k where D changes sign (the width grows by at least 1.2 samples per event on either side, more than the two roundings can
-// take back), and rule (b) on another, so each bound is found by stepping a monotone test from an estimate.  Every D met
-// has |D| <= 2500 * 65535 * 10^6 / (8 * 20) us + one interval: 4 |D| 10^6 stays inside int64.
-SNRX_HD void sync_k_range(const SyncInfo& si, int64_t s, int sps, int64_t base, int64_t n_out, int64_t& k_lo, int64_t& k_hi) {
-    const int64_t I = 1250 * (int64_t)si.interval, U = si.units_us, p = sca_ppm(si.sca);
-    const int64_t O = (int64_t)si.offset * U + (si.adjust ? kSyncOffsetAdjustUs : 0);
-    const int64_t kc = ceil_div(-O, I);                           // the first k with D_lo >= 0; kc - 1 and kc satisfy (a)
-    const int64_t dmax = (2500 * (int64_t)si.interval) * 1000000 / (8 * p);
-    int64_t a_hi = kc + dmax / I, a_lo = kc - 1 - dmax / I;
-    while (!sync_rule_a(si, a_hi)) a_hi--;
-    while (sync_rule_a(si, a_hi + 1)) a_hi++;
-    while (!sync_rule_a(si, a_lo)) a_lo++;
-    while (sync_rule_a(si, a_lo - 1)) a_lo--;
-    // rule (b): win_hi + 31 sps >= base (false, then true as k grows) and win_lo <= base + n_out - 2 (true, then false)
+// Rule (b) of a schedule list on the rule-(a) range [a_lo, a_hi]: the listed [k_lo, k_hi] (empty when k_lo > k_hi) of a
+// schedule whose source's AA bit 0 is at capture index s, in a buffer of local decisions [0, n_out - 2] whose sample 0 is
+// capture index base.  win_lo(k) is the start of event k's first window and win_hi(k) the end of its last one, relative to
+// s.  Both grow with k, so s + win_hi(k) + 31 sps >= base is false, then true as k grows, and s + win_lo(k) <= base +
+// n_out - 2 is true, then false: each bound is stepped from the estimate floor((floor((x - s) / 4) - O) / I), the event
+// whose D_lo (O + k I us after the source) is due at capture index x.
+template <class WinLo, class WinHi>
+SNRX_HD void rule_b_range(int64_t a_lo, int64_t a_hi, int64_t O, int64_t I, WinLo win_lo, WinHi win_hi, int64_t s, int sps,
+                          int64_t base, int64_t n_out, int64_t& k_lo, int64_t& k_hi) {
     const int64_t last = base + n_out - 2;
-    auto meets_lo = [&](int64_t k) { int64_t lo, hi; sync_window(si, k, lo, hi); return s + hi + 31 * sps >= base; };
-    auto meets_hi = [&](int64_t k) { int64_t lo, hi; sync_window(si, k, lo, hi); return s + lo <= last; };
+    auto meets_lo = [&](int64_t k) { return s + win_hi(k) + 31 * sps >= base; };
+    auto meets_hi = [&](int64_t k) { return s + win_lo(k) <= last; };
     auto clamp = [](int64_t k, int64_t a, int64_t b) { return k < a ? a : (k > b ? b : k); };
     int64_t k = clamp(floor_div(floor_div(base - s, 4) - O, I), a_lo, a_hi);
     while (k > a_lo && meets_lo(k - 1)) k--;
@@ -147,6 +146,24 @@ SNRX_HD void sync_k_range(const SyncInfo& si, int64_t s, int sps, int64_t base, 
     k_hi = k;
 }
 
+// The listed k of a train (rule_b_range's arguments): rule (a) holds on one contiguous range around the k where D changes
+// sign (the width grows by at least 1.2 samples per event on either side, more than the two roundings can take back), found
+// by stepping a monotone test from an estimate.  Every D met has |D| <= 2500 * 65535 * 10^6 / (8 * 20) us + one interval:
+// 4 |D| 10^6 stays inside int64.
+SNRX_HD void sync_k_range(const SyncInfo& si, int64_t s, int sps, int64_t base, int64_t n_out, int64_t& k_lo, int64_t& k_hi) {
+    const int64_t I = 1250 * (int64_t)si.interval, U = si.units_us, p = sca_ppm(si.sca);
+    const int64_t O = (int64_t)si.offset * U + (si.adjust ? kSyncOffsetAdjustUs : 0);
+    const int64_t kc = ceil_div(-O, I);                           // the first k with D_lo >= 0; kc - 1 and kc satisfy (a)
+    const int64_t dmax = (2500 * (int64_t)si.interval) * 1000000 / (8 * p);
+    int64_t a_hi = kc + dmax / I, a_lo = kc - 1 - dmax / I;
+    while (!sync_rule_a(si, a_hi)) a_hi--;
+    while (sync_rule_a(si, a_hi + 1)) a_hi++;
+    while (!sync_rule_a(si, a_lo)) a_lo++;
+    while (sync_rule_a(si, a_lo - 1)) a_lo--;
+    rule_b_range(a_lo, a_hi, O, I, [&](int64_t k) { int64_t lo, hi; sync_window(si, k, lo, hi); return lo; },
+                 [&](int64_t k) { int64_t lo, hi; sync_window(si, k, lo, hi); return hi; }, s, sps, base, n_out, k_lo, k_hi);
+}
+
 // the CRC register seed of a crc_init given as c0 << 16 | c1 << 8 | c2 (btle_rx.c crc_init_reorder: byte swap, 24-bit
 // bit reversal)
 SNRX_HD uint32_t crc_seed_of(uint32_t crc_init) {
@@ -156,102 +173,138 @@ SNRX_HD uint32_t crc_seed_of(uint32_t crc_init) {
     return r;
 }
 
+// A periodic-advertising train: the group SyncSched builds from its source
 struct SyncTrain {
     SyncInfo si;
     int64_t s;                    // the source's sample_index
-    int64_t k_lo;                 // first listed event (k_ble_sync_count)
+    int64_t k_lo;                 // first listed event (k_ble_sched_count)
     uint32_t capture_id, source;
     int phy;
 };
 
 #if defined(__CUDACC__)
-// aux entry i is a candidate source (status OK, crc_ok, first == i, a valid SyncInfo)
-__device__ __forceinline__ bool sync_candidate(const snrx_ble_aux_t& r, uint32_t i, SyncInfo& si) {
-    return r.status == SNRX_AUX_OK && r.crc_ok && r.first == i && r.len >= 5 && sync_info_parse(r.bytes, (int)r.len - 5, si) &&
-           sync_info_valid(si);
-}
+// The schedule lists (snrx_ble_periodic, snrx_ble_bis) are built by the kernels below, templated on a schedule S that
+// supplies, from its source entries S::Src:
+//   candidate(r, i, key)   entry i is a candidate source, and its key: one group per (capture, key)
+//   group(r, i)            the S::Group a source describes (s, capture_id, source and what its events need)
+//   k_range(grp, g, ..)    the group's listed k; per_event(grp): the entries of one event
+//   entry(grp, k, j, r)    entry j of event k: every field of r but those the kernel sets (zero bytes, sample_index -1,
+//                          capture_id, source, event, OUTSIDE); returns its status inside the buffer
 
-// One warp per aux entry of [0, n): flags[i] = 1 when entry i is the source of its (capture, AA) train -- no other candidate
-// of the same (capture, AA) has a smaller sample_index, or the same one and a lower index.
-__global__ void __launch_bounds__(256) k_ble_sync_flag(const snrx_ble_aux_t* __restrict__ aux, uint32_t n, uint32_t* __restrict__ flags) {
+// One warp per source entry of [0, n): flags[i] = 1 when entry i is the source of its (capture, key) group -- no other
+// candidate of the same (capture, key) has a smaller sample_index, or the same one and a lower index.
+template <class S>
+__global__ void __launch_bounds__(256) k_ble_sched_flag(const typename S::Src* __restrict__ src, uint32_t n, uint32_t* __restrict__ flags) {
     const int lane = threadIdx.x & 31;
     const uint32_t warps = gridDim.x * (blockDim.x >> 5);
     for (uint32_t i = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); i < n; i += warps) {
-        const snrx_ble_aux_t& r = aux[i];
-        SyncInfo si;
-        bool src = sync_candidate(r, i, si);                      // warp-uniform
-        for (uint32_t b = 0; src && b < n; b += 32) {
+        const typename S::Src& r = src[i];
+        uint32_t key, ko;
+        bool first = S::candidate(r, i, key);                     // warp-uniform
+        for (uint32_t b = 0; first && b < n; b += 32) {
             const uint32_t j = b + lane;
             bool earlier = false;
             if (j < n && j != i) {
-                const snrx_ble_aux_t& o = aux[j];
-                SyncInfo so;
-                earlier = o.capture_id == r.capture_id && sync_candidate(o, j, so) && so.aa == si.aa &&
-                          (o.sample_index < r.sample_index || (o.sample_index == r.sample_index && j < i));
+                const typename S::Src& o = src[j];
+                earlier = o.capture_id == r.capture_id && (o.sample_index < r.sample_index || (o.sample_index == r.sample_index && j < i)) &&
+                          S::candidate(o, j, ko) && ko == key;
             }
-            if (__ballot_sync(0xffffffffu, earlier)) src = false;
+            if (__ballot_sync(0xffffffffu, earlier)) first = false;
         }
-        if (lane == 0) flags[i] = src ? 1u : 0u;
+        if (lane == 0) flags[i] = first ? 1u : 0u;
     }
 }
 
-__global__ void __launch_bounds__(256) k_ble_sync_fill(const snrx_ble_aux_t* __restrict__ aux, uint32_t n, const uint32_t* __restrict__ flags,
-                                                       const uint32_t* __restrict__ offsets, SyncTrain* __restrict__ trains) {
+template <class S>
+__global__ void __launch_bounds__(256) k_ble_sched_fill(const typename S::Src* __restrict__ src, uint32_t n, const uint32_t* __restrict__ flags,
+                                                        const uint32_t* __restrict__ offsets, typename S::Group* __restrict__ groups) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n || !flags[i]) return;
-    const snrx_ble_aux_t& r = aux[i];
-    SyncTrain t{};
-    sync_info_parse(r.bytes, (int)r.len - 5, t.si);
-    t.s = r.sample_index; t.capture_id = r.capture_id; t.source = i; t.phy = r.phy;
-    trains[offsets[i]] = t;
+    groups[offsets[i]] = S::group(src[i], i);
 }
 
-// one thread per train: its listed k range, counts[t] events
-__global__ void __launch_bounds__(256) k_ble_sync_count(SyncTrain* __restrict__ trains, uint32_t n_trains, AuxGeom g,
-                                                        uint32_t* __restrict__ counts) {
+// one thread per group: its listed k range, counts[t] = its entries, capped at max_frames + 1 (the caller sums the counts
+// in 64 bits and refuses more than max_frames before it scans them)
+template <class S>
+__global__ void __launch_bounds__(256) k_ble_sched_count(typename S::Group* __restrict__ groups, uint32_t n_groups, AuxGeom g, uint32_t cap,
+                                                         uint32_t* __restrict__ counts) {
     const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= n_trains) return;
-    SyncTrain& tr = trains[t];
+    if (t >= n_groups) return;
+    typename S::Group& grp = groups[t];
     int64_t k_lo, k_hi;
-    sync_k_range(tr.si, tr.s, tr.phy == SNRX_AUX_PHY_2M ? 2 : 4, g.base, g.n_out, k_lo, k_hi);
-    tr.k_lo = k_lo;
-    counts[t] = k_hi >= k_lo ? (uint32_t)(k_hi - k_lo + 1) : 0u;
+    S::k_range(grp, g, k_lo, k_hi);
+    grp.k_lo = k_lo;
+    const int64_t m = k_hi >= k_lo ? (k_hi - k_lo + 1) * S::per_event(grp) : 0;
+    counts[t] = (uint32_t)(m > (int64_t)cap ? (int64_t)cap + 1 : m);
 }
 
-// one thread per listed event: the entry with its counter, channel, window and OUTSIDE (or pending); offsets[0..n_trains]
-// are the trains' first entries
-__global__ void __launch_bounds__(256) k_ble_sync_events(const SyncTrain* __restrict__ trains, uint32_t n_trains,
-                                                         const uint32_t* __restrict__ offsets, uint32_t total, AuxGeom g,
-                                                         snrx_ble_sync_t* __restrict__ list) {
+// one thread per listed entry: S::entry's fields, then OUTSIDE or its status; offsets[0..n_groups] are the groups' first
+// entries
+template <class S>
+__global__ void __launch_bounds__(256) k_ble_sched_entries(const typename S::Group* __restrict__ groups, uint32_t n_groups,
+                                                           const uint32_t* __restrict__ offsets, uint32_t total, AuxGeom g,
+                                                           typename S::Entry* __restrict__ list) {
+    using E = typename S::Entry;
     const uint32_t e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= total) return;
-    uint32_t a = 0, b = n_trains;                                 // the last t with offsets[t] <= e
+    uint32_t a = 0, b = n_groups;                                 // the last t with offsets[t] <= e
     while (b - a > 1) { const uint32_t m = (a + b) >> 1; if (offsets[m] <= e) a = m; else b = m; }
-    const SyncTrain& tr = trains[a];
-    const int64_t k = tr.k_lo + (int64_t)(e - offsets[a]);
-    snrx_ble_sync_t& r = list[e];
+    const typename S::Group& grp = groups[a];
+    const uint32_t local = e - offsets[a], per_event = S::per_event(grp);
+    const int64_t k = grp.k_lo + (int64_t)(local / per_event);
+    E& r = list[e];
     uint4* d = reinterpret_cast<uint4*>(&r);
 #pragma unroll
-    for (int q = 0; q < (int)(sizeof(snrx_ble_sync_t) / 16); q++) d[q] = make_uint4(0u, 0u, 0u, 0u);
-    int64_t lo, hi;
-    sync_window(tr.si, k, lo, hi);
-    const uint32_t counter = (tr.si.pa_counter + (uint32_t)k) & 0xFFFFu;
+    for (int q = 0; q < (int)(sizeof(E) / 16); q++) d[q] = make_uint4(0u, 0u, 0u, 0u);
+    const uint8_t st = S::entry(grp, k, local % per_event, r);
     r.sample_index = -1;
-    r.win_lo = tr.s + lo; r.win_hi = tr.s + hi;
-    r.capture_id = tr.capture_id;
-    r.source = tr.source;
-    r.access_addr = tr.si.aa;
-    r.crc_init = tr.si.crc_init;
+    r.capture_id = grp.capture_id;
+    r.source = grp.source;
     r.event = (int32_t)k;
-    r.event_counter = (uint16_t)counter;
-    r.interval = (uint16_t)tr.si.interval;
-    r.channel = (uint8_t)csa2_channel(counter, tr.si.aa, tr.si.chm);
-    r.phy = (uint8_t)tr.phy;
-    r.sca = (uint8_t)tr.si.sca;
-    const int sps = tr.phy == SNRX_AUX_PHY_2M ? 2 : 4;
+    const int sps = r.phy == SNRX_AUX_PHY_2M ? 2 : 4;
     const int64_t l = r.win_lo - g.base, x = r.win_hi - g.base + 31 * sps;      // local first / last decision of the search
-    r.status = (l < 0 || x + 1 >= g.n_out) ? SNRX_AUX_OUTSIDE : kAuxPending;
+    r.status = (l < 0 || x + 1 >= g.n_out) ? SNRX_AUX_OUTSIDE : st;
 }
+
+// snrx_ble_periodic: aux entry -> SyncTrain -> one event per listed k
+struct SyncSched {
+    using Src = snrx_ble_aux_t;
+    using Group = SyncTrain;
+    using Entry = snrx_ble_sync_t;
+    // status OK, crc_ok, first == i, a valid SyncInfo; grouped by its AA
+    static __device__ __forceinline__ bool candidate(const Src& r, uint32_t i, uint32_t& key) {
+        SyncInfo si;
+        if (!(r.status == SNRX_AUX_OK && r.crc_ok && r.first == i && r.len >= 5 && sync_info_parse(r.bytes, (int)r.len - 5, si) &&
+              sync_info_valid(si)))
+            return false;
+        key = si.aa;
+        return true;
+    }
+    static __device__ __forceinline__ Group group(const Src& r, uint32_t i) {
+        SyncTrain t{};
+        sync_info_parse(r.bytes, (int)r.len - 5, t.si);
+        t.s = r.sample_index; t.capture_id = r.capture_id; t.source = i; t.phy = r.phy;
+        return t;
+    }
+    static __device__ __forceinline__ void k_range(const Group& t, const AuxGeom& g, int64_t& k_lo, int64_t& k_hi) {
+        sync_k_range(t.si, t.s, t.phy == SNRX_AUX_PHY_2M ? 2 : 4, g.base, g.n_out, k_lo, k_hi);
+    }
+    static __device__ __forceinline__ uint32_t per_event(const Group&) { return 1u; }
+    static __device__ __forceinline__ uint8_t entry(const Group& t, int64_t k, uint32_t, Entry& r) {
+        int64_t lo, hi;
+        sync_window(t.si, k, lo, hi);
+        const uint32_t counter = (t.si.pa_counter + (uint32_t)k) & 0xFFFFu;
+        r.win_lo = t.s + lo; r.win_hi = t.s + hi;
+        r.access_addr = t.si.aa;
+        r.crc_init = t.si.crc_init;
+        r.event_counter = (uint16_t)counter;
+        r.interval = (uint16_t)t.si.interval;
+        r.channel = (uint8_t)csa2_channel(counter, t.si.aa, t.si.chm);
+        r.phy = (uint8_t)t.phy;
+        r.sca = (uint8_t)t.si.sca;
+        return kAuxPending;
+    }
+};
 
 // One warp per pending entry of [0, n): the earliest full match of the entry's access address in its window, then the
 // decode with its CRC init.  E is snrx_ble_sync_t (a periodic event) or snrx_ble_bis_t (a BIS subevent, ble_bis.cuh).
@@ -273,7 +326,7 @@ __global__ void __launch_bounds__(128) k_ble_sync_search(E* __restrict__ list, u
         tabs_s[wib].dont_care[lane] = 0u;
         __syncwarp();
         const int sps = r.phy == SNRX_AUX_PHY_2M ? 2 : 4;
-        const int lo = (int)(r.win_lo - g.base), hi = (int)(r.win_hi - g.base);   // inside the buffer (k_ble_sync_events)
+        const int lo = (int)(r.win_lo - g.base), hi = (int)(r.win_hi - g.base);   // inside the buffer (k_ble_sched_entries)
         const uint32_t* pw = g.bits + g.lay.index(r.capture_id - g.first_capture, r.channel, 0);
         const int nf = aux_find(pw, g.lay.words_per_stream, lo, hi, sps, tabs_s[wib], lane);
         if (nf < 0) { if (lane == 0) r.status = SNRX_AUX_NOT_FOUND; __syncwarp(); continue; }

@@ -1194,54 +1194,71 @@ static int copy_list_out(snrx_handle* h, const char* name, const E* list, uint32
     return SNRX_OK;
 }
 
+// The snrx_ble_aux list of the polled batch into h->d_aux (*total entries): the pointers of the polled records, then the
+// pointer rounds behind them.  Shared by snrx_ble_aux and snrx_ble_periodic.
+static int aux_list(snrx_handle* h, const Lane& ln, cudaStream_t st, uint32_t* total, const char* overflow) {
+    int r = round_buffers_init(h);
+    if (r != SNRX_OK) return r;
+    if (!h->d_aux) CK(cudaMalloc((void**)&h->d_aux, sizeof(snrx_ble_aux_t) * (size_t)h->frame_cap));
+    AuxSrc src{};                                                // depth 0: the pointers of the polled records
+    src.frames = h->polled_frames_dev; src.list = h->d_aux; src.first = 0; src.n = ln.n_frames; src.depth = 0;
+    return run_pointer_rounds(h, src, h->d_aux, aux_geom_of(ln), st, total, overflow);
+}
+
+// A schedule list (ble_sync.cuh) into `list` (*total entries): the groups of the n_src source entries src into `groups`,
+// every group's listed entries, then the search.  SNRX_EOVERFLOW with `overflow` if there are more entries than max_frames.
+// The round buffers hold the flags, counts and offsets (n_src and the group count are at most max_frames).  The counts are
+// summed on the host in 64 bits before the (32-bit) scan: each is at most max_frames + 1, but the groups' counts could wrap a
+// 32-bit sum past the overflow test.  Once the sum is at most max_frames the scan cannot wrap.
+template <class S>
+static int run_schedule(snrx_handle* h, const typename S::Src* src, uint32_t n_src, typename S::Group* groups, typename S::Entry* list,
+                        const AuxGeom& g, cudaStream_t st, uint32_t* total, const char* overflow) {
+    *total = 0;
+    if (n_src == 0) return SNRX_OK;
+    k_ble_sched_flag<S><<<grid_for(h, n_src, 8, 8), 256, 0, st>>>(src, n_src, h->d_round_flags);
+    exclusive_scan(h->d_round_flags, n_src, h->d_round_offsets, h->d_round_scratch, st);
+    k_ble_sched_fill<S><<<div_up(n_src, 256), 256, 0, st>>>(src, n_src, h->d_round_flags, h->d_round_offsets, groups);
+    uint32_t n_groups = 0;
+    CK(cudaMemcpyAsync(&n_groups, h->d_round_offsets + n_src, sizeof n_groups, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (n_groups) {
+        k_ble_sched_count<S><<<div_up(n_groups, 256), 256, 0, st>>>(groups, n_groups, g, h->frame_cap, h->d_round_flags);
+        std::vector<uint32_t> counts(n_groups);
+        CK(cudaMemcpyAsync(counts.data(), h->d_round_flags, sizeof(uint32_t) * (size_t)n_groups, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        uint64_t sum = 0;
+        for (uint32_t c : counts) sum += c;
+        if (sum > h->frame_cap) return fail(h, SNRX_EOVERFLOW, overflow);
+        exclusive_scan(h->d_round_flags, n_groups, h->d_round_offsets, h->d_round_scratch, st);
+        if (sum) {
+            k_ble_sched_entries<S><<<div_up((uint32_t)sum, 256), 256, 0, st>>>(groups, n_groups, h->d_round_offsets, (uint32_t)sum, g, list);
+            k_ble_sync_search<<<grid_for(h, (uint32_t)sum, 4, 8), 128, 0, st>>>(list, (uint32_t)sum, g, h->d_crc_tab, h->d_aux_whiten);
+        }
+        *total = (uint32_t)sum;
+    }
+    CK(cudaGetLastError());
+    return SNRX_OK;
+}
+
 // The snrx_ble_periodic list of the polled batch into h->d_sync (*total entries), the aux list it comes from built into
-// h->d_aux first with the pointer rounds of snrx_ble_aux; *ln is the polled lane.  Shared by snrx_ble_periodic and
-// snrx_ble_bis (`name` in their errors).
-static int periodic_list(snrx_handle* h, const char* name, Lane** ln_out, uint32_t* total_out) {
+// h->d_aux first; *ln is the polled lane.  Shared by snrx_ble_periodic and snrx_ble_bis (`name` in their errors).
+static int periodic_list(snrx_handle* h, const char* name, Lane** ln_out, uint32_t* total) {
     const std::string nm = name;
     Lane* ln = nullptr;
     int r = polled_bits_lane(h, name, true, &ln);
     if (r != SNRX_OK) return r;
     *ln_out = ln;
     CK(cudaSetDevice(h->device));
-    if ((r = round_buffers_init(h)) != SNRX_OK) return r;
-    if (!h->d_aux) CK(cudaMalloc((void**)&h->d_aux, sizeof(snrx_ble_aux_t) * (size_t)h->frame_cap));
     if (!h->d_sync) {
         CK(cudaMalloc((void**)&h->d_sync_trains, sizeof(SyncTrain) * (size_t)h->frame_cap));
         CK(cudaMalloc((void**)&h->d_sync, sizeof(snrx_ble_sync_t) * (size_t)h->frame_cap));
     }
     cudaStream_t st = ln->tail;                                  // the lane is idle: its bit streams stay as the batch left them
-    const AuxGeom g = aux_geom_of(*ln);
-    AuxSrc src{};                                                // the aux list, exactly as snrx_ble_aux builds it
-    src.frames = h->polled_frames_dev; src.list = h->d_aux; src.first = 0; src.n = ln->n_frames; src.depth = 0;
     uint32_t n_aux = 0;
-    r = run_pointer_rounds(h, src, h->d_aux, g, st, &n_aux, (nm + ": more auxiliary pointers than max_frames").c_str());
+    r = aux_list(h, *ln, st, &n_aux, (nm + ": more auxiliary pointers than max_frames").c_str());
     if (r != SNRX_OK) return r;
-    uint32_t total = 0;
-    if (n_aux) {
-        // the trains: flags / offsets over the aux list (n_aux <= max_frames fits the round buffers)
-        k_ble_sync_flag<<<grid_for(h, n_aux, 8, 8), 256, 0, st>>>(h->d_aux, n_aux, h->d_round_flags);
-        exclusive_scan(h->d_round_flags, n_aux, h->d_round_offsets, h->d_round_scratch, st);
-        k_ble_sync_fill<<<div_up(n_aux, 256), 256, 0, st>>>(h->d_aux, n_aux, h->d_round_flags, h->d_round_offsets, h->d_sync_trains);
-        uint32_t n_trains = 0;
-        CK(cudaMemcpyAsync(&n_trains, h->d_round_offsets + n_aux, sizeof n_trains, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        if (n_trains) {
-            // the events: counts / offsets per train, then one entry per listed event, then the search
-            k_ble_sync_count<<<div_up(n_trains, 256), 256, 0, st>>>(h->d_sync_trains, n_trains, g, h->d_round_flags);
-            exclusive_scan(h->d_round_flags, n_trains, h->d_round_offsets, h->d_round_scratch, st);
-            CK(cudaMemcpyAsync(&total, h->d_round_offsets + n_trains, sizeof total, cudaMemcpyDeviceToHost, st));
-            CK(cudaStreamSynchronize(st));
-            if (total > h->frame_cap) return fail(h, SNRX_EOVERFLOW, (nm + ": more periodic events than max_frames").c_str());
-            if (total) {
-                k_ble_sync_events<<<div_up(total, 256), 256, 0, st>>>(h->d_sync_trains, n_trains, h->d_round_offsets, total, g, h->d_sync);
-                k_ble_sync_search<<<grid_for(h, total, 4, 8), 128, 0, st>>>(h->d_sync, total, g, h->d_crc_tab, h->d_aux_whiten);
-            }
-        }
-        CK(cudaGetLastError());
-    }
-    *total_out = total;
-    return SNRX_OK;
+    return run_schedule<SyncSched>(h, h->d_aux, n_aux, h->d_sync_trains, h->d_sync, aux_geom_of(*ln), st, total,
+                                   (nm + ": more periodic events than max_frames").c_str());
 }
 
 extern "C" {
@@ -1283,13 +1300,9 @@ int snrx_ble_aux(snrx_t* h, snrx_ble_aux_t* out, uint32_t cap, uint32_t* n_out) 
     int r = polled_bits_lane(h, "snrx_ble_aux", true, &ln);
     if (r != SNRX_OK) return r;
     CK(cudaSetDevice(h->device));
-    if ((r = round_buffers_init(h)) != SNRX_OK) return r;
-    if (!h->d_aux) CK(cudaMalloc((void**)&h->d_aux, sizeof(snrx_ble_aux_t) * (size_t)h->frame_cap));
     cudaStream_t st = ln->tail;                                  // the lane is idle: its bit streams stay as the batch left them
-    AuxSrc src{};                                                // depth 0: the pointers of the polled records
-    src.frames = h->polled_frames_dev; src.list = h->d_aux; src.first = 0; src.n = ln->n_frames; src.depth = 0;
     uint32_t total = 0;
-    r = run_pointer_rounds(h, src, h->d_aux, aux_geom_of(*ln), st, &total, "snrx_ble_aux: more auxiliary pointers than max_frames");
+    r = aux_list(h, *ln, st, &total, "snrx_ble_aux: more auxiliary pointers than max_frames");
     if (r != SNRX_OK) return r;
     return copy_list_out(h, "snrx_ble_aux", h->d_aux, total, out, cap, n_out, st);
 }
@@ -1359,37 +1372,10 @@ int snrx_ble_bis(snrx_t* h, snrx_ble_bis_t* out, uint32_t cap, uint32_t* n_out) 
         CK(cudaMalloc((void**)&h->d_bis, sizeof(snrx_ble_bis_t) * (size_t)h->frame_cap));
     }
     cudaStream_t st = ln->tail;                                  // the lane is idle: its bit streams stay as the batch left them
-    const AuxGeom g = aux_geom_of(*ln);
     uint32_t total = 0;
-    if (n_sync) {
-        // the BIGs: flags / offsets over the periodic list (n_sync <= max_frames fits the round buffers)
-        k_ble_big_flag<<<grid_for(h, n_sync, 8, 8), 256, 0, st>>>(h->d_sync, n_sync, h->d_round_flags);
-        exclusive_scan(h->d_round_flags, n_sync, h->d_round_offsets, h->d_round_scratch, st);
-        k_ble_big_fill<<<div_up(n_sync, 256), 256, 0, st>>>(h->d_sync, n_sync, h->d_round_flags, h->d_round_offsets, h->d_bigs);
-        uint32_t n_bigs = 0;
-        CK(cudaMemcpyAsync(&n_bigs, h->d_round_offsets + n_sync, sizeof n_bigs, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        if (n_bigs) {
-            // the subevents: counts / offsets per BIG, then one entry per subevent of a listed event, then the search
-            // The counts are summed on the host in 64 bits before the (32-bit) scan: each is at most max_frames + 1, but
-            // n_bigs of them could wrap a 32-bit sum past the overflow test.  Once the sum is at most max_frames the scan
-            // cannot wrap.
-            k_ble_big_count<<<div_up(n_bigs, 256), 256, 0, st>>>(h->d_bigs, n_bigs, g, h->frame_cap, h->d_round_flags);
-            std::vector<uint32_t> counts(n_bigs);
-            CK(cudaMemcpyAsync(counts.data(), h->d_round_flags, sizeof(uint32_t) * (size_t)n_bigs, cudaMemcpyDeviceToHost, st));
-            CK(cudaStreamSynchronize(st));
-            uint64_t sum = 0;
-            for (uint32_t c : counts) sum += c;
-            if (sum > h->frame_cap) return fail(h, SNRX_EOVERFLOW, "snrx_ble_bis: more BIS subevents than max_frames");
-            total = (uint32_t)sum;
-            exclusive_scan(h->d_round_flags, n_bigs, h->d_round_offsets, h->d_round_scratch, st);
-            if (total) {
-                k_ble_bis_events<<<div_up(total, 256), 256, 0, st>>>(h->d_bigs, n_bigs, h->d_round_offsets, total, g, h->d_bis);
-                k_ble_sync_search<<<grid_for(h, total, 4, 8), 128, 0, st>>>(h->d_bis, total, g, h->d_crc_tab, h->d_aux_whiten);
-            }
-        }
-        CK(cudaGetLastError());
-    }
+    r = run_schedule<BigSched>(h, h->d_sync, n_sync, h->d_bigs, h->d_bis, aux_geom_of(*ln), st, &total,
+                               "snrx_ble_bis: more BIS subevents than max_frames");
+    if (r != SNRX_OK) return r;
     return copy_list_out(h, "snrx_ble_bis", h->d_bis, total, out, cap, n_out, st);
 }
 

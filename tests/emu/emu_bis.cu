@@ -1,6 +1,6 @@
 // TEST INFRASTRUCTURE ONLY.  Host-side stepping of the BLE broadcast-isochronous cores of snout_b200/csrc/ble_bis.cuh (the
 // BIGInfo parse, the BIS access address and CRC init, the subevent channels, the payload number, the subevent window and the
-// listed k range that k_ble_big_* / k_ble_bis_events call), built by nvcc into a temporary shared library by
+// listed k range that the schedule kernels call with BigSched), built by nvcc into a temporary shared library by
 // tests/test_ble_bis.py and run on the CPU (no GPU needed).  Never part of libsnoutrx.so.  A BIGInfo is passed as its bytes.
 #include <cstdint>
 #include "../../snout_b200/csrc/ble_bis.cuh"

@@ -1,7 +1,7 @@
 // TEST INFRASTRUCTURE ONLY.  Host-side stepping of the BLE periodic-advertising cores of snout_b200/csrc/ble_sync.cuh (the
-// SyncInfo parse, CSA#2, the event window and the listed k range that k_ble_sync_count / k_ble_sync_events call), built by
-// nvcc into a temporary shared library by tests/test_ble_periodic.py and run on the CPU (no GPU needed).  Never part of
-// libsnoutrx.so.
+// SyncInfo parse, CSA#2, the event window and the listed k range that the schedule kernels call) and the AuxPtr parse of
+// ble_aux.cuh, built by nvcc into a temporary shared library by tests/test_ble_periodic.py and run on the CPU (no GPU
+// needed).  Never part of libsnoutrx.so.
 #include <cstdint>
 #include "../../snout_b200/csrc/ble_sync.cuh"
 
@@ -15,6 +15,13 @@ static SyncInfo emu_si(int offset, int units_us, int adjust, int interval, int s
 
 extern "C" {
 
+// f = channel, ca, units_us, offset, phy; -1 if the PDU carries no AuxPtr (ble_aux.cuh)
+int emu_aux_ptr_parse(const uint8_t* pdu, int n_payload, int32_t* f /*[5]*/) {
+    AuxPtr a{};
+    if (!aux_ptr_parse(pdu, n_payload, a)) return -1;
+    f[0] = a.channel; f[1] = a.ca; f[2] = a.units_us; f[3] = a.offset; f[4] = a.phy;
+    return 0;
+}
 // f = offset, units_us, adjust, interval, sca, aa, crc_init, pa_counter, valid; -1 if the PDU carries no SyncInfo
 int emu_sync_info_parse(const uint8_t* pdu, int n_payload, int32_t* f /*[9]*/, uint64_t* chm) {
     SyncInfo si{};

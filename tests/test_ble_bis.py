@@ -21,7 +21,7 @@ from oracle import aux_oracle as ao
 from oracle import bis_oracle as bo
 from oracle import periodic_oracle as po
 from snout_b200 import _abi, btle_cli, formats, messages, synth
-from test_ble_periodic import KAT_NINE, Scene, Train, case
+from test_ble_periodic import KAT_NINE, Scene, Train, case, ext_header_sweep
 from test_ble_periodic import _unmapped as unmapped_channel
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -174,6 +174,34 @@ def test_acad_walk(bis_emu):
     si = synth.sync_info_bytes(100, 30, 6, 3, 0, 1, 2, 3)
     pdu = synth.ext_pdu(synth.ext_header(0, None, 0, None, None, None, sync_info=si, acad=big))
     assert bo.find_big_info(pdu, pdu[1]).saa == 0x3A1B5C2D and _emu_find(bis_emu, pdu) is not None
+
+
+def test_big_info_find_on_every_header(bis_emu):
+    """The kernels' ACAD walk equals the oracle's on every flags byte and header length, with a 0x2C structure (length 34, 58
+    or random; a valid BIGInfo or random bytes) first in the ACAD or behind another structure."""
+    rng = np.random.default_rng(20262)
+    valid = (big_bytes(), big_bytes(enc=True))
+    f, chm, pc = (ctypes.c_int64 * 19)(), ctypes.c_uint64(), ctypes.c_uint64()
+    found = [0, 0]
+    for buf, n_payload, flags, hlen in ext_header_sweep(20263):
+        later = (flags + hlen + n_payload) % 2
+        at = 2 + sum(size for bit, size in ((0, 6), (1, 6), (2, 1), (3, 2), (4, 3), (5, 18), (6, 1)) if flags >> bit & 1)
+        ln = int(rng.choice([34, 58, rng.integers(1, 64)]))
+        value = valid[ln == 58] if rng.integers(0, 2) else rng.integers(0, 256, 57, dtype=np.uint8).tobytes()
+        ad = bytes([ln, 0x2C]) + value
+        if later:
+            m = int(rng.integers(1, 9))
+            ad = bytes([m, 0xFF]) + rng.integers(0, 256, m - 1, dtype=np.uint8).tobytes() + ad
+        ad = ad[: max(0, len(buf) - 2 - at)]
+        buf[2 + at: 2 + at + len(ad)] = np.frombuffer(ad, np.uint8)
+        want = bo.find_big_info(buf.tobytes(), n_payload)
+        rc = bis_emu.emu_big_info_find(buf.ctypes.data_as(ctypes.c_void_p), n_payload, f, ctypes.byref(chm), ctypes.byref(pc))
+        assert (rc == 0) == (want is not None), (flags, hlen, n_payload, later)
+        if want is not None:
+            assert list(f) == [int(getattr(want, k)) for k in FIELDS] + [int(want.valid())], (flags, hlen, n_payload, later)
+            assert chm.value == want.chm and pc.value == want.payload_count, (flags, hlen, n_payload, later)
+            found[later] += 1
+    assert min(found) > 100                                        # hits at the first and at a later position
 
 
 def test_validity_rules():

@@ -188,6 +188,46 @@ def test_sync_info_parsing(sync_emu):
     assert sync_emu.emu_crc_seed_of(ctypes.c_uint32(0xABCDEF)) == bb.crc_internal(synth.sync_crc_seed(0xABCDEF)) == bb.crc_internal(0xEFCDAB)
 
 
+def ext_header_sweep(seed):
+    """(buffer, n_payload, flags, hlen) for every flags byte, every extended header length 0..63 and payloads of hlen,
+    hlen + 1 and hlen + 2 bytes: a PDU of type 7 with seeded random bytes everywhere else.  The buffer always holds the
+    header length and flags bytes, whatever n_payload says."""
+    rng = np.random.default_rng(seed)
+    noise = rng.integers(0, 256, (256, 64, 3, 2 + 65), dtype=np.uint8)
+    for flags in range(256):
+        for hlen in range(64):
+            for j, n_payload in enumerate((hlen, hlen + 1, hlen + 2)):
+                buf = noise[flags, hlen, j, : 2 + max(n_payload, 2)].copy()
+                buf[0] = (buf[0] & 0xF0) | 7
+                buf[1] = n_payload
+                buf[2] = (buf[2] & 0xC0) | hlen
+                buf[3] = flags
+                yield buf, n_payload, flags, hlen
+
+
+def test_aux_ptr_and_sync_info_parse_on_every_header(sync_emu):
+    """The kernels' AuxPtr and SyncInfo parsers equal the oracles' on every flags byte and header length, including the
+    headers too short for the field and the payloads too short for the header."""
+    fa, fs, chm = (ctypes.c_int32 * 5)(), (ctypes.c_int32 * 9)(), ctypes.c_uint64()
+    n_aux = n_sync = 0
+    for buf, n_payload, flags, hlen in ext_header_sweep(20261):
+        ptr, pdu = buf.ctypes.data_as(ctypes.c_void_p), buf.tobytes()
+        want = ao.parse_aux_ptr(pdu, n_payload)
+        rc = sync_emu.emu_aux_ptr_parse(ptr, n_payload, fa)
+        assert (rc == 0) == (want is not None), (flags, hlen, n_payload)
+        if want is not None:
+            assert tuple(fa) == want, (flags, hlen, n_payload)
+            n_aux += 1
+        si = po.parse_sync_info(pdu, n_payload)
+        rc = sync_emu.emu_sync_info_parse(ptr, n_payload, fs, ctypes.byref(chm))
+        assert (rc == 0) == (si is not None), (flags, hlen, n_payload)
+        if si is not None:
+            assert list(fs) == [si.offset, si.units_us, si.adjust, si.interval, si.sca, ctypes.c_int32(si.aa).value, si.crc_init,
+                                si.pa_counter, int(si.valid())] and chm.value == si.chm, (flags, hlen, n_payload)
+            n_sync += 1
+    assert n_aux > 10000 and n_sync > 1000                      # both parsers find their field on a good share of the sweep
+
+
 # ------------------------------------------------------------------------------------------------ constructed streams
 class Train:
     """A periodic-advertising train's SyncInfo and the symbols of its packets."""
